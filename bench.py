@@ -23,6 +23,9 @@ step (juliet): pivot sample -> K1 pileup -> (N>1: one NCCL all-reduce of the cou
 
 `--impl reference` times the CPU restatement with all host threads on its own C-generated reads (states resident in host
 memory before the timed region: no unpacking is timed).
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0, float64 .npy files, at most 64 MB in all) so that
+two builds can be compared output for output: the inputs depend only on the arguments.
 """
 import argparse
 import ctypes as C
@@ -38,6 +41,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "aligned CCS reads/sec pileup+call+phase"
 MIN_PERC = 0.5   # juliet --min-perc (doc/JULIET.md:342-344): keeps the called set independent of the total read count
@@ -79,7 +83,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-digest", action="store_true")
     ap.add_argument("--write-digest", action="store_true", help="N=1 only: (re)write tests/golden/bench_digest.json")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="", help="write the last timed step's outputs as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU pass's outputs: it needs --impl ours")
+    return args
 
 
 def resolve(args, world):
@@ -295,6 +305,52 @@ def result_digest(j, res, lo, world, dist, torch, device):
             "hap_id_checksum": int(chk.item())}
 
 
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+DUMP_LIMIT = 64 << 20
+HAP_COUNTERS = ("reported", "insufficient", "damaged", "gaps", "heteroduplex", "partial")
+
+
+def step_outputs(kind, j, res, cooc):
+    """What a caller of the timed pass holds after it, as float64 arrays (every count and id here is exact in float64).
+    variants: one row per call, columns gene, codon_index, col, ref_codon, codon, count, coverage, expected, ntests, pvalue.
+    haplotype_summary: nreported, ndistinct, then the six read categories of HAP_COUNTERS."""
+    def f8(a):
+        return np.asarray(a, dtype=np.float64)
+
+    if kind == "fuse":
+        return {"consensus": f8(np.frombuffer(res.encode(), dtype=np.uint8))}
+    col, codon = j.get_counts()
+    out = {"col_counts": f8(col), "codon_counts": f8(codon)}
+    hap = res
+    if kind == "juliet":
+        out["variants"] = f8([[v.gene, v.codon_index, v.col, v.ref_codon, v.codon, v.count, v.coverage, v.expected, v.ntests, v.pvalue]
+                              for v in res.variants]).reshape(-1, 10)
+        out["keys"] = f8(res.keys).reshape(-1, 2)
+        hap = res.haplotypes
+    else:
+        out["cooccurrence"] = f8(cooc.cpu().numpy())
+    if hap is not None:
+        out["haplotype_patterns"] = f8(hap.patterns)
+        out["haplotype_counts"] = f8(hap.counts)
+        out["haplotype_summary"] = f8([hap.nreported, hap.ndistinct] + [hap.counters[k] for k in HAP_COUNTERS])
+    return out
+
+
+def dump_outputs(d, out):
+    """Writes out as d/<name>.npy.  When the arrays exceed DUMP_LIMIT in all, each large one is cut to a fixed, seeded
+    sample of its rows and the row indices go beside it as <name>_rows.npy."""
+    os.makedirs(d, exist_ok=True)
+    if sum(a.nbytes for a in out.values()) > DUMP_LIMIT:
+        per = DUMP_LIMIT // (2 * len(out))
+        for name, a in list(out.items()):
+            if a.nbytes > per:
+                keep = max(1, per // max(1, a.nbytes // len(a)))
+                rows = np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+                out[name], out[name + "_rows"] = a[rows], rows.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 def main():
     args = parse()
     if os.environ.get("BENCH_WATCHDOG"):
@@ -362,8 +418,7 @@ def main():
     def tail_stress(ptr):
         _lib.check(lib.ms_allreduce_counts(j.hd.h), j.hd.h)
         hap, _ = j.phase_device(site_vars, ptr, Rg, want_hap_id=False)
-        j.cooccurrence()
-        return hap
+        return hap, j.cooccurrence()
 
     def step():
         if c["kind"] == "juliet":
@@ -405,6 +460,11 @@ def main():
         elapsed_ms = el.value
     barrier()
     launches = j.hd.launches - launches0
+    cooc = None
+    if c["kind"] == "stress":
+        res, cooc = res
+    if args.dump_outputs and rank == 0:      # before the e2e pass below reuses the handle's buffers
+        dump_outputs(args.dump_outputs, step_outputs(c["kind"], j, res, cooc))
 
     def stage_ms(stage):
         ms = C.c_double()
@@ -440,12 +500,12 @@ def main():
             if c["kind"] == "fuse":
                 j.allreduce_counts()
                 return len(j.consensus()) + L * 32
-            hap = tail_stress(keep.value)
+            hap, _ = tail_stress(keep.value)
             return hap.patterns.nbytes + hap.counts.nbytes + L * 288
         for _ in range(2):
             e2e_step()
         barrier()
-        esteps = max(2, min(args.steps, 5))
+        esteps = args.steps
         d2h = 0
         t0 = time.perf_counter()
         for _ in range(esteps):

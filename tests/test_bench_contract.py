@@ -28,6 +28,31 @@ def test_reference_arm_line_has_the_contract_keys():
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_bad_arguments_are_refused():
+    out = _run("--impl", "reference", "--steps", "0")
+    assert out.returncode != 0 and "--steps must be at least 1" in out.stderr and not out.stdout.strip()
+    out = _run("--impl", "reference", "--dump-outputs", "unused")
+    assert out.returncode != 0 and "needs --impl ours" in out.stderr and not os.path.exists(os.path.join(ROOT, "unused"))
+
+
+def test_dump_outputs_stay_within_the_limit_and_repeat(tmp_path):
+    """--dump-outputs: small outputs are written whole; oversize ones become the same seeded row sample every time."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    small = {"col_counts": np.arange(24, dtype=np.float64).reshape(3, 8)}
+    bench.dump_outputs(str(tmp_path / "s"), dict(small))
+    assert np.array_equal(np.load(tmp_path / "s" / "col_counts.npy"), small["col_counts"])
+    big = {"cooccurrence": np.arange(3000 * 3000, dtype=np.float64).reshape(3000, 3000), "keys": np.ones((5, 2))}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), dict(big))
+        assert sum(f.stat().st_size for f in (tmp_path / d).iterdir()) <= bench.DUMP_LIMIT
+    a, rows = np.load(tmp_path / "a" / "cooccurrence.npy"), np.load(tmp_path / "a" / "cooccurrence_rows.npy")
+    assert np.array_equal(a, big["cooccurrence"][rows.astype(np.int64)])
+    assert np.array_equal(a, np.load(tmp_path / "b" / "cooccurrence.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "keys.npy"), big["keys"])
+
+
 def test_product_arm_refuses_to_run_without_a_gpu():
     import torch
     if torch.cuda.is_available():
