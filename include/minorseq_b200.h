@@ -113,8 +113,10 @@ int ms_pileup_kernel_ms(ms_handle *h, double *ms, int64_t *reads);
  * attached the two exchanges: the count all-reduce, and the haplotype-list all-gather + merge kernels.  Two spans of
  * the host-buffer pass (ms_juliet_pass_events_host) as well: MS_STAGE_UPLOAD = first to last host->device copy on the
  * copy stream, MS_STAGE_PASS = start of the pass to the arrival of its last result on the main stream.             */
+/* Pairwise linkage adds two: MS_STAGE_LINKAGE_STATS = its statistics kernels (m, tests, row offsets), MS_STAGE_LINKAGE_ALLREDUCE
+ * = the all-reduce of its Gram matrix; its contraction is timed as MS_STAGE_COOCCURRENCE.                                      */
 enum { MS_STAGE_PHASE_BITS = 1, MS_STAGE_COOCCURRENCE = 2, MS_STAGE_EXPAND = 3, MS_STAGE_ALLREDUCE = 4, MS_STAGE_HAPMERGE = 5,
-       MS_STAGE_UPLOAD = 6, MS_STAGE_PASS = 7 };
+       MS_STAGE_UPLOAD = 6, MS_STAGE_PASS = 7, MS_STAGE_LINKAGE_STATS = 8, MS_STAGE_LINKAGE_ALLREDUCE = 9 };
 int ms_stage_kernel_ms(ms_handle *h, int stage, double *ms);
 
 /* ---- K1: pileup (juliet "MSA counts", doc/JULIET.md:96-100; fuse doc/FUSE.md:17-20) -- */
@@ -261,6 +263,39 @@ int ms_phase_device(ms_handle *h, uint32_t **d_bits, uint8_t **d_flags, int64_t 
 int ms_cooccurrence(ms_handle *h, int32_t **d_C);
 /* 0 = choose by size (default), 1 = popcount-AND kernel, 2 = tensor-core kernel (A/B measurements, tests) */
 int ms_set_cooccurrence_variant(ms_handle *h, int32_t variant);
+
+/* ---- pairwise variant linkage (restatement choice U14) ------------------------------------------
+ * Do two called variants sit on the same genomes?  Unlike phasing, a read counts for a pair whenever its codons at
+ * BOTH variants are clean (all three states A/C/G/T), whatever it holds elsewhere.  For the pooled phasing keys v < w
+ * whose codons share no column (|col_v - col_w| >= 3) and with n >= min_reads informative reads, the 2x2 table
+ *     a = both, b = v only, c = w only, d = neither   (a+b+c+d = n)
+ * gives D' and r^2, and two one-sided Fisher tests: p_together = P(>= a carry both), p_apart = P(<= a carry both).
+ * With m = the number of tested pairs (Bonferroni), a pair is "linked" if p_together * m < alpha and "exclusive" if
+ * p_apart * m < alpha; only these significant pairs are listed.  Every rank computes the same list from the same,
+ * all-reduced counts.                                                                                               */
+typedef struct { double alpha; int32_t min_reads; } ms_linkage_params;
+enum { MS_LINKED = 1, MS_EXCLUSIVE = 2 };
+typedef struct {
+    int32_t v, w;                               /* indices in the ms_phase_begin list, v < w */
+    uint32_t both, v_only, w_only, neither;     /* the 2x2 table over the informative reads */
+    double d_prime, r2;
+    double pvalue;                              /* uncorrected one-sided Fisher p of the reported relation (fp64) */
+    int32_t relation;                           /* MS_LINKED or MS_EXCLUSIVE */
+} ms_linkage_pair;
+/* alpha 0.01 (juliet's --alpha), min_reads 10 */
+void ms_linkage_params_default(ms_linkage_params *p);
+/* on: the next ms_phase_begin also allocates the clean-codon matrix and ms_phase_dev fills it (off by default). */
+int ms_set_linkage(ms_handle *h, int on);
+/* The significant pairs of the phased reads (with a communicator attached: of all ranks' reads), ordered by v, then w.
+ * *n receives their number (may exceed cap: call again, the counts are cached until the next ms_phase_begin /
+ * ms_phase_dev); *ntested the Bonferroni m.  A collective when a communicator is attached: every rank calls it.       */
+int ms_linkage(ms_handle *h, const ms_linkage_params *prm, ms_linkage_pair *out, int64_t cap, int64_t *n,
+               int64_t *ntested);
+/* The (all-reduced) stacked Gram matrix [B | M]^T [B | M] in device memory, dim x dim int32 with dim = 64*ceil(V/32):
+ * B = the phasing bits (rows 0..), M = the clean-codon bits (rows dim/2..).  So for variants v, w (h = dim/2):
+ * both = G[v][w], v carried and w clean = G[v][h+w], n = G[h+v][h+w], diag(M^T M) = K2 coverage, diag(B^T B) = K2 count.
+ * Owned by the handle; same caching and collective rule as ms_linkage.                                              */
+int ms_linkage_device(ms_handle *h, int32_t **d_gram, int32_t *dim);
 
 /* ---- the whole juliet pass in one call ------------------------------------------------------
  * reset -> pileup -> (all-reduce when a communicator is attached) -> codon test -> phasing, i.e. everything

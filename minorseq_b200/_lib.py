@@ -43,6 +43,15 @@ class JulietResult(C.Structure):
                 ("npatterns", C.c_int64), ("nreported", C.c_int64), ("counters", PhaseCounters), ("hap_id", C.POINTER(C.c_int32))]
 
 
+class LinkageParams(C.Structure):
+    _fields_ = [("alpha", C.c_double), ("min_reads", C.c_int32)]
+
+
+class LinkagePair(C.Structure):
+    _fields_ = [("v", C.c_int32), ("w", C.c_int32), ("both", C.c_uint32), ("v_only", C.c_uint32), ("w_only", C.c_uint32),
+                ("neither", C.c_uint32), ("d_prime", C.c_double), ("r2", C.c_double), ("pvalue", C.c_double), ("relation", C.c_int32)]
+
+
 class ReadHdr(C.Structure):
     _fields_ = [("ev_off", C.c_uint32), ("begin", C.c_uint16), ("end", C.c_uint16)]
 
@@ -104,6 +113,11 @@ _SIGNATURES = {
     "ms_phase_haplotypes": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "ms_phase_device": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_P), C.POINTER(C.c_int64)]),
     "ms_cooccurrence": (C.c_int, [_P, C.POINTER(_P)]),
+    "ms_linkage_params_default": (None, [C.POINTER(LinkageParams)]),
+    "ms_set_linkage": (C.c_int, [_P, C.c_int]),
+    "ms_linkage": (C.c_int, [_P, C.POINTER(LinkageParams), C.POINTER(LinkagePair), C.c_int64, C.POINTER(C.c_int64),
+                             C.POINTER(C.c_int64)]),
+    "ms_linkage_device": (C.c_int, [_P, C.POINTER(_P), C.POINTER(C.c_int32)]),
     "ms_juliet_pass_dev": (C.c_int, [_P, _P, C.c_int64, C.POINTER(Gene), C.c_int32, C.c_char_p, C.POINTER(CallParams), C.c_int32,
                                    C.c_int32, C.POINTER(JulietResult)]),
     "ms_juliet_pass_host": (C.c_int, [_P, _P, C.c_int64, C.POINTER(Gene), C.c_int32, C.c_char_p, C.POINTER(CallParams), C.c_int32,

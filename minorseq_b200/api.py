@@ -13,7 +13,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _lib
-from ._lib import (CallParams, FuseParams, Gene, PhaseCounters, SynthParams, Variant, check)
+from ._lib import (CallParams, FuseParams, Gene, LinkagePair, LinkageParams, PhaseCounters, SynthParams, Variant, check)
 from .synth import start_mask_words, tile_rows, untile_rows
 
 CODONS = [a + b + c for a in "ACGT" for b in "ACGT" for c in "ACGT"]
@@ -45,6 +45,29 @@ class Haplotypes:
     counters: dict
     hap_id: np.ndarray = None       # per local read, -1 = damaged
     ndistinct: int = -1             # distinct patterns in total (patterns/counts may hold only the first ones of the order)
+
+
+@dataclass
+class Linkage:
+    """Pairwise linkage of the phasing keys (Juliet.linkage).  The significant pairs, ordered by v then w, as parallel arrays;
+    and, for every pair, the counts behind the tests as dense [V, V] int64 matrices: n[v, w] informative reads (both codons
+    clean), a[v, w] reads carrying both, b[v, w] v but not w, c[v, w] w but not v (over the informative reads)."""
+    v: np.ndarray
+    w: np.ndarray
+    both: np.ndarray
+    v_only: np.ndarray
+    w_only: np.ndarray
+    neither: np.ndarray
+    d_prime: np.ndarray
+    r2: np.ndarray
+    pvalue: np.ndarray
+    relation: np.ndarray            # 1 linked, 2 exclusive
+    ntested: int                    # Bonferroni m
+    keys: list
+    n: np.ndarray
+    a: np.ndarray
+    b: np.ndarray
+    c: np.ndarray
 
 
 @dataclass
@@ -210,7 +233,9 @@ class Juliet:
         return [Variant.from_buffer_copy(out[i]) for i in range(n.value)]
 
     # -- K3
-    def phase_device(self, variants, d_packed_ptr: int, nreads: int, want_hap_id=True, host_merge=False, cap=4096) -> Haplotypes:
+    def phase_device(self, variants, d_packed_ptr: int, nreads: int, want_hap_id=True, host_merge=False, cap=4096,
+                     linkage=False) -> Haplotypes:
+        """linkage: also record which reads are clean at each key, for Juliet.linkage afterwards"""
         import torch.distributed as dist
         keys = sorted({(v.col, v.codon) for v in variants})
         V = len(keys)
@@ -218,6 +243,8 @@ class Juliet:
         vd = np.array([k[1] for k in keys], dtype=np.int32)
         nw = max(1, (V + 31) // 32)
         self._V = V
+        self._keys = keys
+        check(self.lib.ms_set_linkage(self.hd.h, 1 if linkage else 0), self.hd.h)
         check(self.lib.ms_phase_begin(self.hd.h, _ptr(vc), _ptr(vd), V, nreads), self.hd.h)
         check(self.lib.ms_phase_dev(self.hd.h, C.c_void_p(d_packed_ptr), nreads), self.hd.h)
         if not host_merge and (getattr(self.hd, "native_comm", False) or _torch_world() == 1):
@@ -295,6 +322,36 @@ class Juliet:
             dist.all_reduce(t, op=dist.ReduceOp.SUM)
             torch.cuda.current_stream(self.hd.device).synchronize()
         return t[: self._V * self._V].view(self._V, self._V)
+
+    def linkage(self, alpha=None, min_reads=10, cap=1024) -> Linkage:
+        """Pairwise linkage of the keys of the last phase_device(..., linkage=True) (ms_linkage): the pairs that are
+        significantly "linked" (relation 1) or "exclusive" (relation 2) after Bonferroni over the tested pairs, and the dense
+        counts.  alpha None = the codon test's alpha.  With several ranks the handle needs its own communicator
+        (Handle.attach_comm): the counts are summed inside the library."""
+        import torch
+        if not getattr(self.hd, "native_comm", False) and _torch_world() > 1:
+            raise _lib.MsError("linkage over several ranks needs the handle's own communicator (Handle.attach_comm)")
+        p = LinkageParams()
+        self.lib.ms_linkage_params_default(C.byref(p))
+        p.alpha = self.params.alpha if alpha is None else float(alpha)
+        p.min_reads = int(min_reads)
+        n, m = C.c_int64(), C.c_int64()
+        while True:
+            out = (LinkagePair * max(1, cap))()
+            check(self.lib.ms_linkage(self.hd.h, C.byref(p), out, cap, C.byref(n), C.byref(m)), self.hd.h)
+            if n.value <= cap:
+                break
+            cap = int(n.value)             # the counts are cached: only the statistics run again
+        rec = np.ctypeslib.as_array(out)[: n.value].copy()
+        g, dim = C.c_void_p(), C.c_int32()
+        check(self.lib.ms_linkage_device(self.hd.h, C.byref(g), C.byref(dim)), self.hd.h)
+        check(self.lib.ms_synchronize(self.hd.h), self.hd.h)
+        G = _as_tensor(g.value, (dim.value, dim.value), torch.int32, self.hd.device).cpu().numpy().astype(np.int64)
+        V, h = self._V, dim.value // 2
+        a = G[:V, :V]
+        return Linkage(v=rec["v"], w=rec["w"], both=rec["both"], v_only=rec["v_only"], w_only=rec["w_only"], neither=rec["neither"],
+                       d_prime=rec["d_prime"], r2=rec["r2"], pvalue=rec["pvalue"], relation=rec["relation"], ntested=int(m.value),
+                       keys=list(self._keys), n=G[h:h + V, h:h + V].copy(), a=a.copy(), b=G[:V, h:h + V] - a, c=G[h:h + V, :V] - a)
 
     # -- the whole pass in one C-ABI call (what bench.py times)
     @staticmethod

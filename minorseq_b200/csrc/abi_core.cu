@@ -50,7 +50,9 @@ int ms_create(int device, ms_handle** out) {
         cudaEventCreate(&h->ev_stage[4][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[4][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[5][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[5][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[6][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[6][1]) != cudaSuccess ||
-        cudaEventCreate(&h->ev_stage[7][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[7][1]) != cudaSuccess) {
+        cudaEventCreate(&h->ev_stage[7][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[7][1]) != cudaSuccess ||
+        cudaEventCreate(&h->ev_stage[8][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[8][1]) != cudaSuccess ||
+        cudaEventCreate(&h->ev_stage[9][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[9][1]) != cudaSuccess) {
         g_create_error = cudaGetErrorString(cudaGetLastError());
         delete h;
         return MS_ERR_CUDA;
@@ -106,7 +108,7 @@ void ms_destroy(ms_handle* h) {
     cudaEventDestroy(h->ev_copy[0]); cudaEventDestroy(h->ev_copy[1]);
     cudaEventDestroy(h->ev_k1[0]); cudaEventDestroy(h->ev_k1[1]);
     cudaEventDestroy(h->ev_timer[0]); cudaEventDestroy(h->ev_timer[1]);
-    for (int s = 1; s < 8; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
+    for (int s = 1; s < 10; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
     cudaStreamDestroy(h->own_stream); cudaStreamDestroy(h->copy_stream);
     delete h;
 }
@@ -173,7 +175,7 @@ int ms_pileup_kernel_ms(ms_handle* h, double* ms, int64_t* reads) {
 }
 
 int ms_stage_kernel_ms(ms_handle* h, int stage, double* ms) {
-    if (!h || !ms || stage < 1 || stage > 7 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
+    if (!h || !ms || stage < 1 || stage > 9 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
     MS_CUDA(h, cudaSetDevice(h->device));
     MS_CUDA(h, cudaEventSynchronize(h->ev_stage[stage][1]));
     float f = 0.f;

@@ -61,6 +61,16 @@ int ms_comm_allgather_bytes(ms_handle* h, const void* d_send, void* d_recv, size
     return MS_OK;
 }
 
+// used by linkage.cu: in-place int32 sum of the stacked Gram matrix over the ranks, on the handle's stream
+int ms_comm_allreduce_i32(ms_handle* h, int32_t* d, size_t count) {
+    if (!h->comm) return MS_ERR_ARG;
+    MS_STAGE_BEGIN(h, MS_STAGE_LINKAGE_ALLREDUCE);
+    MS_NCCL(h, api().AllReduce(d, d, count, ncclInt32, ncclSum, static_cast<ncclComm_t>(h->comm), h->stream));
+    MS_STAGE_END(h, MS_STAGE_LINKAGE_ALLREDUCE);
+    h->launches++;
+    return MS_OK;
+}
+
 extern "C" void ms_comm_free_internal(ms_handle* h) {
     if (h->comm && api().ok) api().CommDestroy(static_cast<ncclComm_t>(h->comm));
     h->comm = nullptr;

@@ -43,8 +43,8 @@ struct ms_handle {
     cudaEvent_t ev_k1[2] = {nullptr, nullptr};  // around the last K1 launch when timing is on
     cudaEvent_t ev_timer[2] = {nullptr, nullptr};  // ms_timer_start / ms_timer_stop
     int expand_ctas = 0, expand_ctas_nblk = -1;   // expand_events_kernel: resident CTAs per SM for row length nblk
-    cudaEvent_t ev_stage[8][2] = {};               // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
-    bool stage_seen[8] = {false, false, false, false, false, false, false, false};
+    cudaEvent_t ev_stage[10][2] = {};              // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
+    bool stage_seen[10] = {false, false, false, false, false, false, false, false, false, false};
     bool timing = false;
     int64_t k1_reads = 0;
     std::string err;
@@ -110,6 +110,13 @@ struct ms_handle {
     DevBuf b_nw_seq, b_nw_hrow, b_nw_hcol, b_nw_dir;   // nw.cu (cleric's reference-to-reference alignment)
     int32_t tc_tiles_V = -1;     // variant count the uploaded tcgen05 tile list belongs to
     int cooc_variant = 0;        // 0 auto, 1 popcount-AND, 2 tcgen05 int8
+    // pairwise linkage (linkage.cu): ms_set_linkage before ms_phase_begin makes phase_bits_kernel also write the clean-codon
+    // matrix b_mbits; the stacked Gram matrix of [B | M] is computed (and all-reduced) once per phased read set
+    bool linkage = false;        // ms_set_linkage
+    bool link_ready = false;     // b_mbits belongs to the current phased read set
+    bool gram_valid = false;     // b_link_gram holds the (reduced) Gram matrix of the current read set
+    std::vector<int32_t> link_col;   // start column of each variant of the current ms_phase_begin
+    DevBuf b_mbits, b_link_gram, b_link_col, b_link_sig, b_link_rows, b_link_out;
     std::vector<uint32_t> groups_cnt, groups_pat;   // host copy of the last grouping pass (all ranks when a comm is attached)
     uint64_t groups_marg[4] = {0, 0, 0, 0};
     bool groups_valid = false;

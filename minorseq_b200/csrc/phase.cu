@@ -48,10 +48,15 @@ constexpr int kPhaseChunkMax = 16;   // distinct blocks staged per pass (+1: the
 // No ballots, no shuffles.  `ordered`: the stream visits the words of the bit-vector one after the other (the usual,
 // sorted variant list), so a finished word is stored; otherwise it is ORed into the zeroed vector.  `partial_all`: some
 // variant lies outside the reference, which makes every read partial.
+// kClean (pairwise linkage, restatement choice U14): also the clean-codon matrix `mbits` (same row stride): bit v = the three
+// columns of v's codon all hold A/C/G/T in this read.  It is `hit`'s construction on the state plane q.z instead of X, taken
+// through the same compress / per-variant shift, so it costs a few logic operations per layer and one more store per word.
+template <bool kClean>
 __global__ void __launch_bounds__(kPhaseWarps * 32, 4) phase_bits_kernel(
     const uint4* __restrict__ packed, int64_t R, int32_t nblk, const int32_t* __restrict__ blocklist, int32_t NB, int32_t chunk, int32_t dbuf,
     const uint32_t* __restrict__ stream, int32_t nwords, int32_t vwords, int32_t ordered, int32_t partial_all,
-    uint32_t* __restrict__ bits, uint8_t* __restrict__ flags, unsigned long long* __restrict__ ctr, const PhasePlan* __restrict__ plan) {
+    uint32_t* __restrict__ bits, uint8_t* __restrict__ flags, unsigned long long* __restrict__ ctr, const PhasePlan* __restrict__ plan,
+    uint32_t* __restrict__ mbits) {
     extern __shared__ __align__(16) uint4 stage_sm[];   // [warp][chunk + 1][32]
     if (plan) {     // the sizes come from the device-built plan (one-word bit-vectors); a plan that gave up leaves everything to the host
         if (plan->fallback) return;
@@ -68,7 +73,18 @@ __global__ void __launch_bounds__(kPhaseWarps * 32, 4) phase_bits_kernel(
         const uint32_t pos = static_cast<uint32_t>(r & 7);
         uint32_t fg = 0, fh = 0, fp = partial_all ? 1u : 0u;
         uint32_t word = 0, widx = 0xffffffffu;
+        uint32_t mword = 0;      // kClean: the clean-codon bits of word widx
         uint32_t* myrow = bits + static_cast<size_t>(r) * vwords;
+        uint32_t* mrow = kClean ? mbits + static_cast<size_t>(r) * vwords : nullptr;
+        // store the finished word widx of both matrices
+        auto flush = [&]() {
+            if (ordered) myrow[widx] = word;
+            else if (word) myrow[widx] |= word;
+            if constexpr (kClean) {
+                if (ordered) mrow[widx] = mword;
+                else if (mword) mrow[widx] |= mword;
+            }
+        };
         int32_t p = 0;     // position in the stream
         // per-lane 16-byte asynchronous copies global -> shared (LDGSTS): every block of a chunk is in flight at once, no
         // registers in between.  A list of more than one chunk (dbuf) alternates between two buffers: chunk c + 1 is on its way
@@ -119,32 +135,36 @@ __global__ void __launch_bounds__(kPhaseWarps * 32, 4) phase_bits_kernel(
                 const uint32_t X = ((q.x ^ e0) | (q.y ^ e1)) | q.z;                       // column is not the clean expected base
                 const uint32_t Xn = ((nx.x ^ en) | (nx.y ^ (en >> 2))) | nx.z;            // columns 32, 33 (bits 0, 1)
                 const uint32_t hit = ~(X | __funnelshift_r(X, Xn, 1) | __funnelshift_r(X, Xn, 2));   // bit c: the codon starting at c matches
+                uint32_t clean = 0;                                                       // bit c: the codon starting at c is all A/C/G/T
+                if constexpr (kClean) clean = ~(q.z | __funnelshift_r(q.z, nx.z, 1) | __funnelshift_r(q.z, nx.z, 2));
                 if (h0 & kHdrPacked) {
                     // compress the bits of `hit` at the start columns into the low nv bits (indices v0 .. v0 + nv - 1)
                     uint32_t x = hit & stream[p];
+                    uint32_t xm = clean & stream[p];
 #pragma unroll
                     for (int i = 0; i < 5; ++i) {
                         const uint32_t t = x & stream[p + 1 + i];
                         x = (x ^ t) | (t >> (1 << i));
+                        if constexpr (kClean) {
+                            const uint32_t tm = xm & stream[p + 1 + i];
+                            xm = (xm ^ tm) | (tm >> (1 << i));
+                        }
                     }
                     const uint32_t v0 = stream[p + 6];
                     p += 7;
                     const uint32_t sh = v0 & 31u;
                     if ((v0 >> 5) != widx) {
-                        if (live && widx != 0xffffffffu) {
-                            if (ordered) myrow[widx] = word;
-                            else if (word) myrow[widx] |= word;
-                        }
+                        if (live && widx != 0xffffffffu) flush();
                         widx = v0 >> 5; word = 0;
+                        if constexpr (kClean) mword = 0;
                     }
                     word |= x << sh;
+                    if constexpr (kClean) mword |= xm << sh;
                     if (sh + static_cast<uint32_t>(nv) > 32u) {                             // the layer runs over into the next word
-                        if (live) {
-                            if (ordered) myrow[widx] = word;
-                            else if (word) myrow[widx] |= word;
-                        }
+                        if (live) flush();
                         ++widx;
                         word = x >> (32u - sh);
+                        if constexpr (kClean) mword = xm >> (32u - sh);
                     }
                     continue;
                 }
@@ -153,13 +173,12 @@ __global__ void __launch_bounds__(kPhaseWarps * 32, 4) phase_bits_kernel(
                     const uint32_t bit = __funnelshift_r(hit, 0u, w) & 1u;                 // shift by the low 5 bits of w: the start column
                     const uint32_t v = w >> 5;
                     if ((v >> 5) != widx) {                                                // warp-uniform: all lanes are at the same variant
-                        if (live && widx != 0xffffffffu) {
-                            if (ordered) myrow[widx] = word;
-                            else if (word) myrow[widx] |= word;
-                        }
+                        if (live && widx != 0xffffffffu) flush();
                         widx = v >> 5; word = 0;
+                        if constexpr (kClean) mword = 0;
                     }
                     word |= __funnelshift_l(0u, bit, v);                                    // bit << (v & 31)
+                    if constexpr (kClean) mword |= __funnelshift_l(0u, __funnelshift_r(clean, 0u, w) & 1u, v);
                 }
                 p += nv;
             }
@@ -169,9 +188,9 @@ __global__ void __launch_bounds__(kPhaseWarps * 32, 4) phase_bits_kernel(
         if (live) {
             if (ordered && vwords == 1) {
                 myrow[0] = word;                 // the only word: written whether or not any variant maps to it (no zeroing by the caller)
+                if constexpr (kClean) mrow[0] = mword;
             } else if (widx != 0xffffffffu) {
-                if (ordered) myrow[widx] = word;
-                else if (word) myrow[widx] |= word;
+                flush();
             }
             const uint32_t f = (fg ? MS_FLAG_GAP : 0) | (fh ? MS_FLAG_HET : 0) | (fp ? MS_FLAG_PARTIAL : 0);
             flags[r] = static_cast<uint8_t>(f);
@@ -607,11 +626,12 @@ int phase_groups_copy_out(ms_handle* h, uint32_t* patterns, uint64_t* counts, in
 
 // opt the bit-vector kernel in to its largest staging area (8 warps x 17 blocks x 512 B), on the current device (ms_create)
 void ms_phase_set_smem_attr() {
-    cudaFuncSetAttribute(ms::phase_bits_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         ms::kPhaseWarps * 2 * (ms::kPhaseChunkMax / 2 + 1) * 32 * static_cast<int>(sizeof(uint4)) >
-                                 ms::kPhaseWarps * (ms::kPhaseChunkMax + 1) * 32 * static_cast<int>(sizeof(uint4))
-                             ? ms::kPhaseWarps * 2 * (ms::kPhaseChunkMax / 2 + 1) * 32 * static_cast<int>(sizeof(uint4))
-                             : ms::kPhaseWarps * (ms::kPhaseChunkMax + 1) * 32 * static_cast<int>(sizeof(uint4)));
+    const int bytes = ms::kPhaseWarps * 2 * (ms::kPhaseChunkMax / 2 + 1) * 32 * static_cast<int>(sizeof(uint4)) >
+                              ms::kPhaseWarps * (ms::kPhaseChunkMax + 1) * 32 * static_cast<int>(sizeof(uint4))
+                          ? ms::kPhaseWarps * 2 * (ms::kPhaseChunkMax / 2 + 1) * 32 * static_cast<int>(sizeof(uint4))
+                          : ms::kPhaseWarps * (ms::kPhaseChunkMax + 1) * 32 * static_cast<int>(sizeof(uint4));
+    cudaFuncSetAttribute(ms::phase_bits_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    cudaFuncSetAttribute(ms::phase_bits_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
 }
 
 extern "C" {
@@ -621,13 +641,15 @@ void ms_phase_free_internal(ms_handle* h) {
                      &h->b_ctr, &h->b_groups, &h->b_gather, &h->b_rank, &h->b_hap, &h->b_pat, &h->b_cooc, &h->b_bits_t,
                      &h->b_gslot, &h->b_mt_key, &h->b_mt_cnt, &h->b_mt_rep, &h->b_mslot, &h->b_mindex, &h->b_m_cnt, &h->b_m_pat, &h->b_m_rank,
                      &h->b_ord, &h->b_keys, &h->b_out, &h->b_tc_tiles,
-                     &h->b_nw_seq, &h->b_nw_hrow, &h->b_nw_hcol, &h->b_nw_dir};
+                     &h->b_nw_seq, &h->b_nw_hrow, &h->b_nw_hcol, &h->b_nw_dir,
+                     &h->b_mbits, &h->b_link_gram, &h->b_link_col, &h->b_link_sig, &h->b_link_rows, &h->b_link_out};
     for (DevBuf* b : all) b->release();
     if (h->h_stage) cudaFreeHost(h->h_stage);
     h->h_stage = nullptr; h->h_stage_cap = 0;
     if (h->plan_stage) cudaFreeHost(h->plan_stage);
     h->plan_stage = nullptr;
     h->phase_cap = h->phase_n = 0; h->V = 0; h->vwords = 0; h->table_valid = false;
+    h->link_ready = h->gram_valid = false;
 }
 
 int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codon, int32_t V, int64_t max_reads) {
@@ -639,6 +661,8 @@ int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codo
     h->phase_n = 0;
     h->table_valid = false;
     h->groups_valid = false;
+    h->gram_valid = false;
+    h->link_ready = false;
     // distinct 32-column blocks the variants touch
     std::vector<int32_t> blocks;
     for (int32_t v = 0; v < V; ++v) {
@@ -744,8 +768,14 @@ int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codo
     // the previous pass may still be reading these buffers on the stream if they have to move
     const bool grow = vd.size() * 4 > h->b_var.cap || blocks.size() * 4 > h->b_blocklist.cap ||
                       static_cast<size_t>(h->phase_cap) * h->vwords * 4 > h->b_bits.cap || static_cast<size_t>(h->phase_cap) > h->b_flags.cap ||
-                      static_cast<size_t>(ts) * 8 > h->b_tab_key.cap || !h->b_ctr.p;
+                      static_cast<size_t>(ts) * 8 > h->b_tab_key.cap || !h->b_ctr.p ||
+                      (h->linkage && static_cast<size_t>(h->phase_cap) * h->vwords * 4 > h->b_mbits.cap);
     if (grow) MS_CUDA(h, cudaStreamSynchronize(h->stream));
+    if (h->linkage) {   // the clean-codon matrix of pairwise linkage, same shape as the bit matrix
+        MS_CUDA(h, h->b_mbits.ensure(static_cast<size_t>(h->phase_cap) * h->vwords * 4));
+        h->link_col.assign(var_col, var_col + V);
+        h->link_ready = true;
+    }
     MS_CUDA(h, h->b_var.ensure(vd.size() * 4));
     MS_CUDA(h, h->b_blocklist.ensure(blocks.size() * 4));
     MS_CUDA(h, h->b_bits.ensure(static_cast<size_t>(h->phase_cap) * h->vwords * 4));
@@ -781,13 +811,17 @@ int ms_phase_dev(ms_handle* h, const uint32_t* d_packed, int64_t R) {
     MS_CUDA(h, cudaSetDevice(h->device));
     h->table_valid = false;
     h->groups_valid = false;
+    h->gram_valid = false;
     uint32_t* bits = h->b_bits.as<uint32_t>() + static_cast<size_t>(h->phase_n) * h->vwords;
+    uint32_t* mbits = h->link_ready ? h->b_mbits.as<uint32_t>() + static_cast<size_t>(h->phase_n) * h->vwords : nullptr;
     uint8_t* flags = h->b_flags.as<uint8_t>() + h->phase_n;
     const uint4* pk = reinterpret_cast<const uint4*>(d_packed);
     const uint32_t* stream = h->b_var.as<uint32_t>();
     unsigned long long* ctr = ctr_ptr(h);
-    if (!(h->phase_ordered && h->vwords == 1))   // one-word ordered vectors are written in full by the kernel
+    if (!(h->phase_ordered && h->vwords == 1)) {   // one-word ordered vectors are written in full by the kernel
         MS_CUDA(h, cudaMemsetAsync(bits, 0, static_cast<size_t>(R) * h->vwords * 4, h->stream));   // words no variant maps to stay zero
+        if (mbits) MS_CUDA(h, cudaMemsetAsync(mbits, 0, static_cast<size_t>(R) * h->vwords * 4, h->stream));
+    }
     MS_STAGE_BEGIN(h, MS_STAGE_PHASE_BITS);
     {
         // up to 16 touched blocks: one chunk, all of it in flight at once; longer lists: chunks of 8, double-buffered
@@ -797,9 +831,15 @@ int ms_phase_dev(ms_handle* h, const uint32_t* d_packed, int64_t R) {
         const int per_sm = std::max(1, std::min(6, static_cast<int>((h->max_smem + 1024) / (smem + 1024))));
         const int64_t want = (R + ms::kPhaseWarps * 32 - 1) / (ms::kPhaseWarps * 32);
         const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>(want, static_cast<int64_t>(h->num_sms) * per_sm)));
-        ms::phase_bits_kernel<<<grid, ms::kPhaseWarps * 32, smem, h->stream>>>(pk, R, h->nblk, h->b_blocklist.as<int32_t>(), h->nblocklist, chunk, dbuf ? 1 : 0,
-                                                                              stream, h->phase_nrec, h->vwords, h->phase_ordered ? 1 : 0,
-                                                                              h->phase_partial_all ? 1 : 0, bits, flags, ctr, nullptr);
+        if (mbits)     // pairwise linkage was requested: the same walk also writes the clean-codon matrix
+            ms::phase_bits_kernel<true><<<grid, ms::kPhaseWarps * 32, smem, h->stream>>>(pk, R, h->nblk, h->b_blocklist.as<int32_t>(), h->nblocklist, chunk,
+                                                                                        dbuf ? 1 : 0, stream, h->phase_nrec, h->vwords,
+                                                                                        h->phase_ordered ? 1 : 0, h->phase_partial_all ? 1 : 0, bits, flags,
+                                                                                        ctr, nullptr, mbits);
+        else
+            ms::phase_bits_kernel<false><<<grid, ms::kPhaseWarps * 32, smem, h->stream>>>(pk, R, h->nblk, h->b_blocklist.as<int32_t>(), h->nblocklist, chunk, dbuf ? 1 : 0,
+                                                                                         stream, h->phase_nrec, h->vwords, h->phase_ordered ? 1 : 0,
+                                                                                         h->phase_partial_all ? 1 : 0, bits, flags, ctr, nullptr, nullptr);
     }
     MS_STAGE_END(h, MS_STAGE_PHASE_BITS);
     h->launches++;
@@ -820,6 +860,7 @@ int ms_phase_planned_dev(ms_handle* h, const ms_variant* d_calls, const unsigned
     MS_CUDA(h, cudaSetDevice(h->device));
     h->V = 0;                       // known after the download of the plan (ms_phase_planned_adopt)
     h->vwords = 1;
+    h->link_ready = h->gram_valid = false;   // this pass writes no clean-codon matrix
     h->phase_cap = std::max<int64_t>(1, R);
     h->phase_n = 0;
     h->table_valid = false;
@@ -857,9 +898,10 @@ int ms_phase_planned_dev(ms_handle* h, const ms_variant* d_calls, const unsigned
         const int per_sm = std::max(1, std::min(6, static_cast<int>((h->max_smem + 1024) / (smem + 1024))));
         const int64_t want = (R + ms::kPhaseWarps * 32 - 1) / (ms::kPhaseWarps * 32);
         const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>(want, static_cast<int64_t>(h->num_sms) * per_sm)));
-        ms::phase_bits_kernel<<<grid, ms::kPhaseWarps * 32, smem, h->stream>>>(reinterpret_cast<const uint4*>(d_packed), R, h->nblk, h->b_blocklist.as<int32_t>(),
-                                                                              0, chunk, 0, h->b_var.as<uint32_t>(), 0, 1, 1, 0, h->b_bits.as<uint32_t>(),
-                                                                              h->b_flags.as<uint8_t>(), ctr_ptr(h), d_plan);
+        ms::phase_bits_kernel<false><<<grid, ms::kPhaseWarps * 32, smem, h->stream>>>(reinterpret_cast<const uint4*>(d_packed), R, h->nblk,
+                                                                                     h->b_blocklist.as<int32_t>(), 0, chunk, 0, h->b_var.as<uint32_t>(), 0, 1,
+                                                                                     1, 0, h->b_bits.as<uint32_t>(), h->b_flags.as<uint8_t>(), ctr_ptr(h),
+                                                                                     d_plan, nullptr);
         MS_STAGE_END(h, MS_STAGE_PHASE_BITS);
         h->launches++;
     }
@@ -871,6 +913,43 @@ int ms_phase_planned_dev(ms_handle* h, const ms_variant* d_calls, const unsigned
 
 // after the plan has been read back: the handle learns the number of keys (ms_cooccurrence, ms_phase_device need it)
 void ms_phase_planned_adopt(ms_handle* h, int32_t V) { h->V = V; }
+
+// G (dim x dim int32, full symmetric) = S^T S over the phased reads, S = the nmat bit matrices mats[k] (R rows of h->vwords
+// words each) side by side, matrix k's variants at rows 32 * vwords * k of the stacked transpose.  ms_cooccurrence is the
+// one-matrix case (dim = V); pairwise linkage stacks the bit matrix and the clean-codon matrix (dim = 64 * vwords).  The
+// contraction goes to the tensor cores when it is big enough to be one (cooc_tc.cu: V >= 256 variants and >= 32768 reads);
+// the popcount-AND kernel serves the usual few-dozen-variant case, where the matrix is tiny.  Same integers either way.
+int ms_gram_dev(ms_handle* h, const uint32_t* const* mats, int nmat, int32_t dim, int32_t* G) {
+    const int32_t V = h->V, nw = h->vwords;
+    const int64_t R = h->phase_n;
+    const bool tensor = h->cooc_variant == 2 || (h->cooc_variant == 0 && V >= 256 && R >= 32768);
+    // row stride of the transposed bit matrix: whole 128-read stages for the tensor path (zero padded)
+    const int64_t rwords = tensor ? 4 * ((R + 127) / 128) : std::max<int64_t>(1, (R + 31) / 32);
+    const size_t gbytes = std::max<size_t>(4, static_cast<size_t>(dim) * dim * 4);
+    const size_t mat_words = static_cast<size_t>(nw) * 32 * rwords;
+    MS_CUDA(h, h->b_bits_t.ensure(std::max<size_t>(16, nmat * mat_words * 4)));
+    MS_CUDA(h, cudaMemsetAsync(G, 0, gbytes, h->stream));
+    if (V > 0 && rwords > 0) {
+        const int64_t nwarps = rwords * nw;
+        for (int k = 0; k < nmat; ++k) {
+            ms::bits_transpose_kernel<<<static_cast<unsigned>((nwarps * 32 + 255) / 256), 256, 0, h->stream>>>(mats[k], R, nw, rwords,
+                                                                                                             h->b_bits_t.as<uint32_t>() + k * mat_words);
+            h->launches++;
+        }
+        MS_STAGE_BEGIN(h, MS_STAGE_COOCCURRENCE);
+        if (tensor) {
+            int rc = ms_cooccurrence_tc_launch(h, h->b_bits_t.as<uint32_t>(), dim, rwords, R, G);
+            if (rc != MS_OK) return rc;
+        } else {
+            dim3 grid((dim + ms::kCoTile - 1) / ms::kCoTile, (dim + ms::kCoTile - 1) / ms::kCoTile);
+            ms::cooccurrence_kernel<<<grid, 256, 0, h->stream>>>(h->b_bits_t.as<uint32_t>(), dim, rwords, G);
+            h->launches++;
+        }
+        MS_STAGE_END(h, MS_STAGE_COOCCURRENCE);
+    }
+    MS_CUDA(h, cudaGetLastError());
+    return MS_OK;
+}
 
 extern "C" {
 
@@ -1076,34 +1155,12 @@ int ms_cooccurrence(ms_handle* h, int32_t** d_C) {
     MsRange nvtx_range("K3 co-occurrence");
     if (!h || !h->b_bits.p || !d_C) return MS_ERR_ARG;
     MS_CUDA(h, cudaSetDevice(h->device));
-    const int32_t V = h->V, nw = h->vwords;
-    const int64_t R = h->phase_n;
-    // the contraction goes to the tensor cores when it is big enough to be one (cooc_tc.cu); the popcount-AND
-    // kernel serves the usual few-dozen-variant case, where the matrix is tiny
-    const bool tensor = h->cooc_variant == 2 || (h->cooc_variant == 0 && V >= 256 && R >= 32768);
-    // row stride of the transposed bit matrix: whole 128-read stages for the tensor path (zero padded)
-    const int64_t rwords = tensor ? 4 * ((R + 127) / 128) : std::max<int64_t>(1, (R + 31) / 32);
+    const int32_t V = h->V;
     const size_t cbytes = std::max<size_t>(4, static_cast<size_t>(V) * V * 4);
     MS_CUDA(h, h->b_cooc.ensure(cbytes));
-    MS_CUDA(h, h->b_bits_t.ensure(std::max<size_t>(16, static_cast<size_t>(nw) * 32 * rwords * 4)));
-    MS_CUDA(h, cudaMemsetAsync(h->b_cooc.p, 0, cbytes, h->stream));
-    if (V > 0 && rwords > 0) {
-        const int64_t nwarps = rwords * nw;
-        ms::bits_transpose_kernel<<<static_cast<unsigned>((nwarps * 32 + 255) / 256), 256, 0, h->stream>>>(h->b_bits.as<uint32_t>(), R, nw, rwords,
-                                                                                                         h->b_bits_t.as<uint32_t>());
-        h->launches++;
-        MS_STAGE_BEGIN(h, MS_STAGE_COOCCURRENCE);
-        if (tensor) {
-            int rc = ms_cooccurrence_tc_launch(h, h->b_bits_t.as<uint32_t>(), V, rwords, R, h->b_cooc.as<int32_t>());
-            if (rc != MS_OK) return rc;
-        } else {
-            dim3 grid((V + ms::kCoTile - 1) / ms::kCoTile, (V + ms::kCoTile - 1) / ms::kCoTile);
-            ms::cooccurrence_kernel<<<grid, 256, 0, h->stream>>>(h->b_bits_t.as<uint32_t>(), V, rwords, h->b_cooc.as<int32_t>());
-            h->launches++;
-        }
-        MS_STAGE_END(h, MS_STAGE_COOCCURRENCE);
-    }
-    MS_CUDA(h, cudaGetLastError());
+    const uint32_t* mats[1] = {h->b_bits.as<uint32_t>()};
+    const int rc = ms_gram_dev(h, mats, 1, V, h->b_cooc.as<int32_t>());
+    if (rc != MS_OK) return rc;
     *d_C = h->b_cooc.as<int32_t>();
     return MS_OK;
 }

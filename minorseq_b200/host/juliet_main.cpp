@@ -3,7 +3,8 @@
 // Keeps the reference's process interface (/root/reference/doc/JULIET.md): outputs chosen by file
 // extension, either or both (:61-66); --config/-c <HIV|ABL1|file.json> (:118-162); --region b-e (:270-271);
 // --mode-phasing (:192-211); --min-perc / --max-perc (:342-354); --drm-only (:370).  The unpinned model
-// constants (SURVEY App. B) are options with the restatement's defaults.
+// constants (SURVEY App. B) are options with the restatement's defaults.  --linkage adds pairwise variant linkage
+// (restatement choice U14): per pair of called variants, the reads clean at both codons, D', r^2 and two Fisher tests.
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -28,6 +29,8 @@ static void usage() {
          "                                     target screenshot), not PacBio's full tables: pass the real config as a file\n"
          "      --region <begin-end>           1-based window to subset the target config\n"
          "      --mode-phasing                 phase variants into haplotypes\n"
+         "      --linkage                      pairwise linkage of the called variants (reads clean at both codons; D', r^2,\n"
+         "                                     Fisher tests for \"linked\" / \"exclusive\" after Bonferroni at --alpha)\n"
          "      --min-perc <p>                 only variants with abundance > p %\n"
          "      --max-perc <p>                 only variants with abundance < p %\n"
          "      --drm-only                     only known drug-resistance mutations\n"
@@ -53,9 +56,10 @@ static bool ends_with(const std::string& s, const std::string& e) { return s.siz
 
 int main(int argc, char** argv) {
     std::string config, region, cmdline, timing_json;
-    bool phasing = false, drm_only = false;
+    bool phasing = false, drm_only = false, linkage = false;
     double min_perc = -1, max_perc = -1, sub = 5e-4, del = 3e-3, alpha = 0.01;
     int min_hap = 10, device = 0, ngpus = 1;
+    const int link_min_reads = 10;   // reads clean at both codons that a tested pair needs (the haplotype default, F21)
     mshost::QvFilter qv;
     std::vector<std::string> pos;
     for (int i = 0; i < argc; ++i) cmdline += (i ? " " : "") + std::string(argv[i]);
@@ -70,6 +74,7 @@ int main(int argc, char** argv) {
         else if (a == "-c" || a == "--config") config = need("--config");
         else if (a == "--region") region = need("--region");
         else if (a == "--mode-phasing") phasing = true;
+        else if (a == "--linkage") linkage = true;
         else if (a == "--drm-only") drm_only = true;
         else if (a == "--min-perc") min_perc = atof(need("--min-perc").c_str());
         else if (a == "--max-perc") max_perc = atof(need("--max-perc").c_str());
@@ -167,6 +172,8 @@ int main(int argc, char** argv) {
         std::vector<uint32_t> pat;
         std::vector<uint64_t> cnt;
         int64_t nrep_all = 0;
+        std::vector<ms_linkage_pair> link_pairs;
+        int64_t link_tested = 0;
         std::vector<std::string> errs(static_cast<size_t>(ngpus));
 #define CKR(call)                                                                                      \
     do {                                                                                               \
@@ -218,7 +225,7 @@ int main(int argc, char** argv) {
                 lap("call + DRM annotation");
                 CKR(ms_get_counts(h, col.data(), nullptr));
             }
-            if (phasing) {
+            if (phasing || linkage) {
                 // one global variant list over all genes (screenshot juliet_hiv-phasing.png: same columns in every table)
                 std::vector<std::pair<int, int>> my_keys;
                 for (const msreport::VariantRow& vr : my_rows) my_keys.emplace_back(vr.col, vr.codon);
@@ -228,26 +235,46 @@ int main(int argc, char** argv) {
                 const int32_t nw = std::max(1, (V + 31) / 32);
                 std::vector<int32_t> vc(V), vk(V);
                 for (int32_t i = 0; i < V; ++i) { vc[i] = my_keys[i].first; vk[i] = my_keys[i].second; }
+                CKR(ms_set_linkage(h, linkage ? 1 : 0));
                 CKR(ms_phase_begin(h, vc.data(), vk.data(), V, r1 - r0));
                 CKR(ms_phase_dev(h, d_rows, r1 - r0));
-                // grouping, merge over the ranks, haplotype order and per-read ids in one device-side call; only the reported
-                // haplotypes are read back (every rank takes the same turns through this loop: nrep is a merged result)
-                int64_t H = 0, nrep = 0, cap = 256;
-                std::vector<uint32_t> my_pat;
-                std::vector<uint64_t> my_cnt;
-                ms_phase_counters c2;
-                for (;;) {
-                    my_pat.assign(static_cast<size_t>(cap) * nw, 0u);
-                    my_cnt.assign(cap, 0);
-                    CKR(ms_phase_haplotypes(h, min_hap, my_pat.data(), my_cnt.data(), cap, &H, &nrep, &c2, hap.data() + r0));
-                    if (nrep <= cap) break;
-                    cap = nrep;
+                if (linkage) {
+                    // every rank computes the same list from the all-reduced counts (a collective: all ranks call it)
+                    ms_linkage_params lp;
+                    ms_linkage_params_default(&lp);
+                    lp.alpha = alpha;
+                    lp.min_reads = link_min_reads;
+                    std::vector<ms_linkage_pair> my_pairs(64);
+                    int64_t np = 0, nt = 0;
+                    for (;;) {
+                        CKR(ms_linkage(h, &lp, my_pairs.data(), static_cast<int64_t>(my_pairs.size()), &np, &nt));
+                        if (np <= static_cast<int64_t>(my_pairs.size())) break;
+                        my_pairs.resize(np);
+                    }
+                    my_pairs.resize(np);
+                    if (r == 0) { link_pairs.swap(my_pairs); link_tested = nt; }
                 }
-                if (r == 0) {
-                    counters[0] = c2.reported; counters[1] = c2.insufficient; counters[2] = c2.damaged;
-                    counters[3] = c2.gaps; counters[4] = c2.heteroduplex; counters[5] = c2.partial;
-                    keys.swap(my_keys); pat.swap(my_pat); cnt.swap(my_cnt); nrep_all = nrep;
+                if (phasing) {
+                    // grouping, merge over the ranks, haplotype order and per-read ids in one device-side call; only the reported
+                    // haplotypes are read back (every rank takes the same turns through this loop: nrep is a merged result)
+                    int64_t H = 0, nrep = 0, cap = 256;
+                    std::vector<uint32_t> my_pat;
+                    std::vector<uint64_t> my_cnt;
+                    ms_phase_counters c2;
+                    for (;;) {
+                        my_pat.assign(static_cast<size_t>(cap) * nw, 0u);
+                        my_cnt.assign(cap, 0);
+                        CKR(ms_phase_haplotypes(h, min_hap, my_pat.data(), my_cnt.data(), cap, &H, &nrep, &c2, hap.data() + r0));
+                        if (nrep <= cap) break;
+                        cap = nrep;
+                    }
+                    if (r == 0) {
+                        counters[0] = c2.reported; counters[1] = c2.insufficient; counters[2] = c2.damaged;
+                        counters[3] = c2.gaps; counters[4] = c2.heteroduplex; counters[5] = c2.partial;
+                        pat.swap(my_pat); cnt.swap(my_cnt); nrep_all = nrep;
+                    }
                 }
+                if (r == 0) keys.swap(my_keys);
             }
             if (r == 0) rows.swap(my_rows);
         });
@@ -282,7 +309,35 @@ int main(int argc, char** argv) {
             }
         }
 
-        lap("phasing");
+        msreport::LinkageBlock link;
+        if (linkage) {
+            link.min_reads = link_min_reads;
+            link.alpha = alpha;
+            link.tested_pairs = link_tested;
+            auto variant = [&](int32_t v) {
+                msreport::LinkageVariant o;
+                char cb[4];
+                o.abs_pos = keys[v].first + 1;
+                o.codon = mscfg::codon_string(keys[v].second, cb);
+                for (const msreport::VariantRow& r : rows)
+                    if (r.col == keys[v].first && r.codon == keys[v].second)
+                        o.labels.push_back(genes[r.gene].name + " " + mscfg::translate(r.ref_codon) + std::to_string(r.aa_pos) + mscfg::translate(r.codon));
+                return o;
+            };
+            for (const ms_linkage_pair& p : link_pairs) {
+                msreport::LinkageRow lr;
+                lr.a = variant(p.v);
+                lr.b = variant(p.w);
+                lr.reads = static_cast<unsigned long long>(p.both) + p.v_only + p.w_only + p.neither;
+                lr.both = p.both; lr.a_only = p.v_only; lr.b_only = p.w_only; lr.neither = p.neither;
+                lr.d_prime = p.d_prime; lr.r2 = p.r2; lr.pvalue = p.pvalue;
+                lr.pvalue_corrected = std::min(1.0, p.pvalue * static_cast<double>(link_tested));
+                lr.relation = p.relation == MS_LINKED ? "linked" : "exclusive";
+                link.pairs.push_back(lr);
+            }
+        }
+
+        lap(linkage ? "phasing + linkage" : "phasing");
         char ts[40];
         const auto now = std::chrono::system_clock::now();
         const std::time_t tt = std::chrono::system_clock::to_time_t(now);
@@ -294,7 +349,8 @@ int main(int argc, char** argv) {
         snprintf(ts, sizeof ts, "%s.%03ldZ", base, ms);
         if (getenv("MS_FIXED_TIMESTAMP")) snprintf(ts, sizeof ts, "%s", getenv("MS_FIXED_TIMESTAMP"));
 
-        const msjson::Value report = msreport::build(ts, pos[0], cmdline, MS_VERSION, cfg, L, genes, rows, col, L, phasing, haps, counters);
+        const msjson::Value report = msreport::build(ts, pos[0], cmdline, MS_VERSION, cfg, L, genes, rows, col, L, phasing, haps, counters,
+                                                     linkage ? &link : nullptr);
         if (!out_json.empty()) {
             std::ofstream f(out_json);
             if (!f) mshost::die("cannot write " + out_json);

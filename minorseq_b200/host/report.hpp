@@ -37,6 +37,25 @@ struct HaplotypeRow {
     std::vector<std::string> read_names;
 };
 
+// pairwise linkage of two called variants (--linkage, restatement choice U14): one row per significant pair
+struct LinkageVariant {
+    int abs_pos = 0;                  // 1-based first column of the codon
+    std::string codon;
+    std::vector<std::string> labels;  // the variant's report rows, e.g. "Reverse Transcriptase K65R"
+};
+struct LinkageRow {
+    LinkageVariant a, b;
+    unsigned long long reads = 0, both = 0, a_only = 0, b_only = 0, neither = 0;
+    double d_prime = 0, r2 = 0, pvalue = 0, pvalue_corrected = 0;
+    std::string relation;             // "linked" or "exclusive"
+};
+struct LinkageBlock {
+    int min_reads = 0;
+    double alpha = 0;
+    long long tested_pairs = 0;
+    std::vector<LinkageRow> pairs;
+};
+
 // "%": two significant digits as in the screenshots (1.1, 0.91, 98, 100)
 inline std::string perc2(double p) {
     char b[32];
@@ -56,7 +75,8 @@ inline std::string perc1(double p) {  // haplotype %: one decimal, trailing ".0"
 inline Value build(const std::string& timestamp, const std::string& input_file, const std::string& cmdline, const std::string& version,
                    const mscfg::TargetConfig& cfg, int ref_length, const std::vector<mscfg::Gene>& genes,
                    const std::vector<VariantRow>& variants, const std::vector<unsigned>& col_counts /* L*8 */, int L,
-                   bool phasing, const std::vector<HaplotypeRow>& haps, const unsigned long long counters[6]) {
+                   bool phasing, const std::vector<HaplotypeRow>& haps, const unsigned long long counters[6],
+                   const LinkageBlock* linkage = nullptr) {
     Value root = Value::object();
     Value& in = root.set("input", Value::object());
     in.set("timestamp", Value::string(timestamp));
@@ -169,6 +189,36 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
         Value& hc = root.set("haplotype_read_categories", Value::object());
         static const char* names[6] = {"reported", "insufficient_coverage", "unsuitable", "unsuitable_gaps", "unsuitable_heteroduplex", "unsuitable_partial"};
         for (int i = 0; i < 6; ++i) hc.set(names[i], Value::integer(static_cast<long long>(counters[i])));
+    }
+    if (linkage) {
+        Value& lk = root.set("linkage", Value::object());
+        lk.set("min_reads", Value::integer(linkage->min_reads));
+        lk.set("alpha", Value::number(linkage->alpha));
+        lk.set("tested_pairs", Value::integer(linkage->tested_pairs));
+        Value& ps = lk.set("pairs", Value::array());
+        auto variant = [](const LinkageVariant& v) {
+            Value o = Value::object();
+            o.set("abs_pos", Value::integer(v.abs_pos));
+            o.set("codon", Value::string(v.codon));
+            Value& ls = o.set("labels", Value::array());
+            for (const std::string& l : v.labels) ls.push(Value::string(l));
+            return o;
+        };
+        for (const LinkageRow& r : linkage->pairs) {
+            Value& o = ps.push(Value::object());
+            o.set("a", variant(r.a));
+            o.set("b", variant(r.b));
+            o.set("reads", Value::integer(static_cast<long long>(r.reads)));
+            o.set("both", Value::integer(static_cast<long long>(r.both)));
+            o.set("a_only", Value::integer(static_cast<long long>(r.a_only)));
+            o.set("b_only", Value::integer(static_cast<long long>(r.b_only)));
+            o.set("neither", Value::integer(static_cast<long long>(r.neither)));
+            o.set("d_prime", Value::number(r.d_prime));
+            o.set("r2", Value::number(r.r2));
+            o.set("pValue", Value::number(r.pvalue));
+            o.set("pValueCorrected", Value::number(r.pvalue_corrected));
+            o.set("relation", Value::string(r.relation));
+        }
     }
     return root;
 }
@@ -301,7 +351,38 @@ inline std::string to_html(const Value& root) {
             if (const Value* vs = d.get("variants")) for (const Value& v : vs->arr) h += esc(v.str) + "<br>";
             h += "</p>";
         }
-    h += "</details>\n</body></html>\n";
+    h += "</details>\n";
+    if (const Value* lk = root.get("linkage")) {
+        char b[64];
+        snprintf(b, sizeof b, "%g", lk->get_number("alpha"));
+        h += "<details open><summary>Variant Linkage</summary><p>Pairs of variants tested: " +
+             std::to_string(static_cast<long long>(lk->get_number("tested_pairs"))) + " (at least " +
+             std::to_string(static_cast<long long>(lk->get_number("min_reads"))) + " reads clean at both codons; significance " + b +
+             " after Bonferroni)</p>";
+        const Value* ps = lk->get("pairs");
+        if (ps && !ps->arr.empty()) {
+            h += "<table><tr><th>Variant A</th><th>Codon</th><th>Variant B</th><th>Codon</th><th>Reads</th><th>Both</th><th>A only</th>"
+                 "<th>B only</th><th>Neither</th><th>D'</th><th>r&sup2;</th><th>p (corrected)</th><th>Relation</th></tr>\n";
+            auto cell = [](const Value* v) {
+                std::string t;
+                if (const Value* ls = v ? v->get("labels") : nullptr)
+                    for (const Value& l : ls->arr) t += (t.empty() ? "" : "<br>") + esc(l.str);
+                if (t.empty() && v) t = "Pos " + std::to_string(static_cast<long long>(v->get_number("abs_pos")));
+                return "<td>" + t + "</td><td><tt>" + esc(v ? v->get_string("codon") : "") + "</tt></td>";
+            };
+            for (const Value& r : ps->arr) {
+                h += "<tr>" + cell(r.get("a")) + cell(r.get("b"));
+                for (const char* k : {"reads", "both", "a_only", "b_only", "neither"})
+                    h += "<td>" + std::to_string(static_cast<long long>(r.get_number(k))) + "</td>";
+                snprintf(b, sizeof b, "<td>%.3f</td><td>%.3f</td><td>%.2e</td>", r.get_number("d_prime"), r.get_number("r2"), r.get_number("pValueCorrected"));
+                h += b;
+                h += "<td>" + esc(r.get_string("relation")) + "</td></tr>\n";
+            }
+            h += "</table>";
+        }
+        h += "</details>\n";
+    }
+    h += "</body></html>\n";
     return h;
 }
 
