@@ -114,9 +114,11 @@ int ms_pileup_kernel_ms(ms_handle *h, double *ms, int64_t *reads);
  * the host-buffer pass (ms_juliet_pass_events_host) as well: MS_STAGE_UPLOAD = first to last host->device copy on the
  * copy stream, MS_STAGE_PASS = start of the pass to the arrival of its last result on the main stream.             */
 /* Pairwise linkage adds two: MS_STAGE_LINKAGE_STATS = its statistics kernels (m, tests, row offsets), MS_STAGE_LINKAGE_ALLREDUCE
- * = the all-reduce of its Gram matrix; its contraction is timed as MS_STAGE_COOCCURRENCE.                                      */
+ * = the all-reduce of its Gram matrix; its contraction is timed as MS_STAGE_COOCCURRENCE.  MS_STAGE_GROUP_PILEUP = the
+ * grouped pile-up kernel of ms_group_pileup_dev (without the counting sort in front of it).                                  */
 enum { MS_STAGE_PHASE_BITS = 1, MS_STAGE_COOCCURRENCE = 2, MS_STAGE_EXPAND = 3, MS_STAGE_ALLREDUCE = 4, MS_STAGE_HAPMERGE = 5,
-       MS_STAGE_UPLOAD = 6, MS_STAGE_PASS = 7, MS_STAGE_LINKAGE_STATS = 8, MS_STAGE_LINKAGE_ALLREDUCE = 9 };
+       MS_STAGE_UPLOAD = 6, MS_STAGE_PASS = 7, MS_STAGE_LINKAGE_STATS = 8, MS_STAGE_LINKAGE_ALLREDUCE = 9,
+       MS_STAGE_GROUP_PILEUP = 10 };
 int ms_stage_kernel_ms(ms_handle *h, int stage, double *ms);
 
 /* ---- K1: pileup (juliet "MSA counts", doc/JULIET.md:96-100; fuse doc/FUSE.md:17-20) -- */
@@ -335,6 +337,31 @@ int ms_fuse(ms_handle *h, const ms_fuse_params *prm,
             const int32_t *ins_col, const int64_t *ins_off, const int32_t *ins_len,
             int64_t nins, const char *ins_pool, int64_t pool_len,
             char *seq, int64_t cap, int64_t *len);
+
+/* ---- grouped pile-up and per-group consensus (restatement choice U15) -------------------------------------------
+ * What is the full sequence of each haplotype?  K1's column counts per group of reads: every read carries an int32 label
+ * (device memory, one per read, in read order); a read labelled g in [0, ngroups) is counted into group g's columns, any
+ * other label is skipped.  The group tensor is [ngroups][L][8] u32, each [L][8] laid out as ms_get_counts' col
+ * (A,C,G,T,-,N,ins,coverage).  ms_set_groups allocates and zeroes it (after ms_set_layout; a new layout forgets it),
+ * ms_group_pileup_dev accumulates R more device-resident reads (tiles) into it.                                      */
+int ms_set_groups(ms_handle *h, int32_t ngroups);
+int ms_group_pileup_dev(ms_handle *h, const uint32_t *d_packed, const int32_t *d_group, int64_t R);
+/* In-place u32 sum of the group tensor over the ranks (ncclAllReduce); a collective, a no-op without a communicator. */
+int ms_allreduce_group_counts(ms_handle *h);
+int ms_get_group_counts(ms_handle *h, uint32_t *col /* ngroups*L*8 */);
+/* Device pointer (owned by the handle) to the per-read position in juliet's haplotype order of the last ms_phase_haplotypes
+ * (-1 = damaged; R = the reads phased on this handle), e.g. the labels of ms_group_pileup_dev.  Valid until the next phasing
+ * call.  Computed here if ms_phase_haplotypes was called with hap_id == NULL.                                          */
+int ms_phase_hap_device(ms_handle *h, int32_t **d_hap, int64_t *R);
+/* fuse's consensus (U6-U8) of every group's (all-reduced) counts, with U15's one difference: inside the span from the first
+ * to the last column with votes >= min_coverage, a column with fewer votes is written as 'N' instead of being dropped
+ * (columns outside the span are trimmed).  Insertion events carry their group (ins_group; events of other groups are
+ * skipped) and are tallied and judged against their own group's votes; only insertions after a column inside the span
+ * are candidates.  Group g's sequence is seq[seq_off[g] .. seq_off[g+1]) (seq_off: ngroups + 1 entries, always filled);
+ * MS_ERR_CAPACITY when cap < seq_off[ngroups] (seq may be NULL to query the size).                                     */
+int ms_group_consensus(ms_handle *h, const ms_fuse_params *prm, const int32_t *ins_group, const int32_t *ins_col,
+                       const int64_t *ins_off, const int32_t *ins_len, int64_t nins, const char *ins_pool, int64_t pool_len,
+                       char *seq, int64_t cap, int64_t *seq_off);
 
 /* ---- cleric's alignment step (doc/CLERIC.md:19-23,41-44; SURVEY 8f row 4) ------------------------
  * Global Needleman-Wunsch of the original reference a against the target reference b on the GPU

@@ -137,6 +137,12 @@ _SIGNATURES = {
     "ms_fuse": (C.c_int, [_P, C.POINTER(FuseParams), _P, _P, _P, C.c_int64, _P, C.c_int64, _P, C.c_int64,
                           C.POINTER(C.c_int64)]),
     "ms_synth_dev": (C.c_int, [_P, C.POINTER(SynthParams), _P, _P, _P, C.c_int64, C.c_int64, _P]),
+    "ms_set_groups": (C.c_int, [_P, C.c_int32]),
+    "ms_group_pileup_dev": (C.c_int, [_P, _P, _P, C.c_int64]),
+    "ms_allreduce_group_counts": (C.c_int, [_P]),
+    "ms_get_group_counts": (C.c_int, [_P, _P]),
+    "ms_phase_hap_device": (C.c_int, [_P, C.POINTER(_P), C.POINTER(C.c_int64)]),
+    "ms_group_consensus": (C.c_int, [_P, C.POINTER(FuseParams), _P, _P, _P, _P, C.c_int64, _P, C.c_int64, _P, C.c_int64, _P]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -244,6 +244,7 @@ class Juliet:
         nw = max(1, (V + 31) // 32)
         self._V = V
         self._keys = keys
+        self._nreported = None             # set when the device path below leaves per-read ranks on the device
         check(self.lib.ms_set_linkage(self.hd.h, 1 if linkage else 0), self.hd.h)
         check(self.lib.ms_phase_begin(self.hd.h, _ptr(vc), _ptr(vd), V, nreads), self.hd.h)
         check(self.lib.ms_phase_dev(self.hd.h, C.c_void_p(d_packed_ptr), nreads), self.hd.h)
@@ -300,6 +301,7 @@ class Juliet:
                 break
             cap = int(nrep.value)
         k = min(cap, int(H.value))
+        self._nreported = int(nrep.value)
         names = []
         buf = C.create_string_buffer(3)
         for i in range(nrep.value):
@@ -352,6 +354,75 @@ class Juliet:
         return Linkage(v=rec["v"], w=rec["w"], both=rec["both"], v_only=rec["v_only"], w_only=rec["w_only"], neither=rec["neither"],
                        d_prime=rec["d_prime"], r2=rec["r2"], pvalue=rec["pvalue"], relation=rec["relation"], ntested=int(m.value),
                        keys=list(self._keys), n=G[h:h + V, h:h + V].copy(), a=a.copy(), b=G[:V, h:h + V] - a, c=G[h:h + V, :V] - a)
+
+    # -- grouped pile-up and per-haplotype consensus (restatement choice U15)
+    def group_pileup(self, d_packed_ptr: int, d_group_ptr: int, nreads: int, ngroups: int, accumulate=False):
+        """K1's column counts per group of reads (ms_group_pileup_dev): read r of the device tiles is counted into group
+        g = label[r] (d_group_ptr: device int32, one per read) when 0 <= g < ngroups and skipped otherwise.  accumulate=False
+        starts from zero counts; True adds to the counts of the previous call with the same ngroups."""
+        if accumulate and getattr(self, "_ngroups", None) != ngroups:
+            raise ValueError("accumulate=True needs a previous group_pileup with the same ngroups")
+        if not accumulate:
+            check(self.lib.ms_set_groups(self.hd.h, int(ngroups)), self.hd.h)
+            self._ngroups = int(ngroups)
+        check(self.lib.ms_group_pileup_dev(self.hd.h, C.c_void_p(d_packed_ptr), C.c_void_p(d_group_ptr), int(nreads)), self.hd.h)
+
+    def group_counts(self) -> np.ndarray:
+        """[ngroups, L, 8] uint32: A, C, G, T, -, N, insertion flags and coverage of each group's reads (after haplotype_consensus:
+        summed over the ranks)."""
+        out = np.empty((self._ngroups, self.L, 8), dtype=np.uint32)
+        check(self.lib.ms_get_group_counts(self.hd.h, _ptr(out)), self.hd.h)
+        return out
+
+    def haplotype_consensus(self, d_packed_ptr: int, nreads: int, insertions=None, min_coverage=10, ins_fraction=0.5,
+                            ins_distance=20) -> list:
+        """The sequence of every reported haplotype of the last phase_device, in report order (restatement choice U15): fuse's
+        consensus over the haplotype's reads, with columns of fewer than min_coverage votes inside the covered span written as
+        'N'.  d_packed_ptr / nreads: the reads that were phased.  insertions: (read, col, off, len, pool) insertion events of
+        these reads (read = index among them, pool = bytes); each event belongs to its read's haplotype.  With several ranks
+        the handle needs its own communicator (Handle.attach_comm), the counts are summed inside the library, and insertion
+        events are not supported (their read indices are local to a rank)."""
+        import torch
+        if not getattr(self.hd, "native_comm", False) and _torch_world() > 1:
+            raise _lib.MsError("haplotype consensus over several ranks needs the handle's own communicator (Handle.attach_comm)")
+        nrep = getattr(self, "_nreported", None)
+        if nrep is None:
+            raise _lib.MsError("haplotype_consensus needs the per-read haplotype ranks of a phase_device call on this handle")
+        d_hap, R = C.c_void_p(), C.c_int64()
+        check(self.lib.ms_phase_hap_device(self.hd.h, C.byref(d_hap), C.byref(R)), self.hd.h)
+        if R.value != nreads:
+            raise ValueError(f"{nreads} reads given, {R.value} were phased")
+        self.group_pileup(d_packed_ptr, d_hap.value or 0, nreads, nrep)
+        check(self.lib.ms_allreduce_group_counts(self.hd.h), self.hd.h)
+        nins, ig, ic, io, il, pool = 0, None, None, None, None, b""
+        if insertions is not None and len(insertions[0]):
+            if _torch_world() > 1:
+                raise _lib.MsError("haplotype_consensus: insertion events are not supported with several ranks")
+            read, col, off, ln, pool = insertions
+            read = np.asarray(read, dtype=np.int64)
+            if read.min() < 0 or read.max() >= nreads:
+                raise ValueError("insertion read index outside the phased reads")
+            check(self.lib.ms_synchronize(self.hd.h), self.hd.h)
+            hap = _as_tensor(d_hap.value, (max(1, nreads),), torch.int32, self.hd.device).cpu().numpy()[:nreads]
+            ig = np.ascontiguousarray(hap[read], dtype=np.int32)
+            ic = np.ascontiguousarray(col, dtype=np.int32)
+            io = np.ascontiguousarray(off, dtype=np.int64)
+            il = np.ascontiguousarray(ln, dtype=np.int32)
+            nins = len(ig)
+        pl = np.frombuffer(pool, dtype=np.uint8) if nins else None
+        prm = FuseParams(int(min_coverage), float(ins_fraction), int(ins_distance))
+        seq_off = np.zeros(nrep + 1, dtype=np.int64)
+        cap = nrep * (self.L + 16)
+        while True:
+            seq = np.empty(max(1, cap), dtype=np.uint8)
+            rc = self.lib.ms_group_consensus(self.hd.h, C.byref(prm), _ptr(ig), _ptr(ic), _ptr(io), _ptr(il), nins, _ptr(pl), len(pool),
+                                             _ptr(seq), cap, _ptr(seq_off))
+            if rc == -4:   # MS_ERR_CAPACITY: seq_off holds the size
+                cap = int(seq_off[-1])
+                continue
+            check(rc, self.hd.h)
+            break
+        return [seq[seq_off[g]: seq_off[g + 1]].tobytes().decode() for g in range(nrep)]
 
     # -- the whole pass in one C-ABI call (what bench.py times)
     @staticmethod

@@ -10,6 +10,7 @@ static std::string g_create_error;
 void ms_events_set_smem_attr(int max_smem);
 void ms_cooc_tc_set_smem_attr();
 void ms_phase_set_smem_attr();
+void ms_group_set_smem_attr();
 int ms_tile_rows_launch(ms_handle* h, const uint32_t* d_rows, int64_t R, uint32_t* d_tiled);
 
 extern "C" {
@@ -52,7 +53,8 @@ int ms_create(int device, ms_handle** out) {
         cudaEventCreate(&h->ev_stage[6][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[6][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[7][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[7][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[8][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[8][1]) != cudaSuccess ||
-        cudaEventCreate(&h->ev_stage[9][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[9][1]) != cudaSuccess) {
+        cudaEventCreate(&h->ev_stage[9][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[9][1]) != cudaSuccess ||
+        cudaEventCreate(&h->ev_stage[10][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[10][1]) != cudaSuccess) {
         g_create_error = cudaGetErrorString(cudaGetLastError());
         delete h;
         return MS_ERR_CUDA;
@@ -74,6 +76,7 @@ int ms_create(int device, ms_handle** out) {
     ms_events_set_smem_attr(h->max_smem);
     ms_cooc_tc_set_smem_attr();
     ms_phase_set_smem_attr();
+    ms_group_set_smem_attr();
     *out = h;
     return MS_OK;
 }
@@ -100,6 +103,7 @@ void ms_destroy(ms_handle* h) {
     cudaFree(h->d_upload); cudaFree(h->d_call_buf); cudaFree(h->d_seq);
     h->b_exc_list.release(); h->b_exc_cnt.release();
     h->b_base.release(); h->b_ev_hdr.release(); h->b_ev.release();
+    for (DevBuf* b : {&h->b_gcol, &h->b_ghist, &h->b_gtot, &h->b_goff, &h->b_gioff, &h->b_glist}) b->release();
     for (cudaEvent_t ev : h->ev_chunk) cudaEventDestroy(ev);
     for (cudaEvent_t ev : h->ev_stagefree) cudaEventDestroy(ev);
     h->b_rowstage[0].release(); h->b_rowstage[1].release();
@@ -108,7 +112,7 @@ void ms_destroy(ms_handle* h) {
     cudaEventDestroy(h->ev_copy[0]); cudaEventDestroy(h->ev_copy[1]);
     cudaEventDestroy(h->ev_k1[0]); cudaEventDestroy(h->ev_k1[1]);
     cudaEventDestroy(h->ev_timer[0]); cudaEventDestroy(h->ev_timer[1]);
-    for (int s = 1; s < 10; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
+    for (int s = 1; s < 11; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
     cudaStreamDestroy(h->own_stream); cudaStreamDestroy(h->copy_stream);
     delete h;
 }
@@ -175,7 +179,7 @@ int ms_pileup_kernel_ms(ms_handle* h, double* ms, int64_t* reads) {
 }
 
 int ms_stage_kernel_ms(ms_handle* h, int stage, double* ms) {
-    if (!h || !ms || stage < 1 || stage > 9 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
+    if (!h || !ms || stage < 1 || stage > 10 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
     MS_CUDA(h, cudaSetDevice(h->device));
     MS_CUDA(h, cudaEventSynchronize(h->ev_stage[stage][1]));
     float f = 0.f;
@@ -235,6 +239,8 @@ int ms_set_layout(ms_handle* h, int32_t L, const uint32_t* start_mask) {
     const int32_t W = best_W;
     MS_CUDA(h, cudaStreamSynchronize(h->stream));
     free_layout(h);
+    h->label_groups = -1;   // group counts belong to the old layout
+    h->b_gcol.release();
     h->L = L; h->nblk = nblk; h->count_codons = start_mask != nullptr; h->have_pivot = false;
     h->have_base = false;
     h->wpg = W;

@@ -118,4 +118,15 @@ int ms_allreduce_counts(ms_handle* h) {
     return MS_OK;
 }
 
+int ms_allreduce_group_counts(ms_handle* h) {
+    MsRange nvtx_range("all-reduce group counts");
+    if (!h || h->label_groups < 0 || h->label_L != h->L) return MS_ERR_ARG;
+    if (!h->comm || h->label_groups == 0) return MS_OK;
+    MS_CUDA(h, cudaSetDevice(h->device));
+    MS_NCCL(h, api().AllReduce(h->b_gcol.p, h->b_gcol.p, static_cast<size_t>(h->label_groups) * h->L * 8, ncclUint32, ncclSum,
+                               static_cast<ncclComm_t>(h->comm), h->stream));
+    h->launches++;
+    return MS_OK;
+}
+
 }  // extern "C"

@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <cstring>
 #include <vector>
+#include "fuse.cuh"
 #include "handle.h"
 
 namespace ms {
@@ -43,8 +44,6 @@ __global__ void ins_tally_kernel(const int32_t* __restrict__ col, const long lon
     atomicAdd(tab_cnt + idx, 1u);
     atomicMin(tab_rep + idx, static_cast<long long>(i));
 }
-
-struct InsCand { int32_t col, len; long long rep; uint32_t cnt, pad; };
 
 __global__ void ins_eval_kernel(const uint32_t* __restrict__ tab_cnt, const long long* __restrict__ tab_rep, int64_t tab_size,
                                 const int32_t* __restrict__ col, const int32_t* __restrict__ len,

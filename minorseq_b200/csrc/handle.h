@@ -43,8 +43,8 @@ struct ms_handle {
     cudaEvent_t ev_k1[2] = {nullptr, nullptr};  // around the last K1 launch when timing is on
     cudaEvent_t ev_timer[2] = {nullptr, nullptr};  // ms_timer_start / ms_timer_stop
     int expand_ctas = 0, expand_ctas_nblk = -1;   // expand_events_kernel: resident CTAs per SM for row length nblk
-    cudaEvent_t ev_stage[10][2] = {};              // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
-    bool stage_seen[10] = {false, false, false, false, false, false, false, false, false, false};
+    cudaEvent_t ev_stage[11][2] = {};              // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
+    bool stage_seen[11] = {false, false, false, false, false, false, false, false, false, false, false};
     bool timing = false;
     int64_t k1_reads = 0;
     std::string err;
@@ -118,6 +118,8 @@ struct ms_handle {
     std::vector<int32_t> link_col;   // start column of each variant of the current ms_phase_begin
     DevBuf b_mbits, b_link_gram, b_link_col, b_link_sig, b_link_rows, b_link_out;
     std::vector<uint32_t> groups_cnt, groups_pat;   // host copy of the last grouping pass (all ranks when a comm is attached)
+    bool hap_ranked = false;     // b_rank maps the table slots of the current phased reads to the last ms_phase_haplotypes order
+    bool hap_assigned = false;   // ... and b_hap holds the per-read positions in it (ms_phase_hap_device)
     uint64_t groups_marg[4] = {0, 0, 0, 0};
     bool groups_valid = false;
     void* h_stage = nullptr;      // pinned host staging for small D2H reads
@@ -129,6 +131,11 @@ struct ms_handle {
 
     // fuse
     char* d_seq = nullptr;
+
+    // grouped pile-up (group.cu): column counts [label_groups][L][8] of the reads of each label, and the counting sort's buffers
+    int32_t label_groups = -1;   // ms_set_groups; -1 = not set
+    int32_t label_L = 0;         // L of the layout the group counts belong to
+    DevBuf b_gcol, b_ghist, b_gtot, b_goff, b_gioff, b_glist;
 };
 
 #define MS_CUDA(h, call)                                                                    \

@@ -555,6 +555,7 @@ int phase_ensure_stage(ms_handle* h, size_t bytes) {
 
 int phase_build_table(ms_handle* h, int attempt) {
     const int64_t R = h->phase_n;
+    h->hap_ranked = h->hap_assigned = false;   // new table slots: the order positions of ms_phase_haplotypes no longer apply
     unsigned long long* ctr = phase_ctr(h);
     // spare word of the exchanged header (ctr[7]): 1 = this build was this rank's last resort (table at its maximum size, or the
     // fourth hash seed), so that an overflow / a collision reported with it makes EVERY rank give up in the same iteration
@@ -650,6 +651,7 @@ void ms_phase_free_internal(ms_handle* h) {
     h->plan_stage = nullptr;
     h->phase_cap = h->phase_n = 0; h->V = 0; h->vwords = 0; h->table_valid = false;
     h->link_ready = h->gram_valid = false;
+    h->hap_ranked = h->hap_assigned = false;
 }
 
 int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codon, int32_t V, int64_t max_reads) {
@@ -663,6 +665,7 @@ int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codo
     h->groups_valid = false;
     h->gram_valid = false;
     h->link_ready = false;
+    h->hap_ranked = h->hap_assigned = false;
     // distinct 32-column blocks the variants touch
     std::vector<int32_t> blocks;
     for (int32_t v = 0; v < V; ++v) {
@@ -812,6 +815,7 @@ int ms_phase_dev(ms_handle* h, const uint32_t* d_packed, int64_t R) {
     h->table_valid = false;
     h->groups_valid = false;
     h->gram_valid = false;
+    h->hap_ranked = h->hap_assigned = false;
     uint32_t* bits = h->b_bits.as<uint32_t>() + static_cast<size_t>(h->phase_n) * h->vwords;
     uint32_t* mbits = h->link_ready ? h->b_mbits.as<uint32_t>() + static_cast<size_t>(h->phase_n) * h->vwords : nullptr;
     uint8_t* flags = h->b_flags.as<uint8_t>() + h->phase_n;
@@ -861,6 +865,7 @@ int ms_phase_planned_dev(ms_handle* h, const ms_variant* d_calls, const unsigned
     h->V = 0;                       // known after the download of the plan (ms_phase_planned_adopt)
     h->vwords = 1;
     h->link_ready = h->gram_valid = false;   // this pass writes no clean-codon matrix
+    h->hap_ranked = h->hap_assigned = false;
     h->phase_cap = std::max<int64_t>(1, R);
     h->phase_n = 0;
     h->table_valid = false;
@@ -1115,6 +1120,7 @@ int ms_phase_assign(ms_handle* h, const uint32_t* ordered_patterns, int64_t H, i
     }
     const int64_t R = h->phase_n;
     const int32_t nw = h->vwords;
+    h->hap_ranked = h->hap_assigned = false;   // b_rank / b_hap now follow the caller's pattern list
     MS_CUDA(h, h->b_rank.ensure(static_cast<size_t>(h->tab_size) * 4));
     MS_CUDA(h, h->b_hap.ensure(static_cast<size_t>(std::max<int64_t>(1, R)) * 4));
     MS_CUDA(h, h->b_pat.ensure(static_cast<size_t>(std::max<int64_t>(1, H)) * nw * 4));

@@ -478,10 +478,31 @@ extern "C" int ms_phase_haplotypes(ms_handle* h, int32_t min_reads, uint32_t* pa
     }
     if (pending) MS_CUDA(h, cudaStreamSynchronize(h->stream));
     MS_CUDA(h, cudaGetLastError());
+    h->hap_ranked = true;
+    h->hap_assigned = hap_id && h->phase_n > 0;
     if (need > 0) {
         memcpy(patterns, st + off_pat, static_cast<size_t>(need) * nw * 4);
         const uint32_t* c = reinterpret_cast<const uint32_t*>(st + off_cnt);
         for (int64_t i = 0; i < need; ++i) counts[i] = c[i];
     }
+    return MS_OK;
+}
+
+// The per-read positions in the order of the last ms_phase_haplotypes, on the device (b_hap); hap_assign_kernel runs here when
+// that call was made without hap_id.
+extern "C" int ms_phase_hap_device(ms_handle* h, int32_t** d_hap, int64_t* R) {
+    if (!h || !d_hap || !R) return MS_ERR_ARG;
+    if (!h->hap_ranked) MS_FAIL(h, MS_ERR_ARG, "ms_phase_hap_device: call ms_phase_haplotypes on the phased reads first");
+    MS_CUDA(h, cudaSetDevice(h->device));
+    MS_CUDA(h, h->b_hap.ensure(static_cast<size_t>(std::max<int64_t>(1, h->phase_n)) * 4));
+    if (!h->hap_assigned && h->phase_n > 0) {
+        ms::hap_assign_kernel<<<grid_for(h->phase_n, 256), 256, 0, h->stream>>>(h->b_slot.as<int32_t>(), h->b_rank.as<int32_t>(), h->phase_n,
+                                                                               h->b_hap.as<int32_t>());
+        h->launches++;
+        MS_CUDA(h, cudaGetLastError());
+        h->hap_assigned = true;
+    }
+    *d_hap = h->b_hap.as<int32_t>();
+    *R = h->phase_n;
     return MS_OK;
 }

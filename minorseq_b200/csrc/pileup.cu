@@ -45,23 +45,8 @@ __device__ __forceinline__ uint4 lds128(uint32_t addr) {
     asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
     return v;
 }
-__device__ __forceinline__ uint32_t lds32(uint32_t addr) {
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ void sts32(uint32_t addr, uint32_t v) {
-    asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
-}
 __device__ __forceinline__ void consumer_barrier(int nthreads) {
     asm volatile("bar.sync 1, %0;" ::"r"(nthreads) : "memory");
-}
-
-// carry-save adder: (h,l) = a + b + c per bit position.  Two LOP3.
-__device__ __forceinline__ void csa(uint32_t& h, uint32_t& l, uint32_t a, uint32_t b, uint32_t c) {
-    const uint32_t u = a ^ b;
-    h = (a & b) | (u & c);
-    l = u ^ c;
 }
 
 // DENSE: a second bit-sliced codon count per start column -- the "designated" codon (runner-up base of the pivot sample
@@ -76,50 +61,7 @@ struct Traits {
     static constexpr int iND = iNP + 1;                    // "not the designated codon" (DENSE only)
 };
 
-// ---------------------------------------------------------------- per-thread state
-template <int NM>
-struct Vert {
-    uint32_t c[NM][kPlanes];  // vertical counters, plane k has weight 2^k
-    uint32_t p3[NM], p4[NM], p5[NM];  // pending carry-save inputs of weight 8, 16 and 32
-};
-
-// Planes kPlanes and kPlanes+1 (weights 2048 and 4096) live in shared memory, one word per thread and mask: a carry out of
-// the register planes reaches them once per 2048 reads of a column, so they cost nothing in the hot loop and lift the
-// capacity of a row-group from 2047 to 8191 reads -- which keeps the barrier-ordered mid-kernel flush out of every
-// workload of ordinary size (it costs G serialised read-modify-write rounds over the CTA's slice).  HI is a template
-// switch: K1 sits at its register limit, and carrying the two extra values cost the 1M x 3 kb kernel 5 %, so launches
-// whose row-groups stay below 2048 reads use the instantiation without it.
-struct HiPlanes {
-    uint32_t base;     // shared-memory address of this thread's word of (plane kPlanes, mask 0)
-    uint32_t stride;   // bytes between consecutive masks (= threads * 4); plane kPlanes+1 follows the NM masks of plane kPlanes
-};
-template <int NM>
-__device__ __forceinline__ void hi_add(const HiPlanes& hp, int i, uint32_t x) {
-    const uint32_t a0 = hp.base + static_cast<uint32_t>(i) * hp.stride;
-    const uint32_t p = lds32(a0);
-    sts32(a0, p ^ x);
-    const uint32_t c = p & x;
-    if (c) {
-        const uint32_t a1 = a0 + static_cast<uint32_t>(NM) * hp.stride;
-        sts32(a1, lds32(a1) ^ c);     // capacity checked by the caller (kMaxReadsPerFlush): no carry out of this one
-    }
-}
-
-template <bool HI, int NM>
-__device__ __forceinline__ void ripple(Vert<NM>& v, const HiPlanes& hp, int i, int level, uint32_t x) {
-#pragma unroll
-    for (int k = 0; k < kPlanes; ++k) {
-        if (k >= level) {
-            const uint32_t t = v.c[i][k] & x;
-            v.c[i][k] ^= x;
-            x = t;
-        }
-    }
-    if (HI) {
-        if (x) hi_add<NM>(hp, i, x);
-    }
-}
-
+// ---------------------------------------------------------------- per-thread state (Vert, HiPlanes: pileup.cuh)
 // Per-thread constants for codon work
 struct CodonCtx {
     uint32_t r0, r1, r0n, r1n;  // pivot planes of this block and the next (the latter only for the rare path)
@@ -297,22 +239,6 @@ __device__ __forceinline__ void log_or_handle(uint32_t pm, ExcLog& lg, uint32_t 
 }
 
 // ---------------------------------------------------------------- flush (cold path)
-// 16 words x 32 bits holding two 16x16 bit matrices side by side: after the call, word j has
-// bit k (low half) = old word k bit j, and bit 16+k (high half) = old word k bit 16+j.
-__device__ __forceinline__ void transpose16x2(uint32_t (&a)[16]) {
-#pragma unroll
-    for (int s = 8; s >= 1; s >>= 1) {
-        const uint32_t m = s == 8 ? 0x00FF00FFu : s == 4 ? 0x0F0F0F0Fu : s == 2 ? 0x33333333u : 0x55555555u;
-#pragma unroll
-        for (int k = 0; k < 16; ++k) {
-            if (k & s) continue;
-            const uint32_t t = ((a[k] >> s) ^ a[k + s]) & m;
-            a[k + s] ^= t;
-            a[k] ^= t << s;
-        }
-    }
-}
-
 // planes: this thread's counters (pendings already folded), [NM][NP] in local memory (NP = kPlanes, or kPlanesAll with the shared-memory planes).
 // Adds the other groups' planes from shared memory (bit-sliced ripple-carry), transposes to
 // per-column integers and stores / adds them into the CTA's slice.
@@ -352,18 +278,8 @@ __device__ __noinline__ void emit_slice(const uint32_t* planes, uint32_t merge_b
             uint32_t s[NM];
 #pragma unroll
             for (int i = 0; i < NM; ++i) s[i] = half ? (tr[i][j] >> 16) : (tr[i][j] & 0xffffu);
-            // states: A=000 C=001 G=010 T=011 -=100 N=101 U=111 ; s0=sum p0, s1=sum p1, s2=sum p2,
-            // s3=sum p0&p1, s4=sum p0&p2, s5=sum p1&p2
-            const uint32_t nU = s[5];
-            const uint32_t nN = s[4] - nU;
-            const uint32_t nT = s[3] - nU;
-            const uint32_t nD = s[2] - nN - nU;
-            const uint32_t nG = s[1] - nT - nU;
-            const uint32_t nC = s[0] - nT - nN - nU;
-            const uint32_t cov = n - nU;
-            const uint32_t nA = cov - (nC + nG + nT + nD + nN);
-            uint4 lo = make_uint4(nA, nC, nG, nT);
-            uint4 hi = make_uint4(nD, nN, T::INS ? s[T::iINS] : 0u, cov);
+            uint4 lo, hi;
+            decode_counts(s, T::INS ? s[T::iINS] : 0u, n, lo, hi);
             uint4* dst = reinterpret_cast<uint4*>(pc + colj * 8);
             if (add) {
                 const uint4 x = dst[0], y = dst[1];
@@ -382,30 +298,6 @@ __device__ __noinline__ void emit_slice(const uint32_t* planes, uint32_t merge_b
                     pd[colj] = des;
                 }
             }
-        }
-    }
-}
-
-template <bool HI, int NM>
-__device__ __forceinline__ void fold_pendings(Vert<NM>& v, const HiPlanes& hp, uint32_t bi) {
-#pragma unroll
-    for (int i = 0; i < NM; ++i) {
-        if (bi & 1u) ripple<HI>(v, hp, i, 3, v.p3[i]);
-        if (bi & 2u) ripple<HI>(v, hp, i, 4, v.p4[i]);
-        if (bi & 4u) ripple<HI>(v, hp, i, 5, v.p5[i]);
-    }
-}
-
-template <bool HI, int NM>
-__device__ __forceinline__ void clear(Vert<NM>& v, const HiPlanes& hp) {
-#pragma unroll
-    for (int i = 0; i < NM; ++i) {
-#pragma unroll
-        for (int k = 0; k < kPlanes; ++k) v.c[i][k] = 0;
-        v.p3[i] = v.p4[i] = v.p5[i] = 0;
-        if (HI) {
-            sts32(hp.base + static_cast<uint32_t>(i) * hp.stride, 0u);
-            sts32(hp.base + static_cast<uint32_t>(NM + i) * hp.stride, 0u);
         }
     }
 }

@@ -84,9 +84,9 @@ struct Alignments {
     uint8_t* events = nullptr;         // pinned, ev_bytes
     int64_t ev_bytes = 0;
     std::vector<std::string> names;
-    // insertion events (only when want_insertions)
+    // insertion events (only when want_insertions); ins_read = the index of the event's read (in read order)
     std::vector<int32_t> ins_col, ins_len;
-    std::vector<int64_t> ins_off;
+    std::vector<int64_t> ins_off, ins_read;
     std::string ins_pool;
     ~Alignments() { ms_free_pinned(hdr); ms_free_pinned(events); }
 };
@@ -240,7 +240,7 @@ inline void expand_alignments(const Decoded& d, const QvFilter& qv, bool want_na
     if (ms_base_planes(out.base.data(), L, planes.data()) != MS_OK) throw std::runtime_error("ms_base_planes failed");
     // ---- every thread expands and encodes its contiguous range of the reads into buffers of its own
     struct Part {
-        std::vector<int32_t> col, len; std::vector<int64_t> off; std::string pool;
+        std::vector<int32_t> col, len; std::vector<int64_t> off, read; std::string pool;
         std::vector<ms_read_hdr> hdr; std::vector<uint8_t> ev; int64_t nbytes = 0;
     };
     nt = static_cast<unsigned>(std::min<size_t>(nt, keep.size()));
@@ -262,6 +262,7 @@ inline void expand_alignments(const Decoded& d, const QvFilter& qv, bool want_na
             const auto& rr = bx.records[keep[k]];
             msbam::BamReader::parse_record(u.data() + rr.first, rr.second, rec);
             expand_record(rec, qv, L, row.data(), want_insertions, mask, ic, io, il, pool, P.col, P.len, P.off, P.pool);
+            P.read.resize(P.col.size(), static_cast<int64_t>(k));
             if (static_cast<int64_t>(P.ev.size()) - P.nbytes < bound) P.ev.resize(P.ev.size() * 2 + static_cast<size_t>(bound));
             if (ms_encode_row(row.data(), L, planes.data(), &P.hdr[k - i0], P.ev.data(), static_cast<int64_t>(P.ev.size()), &P.nbytes) != MS_OK)
                 throw std::runtime_error("record " + rec.name + ": cannot encode the expanded row");
@@ -301,6 +302,7 @@ inline void expand_alignments(const Decoded& d, const QvFilter& qv, bool want_na
         const int64_t base = static_cast<int64_t>(out.ins_pool.size());
         out.ins_col.insert(out.ins_col.end(), p.col.begin(), p.col.end());
         out.ins_len.insert(out.ins_len.end(), p.len.begin(), p.len.end());
+        out.ins_read.insert(out.ins_read.end(), p.read.begin(), p.read.end());
         for (int64_t o : p.off) out.ins_off.push_back(base + o);
         out.ins_pool += p.pool;
     }

@@ -5,6 +5,8 @@
 // --mode-phasing (:192-211); --min-perc / --max-perc (:342-354); --drm-only (:370).  The unpinned model
 // constants (SURVEY App. B) are options with the restatement's defaults.  --linkage adds pairwise variant linkage
 // (restatement choice U14): per pair of called variants, the reads clean at both codons, D', r^2 and two Fisher tests.
+// A third output kind, out.fasta (with --mode-phasing), holds the consensus sequence of every reported haplotype (restatement
+// choice U15): a grouped pile-up of each haplotype's reads on the GPU and fuse's column rule with thin columns written as 'N'.
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -23,7 +25,8 @@
 #define MS_VERSION "minorseq_b200 juliet 0.1.0 (B200-native restatement; not PacBio juliet)"
 
 static void usage() {
-    puts("Usage: juliet [options] <in.bam> <out.json|out.html> [<out.html|out.json>]\n"
+    puts("Usage: juliet [options] <in.bam> <out.json|out.html|out.fasta> ...\n"
+         "  outputs by extension, one or more: .json report, .html report, .fasta haplotype sequences (needs --mode-phasing)\n"
          "  -c, --config <HIV|ABL1|file.json>  target configuration (genes, DRMs, referenceSequence); the built-in HIV and ABL1\n"
          "                                     hold only what the public documentation shows (doc/JULIET.md:138-157 and the\n"
          "                                     target screenshot), not PacBio's full tables: pass the real config as a file\n"
@@ -38,6 +41,8 @@ static void usage() {
          "      --deletion-rate <r>            error model (default 3e-3)\n"
          "      --alpha <a>                    significance after Bonferroni (default 0.01)\n"
          "      --min-haplotype-reads <n>      reads needed to report a haplotype (default 10)\n"
+         "      --hap-min-coverage <n>         .fasta: a column with fewer votes of the haplotype's reads is written 'N'\n"
+         "                                     (default 10; leading and trailing runs of such columns are trimmed)\n"
          "      --qv-threshold <q>             rich-QV base filter, 0 = off (default 20 on dq,iq,sq when present)\n"
          "      --device <n>                   first CUDA device (default 0)\n"
          "      --gpus <n>                     shard the reads over n GPUs (devices n0..n0+n-1) of this machine: contiguous read\n"
@@ -58,7 +63,7 @@ int main(int argc, char** argv) {
     std::string config, region, cmdline, timing_json;
     bool phasing = false, drm_only = false, linkage = false;
     double min_perc = -1, max_perc = -1, sub = 5e-4, del = 3e-3, alpha = 0.01;
-    int min_hap = 10, device = 0, ngpus = 1;
+    int min_hap = 10, device = 0, ngpus = 1, hap_min_cov = 10;
     const int link_min_reads = 10;   // reads clean at both codons that a tested pair needs (the haplotype default, F21)
     mshost::QvFilter qv;
     std::vector<std::string> pos;
@@ -82,6 +87,7 @@ int main(int argc, char** argv) {
         else if (a == "--deletion-rate") del = atof(need("--deletion-rate").c_str());
         else if (a == "--alpha") alpha = atof(need("--alpha").c_str());
         else if (a == "--min-haplotype-reads") min_hap = atoi(need("--min-haplotype-reads").c_str());
+        else if (a == "--hap-min-coverage") hap_min_cov = atoi(need("--hap-min-coverage").c_str());
         else if (a == "--qv-threshold") qv.threshold = atoi(need("--qv-threshold").c_str());
         else if (a == "--device") device = atoi(need("--device").c_str());
         else if (a == "--gpus") ngpus = atoi(need("--gpus").c_str());
@@ -91,12 +97,15 @@ int main(int argc, char** argv) {
     }
     if (pos.size() < 2) { usage(); return 1; }
     if (ngpus < 1 || ngpus > 64) mshost::die("--gpus expects 1..64");
-    std::string out_json, out_html;
+    std::string out_json, out_html, out_fasta;
     for (size_t i = 1; i < pos.size(); ++i) {
         if (ends_with(pos[i], ".json")) out_json = pos[i];
         else if (ends_with(pos[i], ".html")) out_html = pos[i];
-        else mshost::die("output must end in .json or .html: " + pos[i]);
+        else if (ends_with(pos[i], ".fasta")) out_fasta = pos[i];
+        else mshost::die("output must end in .json, .html or .fasta: " + pos[i]);
     }
+    if (!out_fasta.empty() && !phasing) mshost::die("a .fasta output holds the haplotypes' sequences: it needs --mode-phasing");
+    if (hap_min_cov < 0) mshost::die("--hap-min-coverage expects a count >= 0");
     int rb = 0, re = 0;
     if (!region.empty()) {
         if (sscanf(region.c_str(), "%d-%d", &rb, &re) != 2 || rb < 1 || re <= rb) mshost::die("--region expects <begin-end>");
@@ -121,7 +130,8 @@ int main(int argc, char** argv) {
         // with --gpus N every GPU gets its own handle and the handles share one NCCL communicator (one rank per thread)
         std::vector<ms_handle*> hs(static_cast<size_t>(ngpus), nullptr);
         mshost::Alignments aln;
-        mshost::load_alignments_overlapped(pos[0], qv, phasing, false, cfg.reference_sequence, aln, [&] {
+        const bool fasta = !out_fasta.empty();
+        mshost::load_alignments_overlapped(pos[0], qv, phasing, fasta, cfg.reference_sequence, aln, [&] {
             char id[128];
             if (ngpus > 1 && ms_comm_unique_id(id) != MS_OK) mshost::die("NCCL is not available (libnccl.so.2): --gpus needs it");
             std::vector<std::string> errs(static_cast<size_t>(ngpus));
@@ -174,6 +184,7 @@ int main(int argc, char** argv) {
         int64_t nrep_all = 0;
         std::vector<ms_linkage_pair> link_pairs;
         int64_t link_tested = 0;
+        std::vector<const uint32_t*> rows_dev(static_cast<size_t>(ngpus), nullptr);   // each rank's reads on its GPU (tiles)
         std::vector<std::string> errs(static_cast<size_t>(ngpus));
 #define CKR(call)                                                                                      \
     do {                                                                                               \
@@ -195,6 +206,7 @@ int main(int argc, char** argv) {
             if (prc == MS_OK && ngpus > 1) ms_synchronize(h);     // the shard's header copy is ours to free once the upload is done
             if (ngpus > 1) ms_free_pinned(my_hdr);
             if (prc != MS_OK) { errs[r] = std::string("ms_pileup_events_host failed: ") + ms_last_error(h); return; }
+            rows_dev[r] = d_rows;
             CKR(ms_allreduce_counts(h));
             CKR(ms_synchronize(h));
             if (r == 0) lap(ngpus > 1 ? "H2D events + expand + pileup + all-reduce" : "H2D events + expand + pileup");
@@ -278,7 +290,6 @@ int main(int argc, char** argv) {
             }
             if (r == 0) rows.swap(my_rows);
         });
-#undef CKR
         for (const std::string& e : errs)
             if (!e.empty()) mshost::die(e);
         ms_handle* h = hs[0];
@@ -338,6 +349,53 @@ int main(int argc, char** argv) {
         }
 
         lap(linkage ? "phasing + linkage" : "phasing");
+
+        // haplotype sequences: every rank piles up its reads per haplotype (labels: the ranks' positions in the haplotype
+        // order, on the device), one all-reduce sums the group counts, rank 0 calls them with all insertion events
+        std::string fasta_text;
+        if (fasta) {
+            const int32_t nrep = static_cast<int32_t>(nrep_all);
+            mshost::run_ranks(ngpus, [&](int r) {
+                ms_handle* h = hs[r];
+                const int64_t r0 = aln.nreads * r / ngpus, r1 = aln.nreads * (r + 1) / ngpus;
+                int32_t* d_hap = nullptr;
+                int64_t nh = 0;
+                CKR(ms_phase_hap_device(h, &d_hap, &nh));
+                if (nh != r1 - r0) { errs[r] = "ms_phase_hap_device: unexpected read count"; return; }
+                CKR(ms_set_groups(h, nrep));
+                CKR(ms_group_pileup_dev(h, rows_dev[r], d_hap, r1 - r0));
+                CKR(ms_allreduce_group_counts(h));
+                CKR(ms_synchronize(h));
+            });
+            for (const std::string& e : errs)
+                if (!e.empty()) mshost::die(e);
+            ms_fuse_params fp;
+            ms_fuse_params_default(&fp);
+            fp.min_coverage = hap_min_cov;
+            std::vector<int32_t> ins_hap(aln.ins_read.size());
+            for (size_t i = 0; i < ins_hap.size(); ++i) ins_hap[i] = hap[aln.ins_read[i]];
+            std::vector<int64_t> seq_off(static_cast<size_t>(nrep) + 1, 0);
+            std::string seqs(static_cast<size_t>(nrep) * (static_cast<size_t>(L) + 16), '\0');
+            for (;;) {
+                const int rc = ms_group_consensus(h, &fp, ins_hap.data(), aln.ins_col.data(), aln.ins_off.data(), aln.ins_len.data(),
+                                                  static_cast<int64_t>(ins_hap.size()), aln.ins_pool.data(), static_cast<int64_t>(aln.ins_pool.size()),
+                                                  seqs.empty() ? nullptr : &seqs[0], static_cast<int64_t>(seqs.size()), seq_off.data());
+                if (rc == MS_ERR_CAPACITY) { seqs.resize(static_cast<size_t>(seq_off[nrep])); continue; }
+                if (rc != MS_OK) mshost::die(std::string("ms_group_consensus failed: ") + ms_last_error(h));
+                break;
+            }
+            std::string stem = pos[0];
+            const size_t sl = stem.find_last_of('/');
+            if (sl != std::string::npos) stem = stem.substr(sl + 1);
+            for (int32_t k = 0; k < nrep; ++k) {
+                char nb[3];
+                ms_haplotype_name(k, nb);
+                fasta_text += ">" + stem + "|haplotype_" + nb + "|" + aln.ref_name + " reads=" + std::to_string(cnt[k]) + "\n";
+                for (int64_t i = seq_off[k]; i < seq_off[k + 1]; i += 70)
+                    fasta_text += seqs.substr(static_cast<size_t>(i), static_cast<size_t>(std::min<int64_t>(70, seq_off[k + 1] - i))) + "\n";
+            }
+            lap("haplotype consensus");
+        }
         char ts[40];
         const auto now = std::chrono::system_clock::now();
         const std::time_t tt = std::chrono::system_clock::to_time_t(now);
@@ -361,7 +419,13 @@ int main(int argc, char** argv) {
             if (!f) mshost::die("cannot write " + out_html);
             f << msreport::to_html(report);
         }
+        if (fasta) {
+            std::ofstream f(out_fasta);
+            if (!f) mshost::die("cannot write " + out_fasta);
+            f << fasta_text;
+        }
         lap("report writing");
+#undef CKR
         if (!timing_json.empty()) {
             msjson::Value t = msjson::Value::object();
             msjson::Value st = msjson::Value::array();
