@@ -115,10 +115,12 @@ int ms_pileup_kernel_ms(ms_handle *h, double *ms, int64_t *reads);
  * copy stream, MS_STAGE_PASS = start of the pass to the arrival of its last result on the main stream.             */
 /* Pairwise linkage adds two: MS_STAGE_LINKAGE_STATS = its statistics kernels (m, tests, row offsets), MS_STAGE_LINKAGE_ALLREDUCE
  * = the all-reduce of its Gram matrix; its contraction is timed as MS_STAGE_COOCCURRENCE.  MS_STAGE_GROUP_PILEUP = the
- * grouped pile-up kernel of ms_group_pileup_dev (without the counting sort in front of it).                                  */
+ * grouped pile-up kernel of ms_group_pileup_dev (without the counting sort in front of it).  Read alignment adds two:
+ * MS_STAGE_ALIGN_SEED = align_seed_kernel, MS_STAGE_ALIGN_BAND = align_band_kernel (banded DP and traceback) of the last
+ * chunk of ms_align_reads.                                                                                                 */
 enum { MS_STAGE_PHASE_BITS = 1, MS_STAGE_COOCCURRENCE = 2, MS_STAGE_EXPAND = 3, MS_STAGE_ALLREDUCE = 4, MS_STAGE_HAPMERGE = 5,
        MS_STAGE_UPLOAD = 6, MS_STAGE_PASS = 7, MS_STAGE_LINKAGE_STATS = 8, MS_STAGE_LINKAGE_ALLREDUCE = 9,
-       MS_STAGE_GROUP_PILEUP = 10 };
+       MS_STAGE_GROUP_PILEUP = 10, MS_STAGE_ALIGN_SEED = 11, MS_STAGE_ALIGN_BAND = 12 };
 int ms_stage_kernel_ms(ms_handle *h, int stage, double *ms);
 
 /* ---- K1: pileup (juliet "MSA counts", doc/JULIET.md:96-100; fuse doc/FUSE.md:17-20) -- */
@@ -371,6 +373,28 @@ int ms_group_consensus(ms_handle *h, const ms_fuse_params *prm, const int32_t *i
  * The per-read CIGAR projection through this path is host code (minorseq_b200/host/cleric.hpp).   */
 int ms_align_refs(ms_handle *h, const char *a, int32_t la, const char *b, int32_t lb,
                   char *ops, int64_t cap, int64_t *nops, int64_t *score);
+
+/* ---- K6: read alignment (restatement choice U16; DESIGN.md "K6 read alignment") ---------------------------------
+ * Overlap alignment of unaligned CCS reads to one amplicon reference: unique 15-mer seeds pick the strand and a start
+ * diagonal, then a 128-cell adaptive band (Suzuki & Kasahara) with U13's scores (match +2, mismatch -3, linear gap -4)
+ * finds the best path from the top or left edge to the bottom or right edge.  Reads and references are at most 65535
+ * bases.  A read is its native sequence (the caller reverse-complements a BAM record with flag 0x10 first).
+ * ms_align_set_reference builds the seed index (host) and uploads it with the reference; it stays until the next call. */
+typedef struct { int32_t min_seeds; } ms_align_params;    /* the winning strand's seed support must reach min_seeds (>= 1) */
+typedef struct {
+    int32_t mapped;        /* 0: no strand reached min_seeds; the other fields are strand 0, pos -1, score 0, no CIGAR */
+    int32_t strand;        /* 1: the reverse complement of the read was aligned (BAM flag 0x10) */
+    int32_t pos;           /* 0-based reference position of the first aligned base */
+    int32_t score;         /* the alignment's score (AS:i) */
+    int64_t cigar_off;     /* first op in the caller's cigar array */
+    int32_t ncigar;        /* ops: BAM-encoded len << 4 | op, only S = X I D, in the aligned strand's orientation */
+} ms_read_alignment;
+void ms_align_params_default(ms_align_params *p);    /* min_seeds 10 */
+int ms_align_set_reference(ms_handle *h, const char *ref, int32_t L);
+/* R reads, read r = seq[off[r] .. off[r+1]) (off: R + 1 entries).  out: R entries, in read order.  *ncigar receives the
+ * total number of ops; MS_ERR_CAPACITY when it exceeds cap (out is filled all the same; call again with a larger cigar). */
+int ms_align_reads(ms_handle *h, const ms_align_params *prm, const char *seq, const int64_t *off, int64_t R,
+                   ms_read_alignment *out, uint32_t *cigar, int64_t cap, int64_t *ncigar);
 
 /* ---- synthetic amplicon generator (bench/tests; SURVEY 8d) ------------------------- */
 typedef struct {

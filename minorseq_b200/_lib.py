@@ -56,6 +56,15 @@ class ReadHdr(C.Structure):
     _fields_ = [("ev_off", C.c_uint32), ("begin", C.c_uint16), ("end", C.c_uint16)]
 
 
+class AlignParams(C.Structure):
+    _fields_ = [("min_seeds", C.c_int32)]
+
+
+class ReadAlignment(C.Structure):
+    _fields_ = [("mapped", C.c_int32), ("strand", C.c_int32), ("pos", C.c_int32), ("score", C.c_int32), ("cigar_off", C.c_int64),
+                ("ncigar", C.c_int32)]
+
+
 class SynthParams(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("L", C.c_int32), ("nstrains", C.c_int32), ("thr_N", C.c_uint32),
                 ("thr_sub", C.c_uint32), ("thr_ins20", C.c_uint32), ("thr_trunc16", C.c_uint32)]
@@ -109,6 +118,9 @@ _SIGNATURES = {
     "ms_haplotype_name": (None, [C.c_int64, C.c_char_p]),
     "ms_phase_assign": (C.c_int, [_P, _P, C.c_int64, _P]),
     "ms_align_refs": (C.c_int, [_P, C.c_char_p, C.c_int32, C.c_char_p, C.c_int32, _P, C.c_int64, _P, _P]),
+    "ms_align_params_default": (None, [C.POINTER(AlignParams)]),
+    "ms_align_set_reference": (C.c_int, [_P, C.c_char_p, C.c_int32]),
+    "ms_align_reads": (C.c_int, [_P, C.POINTER(AlignParams), C.c_char_p, _P, C.c_int64, _P, _P, C.c_int64, C.POINTER(C.c_int64)]),
     "ms_set_cooccurrence_variant": (C.c_int, [_P, C.c_int32]),
     "ms_phase_haplotypes": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "ms_phase_device": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_P), C.POINTER(C.c_int64)]),

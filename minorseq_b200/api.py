@@ -13,7 +13,8 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _lib
-from ._lib import (CallParams, FuseParams, Gene, LinkagePair, LinkageParams, PhaseCounters, SynthParams, Variant, check)
+from ._lib import (AlignParams, CallParams, FuseParams, Gene, LinkagePair, LinkageParams, PhaseCounters, ReadAlignment, SynthParams, Variant,
+                   check)
 from .synth import start_mask_words, tile_rows, untile_rows
 
 CODONS = [a + b + c for a in "ACGT" for b in "ACGT" for c in "ACGT"]
@@ -734,3 +735,47 @@ def _gather_groups(pat, cnt, marg, device):
         pats.append(b[1: 1 + k, :nw].astype(np.uint32))
         cnts.append(b[1: 1 + k, nw].astype(np.uint64))
     return np.concatenate(pats, axis=0), np.concatenate(cnts), m
+
+
+CIGAR_OPS = "MIDNSHP=X"
+
+
+class Aligner:
+    """Overlap alignment of unaligned reads to one amplicon reference on the GPU (K6, restatement choice U16)."""
+
+    def __init__(self, device=0, min_seeds=10, handle=None):
+        self.hd = handle or Handle(device)
+        self.lib = self.hd.lib
+        self.params = AlignParams(int(min_seeds))
+
+    def set_reference(self, ref: str):
+        b = ref.encode()
+        check(self.lib.ms_align_set_reference(self.hd.h, b, len(b)), self.hd.h)
+
+    def align_raw(self, reads):
+        """reads: list of str (native orientation).  Returns (ms_read_alignment array, u32 BAM-encoded CIGAR ops)."""
+        seq = "".join(reads).encode()
+        off = np.zeros(len(reads) + 1, dtype=np.int64)
+        off[1:] = np.cumsum([len(r) for r in reads])
+        out = (ReadAlignment * max(1, len(reads)))()
+        cap = int(off[-1] // 8 + 16)
+        while True:
+            cig = np.zeros(cap, dtype=np.uint32)
+            n = C.c_int64()
+            rc = self.lib.ms_align_reads(self.hd.h, C.byref(self.params), seq, _ptr(off), len(reads), out, _ptr(cig), cap, C.byref(n))
+            if rc == -4:   # MS_ERR_CAPACITY: n holds the number of ops
+                cap = n.value
+                continue
+            check(rc, self.hd.h)
+            return out, cig[:n.value]
+
+    def align(self, reads):
+        """list of (mapped, strand, pos, score, cigar string) in read order; unmapped reads are (False, 0, -1, 0, "")."""
+        out, cig = self.align_raw(reads)
+        res = []
+        for r in range(len(reads)):
+            a = out[r]
+            ops = cig[a.cigar_off:a.cigar_off + a.ncigar]
+            res.append((bool(a.mapped), int(a.strand), int(a.pos), int(a.score),
+                        "".join(f"{int(x) >> 4}{CIGAR_OPS[int(x) & 15]}" for x in ops)))
+        return res

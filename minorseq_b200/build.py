@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libminorseq_b200.so")
-SOURCES = ["abi_core.cu", "pileup.cu", "format.cu", "synth.cu", "call.cu", "phase.cu", "phase_order.cu", "cooc_tc.cu", "fuse.cu", "comm.cu", "pass.cu", "nw.cu", "events.cu", "tiles.cu", "linkage.cu", "group.cu"]
+SOURCES = ["abi_core.cu", "pileup.cu", "format.cu", "synth.cu", "call.cu", "phase.cu", "phase_order.cu", "cooc_tc.cu", "fuse.cu", "comm.cu", "pass.cu", "nw.cu", "events.cu", "tiles.cu", "linkage.cu", "group.cu", "align.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-fmad=false",  # K2's fp64 path must not contract a*b+c (fisher_core.h)
@@ -41,7 +41,7 @@ def build_library(force=False, verbose=False):
 
 HOST = os.path.join(HERE, "host")
 BIN = os.path.join(HERE, "bin")
-HOST_PROGRAMS = {"juliet": "juliet_main.cpp", "fuse": "fuse_main.cpp", "host_selftest": "host_selftest.cpp", "mixdata": "mixdata_main.cpp", "packed2bam": "packed2bam_main.cpp", "cleric": "cleric_main.cpp"}
+HOST_PROGRAMS = {"juliet": "juliet_main.cpp", "fuse": "fuse_main.cpp", "host_selftest": "host_selftest.cpp", "mixdata": "mixdata_main.cpp", "packed2bam": "packed2bam_main.cpp", "cleric": "cleric_main.cpp", "align": "align_main.cpp", "julietflow": "julietflow_main.cpp"}
 
 
 def build_host(force=False):
@@ -53,7 +53,7 @@ def build_host(force=False):
         if not force and os.path.exists(out) and all(os.path.getmtime(d) <= os.path.getmtime(out) for d in hdrs if os.path.exists(d)):
             continue
         cmd = ["/usr/bin/g++", "-O3", "-std=c++17", "-Wall", "-I/usr/local/cuda/include", "-o", out, os.path.join(HOST, src), "-lz", "-pthread", "-ldl"]
-        if name in ("juliet", "fuse", "cleric"):
+        if name in ("juliet", "fuse", "cleric", "align"):
             cmd += ["-L" + HERE, "-lminorseq_b200", "-Wl,-rpath,$ORIGIN/..", "-Wl,-rpath," + HERE]
         res = subprocess.run(cmd, capture_output=True, text=True)
         if res.returncode != 0:

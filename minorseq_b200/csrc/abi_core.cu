@@ -54,7 +54,9 @@ int ms_create(int device, ms_handle** out) {
         cudaEventCreate(&h->ev_stage[7][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[7][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[8][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[8][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[9][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[9][1]) != cudaSuccess ||
-        cudaEventCreate(&h->ev_stage[10][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[10][1]) != cudaSuccess) {
+        cudaEventCreate(&h->ev_stage[10][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[10][1]) != cudaSuccess ||
+        cudaEventCreate(&h->ev_stage[11][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[11][1]) != cudaSuccess ||
+        cudaEventCreate(&h->ev_stage[12][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[12][1]) != cudaSuccess) {
         g_create_error = cudaGetErrorString(cudaGetLastError());
         delete h;
         return MS_ERR_CUDA;
@@ -104,6 +106,9 @@ void ms_destroy(ms_handle* h) {
     h->b_exc_list.release(); h->b_exc_cnt.release();
     h->b_base.release(); h->b_ev_hdr.release(); h->b_ev.release();
     for (DevBuf* b : {&h->b_gcol, &h->b_ghist, &h->b_gtot, &h->b_goff, &h->b_gioff, &h->b_glist}) b->release();
+    for (DevBuf* b : {&h->b_aln_ref, &h->b_aln_idx, &h->b_aln_seq, &h->b_aln_off, &h->b_aln_seed, &h->b_aln_scratch, &h->b_aln_slab,
+                      &h->b_aln_mbits, &h->b_aln_cig, &h->b_aln_res, &h->b_aln_ctr, &h->b_aln_dst, &h->b_aln_pack})
+        b->release();
     for (cudaEvent_t ev : h->ev_chunk) cudaEventDestroy(ev);
     for (cudaEvent_t ev : h->ev_stagefree) cudaEventDestroy(ev);
     h->b_rowstage[0].release(); h->b_rowstage[1].release();
@@ -112,7 +117,7 @@ void ms_destroy(ms_handle* h) {
     cudaEventDestroy(h->ev_copy[0]); cudaEventDestroy(h->ev_copy[1]);
     cudaEventDestroy(h->ev_k1[0]); cudaEventDestroy(h->ev_k1[1]);
     cudaEventDestroy(h->ev_timer[0]); cudaEventDestroy(h->ev_timer[1]);
-    for (int s = 1; s < 11; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
+    for (int s = 1; s < 13; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
     cudaStreamDestroy(h->own_stream); cudaStreamDestroy(h->copy_stream);
     delete h;
 }
@@ -179,7 +184,7 @@ int ms_pileup_kernel_ms(ms_handle* h, double* ms, int64_t* reads) {
 }
 
 int ms_stage_kernel_ms(ms_handle* h, int stage, double* ms) {
-    if (!h || !ms || stage < 1 || stage > 10 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
+    if (!h || !ms || stage < 1 || stage > 12 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
     MS_CUDA(h, cudaSetDevice(h->device));
     MS_CUDA(h, cudaEventSynchronize(h->ev_stage[stage][1]));
     float f = 0.f;

@@ -43,8 +43,8 @@ struct ms_handle {
     cudaEvent_t ev_k1[2] = {nullptr, nullptr};  // around the last K1 launch when timing is on
     cudaEvent_t ev_timer[2] = {nullptr, nullptr};  // ms_timer_start / ms_timer_stop
     int expand_ctas = 0, expand_ctas_nblk = -1;   // expand_events_kernel: resident CTAs per SM for row length nblk
-    cudaEvent_t ev_stage[11][2] = {};              // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
-    bool stage_seen[11] = {false, false, false, false, false, false, false, false, false, false, false};
+    cudaEvent_t ev_stage[13][2] = {};              // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
+    bool stage_seen[13] = {};
     bool timing = false;
     int64_t k1_reads = 0;
     std::string err;
@@ -136,6 +136,12 @@ struct ms_handle {
     int32_t label_groups = -1;   // ms_set_groups; -1 = not set
     int32_t label_L = 0;         // L of the layout the group counts belong to
     DevBuf b_gcol, b_ghist, b_gtot, b_goff, b_gioff, b_glist;
+
+    // read alignment (align.cu): the reference and its seed hash table, then per chunk of reads their bases and offsets, seeds,
+    // the seed kernel's hit scratch, the band kernel's move-bit slabs and band-move bits, CIGAR slots, results, packed CIGARs
+    int32_t aln_L = -1, aln_bits = 0;   // reference length (-1 = none set), log2 of the hash table's size
+    DevBuf b_aln_ref, b_aln_idx, b_aln_seq, b_aln_off, b_aln_seed, b_aln_scratch, b_aln_slab, b_aln_mbits, b_aln_cig, b_aln_res, b_aln_ctr,
+        b_aln_dst, b_aln_pack;
 };
 
 #define MS_CUDA(h, call)                                                                    \
