@@ -117,10 +117,12 @@ int ms_pileup_kernel_ms(ms_handle *h, double *ms, int64_t *reads);
  * = the all-reduce of its Gram matrix; its contraction is timed as MS_STAGE_COOCCURRENCE.  MS_STAGE_GROUP_PILEUP = the
  * grouped pile-up kernel of ms_group_pileup_dev (without the counting sort in front of it).  Read alignment adds two:
  * MS_STAGE_ALIGN_SEED = align_seed_kernel, MS_STAGE_ALIGN_BAND = align_band_kernel (banded DP and traceback) of the last
- * chunk of ms_align_reads.                                                                                                 */
+ * chunk of ms_align_reads.  Haplotype abundance adds two: MS_STAGE_ABUNDANCE_COMPAT = abundance_compat_kernel,
+ * MS_STAGE_ABUNDANCE_EM = the EM iterations (host checks included).                                                      */
 enum { MS_STAGE_PHASE_BITS = 1, MS_STAGE_COOCCURRENCE = 2, MS_STAGE_EXPAND = 3, MS_STAGE_ALLREDUCE = 4, MS_STAGE_HAPMERGE = 5,
        MS_STAGE_UPLOAD = 6, MS_STAGE_PASS = 7, MS_STAGE_LINKAGE_STATS = 8, MS_STAGE_LINKAGE_ALLREDUCE = 9,
-       MS_STAGE_GROUP_PILEUP = 10, MS_STAGE_ALIGN_SEED = 11, MS_STAGE_ALIGN_BAND = 12 };
+       MS_STAGE_GROUP_PILEUP = 10, MS_STAGE_ALIGN_SEED = 11, MS_STAGE_ALIGN_BAND = 12, MS_STAGE_ABUNDANCE_COMPAT = 13,
+       MS_STAGE_ABUNDANCE_EM = 14 };
 int ms_stage_kernel_ms(ms_handle *h, int stage, double *ms);
 
 /* ---- K1: pileup (juliet "MSA counts", doc/JULIET.md:96-100; fuse doc/FUSE.md:17-20) -- */
@@ -300,6 +302,36 @@ int ms_linkage(ms_handle *h, const ms_linkage_params *prm, ms_linkage_pair *out,
  * both = G[v][w], v carried and w clean = G[v][h+w], n = G[h+v][h+w], diag(M^T M) = K2 coverage, diag(B^T B) = K2 count.
  * Owned by the handle; same caching and collective rule as ms_linkage.                                              */
 int ms_linkage_device(ms_handle *h, int32_t **d_gram, int32_t *dim);
+
+/* ---- haplotype abundance (restatement choice U18) ------------------------------------------------
+ * Phasing counts a haplotype's reads among the reads that are clean at EVERY key; abundance also uses the damaged ones.
+ * With B (read carries key v's codon) and M (key v's three columns are all A/C/G/T) as in linkage, read r is compatible
+ * with pattern h iff B[r][v] == P[h][v] for every v with M[r][v] = 1; S_r = the patterns it is compatible with.  A read is
+ * "incompatible" (S_r empty), "uninformative" (S_r = all H patterns, H >= 2), "unique" (|S_r| = 1) or "ambiguous".  The
+ * unique and ambiguous reads (N of them) give the maximum-likelihood frequencies by EM: pi_h = 1/H to start, then
+ *     pi'_h = (1/N) sum_r [h in S_r] pi_h / sum_{h' in S_r} pi_h'
+ * until max_h |pi' - pi| < tolerance or max_iterations iterations.  Reads with the same S_r form a class; the classes are
+ * merged over the ranks and totally ordered (count desc, then mask words asc), and the EM runs over them in that order with
+ * fixed-order sums: the same bits on every run, rank and number of GPUs.                                                */
+typedef struct { double tolerance; int32_t max_iterations; } ms_abundance_params;
+typedef struct {
+    uint64_t unique_reads;       /* reads with S_r = {h} */
+    uint64_t compatible_reads;   /* reads with h in S_r */
+    double em_frequency;         /* pi_h */
+} ms_abundance_row;
+typedef struct { uint64_t unique, ambiguous, uninformative, incompatible; } ms_abundance_counters;
+/* tolerance 1e-10, max_iterations 10000 */
+void ms_abundance_params_default(ms_abundance_params *p);
+/* on: the next ms_phase_begin also allocates the clean-codon matrix and ms_phase_dev fills it (as ms_set_linkage). */
+int ms_set_abundance(ms_handle *h, int on);
+/* The abundance of H distinct patterns (rows of max(1, ceil(V/32)) words, as ms_phase_haplotypes returns them; bits >= V
+ * are ignored; H <= 4096) over the phased reads (with a communicator attached: all ranks' reads; a collective, and every
+ * rank passes the same patterns).  rows[h] in the order of the patterns; MS_ERR_CAPACITY when cap < H (nothing is
+ * computed).  MS_ERR_ARG for duplicate patterns, H > 4096, or reads phased without ms_set_abundance / ms_set_linkage.
+ * H = 0 or N = 0: no EM (pi = 1/H, *iterations 0, *converged 1).  *loglik = sum over the N reads of log sum_{h in S_r} pi_h. */
+int ms_haplotype_abundance(ms_handle *h, const ms_abundance_params *prm, const uint32_t *patterns, int64_t H,
+                           ms_abundance_row *rows, int64_t cap, ms_abundance_counters *counters, int32_t *iterations,
+                           int32_t *converged, double *loglik);
 
 /* ---- the whole juliet pass in one call ------------------------------------------------------
  * reset -> pileup -> (all-reduce when a communicator is attached) -> codon test -> phasing, i.e. everything

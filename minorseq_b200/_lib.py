@@ -52,6 +52,18 @@ class LinkagePair(C.Structure):
                 ("neither", C.c_uint32), ("d_prime", C.c_double), ("r2", C.c_double), ("pvalue", C.c_double), ("relation", C.c_int32)]
 
 
+class AbundanceParams(C.Structure):
+    _fields_ = [("tolerance", C.c_double), ("max_iterations", C.c_int32)]
+
+
+class AbundanceRow(C.Structure):
+    _fields_ = [("unique_reads", C.c_uint64), ("compatible_reads", C.c_uint64), ("em_frequency", C.c_double)]
+
+
+class AbundanceCounters(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("unique", "ambiguous", "uninformative", "incompatible")]
+
+
 class ReadHdr(C.Structure):
     _fields_ = [("ev_off", C.c_uint32), ("begin", C.c_uint16), ("end", C.c_uint16)]
 
@@ -130,6 +142,10 @@ _SIGNATURES = {
     "ms_linkage": (C.c_int, [_P, C.POINTER(LinkageParams), C.POINTER(LinkagePair), C.c_int64, C.POINTER(C.c_int64),
                              C.POINTER(C.c_int64)]),
     "ms_linkage_device": (C.c_int, [_P, C.POINTER(_P), C.POINTER(C.c_int32)]),
+    "ms_abundance_params_default": (None, [C.POINTER(AbundanceParams)]),
+    "ms_set_abundance": (C.c_int, [_P, C.c_int]),
+    "ms_haplotype_abundance": (C.c_int, [_P, C.POINTER(AbundanceParams), _P, C.c_int64, C.POINTER(AbundanceRow), C.c_int64,
+                                         C.POINTER(AbundanceCounters), C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_double)]),
     "ms_juliet_pass_dev": (C.c_int, [_P, _P, C.c_int64, C.POINTER(Gene), C.c_int32, C.c_char_p, C.POINTER(CallParams), C.c_int32,
                                    C.c_int32, C.POINTER(JulietResult)]),
     "ms_juliet_pass_host": (C.c_int, [_P, _P, C.c_int64, C.POINTER(Gene), C.c_int32, C.c_char_p, C.POINTER(CallParams), C.c_int32,

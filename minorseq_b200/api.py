@@ -13,7 +13,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _lib
-from ._lib import (AlignParams, CallParams, FuseParams, Gene, LinkagePair, LinkageParams, PhaseCounters, ReadAlignment, SynthParams, Variant,
+from ._lib import (AbundanceCounters, AbundanceParams, AbundanceRow, AlignParams, CallParams, FuseParams, Gene, LinkagePair, LinkageParams, PhaseCounters, ReadAlignment, SynthParams, Variant,
                    check)
 from .synth import start_mask_words, tile_rows, untile_rows
 
@@ -69,6 +69,26 @@ class Linkage:
     a: np.ndarray
     b: np.ndarray
     c: np.ndarray
+
+
+@dataclass
+class Abundance:
+    """Haplotype abundance (Juliet.haplotype_abundance, restatement choice U18): per pattern, in the order given, the reads
+    compatible with it alone and with it at all, and the EM's frequency over the unique and ambiguous reads."""
+    unique_reads: np.ndarray        # [H] uint64
+    compatible_reads: np.ndarray    # [H] uint64
+    em_frequency: np.ndarray        # [H] float64
+    counters: dict                  # unique, ambiguous, uninformative, incompatible
+    reads_used: int                 # unique + ambiguous: the EM's reads
+    iterations: int
+    converged: bool
+    log_likelihood: float
+    tolerance: float
+    max_iterations: int
+
+    @property
+    def em_reads(self):
+        return self.em_frequency * self.reads_used
 
 
 @dataclass
@@ -235,8 +255,9 @@ class Juliet:
 
     # -- K3
     def phase_device(self, variants, d_packed_ptr: int, nreads: int, want_hap_id=True, host_merge=False, cap=4096,
-                     linkage=False) -> Haplotypes:
-        """linkage: also record which reads are clean at each key, for Juliet.linkage afterwards"""
+                     linkage=False, abundance=False) -> Haplotypes:
+        """linkage / abundance: also record which reads are clean at each key, for Juliet.linkage / Juliet.haplotype_abundance
+        afterwards"""
         import torch.distributed as dist
         keys = sorted({(v.col, v.codon) for v in variants})
         V = len(keys)
@@ -246,11 +267,15 @@ class Juliet:
         self._V = V
         self._keys = keys
         self._nreported = None             # set when the device path below leaves per-read ranks on the device
+        self._reported = None
         check(self.lib.ms_set_linkage(self.hd.h, 1 if linkage else 0), self.hd.h)
+        check(self.lib.ms_set_abundance(self.hd.h, 1 if abundance else 0), self.hd.h)
         check(self.lib.ms_phase_begin(self.hd.h, _ptr(vc), _ptr(vd), V, nreads), self.hd.h)
         check(self.lib.ms_phase_dev(self.hd.h, C.c_void_p(d_packed_ptr), nreads), self.hd.h)
         if not host_merge and (getattr(self.hd, "native_comm", False) or _torch_world() == 1):
-            return self._haplotypes_device(V, nw, nreads, want_hap_id, cap), keys
+            hap = self._haplotypes_device(V, nw, nreads, want_hap_id, cap)
+            self._reported = hap.patterns[:hap.nreported].copy()
+            return hap, keys
         # torch.distributed exchange (e.g. gloo in the CPU tests): the three-call protocol with a host merge
         while True:
             if getattr(self, "_grp_shape", None) != (cap, nw):   # reused from pass to pass
@@ -284,6 +309,7 @@ class Juliet:
         if want_hap_id:
             hap = np.empty(nreads, dtype=np.int32)
             check(self.lib.ms_phase_assign(self.hd.h, _ptr(pat), len(cnt), _ptr(hap)), self.hd.h)
+        self._reported = pat[:nrep.value].copy()
         return Haplotypes(patterns=pat, counts=cnt, nreported=int(nrep.value), names=names, counters=counters, hap_id=hap), keys
 
     def _haplotypes_device(self, V, nw, nreads, want_hap_id, cap=4096) -> Haplotypes:
@@ -355,6 +381,36 @@ class Juliet:
         return Linkage(v=rec["v"], w=rec["w"], both=rec["both"], v_only=rec["v_only"], w_only=rec["w_only"], neither=rec["neither"],
                        d_prime=rec["d_prime"], r2=rec["r2"], pvalue=rec["pvalue"], relation=rec["relation"], ntested=int(m.value),
                        keys=list(self._keys), n=G[h:h + V, h:h + V].copy(), a=a.copy(), b=G[:V, h:h + V] - a, c=G[h:h + V, :V] - a)
+
+    def haplotype_abundance(self, patterns=None, tol=1e-10, max_iter=10000) -> Abundance:
+        """Haplotype abundance over every phased read of the last phase_device(..., abundance=True) (ms_haplotype_abundance,
+        restatement choice U18).  patterns: [H, ceil(V/32)] uint32 phasing patterns, distinct; None = the reported haplotypes
+        of that phasing, in report order.  With several ranks the handle needs its own communicator (Handle.attach_comm) and
+        every rank passes the same patterns."""
+        if not getattr(self.hd, "native_comm", False) and _torch_world() > 1:
+            raise _lib.MsError("haplotype abundance over several ranks needs the handle's own communicator (Handle.attach_comm)")
+        if patterns is None:
+            patterns = getattr(self, "_reported", None)
+            if patterns is None:
+                raise _lib.MsError("haplotype_abundance needs the haplotypes of a phase_device call on this handle")
+        nw = max(1, (getattr(self, "_V", 0) + 31) // 32)
+        pat = np.ascontiguousarray(np.asarray(patterns, dtype=np.uint32).reshape(-1, nw))
+        H = pat.shape[0]
+        p = AbundanceParams()
+        self.lib.ms_abundance_params_default(C.byref(p))
+        p.tolerance, p.max_iterations = float(tol), int(max_iter)
+        rows = (AbundanceRow * max(1, H))()
+        ctr = AbundanceCounters()
+        it, conv, ll = C.c_int32(), C.c_int32(), C.c_double()
+        check(self.lib.ms_haplotype_abundance(self.hd.h, C.byref(p), _ptr(pat) if H else None, H, rows, H, C.byref(ctr), C.byref(it),
+                                              C.byref(conv), C.byref(ll)), self.hd.h)
+        rec = np.ctypeslib.as_array(rows)[:H]
+        counters = dict(unique=int(ctr.unique), ambiguous=int(ctr.ambiguous), uninformative=int(ctr.uninformative),
+                        incompatible=int(ctr.incompatible))
+        return Abundance(unique_reads=rec["unique_reads"].copy(), compatible_reads=rec["compatible_reads"].copy(),
+                         em_frequency=rec["em_frequency"].copy(), counters=counters, reads_used=counters["unique"] + counters["ambiguous"],
+                         iterations=int(it.value), converged=bool(conv.value), log_likelihood=float(ll.value), tolerance=float(tol),
+                         max_iterations=int(max_iter))
 
     # -- grouped pile-up and per-haplotype consensus (restatement choice U15)
     def group_pileup(self, d_packed_ptr: int, d_group_ptr: int, nreads: int, ngroups: int, accumulate=False):

@@ -56,7 +56,9 @@ int ms_create(int device, ms_handle** out) {
         cudaEventCreate(&h->ev_stage[9][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[9][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[10][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[10][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[11][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[11][1]) != cudaSuccess ||
-        cudaEventCreate(&h->ev_stage[12][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[12][1]) != cudaSuccess) {
+        cudaEventCreate(&h->ev_stage[12][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[12][1]) != cudaSuccess ||
+        cudaEventCreate(&h->ev_stage[13][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[13][1]) != cudaSuccess ||
+        cudaEventCreate(&h->ev_stage[14][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[14][1]) != cudaSuccess) {
         g_create_error = cudaGetErrorString(cudaGetLastError());
         delete h;
         return MS_ERR_CUDA;
@@ -117,7 +119,10 @@ void ms_destroy(ms_handle* h) {
     cudaEventDestroy(h->ev_copy[0]); cudaEventDestroy(h->ev_copy[1]);
     cudaEventDestroy(h->ev_k1[0]); cudaEventDestroy(h->ev_k1[1]);
     cudaEventDestroy(h->ev_timer[0]); cudaEventDestroy(h->ev_timer[1]);
-    for (int s = 1; s < 13; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
+    for (DevBuf* b : {&h->b_ab_pat, &h->b_ab_mask, &h->b_ab_flag, &h->b_ab_slot, &h->b_ab_tab_key, &h->b_ab_tab_cnt, &h->b_ab_tab_rep, &h->b_ab_ctr,
+                      &h->b_ab_blk, &h->b_ab_out, &h->b_ab_em})
+        b->release();
+    for (int s = 1; s < 15; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
     cudaStreamDestroy(h->own_stream); cudaStreamDestroy(h->copy_stream);
     delete h;
 }
@@ -184,7 +189,7 @@ int ms_pileup_kernel_ms(ms_handle* h, double* ms, int64_t* reads) {
 }
 
 int ms_stage_kernel_ms(ms_handle* h, int stage, double* ms) {
-    if (!h || !ms || stage < 1 || stage > 12 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
+    if (!h || !ms || stage < 1 || stage > 14 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
     MS_CUDA(h, cudaSetDevice(h->device));
     MS_CUDA(h, cudaEventSynchronize(h->ev_stage[stage][1]));
     float f = 0.f;

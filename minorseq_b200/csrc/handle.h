@@ -43,8 +43,8 @@ struct ms_handle {
     cudaEvent_t ev_k1[2] = {nullptr, nullptr};  // around the last K1 launch when timing is on
     cudaEvent_t ev_timer[2] = {nullptr, nullptr};  // ms_timer_start / ms_timer_stop
     int expand_ctas = 0, expand_ctas_nblk = -1;   // expand_events_kernel: resident CTAs per SM for row length nblk
-    cudaEvent_t ev_stage[13][2] = {};              // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
-    bool stage_seen[13] = {};
+    cudaEvent_t ev_stage[15][2] = {};              // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
+    bool stage_seen[15] = {};
     bool timing = false;
     int64_t k1_reads = 0;
     std::string err;
@@ -117,6 +117,12 @@ struct ms_handle {
     bool gram_valid = false;     // b_link_gram holds the (reduced) Gram matrix of the current read set
     std::vector<int32_t> link_col;   // start column of each variant of the current ms_phase_begin
     DevBuf b_mbits, b_link_gram, b_link_col, b_link_sig, b_link_rows, b_link_out;
+    // haplotype abundance (abundance.cu): ms_set_abundance before ms_phase_begin records b_mbits as linkage does.  Per call: the
+    // patterns, one compatibility mask per read and its EM flag, the class table, this rank's class list (exchanged block), the
+    // ordered class list and the EM's state.  The merge and sort scratch of phase_order.cu (b_gather, b_mt_*, b_mslot, b_mindex,
+    // b_m_*, b_ord, b_keys) is reused: it holds nothing between calls.
+    bool abundance = false;      // ms_set_abundance
+    DevBuf b_ab_pat, b_ab_mask, b_ab_flag, b_ab_slot, b_ab_tab_key, b_ab_tab_cnt, b_ab_tab_rep, b_ab_ctr, b_ab_blk, b_ab_out, b_ab_em;
     std::vector<uint32_t> groups_cnt, groups_pat;   // host copy of the last grouping pass (all ranks when a comm is attached)
     bool hap_ranked = false;     // b_rank maps the table slots of the current phased reads to the last ms_phase_haplotypes order
     bool hap_assigned = false;   // ... and b_hap holds the per-read positions in it (ms_phase_hap_device)

@@ -772,9 +772,9 @@ int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codo
     const bool grow = vd.size() * 4 > h->b_var.cap || blocks.size() * 4 > h->b_blocklist.cap ||
                       static_cast<size_t>(h->phase_cap) * h->vwords * 4 > h->b_bits.cap || static_cast<size_t>(h->phase_cap) > h->b_flags.cap ||
                       static_cast<size_t>(ts) * 8 > h->b_tab_key.cap || !h->b_ctr.p ||
-                      (h->linkage && static_cast<size_t>(h->phase_cap) * h->vwords * 4 > h->b_mbits.cap);
+                      ((h->linkage || h->abundance) && static_cast<size_t>(h->phase_cap) * h->vwords * 4 > h->b_mbits.cap);
     if (grow) MS_CUDA(h, cudaStreamSynchronize(h->stream));
-    if (h->linkage) {   // the clean-codon matrix of pairwise linkage, same shape as the bit matrix
+    if (h->linkage || h->abundance) {   // the clean-codon matrix of pairwise linkage and haplotype abundance, same shape as the bit matrix
         MS_CUDA(h, h->b_mbits.ensure(static_cast<size_t>(h->phase_cap) * h->vwords * 4));
         h->link_col.assign(var_col, var_col + V);
         h->link_ready = true;
@@ -835,7 +835,7 @@ int ms_phase_dev(ms_handle* h, const uint32_t* d_packed, int64_t R) {
         const int per_sm = std::max(1, std::min(6, static_cast<int>((h->max_smem + 1024) / (smem + 1024))));
         const int64_t want = (R + ms::kPhaseWarps * 32 - 1) / (ms::kPhaseWarps * 32);
         const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>(want, static_cast<int64_t>(h->num_sms) * per_sm)));
-        if (mbits)     // pairwise linkage was requested: the same walk also writes the clean-codon matrix
+        if (mbits)     // linkage or abundance was requested: the same walk also writes the clean-codon matrix
             ms::phase_bits_kernel<true><<<grid, ms::kPhaseWarps * 32, smem, h->stream>>>(pk, R, h->nblk, h->b_blocklist.as<int32_t>(), h->nblocklist, chunk,
                                                                                         dbuf ? 1 : 0, stream, h->phase_nrec, h->vwords,
                                                                                         h->phase_ordered ? 1 : 0, h->phase_partial_all ? 1 : 0, bits, flags,

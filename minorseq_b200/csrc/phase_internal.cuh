@@ -41,6 +41,71 @@ struct PhasePlan {
     int32_t key_col[kPlanMaxKeys], key_codon[kPlanMaxKeys];
 };
 
+// ---- grouping (phase.cu) and ordering (phase_order.cu) kernels; haplotype abundance (abundance.cu) runs them as well, on its
+// per-read compatibility masks instead of the phasing bits ----
+constexpr int64_t kSmallSort = 4096;   // up to this many distinct entries are ranked by counting, more are sorted
+
+__global__ void __launch_bounds__(256) phase_clear_kernel(unsigned long long* __restrict__ tab_key, uint32_t* __restrict__ tab_cnt,
+                                                          long long* __restrict__ tab_rep, int64_t tab_size, unsigned long long* __restrict__ ctr,
+                                                          unsigned long long last_resort);
+__global__ void phase_insert_kernel(const uint32_t* __restrict__ bits, const uint8_t* __restrict__ flags, int64_t R,
+                                    int32_t vwords, uint64_t seed, unsigned long long* tab_key, uint32_t* tab_cnt,
+                                    long long* tab_rep, int64_t mask, int32_t* __restrict__ slot, unsigned long long* overflow);
+__global__ void phase_verify_kernel(const uint32_t* __restrict__ bits, int64_t R, int32_t vwords,
+                                    const long long* __restrict__ tab_rep, const int32_t* __restrict__ slot,
+                                    unsigned long long* collision);
+__global__ void phase_compact_kernel(const uint32_t* __restrict__ tab_cnt, const long long* __restrict__ tab_rep,
+                                     int64_t tab_size, const uint32_t* __restrict__ bits, int32_t vwords,
+                                     unsigned long long* ngroups, uint32_t* __restrict__ g_cnt,
+                                     uint32_t* __restrict__ g_pat, int32_t* __restrict__ g_slot, int64_t cap);
+
+// result header (u64[8]) at the start of the out block:
+// [0] merged distinct M (world > 1)  [1] nreported  [2] reported reads  [3] insufficient reads
+// [4] "too many for counting rank"   [5] merge hash collisions  [6] merge table overflow
+struct OrderOut {
+    unsigned long long* res;
+    uint32_t* rank;    // entry -> position in the order
+    uint32_t* o_cnt;   // position -> count, first ocap positions
+    uint32_t* o_pat;   // position -> pattern, first ocap positions
+    int64_t ocap;
+    uint32_t min_reads;
+};
+
+// ---- merge of the all-gathered compact lists: block r = [64-byte header | cnt u32[gcap] | pat u32[gcap*nw]] ----
+struct Gathered {
+    const uint8_t* base;
+    size_t block;
+    int64_t gcap;
+    int32_t nw;
+    __device__ __forceinline__ int64_t ng(int64_t rnk) const {
+        const unsigned long long n = reinterpret_cast<const unsigned long long*>(base + rnk * block)[5];
+        return n < static_cast<unsigned long long>(gcap) ? static_cast<int64_t>(n) : gcap;
+    }
+    __device__ __forceinline__ uint32_t cnt(int64_t e) const {
+        const int64_t rnk = e / gcap;
+        return reinterpret_cast<const uint32_t*>(base + rnk * block + 64)[e - rnk * gcap];
+    }
+    __device__ __forceinline__ const uint32_t* pat(int64_t e) const {
+        const int64_t rnk = e / gcap;
+        return reinterpret_cast<const uint32_t*>(base + rnk * block + 64) + gcap + static_cast<size_t>(e - rnk * gcap) * nw;
+    }
+};
+
+__global__ void __launch_bounds__(256) rank_small_kernel(const uint32_t* __restrict__ cnt, const uint32_t* __restrict__ pat, int32_t nw,
+                                                         const unsigned long long* __restrict__ Mptr, int64_t bound,
+                                                         const uint8_t* __restrict__ hdr_src, size_t hdr_stride, int32_t world, OrderOut o);
+__global__ void __launch_bounds__(256) emit_sorted_kernel(const uint32_t* __restrict__ ord, const uint32_t* __restrict__ cnt,
+                                                          const uint32_t* __restrict__ pat, int32_t nw, int64_t M, OrderOut o);
+__global__ void merge_insert_kernel(Gathered g, int64_t bound, uint64_t seed, unsigned long long* mt_key, uint32_t* mt_cnt,
+                                    unsigned long long* mt_rep, int64_t mask, int32_t* __restrict__ mslot, unsigned long long* res);
+__global__ void merge_verify_kernel(Gathered g, int64_t bound, const unsigned long long* __restrict__ mt_rep, const int32_t* __restrict__ mslot,
+                                    unsigned long long* res);
+__global__ void merge_compact_kernel(Gathered g, const uint32_t* __restrict__ mt_cnt, const unsigned long long* __restrict__ mt_rep, int64_t tsize,
+                                     unsigned long long* res, uint32_t* __restrict__ m_cnt, uint32_t* __restrict__ m_pat,
+                                     uint32_t* __restrict__ m_index);
+// bitonic sort of the entry indices 0..M-1 by (count desc, pattern asc); result in h->b_ord (n_pad entries, sentinels last)
+int sort_big(ms_handle* h, const uint32_t* cnt, const uint32_t* pat, int32_t nw, int64_t M, int64_t* n_pad_out);
+
 int phase_ensure_stage(ms_handle* h, size_t bytes);
 int phase_build_table(ms_handle* h, int attempt);
 // enqueue: distinct patterns of the local table -> g_cnt/g_pat (and the table slot of each in g_slot, may be null); count in ctr[5]

@@ -18,21 +18,8 @@ int ms_comm_allgather_bytes(ms_handle* h, const void* d_send, void* d_recv, size
 
 namespace ms {
 
-constexpr int64_t kSmallSort = 4096;
 constexpr uint32_t kSentinel = 0xffffffffu;
 constexpr int kLocalSpan = 2048;   // elements one CTA of bitonic_local_kernel sorts in shared memory
-
-// result header (u64[8]) at the start of the out block:
-// [0] merged distinct M (world > 1)  [1] nreported  [2] reported reads  [3] insufficient reads
-// [4] "too many for counting rank"   [5] merge hash collisions  [6] merge table overflow
-struct OrderOut {
-    unsigned long long* res;
-    uint32_t* rank;    // entry -> position in the order
-    uint32_t* o_cnt;   // position -> count, first ocap positions
-    uint32_t* o_pat;   // position -> pattern, first ocap positions
-    int64_t ocap;
-    uint32_t min_reads;
-};
 
 __device__ __forceinline__ unsigned long long warp_sum64(unsigned long long v) {
 #pragma unroll
@@ -199,26 +186,6 @@ __global__ void hap_assign_kernel(const int32_t* __restrict__ slot, const int32_
     hap[r] = slot[r] < 0 ? -1 : slot_rank[slot[r]];
 }
 
-// ---- merge of the all-gathered compact lists: block r = [64-byte header | cnt u32[gcap] | pat u32[gcap*nw]] ----
-struct Gathered {
-    const uint8_t* base;
-    size_t block;
-    int64_t gcap;
-    int32_t nw;
-    __device__ __forceinline__ int64_t ng(int64_t rnk) const {
-        const unsigned long long n = reinterpret_cast<const unsigned long long*>(base + rnk * block)[5];
-        return n < static_cast<unsigned long long>(gcap) ? static_cast<int64_t>(n) : gcap;
-    }
-    __device__ __forceinline__ uint32_t cnt(int64_t e) const {
-        const int64_t rnk = e / gcap;
-        return reinterpret_cast<const uint32_t*>(base + rnk * block + 64)[e - rnk * gcap];
-    }
-    __device__ __forceinline__ const uint32_t* pat(int64_t e) const {
-        const int64_t rnk = e / gcap;
-        return reinterpret_cast<const uint32_t*>(base + rnk * block + 64) + gcap + static_cast<size_t>(e - rnk * gcap) * nw;
-    }
-};
-
 __global__ void merge_insert_kernel(Gathered g, int64_t bound, uint64_t seed, unsigned long long* mt_key, uint32_t* mt_cnt,
                                     unsigned long long* mt_rep, int64_t mask, int32_t* __restrict__ mslot, unsigned long long* res) {
     const int64_t e = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -267,7 +234,10 @@ namespace {
 
 inline unsigned grid_for(int64_t n, int block) { return static_cast<unsigned>(std::max<int64_t>(1, (n + block - 1) / block)); }
 
-// bitonic sort of the entry indices 0..M-1 by (count desc, pattern asc); result in h->b_ord
+}  // namespace
+
+namespace ms {
+
 int sort_big(ms_handle* h, const uint32_t* cnt, const uint32_t* pat, int32_t nw, int64_t M, int64_t* n_pad_out) {
     int64_t n_pad = ms::kLocalSpan;
     while (n_pad < M) n_pad <<= 1;
@@ -292,7 +262,9 @@ int sort_big(ms_handle* h, const uint32_t* cnt, const uint32_t* pat, int32_t nw,
     return MS_OK;
 }
 
-}  // namespace
+}  // namespace ms
+
+using ms::sort_big;
 
 extern "C" int ms_phase_haplotypes(ms_handle* h, int32_t min_reads, uint32_t* patterns, uint64_t* counts, int64_t cap, int64_t* H,
                                    int64_t* nreported, ms_phase_counters* ctr, int32_t* hap_id) {

@@ -7,6 +7,8 @@
 // (restatement choice U14): per pair of called variants, the reads clean at both codons, D', r^2 and two Fisher tests.
 // A third output kind, out.fasta (with --mode-phasing), holds the consensus sequence of every reported haplotype (restatement
 // choice U15): a grouped pile-up of each haplotype's reads on the GPU and fuse's column rule with thin columns written as 'N'.
+// --haplotype-abundance (restatement choice U18) fits every phased read, damaged ones included, to the reported haplotypes and
+// estimates their frequencies by EM over the reads' compatibility sets.
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -34,6 +36,8 @@ static void usage() {
          "      --mode-phasing                 phase variants into haplotypes\n"
          "      --linkage                      pairwise linkage of the called variants (reads clean at both codons; D', r^2,\n"
          "                                     Fisher tests for \"linked\" / \"exclusive\" after Bonferroni at --alpha)\n"
+         "      --haplotype-abundance          with --mode-phasing: fit every read, damaged ones included, to the reported\n"
+         "                                     haplotypes and estimate their frequencies by EM (\"haplotype_abundance\")\n"
          "      --min-perc <p>                 only variants with abundance > p %\n"
          "      --max-perc <p>                 only variants with abundance < p %\n"
          "      --drm-only                     only known drug-resistance mutations\n"
@@ -61,7 +65,7 @@ static bool ends_with(const std::string& s, const std::string& e) { return s.siz
 
 int main(int argc, char** argv) {
     std::string config, region, cmdline, timing_json;
-    bool phasing = false, drm_only = false, linkage = false;
+    bool phasing = false, drm_only = false, linkage = false, abundance = false;
     double min_perc = -1, max_perc = -1, sub = 5e-4, del = 3e-3, alpha = 0.01;
     int min_hap = 10, device = 0, ngpus = 1, hap_min_cov = 10;
     const int link_min_reads = 10;   // reads clean at both codons that a tested pair needs (the haplotype default, F21)
@@ -80,6 +84,7 @@ int main(int argc, char** argv) {
         else if (a == "--region") region = need("--region");
         else if (a == "--mode-phasing") phasing = true;
         else if (a == "--linkage") linkage = true;
+        else if (a == "--haplotype-abundance") abundance = true;
         else if (a == "--drm-only") drm_only = true;
         else if (a == "--min-perc") min_perc = atof(need("--min-perc").c_str());
         else if (a == "--max-perc") max_perc = atof(need("--max-perc").c_str());
@@ -106,6 +111,7 @@ int main(int argc, char** argv) {
     }
     if (!out_fasta.empty() && !phasing) mshost::die("a .fasta output holds the haplotypes' sequences: it needs --mode-phasing");
     if (hap_min_cov < 0) mshost::die("--hap-min-coverage expects a count >= 0");
+    if (abundance && !phasing) mshost::die("--haplotype-abundance fits the reads to the reported haplotypes: it needs --mode-phasing");
     int rb = 0, re = 0;
     if (!region.empty()) {
         if (sscanf(region.c_str(), "%d-%d", &rb, &re) != 2 || rb < 1 || re <= rb) mshost::die("--region expects <begin-end>");
@@ -248,6 +254,7 @@ int main(int argc, char** argv) {
                 std::vector<int32_t> vc(V), vk(V);
                 for (int32_t i = 0; i < V; ++i) { vc[i] = my_keys[i].first; vk[i] = my_keys[i].second; }
                 CKR(ms_set_linkage(h, linkage ? 1 : 0));
+                CKR(ms_set_abundance(h, abundance ? 1 : 0));
                 CKR(ms_phase_begin(h, vc.data(), vk.data(), V, r1 - r0));
                 CKR(ms_phase_dev(h, d_rows, r1 - r0));
                 if (linkage) {
@@ -350,6 +357,47 @@ int main(int argc, char** argv) {
 
         lap(linkage ? "phasing + linkage" : "phasing");
 
+        // haplotype abundance: every rank fits its reads to the same reported patterns; classes and EM are merged inside the library
+        msreport::AbundanceBlock ab;
+        if (abundance) {
+            const int64_t nrep = nrep_all;
+            if (nrep > 4096)
+                mshost::die("--haplotype-abundance handles at most 4096 haplotypes; this run reports " + std::to_string(nrep));
+            ms_abundance_params ap;
+            ms_abundance_params_default(&ap);
+            ab.tolerance = ap.tolerance;
+            ab.max_iterations = ap.max_iterations;
+            std::vector<ms_abundance_row> arows(static_cast<size_t>(std::max<int64_t>(1, nrep)));
+            ms_abundance_counters actr;
+            int32_t it = 0, conv = 0;
+            double ll = 0;
+            mshost::run_ranks(ngpus, [&](int r) {
+                ms_handle* h = hs[r];
+                std::vector<ms_abundance_row> my_rows(arows.size());
+                ms_abundance_counters my_ctr;
+                int32_t my_it = 0, my_conv = 0;
+                double my_ll = 0;
+                CKR(ms_haplotype_abundance(h, &ap, pat.data(), nrep, my_rows.data(), nrep, &my_ctr, &my_it, &my_conv, &my_ll));
+                if (r == 0) { arows.swap(my_rows); actr = my_ctr; it = my_it; conv = my_conv; ll = my_ll; }
+            });
+            for (const std::string& e : errs)
+                if (!e.empty()) mshost::die(e);
+            ab.iterations = it;
+            ab.converged = conv != 0;
+            ab.log_likelihood = ll;
+            ab.unique = actr.unique; ab.ambiguous = actr.ambiguous; ab.uninformative = actr.uninformative; ab.incompatible = actr.incompatible;
+            for (int64_t k = 0; k < nrep; ++k) {
+                msreport::AbundanceRow row;
+                row.name = haps[k].name;
+                row.reads = haps[k].reads;
+                row.unique_reads = arows[k].unique_reads;
+                row.compatible_reads = arows[k].compatible_reads;
+                row.em_frequency = arows[k].em_frequency;
+                ab.haplotypes.push_back(row);
+            }
+            lap("haplotype abundance");
+        }
+
         // haplotype sequences: every rank piles up its reads per haplotype (labels: the ranks' positions in the haplotype
         // order, on the device), one all-reduce sums the group counts, rank 0 calls them with all insertion events
         std::string fasta_text;
@@ -408,7 +456,7 @@ int main(int argc, char** argv) {
         if (getenv("MS_FIXED_TIMESTAMP")) snprintf(ts, sizeof ts, "%s", getenv("MS_FIXED_TIMESTAMP"));
 
         const msjson::Value report = msreport::build(ts, pos[0], cmdline, MS_VERSION, cfg, L, genes, rows, col, L, phasing, haps, counters,
-                                                     linkage ? &link : nullptr);
+                                                     linkage ? &link : nullptr, abundance ? &ab : nullptr);
         if (!out_json.empty()) {
             std::ofstream f(out_json);
             if (!f) mshost::die("cannot write " + out_json);

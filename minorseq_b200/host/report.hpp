@@ -56,6 +56,21 @@ struct LinkageBlock {
     std::vector<LinkageRow> pairs;
 };
 
+// haplotype abundance (--haplotype-abundance, restatement choice U18): every phased read fitted to the reported haplotypes
+struct AbundanceRow {
+    std::string name;
+    unsigned long long reads = 0, unique_reads = 0, compatible_reads = 0;
+    double em_frequency = 0;
+};
+struct AbundanceBlock {
+    double tolerance = 0;
+    int max_iterations = 0, iterations = 0;
+    bool converged = false;
+    double log_likelihood = 0;
+    unsigned long long unique = 0, ambiguous = 0, uninformative = 0, incompatible = 0;
+    std::vector<AbundanceRow> haplotypes;   // report order
+};
+
 // "%": two significant digits as in the screenshots (1.1, 0.91, 98, 100)
 inline std::string perc2(double p) {
     char b[32];
@@ -76,7 +91,7 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
                    const mscfg::TargetConfig& cfg, int ref_length, const std::vector<mscfg::Gene>& genes,
                    const std::vector<VariantRow>& variants, const std::vector<unsigned>& col_counts /* L*8 */, int L,
                    bool phasing, const std::vector<HaplotypeRow>& haps, const unsigned long long counters[6],
-                   const LinkageBlock* linkage = nullptr) {
+                   const LinkageBlock* linkage = nullptr, const AbundanceBlock* abundance = nullptr) {
     Value root = Value::object();
     Value& in = root.set("input", Value::object());
     in.set("timestamp", Value::string(timestamp));
@@ -218,6 +233,34 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             o.set("pValue", Value::number(r.pvalue));
             o.set("pValueCorrected", Value::number(r.pvalue_corrected));
             o.set("relation", Value::string(r.relation));
+        }
+    }
+    if (abundance) {
+        Value& ab = root.set("haplotype_abundance", Value::object());
+        ab.set("tolerance", Value::number(abundance->tolerance));
+        ab.set("max_iterations", Value::integer(abundance->max_iterations));
+        ab.set("iterations", Value::integer(abundance->iterations));
+        ab.set("converged", Value::boolean(abundance->converged));
+        ab.set("log_likelihood", Value::number(abundance->log_likelihood));
+        const unsigned long long used = abundance->unique + abundance->ambiguous;
+        ab.set("reads_used", Value::integer(static_cast<long long>(used)));
+        Value& rc = ab.set("read_categories", Value::object());
+        rc.set("unique", Value::integer(static_cast<long long>(abundance->unique)));
+        rc.set("ambiguous", Value::integer(static_cast<long long>(abundance->ambiguous)));
+        rc.set("uninformative", Value::integer(static_cast<long long>(abundance->uninformative)));
+        rc.set("incompatible", Value::integer(static_cast<long long>(abundance->incompatible)));
+        Value& hs = ab.set("haplotypes", Value::array());
+        for (const AbundanceRow& r : abundance->haplotypes) {
+            Value& o = hs.push(Value::object());
+            o.set("name", Value::string(r.name));
+            o.set("reads", Value::integer(static_cast<long long>(r.reads)));
+            o.set("unique_reads", Value::integer(static_cast<long long>(r.unique_reads)));
+            o.set("compatible_reads", Value::integer(static_cast<long long>(r.compatible_reads)));
+            o.set("em_reads", Value::number(r.em_frequency * static_cast<double>(used)));
+            o.set("em_frequency", Value::number(r.em_frequency));
+            char b[32];
+            snprintf(b, sizeof b, "%.1f", 100.0 * r.em_frequency);
+            o.set("em_percentage", Value::string(b));
         }
     }
     return root;
@@ -381,6 +424,26 @@ inline std::string to_html(const Value& root) {
             h += "</table>";
         }
         h += "</details>\n";
+    }
+    if (const Value* ab = root.get("haplotype_abundance")) {
+        char b[160];
+        const Value* rc = ab->get("read_categories");
+        auto cat = [&](const char* k) { return std::to_string(static_cast<long long>(rc ? rc->get_number(k) : 0)); };
+        snprintf(b, sizeof b, "%lld iterations (%s), log-likelihood %.6g", static_cast<long long>(ab->get_number("iterations")),
+                 ab->get("converged") && ab->get("converged")->b ? "converged" : "not converged", ab->get_number("log_likelihood"));
+        h += "<details open><summary>Haplotype Abundance</summary><p>Reads used: " +
+             std::to_string(static_cast<long long>(ab->get_number("reads_used"))) + " (unique " + cat("unique") + ", ambiguous " + cat("ambiguous") +
+             "; set aside: uninformative " + cat("uninformative") + ", incompatible " + cat("incompatible") + ")<br>EM: " + b + "</p>";
+        h += "<table><tr><th>Haplotype</th><th>Reads</th><th>Unique</th><th>Compatible</th><th>EM reads</th><th>EM %</th></tr>\n";
+        if (const Value* hs = ab->get("haplotypes"))
+            for (const Value& r : hs->arr) {
+                h += "<tr><td>" + esc(r.get_string("name")) + "</td>";
+                for (const char* k : {"reads", "unique_reads", "compatible_reads"}) h += "<td>" + std::to_string(static_cast<long long>(r.get_number(k))) + "</td>";
+                snprintf(b, sizeof b, "<td>%.1f</td>", r.get_number("em_reads"));
+                h += b;
+                h += "<td>" + esc(r.get_string("em_percentage")) + "</td></tr>\n";
+            }
+        h += "</table></details>\n";
     }
     h += "</body></html>\n";
     return h;
