@@ -63,8 +63,9 @@ __global__ void call_kernel(const uint32_t* __restrict__ codon, const CallPos* _
         // p >= 1/2: such a codon can never be called when alpha <= ntests/2, skip the exact tail.
         if (k <= e && 0.5 * static_cast<double>(ps.ntests) >= cc.alpha) continue;
         // a codon is called iff p * ntests < alpha: stop summing the tail once that is out of reach (the p-value of a
-        // codon that is not called is never reported)
-        const double p = fisher_greater(k, n - k, e, n - e, 1.000001 * cc.alpha / static_cast<double>(ps.ntests));
+        // codon that is not called is never reported).  For k > e the mode floor((k+e+1)/2) is <= k and fisher_upper is
+        // fisher_greater itself; a k <= e codon (tested only when alpha > ntests/2) gets 1 - P(X <= k-1), not an underflow.
+        const double p = fisher_upper(k, n - k, e, n - e, 1.000001 * cc.alpha / static_cast<double>(ps.ntests));
         if (!(p * static_cast<double>(ps.ntests) < cc.alpha)) continue;
         const double perc = 100.0 * static_cast<double>(k) / static_cast<double>(n);
         if (cc.min_perc >= 0.0 && !(perc > cc.min_perc)) continue;

@@ -66,6 +66,11 @@ MS_HD double bd0(double x, double np) {
     return x * log(x / np) + np - x;
 }
 
+// kPreciseLog: take log(1 - x/n) as log((n - x) / n) when x > n/2.  log1p(-x/n) loses the low digits of 1 - x/n when x is
+// close to n: relative error ~1e-16 * x / (n - x), 4e-11 in a linkage table such as [[1999999, 0], [0, 1]].  K2 keeps the
+// plain form so that its p-values stay the same bit for bit: in its tables [[k, n-k], [e, n-e]] the loss is x / (n - x) =
+// k / e, and where that is large enough to matter (~1e4) the tail is far below 1e-300.
+template <bool kPreciseLog = false>
 MS_HD double dbinom_raw(double x, double n, double p, double q) {
     const double ln2pi = 1.83787706640934548356065947281;
     if (p == 0.0) return x == 0.0 ? 1.0 : 0.0;
@@ -81,18 +86,19 @@ MS_HD double dbinom_raw(double x, double n, double p, double q) {
     }
     if (x < 0.0 || x > n) return 0.0;
     const double lc = stirlerr(n) - stirlerr(x) - stirlerr(n - x) - bd0(x, n * p) - bd0(n - x, n * q);
-    const double lf = ln2pi + log(x) + log1p(-x / n);
+    const double lf = ln2pi + log(x) + (kPreciseLog && x > 0.5 * n ? log((n - x) / n) : log1p(-x / n));
     return exp(lc - 0.5 * lf);
 }
 
 // P(X = x), X ~ Hypergeometric(white r, black b, draws n)
+template <bool kPreciseLog = false>
 MS_HD double dhyper(double x, double r, double b, double n) {
     if (x < 0.0 || x > r || n - x > b || n - x < 0.0) return 0.0;
     if (n == 0.0) return x == 0.0 ? 1.0 : 0.0;
     const double p = n / (r + b), q = (r + b - n) / (r + b);
-    const double p1 = dbinom_raw(x, r, p, q);
-    const double p2 = dbinom_raw(n - x, b, p, q);
-    const double p3 = dbinom_raw(n, r + b, p, q);
+    const double p1 = dbinom_raw<kPreciseLog>(x, r, p, q);
+    const double p2 = dbinom_raw<kPreciseLog>(n - x, b, p, q);
+    const double p3 = dbinom_raw<kPreciseLog>(n, r + b, p, q);
     return p1 * p2 / p3;
 }
 
@@ -100,12 +106,13 @@ MS_HD double dhyper(double x, double r, double b, double n) {
 // p < enough, so the (monotone) partial sum is returned as soon as it reaches it.  Codons at their expected
 // sequencing-error count have p ~ 0.5 and a tail of a few hundred slowly falling terms; their first term alone is
 // orders of magnitude above a Bonferroni threshold, and they are most of what K2 would otherwise spend its time on.
+template <bool kPreciseLog = false>
 MS_HD double fisher_greater(uint32_t a, uint32_t b, uint32_t c, uint32_t d, double enough = 2.0) {
     const double white = static_cast<double>(a) + c, black = static_cast<double>(b) + d;
     const double draws = static_cast<double>(a) + b;
     const double xmax = white < draws ? white : draws;
     double x = a;
-    double term = dhyper(x, white, black, draws);
+    double term = dhyper<kPreciseLog>(x, white, black, draws);
     double sum = term;
     while (x < xmax && term > 0.0 && sum < enough) {
         const double ratio = (white - x) * (draws - x) / ((x + 1.0) * (black - draws + x + 1.0));
@@ -117,6 +124,23 @@ MS_HD double fisher_greater(uint32_t a, uint32_t b, uint32_t c, uint32_t d, doub
         if (ratio < 1.0 && term < sum * 8.470329472543003e-22) break;
     }
     return sum > 1.0 ? 1.0 : sum;
+}
+
+// true when the top-left cell a of [[a,b],[c,d]] is at or above the mode of its hypergeometric distribution, i.e. the upper
+// tail P(X >= a) is the one that can be small
+MS_HD bool fisher_at_or_above_mode(uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
+    const double n = static_cast<double>(a) + b + c + d;
+    const double mode = floor((static_cast<double>(a) + b + 1.0) * (static_cast<double>(a) + c + 1.0) / (n + 2.0));
+    return static_cast<double>(a) >= mode;
+}
+
+// P(X >= a) on either side of the mode.  At or above it the tail is summed directly (stopped at `enough`, as in
+// fisher_greater).  Below it the tail holds the mode and is taken as 1 - P(X <= a - 1), the upper tail of the mirrored
+// table: summed from a, its first term can lie so far out that it underflows to 0, and the sum would be 0 instead of ~1.
+template <bool kPreciseLog = false>
+MS_HD double fisher_upper(uint32_t a, uint32_t b, uint32_t c, uint32_t d, double enough = 2.0) {
+    if (fisher_at_or_above_mode(a, b, c, d)) return fisher_greater<kPreciseLog>(a, b, c, d, enough);
+    return (a == 0 || d == 0) ? 1.0 : 1.0 - fisher_greater<kPreciseLog>(b + 1, a - 1, d - 1, c + 1);
 }
 
 // P(ref codon -> codon) for nm mismatching bases (restatement choice U1, SURVEY App. B)
