@@ -118,11 +118,12 @@ int ms_pileup_kernel_ms(ms_handle *h, double *ms, int64_t *reads);
  * grouped pile-up kernel of ms_group_pileup_dev (without the counting sort in front of it).  Read alignment adds two:
  * MS_STAGE_ALIGN_SEED = align_seed_kernel, MS_STAGE_ALIGN_BAND = align_band_kernel (banded DP and traceback) of the last
  * chunk of ms_align_reads.  Haplotype abundance adds two: MS_STAGE_ABUNDANCE_COMPAT = abundance_compat_kernel,
- * MS_STAGE_ABUNDANCE_EM = the EM iterations (host checks included).                                                      */
+ * MS_STAGE_ABUNDANCE_EM = the EM iterations (host checks included).  MS_STAGE_INDELS = indel_count_kernel of
+ * ms_indel_count_dev.                                                                                                   */
 enum { MS_STAGE_PHASE_BITS = 1, MS_STAGE_COOCCURRENCE = 2, MS_STAGE_EXPAND = 3, MS_STAGE_ALLREDUCE = 4, MS_STAGE_HAPMERGE = 5,
        MS_STAGE_UPLOAD = 6, MS_STAGE_PASS = 7, MS_STAGE_LINKAGE_STATS = 8, MS_STAGE_LINKAGE_ALLREDUCE = 9,
        MS_STAGE_GROUP_PILEUP = 10, MS_STAGE_ALIGN_SEED = 11, MS_STAGE_ALIGN_BAND = 12, MS_STAGE_ABUNDANCE_COMPAT = 13,
-       MS_STAGE_ABUNDANCE_EM = 14 };
+       MS_STAGE_ABUNDANCE_EM = 14, MS_STAGE_INDELS = 15 };
 int ms_stage_kernel_ms(ms_handle *h, int stage, double *ms);
 
 /* ---- K1: pileup (juliet "MSA counts", doc/JULIET.md:96-100; fuse doc/FUSE.md:17-20) -- */
@@ -332,6 +333,54 @@ int ms_set_abundance(ms_handle *h, int on);
 int ms_haplotype_abundance(ms_handle *h, const ms_abundance_params *prm, const uint32_t *patterns, int64_t H,
                            ms_abundance_row *rows, int64_t cap, ms_abundance_counters *counters, int32_t *iterations,
                            int32_t *converged, double *loglik);
+
+/* ---- in-frame codon deletions and insertions (restatement choice U19) ------------------------------------------
+ * The reads are the ones K1 piles up; codon starts are the layout's start mask, limited by the genes and the region as in
+ * ms_call.  A read is "clean" at a column holding A/C/G/T.
+ *   deletion of the codon at s:  k = reads with '-' at s, s+1 and s+2;  n = k + K2's coverage at s (reads with a clean codon);
+ *   insertion at the boundary c = s+2 between the codons at s and s+3 of one gene (both tested):  n = reads clean at c and
+ *   c+1;  k(x) = those of them whose FIRST insertion event at column c (ms_expand_cigar's ins_col) is the string x, of a
+ *   length that is a multiple of 3 and >= 3, all A/C/G/T (upper-cased).  Other insertions stay in n and count for no x.
+ * Test as K2: e = min(n, ceil(n P)) with P = deletion_rate^3 or insertion_rate^len(x), p = one-sided Fisher of
+ * [[k, n-k], [e, n-e]], called iff p * ntests < alpha (ntests = the gene's tested codons, as K2), then min_perc / max_perc
+ * on 100 k / n.  Needs the (all-reduced) K1 counts of the same reads.                                                 */
+typedef struct {
+    double deletion_rate, insertion_rate;      /* error model: P = deletion_rate^3, insertion_rate^len */
+    double alpha;                              /* call iff p * ntests < alpha */
+    double min_perc, max_perc;                 /* < 0 = off */
+    int32_t region_begin, region_end;          /* 1-based [b,e); 0,0 = off */
+} ms_indel_params;
+enum { MS_INDEL_DELETION = 0, MS_INDEL_INSERTION = 1 };
+typedef struct {
+    int32_t gene, codon_index;                 /* the deleted codon / the codon before the insertion */
+    int32_t col;                               /* deletion: its start column s; insertion: the column c = s+2 it follows */
+    int32_t kind;                              /* MS_INDEL_DELETION or MS_INDEL_INSERTION */
+    int32_t sid;                               /* insertion: string id (ms_indel_inserted); deletion: -1 */
+    int32_t ref_codon;                         /* reference codon at s: referenceSequence, else the majority (-1: no clean read) */
+    int32_t next_codon;                        /* insertion: the same at s+3; deletion: -1 */
+    uint32_t count, coverage, expected, ntests;
+    double pvalue;                             /* uncorrected one-sided Fisher p (fp64) */
+} ms_indel;
+/* deletion_rate 3e-3, insertion_rate 3e-3, alpha 0.01, no percentage filter, no region */
+void ms_indel_params_default(ms_indel_params *p);
+/* Counts R device-resident reads (tiles), which are reads [read0, read0 + R) of the caller's numbering, afresh: k_del and
+ * n_ins of every column, and k(x).  The insertion events (ins_read in that numbering, ins_col, ins_off / ins_len into
+ * ins_pool, in the order ms_expand_cigar appends them) are ALL the events of the run: the string ids are assigned from all of
+ * them (one per (column, upper-cased x), in that order), so every rank that passes the same list gets the same ids; only the
+ * events of this rank's reads are counted.                                                                              */
+int ms_indel_count_dev(ms_handle *h, const uint32_t *d_packed, int64_t R, int64_t read0, const int64_t *ins_read,
+                       const int32_t *ins_col, const int64_t *ins_off, const int32_t *ins_len, int64_t nins,
+                       const char *ins_pool, int64_t pool_len);
+/* Host copy of the counts: cnt[L][2] = k_del, n_ins; tally[sid] (the first min(cap, *nstrings)).  Summed over the ranks once
+ * ms_indel_call has run.                                                                                               */
+int ms_indel_counts(ms_handle *h, uint32_t *cnt, uint32_t *tally, int64_t cap, int64_t *nstrings);
+/* The upper-cased string of id sid and its column (col may be NULL); MS_ERR_CAPACITY when cap < *len. */
+int ms_indel_inserted(ms_handle *h, int32_t sid, int32_t *col, char *buf, int64_t cap, int64_t *len);
+/* The called indels, sorted by (gene, codon, deletion before insertion, string).  *n receives their number; MS_ERR_CAPACITY
+ * when it exceeds cap (out holds the first cap; call again, the counts are kept).  With a communicator attached a collective:
+ * the first call after ms_indel_count_dev sums the counts over the ranks (one all-reduce), and every rank gets the same list. */
+int ms_indel_call(ms_handle *h, const ms_gene *genes, int32_t ngenes, const char *refseq, const ms_indel_params *prm,
+                  ms_indel *out, int64_t cap, int64_t *n);
 
 /* ---- the whole juliet pass in one call ------------------------------------------------------
  * reset -> pileup -> (all-reduce when a communicator is attached) -> codon test -> phasing, i.e. everything

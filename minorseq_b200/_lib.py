@@ -64,6 +64,17 @@ class AbundanceCounters(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("unique", "ambiguous", "uninformative", "incompatible")]
 
 
+class IndelParams(C.Structure):
+    _fields_ = [("deletion_rate", C.c_double), ("insertion_rate", C.c_double), ("alpha", C.c_double), ("min_perc", C.c_double),
+                ("max_perc", C.c_double), ("region_begin", C.c_int32), ("region_end", C.c_int32)]
+
+
+class Indel(C.Structure):
+    _fields_ = [("gene", C.c_int32), ("codon_index", C.c_int32), ("col", C.c_int32), ("kind", C.c_int32), ("sid", C.c_int32),
+                ("ref_codon", C.c_int32), ("next_codon", C.c_int32), ("count", C.c_uint32), ("coverage", C.c_uint32),
+                ("expected", C.c_uint32), ("ntests", C.c_uint32), ("pvalue", C.c_double)]
+
+
 class ReadHdr(C.Structure):
     _fields_ = [("ev_off", C.c_uint32), ("begin", C.c_uint16), ("end", C.c_uint16)]
 
@@ -171,6 +182,12 @@ _SIGNATURES = {
     "ms_get_group_counts": (C.c_int, [_P, _P]),
     "ms_phase_hap_device": (C.c_int, [_P, C.POINTER(_P), C.POINTER(C.c_int64)]),
     "ms_group_consensus": (C.c_int, [_P, C.POINTER(FuseParams), _P, _P, _P, _P, C.c_int64, _P, C.c_int64, _P, C.c_int64, _P]),
+    "ms_indel_params_default": (None, [C.POINTER(IndelParams)]),
+    "ms_indel_count_dev": (C.c_int, [_P, _P, C.c_int64, C.c_int64, _P, _P, _P, _P, C.c_int64, _P, C.c_int64]),
+    "ms_indel_counts": (C.c_int, [_P, _P, _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "ms_indel_inserted": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32), _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "ms_indel_call": (C.c_int, [_P, C.POINTER(Gene), C.c_int32, C.c_char_p, C.POINTER(IndelParams), C.POINTER(Indel), C.c_int64,
+                                C.POINTER(C.c_int64)]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -13,7 +13,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _lib
-from ._lib import (AbundanceCounters, AbundanceParams, AbundanceRow, AlignParams, CallParams, FuseParams, Gene, LinkagePair, LinkageParams, PhaseCounters, ReadAlignment, SynthParams, Variant,
+from ._lib import (AbundanceCounters, AbundanceParams, AbundanceRow, AlignParams, CallParams, FuseParams, Gene, Indel, IndelParams, LinkagePair, LinkageParams, PhaseCounters, ReadAlignment, SynthParams, Variant,
                    check)
 from .synth import start_mask_words, tile_rows, untile_rows
 
@@ -89,6 +89,46 @@ class Abundance:
     @property
     def em_reads(self):
         return self.em_frequency * self.reads_used
+
+
+@dataclass
+class Indels:
+    """In-frame codon deletions and insertions (Juliet.indels, restatement choice U19).  The calls, sorted by (gene, codon,
+    deletion before insertion, string), as parallel arrays; inserted[i] is the upper-cased inserted string ('' for a
+    deletion) and label[i] the amino-acid label (D67del, T69_S70insSS).  The counts behind them: cnt[L, 2] = k_del (reads
+    with '-' at s, s+1, s+2) and n_ins (reads clean at c and c+1) of every column, tally[sid] the reads of each inserted
+    string strings[sid] at column string_col[sid]."""
+    gene: np.ndarray
+    codon_index: np.ndarray
+    col: np.ndarray
+    kind: np.ndarray                # 0 deletion, 1 insertion
+    sid: np.ndarray
+    ref_codon: np.ndarray
+    next_codon: np.ndarray
+    count: np.ndarray
+    coverage: np.ndarray
+    expected: np.ndarray
+    ntests: np.ndarray
+    pvalue: np.ndarray
+    inserted: list
+    label: list
+    cnt: np.ndarray
+    tally: np.ndarray
+    strings: list
+    string_col: np.ndarray
+
+
+def translate_dna(x: str) -> str:
+    """Amino acids of an in-frame string, '*' for a stop (the indel labels)."""
+    return "".join(_AA[CODONS.index(x[i:i + 3])].replace("X", "*") for i in range(0, len(x) - 2, 3))
+
+
+def indel_label(kind, ref_codon, next_codon, aa_pos, inserted):
+    """D67del; T69_S70insSS (flanking reference amino acids, then the inserted ones).  A codon without a clean read is '?'."""
+    aa = lambda c: translate(int(c)) if c >= 0 else "?"
+    if kind == 0:
+        return f"{aa(ref_codon)}{aa_pos}del"
+    return f"{aa(ref_codon)}{aa_pos}_{aa(next_codon)}{aa_pos + 1}ins{translate_dna(inserted)}"
 
 
 @dataclass
@@ -411,6 +451,70 @@ class Juliet:
                          em_frequency=rec["em_frequency"].copy(), counters=counters, reads_used=counters["unique"] + counters["ambiguous"],
                          iterations=int(it.value), converged=bool(conv.value), log_likelihood=float(ll.value), tolerance=float(tol),
                          max_iterations=int(max_iter))
+
+    # -- in-frame indels (restatement choice U19)
+    def indels(self, d_packed_ptr: int, nreads: int, insertions=None, read0=0, deletion_rate=None, insertion_rate=3e-3,
+               alpha=None, min_perc=None, max_perc=None, cap=256) -> Indels:
+        """In-frame codon deletions and insertions of the reads that were piled up (ms_indel_count_dev + ms_indel_call): needs
+        the all-reduced K1 counts of the same reads.  d_packed_ptr / nreads: this rank's reads (device tiles), reads
+        [read0, read0 + nreads) of the run.  insertions: (read, col, off, len, pool) insertion events of ALL the run's reads
+        (read in the run's numbering, pool = bytes), in ms_expand_cigar's order.  The rates, alpha and the percentage filters
+        default to the codon test's.  With several ranks the handle needs its own communicator (Handle.attach_comm)."""
+        if not getattr(self.hd, "native_comm", False) and _torch_world() > 1:
+            raise _lib.MsError("indels over several ranks need the handle's own communicator (Handle.attach_comm)")
+        nins, ir, ic, io, il, pl, pool = 0, None, None, None, None, None, b""
+        if insertions is not None and len(insertions[0]):
+            read, col, off, ln, pool = insertions
+            ir = np.ascontiguousarray(read, dtype=np.int64)
+            ic = np.ascontiguousarray(col, dtype=np.int32)
+            io = np.ascontiguousarray(off, dtype=np.int64)
+            il = np.ascontiguousarray(ln, dtype=np.int32)
+            pl = np.frombuffer(pool, dtype=np.uint8)
+            nins = len(ir)
+        check(self.lib.ms_indel_count_dev(self.hd.h, C.c_void_p(d_packed_ptr), int(nreads), int(read0), _ptr(ir), _ptr(ic), _ptr(io), _ptr(il),
+                                          nins, _ptr(pl), len(pool)), self.hd.h)
+        p = IndelParams()
+        self.lib.ms_indel_params_default(C.byref(p))
+        p.deletion_rate = self.params.deletion_rate if deletion_rate is None else float(deletion_rate)
+        p.insertion_rate = float(insertion_rate)
+        p.alpha = self.params.alpha if alpha is None else float(alpha)
+        p.min_perc = self.params.min_perc if min_perc is None else float(min_perc)
+        p.max_perc = self.params.max_perc if max_perc is None else float(max_perc)
+        p.region_begin, p.region_end = self.params.region_begin, self.params.region_end
+        genes = (Gene * max(1, len(self.genes)))(*[Gene(b, e) for (b, e) in self.genes])
+        ref = self.refseq.encode() if self.refseq else None
+        n = C.c_int64()
+        while True:
+            out = (Indel * max(1, cap))()
+            rc = self.lib.ms_indel_call(self.hd.h, genes, len(self.genes), ref, C.byref(p), out, cap, C.byref(n))
+            if rc == -4:   # MS_ERR_CAPACITY: the counts are kept, only the test runs again
+                cap = int(n.value)
+                continue
+            check(rc, self.hd.h)
+            break
+        rec = np.ctypeslib.as_array(out)[: n.value].copy()
+        cnt = np.empty((self.L, 2), dtype=np.uint32)
+        ns = C.c_int64()
+        check(self.lib.ms_indel_counts(self.hd.h, _ptr(cnt), None, 0, C.byref(ns)), self.hd.h)
+        tally = np.zeros(max(1, ns.value), dtype=np.uint32)
+        check(self.lib.ms_indel_counts(self.hd.h, _ptr(cnt), _ptr(tally), ns.value, C.byref(ns)), self.hd.h)
+        strings, scol = [], np.zeros(ns.value, dtype=np.int32)
+        for sid in range(ns.value):
+            c, ln = C.c_int32(), C.c_int64()
+            buf = C.create_string_buffer(self.L + 1)
+            rc = self.lib.ms_indel_inserted(self.hd.h, sid, C.byref(c), buf, len(buf), C.byref(ln))
+            if rc == -4:
+                buf = C.create_string_buffer(int(ln.value))
+                rc = self.lib.ms_indel_inserted(self.hd.h, sid, C.byref(c), buf, len(buf), C.byref(ln))
+            check(rc, self.hd.h)
+            strings.append(buf.raw[: ln.value].decode())
+            scol[sid] = c.value
+        ins = [strings[s] if k == 1 else "" for k, s in zip(rec["kind"], rec["sid"])]
+        labels = [indel_label(int(r["kind"]), int(r["ref_codon"]), int(r["next_codon"]), int(r["codon_index"]) + 1, x) for r, x in zip(rec, ins)]
+        return Indels(gene=rec["gene"], codon_index=rec["codon_index"], col=rec["col"], kind=rec["kind"], sid=rec["sid"],
+                      ref_codon=rec["ref_codon"], next_codon=rec["next_codon"], count=rec["count"], coverage=rec["coverage"],
+                      expected=rec["expected"], ntests=rec["ntests"], pvalue=rec["pvalue"], inserted=ins, label=labels, cnt=cnt,
+                      tally=tally[: ns.value].copy(), strings=strings, string_col=scol)
 
     # -- grouped pile-up and per-haplotype consensus (restatement choice U15)
     def group_pileup(self, d_packed_ptr: int, d_group_ptr: int, nreads: int, ngroups: int, accumulate=False):

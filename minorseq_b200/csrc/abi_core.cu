@@ -11,6 +11,7 @@ void ms_events_set_smem_attr(int max_smem);
 void ms_cooc_tc_set_smem_attr();
 void ms_phase_set_smem_attr();
 void ms_group_set_smem_attr();
+void ms_indel_set_smem_attr();
 int ms_tile_rows_launch(ms_handle* h, const uint32_t* d_rows, int64_t R, uint32_t* d_tiled);
 
 extern "C" {
@@ -58,7 +59,8 @@ int ms_create(int device, ms_handle** out) {
         cudaEventCreate(&h->ev_stage[11][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[11][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[12][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[12][1]) != cudaSuccess ||
         cudaEventCreate(&h->ev_stage[13][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[13][1]) != cudaSuccess ||
-        cudaEventCreate(&h->ev_stage[14][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[14][1]) != cudaSuccess) {
+        cudaEventCreate(&h->ev_stage[14][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[14][1]) != cudaSuccess ||
+        cudaEventCreate(&h->ev_stage[15][0]) != cudaSuccess || cudaEventCreate(&h->ev_stage[15][1]) != cudaSuccess) {
         g_create_error = cudaGetErrorString(cudaGetLastError());
         delete h;
         return MS_ERR_CUDA;
@@ -81,6 +83,7 @@ int ms_create(int device, ms_handle** out) {
     ms_cooc_tc_set_smem_attr();
     ms_phase_set_smem_attr();
     ms_group_set_smem_attr();
+    ms_indel_set_smem_attr();
     *out = h;
     return MS_OK;
 }
@@ -120,9 +123,9 @@ void ms_destroy(ms_handle* h) {
     cudaEventDestroy(h->ev_k1[0]); cudaEventDestroy(h->ev_k1[1]);
     cudaEventDestroy(h->ev_timer[0]); cudaEventDestroy(h->ev_timer[1]);
     for (DevBuf* b : {&h->b_ab_pat, &h->b_ab_mask, &h->b_ab_flag, &h->b_ab_slot, &h->b_ab_tab_key, &h->b_ab_tab_cnt, &h->b_ab_tab_rep, &h->b_ab_ctr,
-                      &h->b_ab_blk, &h->b_ab_out, &h->b_ab_em})
+                      &h->b_ab_blk, &h->b_ab_out, &h->b_ab_em, &h->b_indel_cnt, &h->b_indel_ev, &h->b_indel_out})
         b->release();
-    for (int s = 1; s < 15; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
+    for (int s = 1; s < 16; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
     cudaStreamDestroy(h->own_stream); cudaStreamDestroy(h->copy_stream);
     delete h;
 }
@@ -189,7 +192,7 @@ int ms_pileup_kernel_ms(ms_handle* h, double* ms, int64_t* reads) {
 }
 
 int ms_stage_kernel_ms(ms_handle* h, int stage, double* ms) {
-    if (!h || !ms || stage < 1 || stage > 14 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
+    if (!h || !ms || stage < 1 || stage > 15 || !h->timing || !h->stage_seen[stage]) return MS_ERR_ARG;
     MS_CUDA(h, cudaSetDevice(h->device));
     MS_CUDA(h, cudaEventSynchronize(h->ev_stage[stage][1]));
     float f = 0.f;
@@ -213,6 +216,7 @@ int ms_set_pileup_variant(ms_handle* h, int variant) {
 int ms_set_layout(ms_handle* h, int32_t L, const uint32_t* start_mask) {
     if (!h || L < 3) return MS_ERR_ARG;
     MS_CUDA(h, cudaSetDevice(h->device));
+    h->indel_L = 0;   // the indel counts belong to the old layout
     const int32_t nblk = (L + 31) / 32;
     // CTA shape.  W warps span a row or a column segment of it (31 counting lanes per warp -- lane 31 is the codon
     // look-ahead provider -- and 32 in the last), G row-groups per CTA with W*G <= 12.  With nseg > 1 CTA c handles

@@ -71,6 +71,14 @@ int ms_comm_allreduce_i32(ms_handle* h, int32_t* d, size_t count) {
     return MS_OK;
 }
 
+// used by indel.cu: in-place u32 sum of the indel counts over the ranks, on the handle's stream
+int ms_comm_allreduce_u32(ms_handle* h, uint32_t* d, size_t count) {
+    if (!h->comm) return MS_ERR_ARG;
+    MS_NCCL(h, api().AllReduce(d, d, count, ncclUint32, ncclSum, static_cast<ncclComm_t>(h->comm), h->stream));
+    h->launches++;
+    return MS_OK;
+}
+
 extern "C" void ms_comm_free_internal(ms_handle* h) {
     if (h->comm && api().ok) api().CommDestroy(static_cast<ncclComm_t>(h->comm));
     h->comm = nullptr;

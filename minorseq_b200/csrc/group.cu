@@ -20,14 +20,11 @@
 #include <unordered_map>
 #include <vector>
 #include "fuse.cuh"
+#include "group.cuh"
 #include "handle.h"
-#include "pileup.cuh"
 
 namespace ms {
 
-constexpr int kGroupChunk = 8 * (kMaxReadsPerFlush / 8);   // reads per work item: whole batches of 8 within K1's counter capacity
-constexpr int kGroupMaxThreads = 256;                      // one thread per 32-column block of a segment
-constexpr int kGroupRing = 3;                              // batches of 8 reads per thread in the cp.async ring
 constexpr int kGroupMasks = 7;                             // P0 P1 P2 P0&P1 P0&P2 P1&P2 P3
 constexpr int kSortThreads = 256;
 constexpr int64_t kSortHistMax = 1 << 22;                  // entries of the [chunk][group] histogram of the counting sort
@@ -155,20 +152,8 @@ struct GroupArgs {
     int32_t ngroups, L, nblk, nseg, seg_len;
 };
 
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ uint4 lds128g(uint32_t addr) {
-    uint4 v;
-    asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ void sts128(uint32_t addr, uint4 v) {
-    asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-
 // K1's masks of one read (kModeFuse's set)
-__device__ __forceinline__ void group_masks(uint32_t addr, uint32_t (&m)[kGroupMasks]) {
+__device__ __forceinline__ void group_masks(uint32_t addr, uint32_t /*stride*/, uint32_t (&m)[kGroupMasks]) {
     const uint4 q = lds128g(addr);
     m[0] = q.x;
     m[1] = q.y;
@@ -177,62 +162,6 @@ __device__ __forceinline__ void group_masks(uint32_t addr, uint32_t (&m)[kGroupM
     m[4] = q.x & q.z;
     m[5] = q.y & q.z;
     m[6] = q.w;
-}
-
-// 8 reads (read i at addr + i * stride) into the counters: K1's carry-save tree (pileup.cu, block8)
-__device__ __forceinline__ void group_add8(Vert<kGroupMasks>& v, const HiPlanes& hp, uint32_t addr, uint32_t stride, uint32_t bi) {
-    constexpr int NM = kGroupMasks;
-    uint32_t m0[NM], m1[NM], twosA[NM], twosB[NM], foursA[NM], foursB[NM];
-    group_masks(addr, m0);
-    group_masks(addr + stride, m1);
-#pragma unroll
-    for (int i = 0; i < NM; ++i) csa(twosA[i], v.c[i][0], v.c[i][0], m0[i], m1[i]);
-    group_masks(addr + 2 * stride, m0);
-    group_masks(addr + 3 * stride, m1);
-#pragma unroll
-    for (int i = 0; i < NM; ++i) {
-        csa(twosB[i], v.c[i][0], v.c[i][0], m0[i], m1[i]);
-        csa(foursA[i], v.c[i][1], v.c[i][1], twosA[i], twosB[i]);
-    }
-    group_masks(addr + 4 * stride, m0);
-    group_masks(addr + 5 * stride, m1);
-#pragma unroll
-    for (int i = 0; i < NM; ++i) csa(twosA[i], v.c[i][0], v.c[i][0], m0[i], m1[i]);
-    group_masks(addr + 6 * stride, m0);
-    group_masks(addr + 7 * stride, m1);
-#pragma unroll
-    for (int i = 0; i < NM; ++i) {
-        csa(twosB[i], v.c[i][0], v.c[i][0], m0[i], m1[i]);
-        csa(foursB[i], v.c[i][1], v.c[i][1], twosA[i], twosB[i]);
-        csa(twosA[i], v.c[i][2], v.c[i][2], foursA[i], foursB[i]);  // twosA now holds the weight-8 carry
-    }
-    if (bi & 1u) {
-        if (bi & 2u) {
-            if (bi & 4u) {
-#pragma unroll
-                for (int i = 0; i < NM; ++i) {
-                    uint32_t x16, x32, x64;
-                    csa(x16, v.c[i][3], v.c[i][3], v.p3[i], twosA[i]);
-                    csa(x32, v.c[i][4], v.c[i][4], v.p4[i], x16);
-                    csa(x64, v.c[i][5], v.c[i][5], v.p5[i], x32);
-                    ripple<false>(v, hp, i, 6, x64);
-                }
-            } else {
-#pragma unroll
-                for (int i = 0; i < NM; ++i) {
-                    uint32_t x16;
-                    csa(x16, v.c[i][3], v.c[i][3], v.p3[i], twosA[i]);
-                    csa(v.p5[i], v.c[i][4], v.c[i][4], v.p4[i], x16);
-                }
-            }
-        } else {
-#pragma unroll
-            for (int i = 0; i < NM; ++i) csa(v.p4[i], v.c[i][3], v.c[i][3], v.p3[i], twosA[i]);
-        }
-    } else {
-#pragma unroll
-        for (int i = 0; i < NM; ++i) v.p3[i] = twosA[i];
-    }
 }
 
 // end of a work item (cold path, as K1's emit_slice): planes [mask][kPlanes] of n reads -> per-column integers, added into
@@ -267,67 +196,30 @@ __device__ __noinline__ void group_flush(const uint32_t* planes, uint32_t n, uin
     }
 }
 
-__global__ void __launch_bounds__(kGroupMaxThreads) group_pileup_kernel(GroupArgs a) {
-    extern __shared__ __align__(16) uint4 ring[];   // [kGroupRing * 8][blockDim]: batch slot s, read i at row s * 8 + i
-    const int tid = threadIdx.x;
-    const uint32_t stride = static_cast<uint32_t>(blockDim.x) * 16u;        // bytes between the reads of a batch
-    const uint32_t ring0 = static_cast<uint32_t>(__cvta_generic_to_shared(ring)) + static_cast<uint32_t>(tid) * 16u;
-    const int64_t nitems = static_cast<int64_t>(a.ioff[a.ngroups]) * a.nseg;
-    HiPlanes hp;
-    hp.base = hp.stride = 0;
-    Vert<kGroupMasks> v;
-    for (int64_t it = blockIdx.x; it < nitems; it += gridDim.x) {
-        const int seg = static_cast<int>(it % a.nseg);
-        const int32_t k = static_cast<int32_t>(it / a.nseg);
-        const int b = seg * a.seg_len + tid;
-        if (tid >= a.seg_len || b >= a.nblk) continue;      // no barriers below: idle lanes may leave the item
-        int32_t lo = 0, hi = a.ngroups;                     // the group of item k: ioff[lo] <= k < ioff[lo + 1]
+// the walk's policy (group.cuh): work item k belongs to the group g with ioff[g] <= k < ioff[g + 1]
+struct GroupPolicy {
+    static constexpr int NM = kGroupMasks, SLOTS = 1;
+    GroupArgs a;
+    __device__ __forceinline__ int32_t item(int32_t k, int32_t& r_begin, int32_t& r_end) const {
+        int32_t lo = 0, hi = a.ngroups;
         while (hi - lo > 1) {
             const int32_t mid = (lo + hi) >> 1;
             if (__ldg(a.ioff + mid) <= k) lo = mid;
             else hi = mid;
         }
-        const int32_t g = lo;
-        const int32_t r_begin = __ldg(a.goff + g) + (k - __ldg(a.ioff + g)) * kGroupChunk;
-        const int32_t r_end = min(__ldg(a.goff + g + 1), r_begin + kGroupChunk);
-        const int32_t nb = (r_end - r_begin + 7) >> 3;      // batches of 8; the slots past r_end hold "not spanned" reads
-        auto load = [&](int32_t batch) {
-            const uint32_t slot = ring0 + static_cast<uint32_t>(batch % kGroupRing) * 8u * stride;
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int32_t idx = r_begin + batch * 8 + i;
-                if (idx < r_end) {
-                    const int64_t r = __ldg(a.list + idx);
-                    cp_async16(slot + static_cast<uint32_t>(i) * stride, a.tiles + (((r >> 3) * a.nblk + b) << 3) + ((r & 7) ^ (b & 7)));
-                } else {
-                    sts128(slot + static_cast<uint32_t>(i) * stride, make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0u));
-                }
-            }
-        };
-        clear<false>(v, hp);
-#pragma unroll
-        for (int p = 0; p < kGroupRing - 1; ++p) {
-            if (p < nb) load(p);
-            asm volatile("cp.async.commit_group;" ::: "memory");
-        }
-        uint32_t bi = 0;
-        for (int32_t j = 0; j < nb; ++j) {
-            if (j + kGroupRing - 1 < nb) load(j + kGroupRing - 1);   // into the slot batch j - 1 has left
-            asm volatile("cp.async.commit_group;" ::: "memory");
-            asm volatile("cp.async.wait_group %0;" ::"n"(kGroupRing - 1) : "memory");   // batch j has landed
-            group_add8(v, hp, ring0 + static_cast<uint32_t>(j % kGroupRing) * 8u * stride, stride, bi);
-            ++bi;
-        }
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        fold_pendings<false>(v, hp, bi);
-        uint32_t planes[kGroupMasks * kPlanes];
-#pragma unroll
-        for (int i = 0; i < kGroupMasks; ++i)
-#pragma unroll
-            for (int q = 0; q < kPlanes; ++q) planes[i * kPlanes + q] = v.c[i][q];
-        group_flush(planes, static_cast<uint32_t>(nb) * 8u, a.gcol + (static_cast<size_t>(g) * a.L + static_cast<size_t>(b) * 32) * 8,
-                    min(32, a.L - b * 32));
+        r_begin = __ldg(a.goff + lo) + (k - __ldg(a.ioff + lo)) * kGroupChunk;
+        r_end = min(__ldg(a.goff + lo + 1), r_begin + kGroupChunk);
+        return lo;
     }
+    __device__ __forceinline__ int64_t read(int32_t idx) const { return __ldg(a.list + idx); }
+    __device__ static __forceinline__ void masks(uint32_t addr, uint32_t stride, uint32_t (&m)[NM]) { group_masks(addr, stride, m); }
+    __device__ __forceinline__ void flush(const uint32_t* planes, uint32_t n, int32_t g, int b) const {
+        group_flush(planes, n, a.gcol + (static_cast<size_t>(g) * a.L + static_cast<size_t>(b) * 32) * 8, min(32, a.L - b * 32));
+    }
+};
+
+__global__ void __launch_bounds__(kGroupMaxThreads) group_pileup_kernel(GroupArgs a) {
+    csa_walk(GroupPolicy{a}, a.tiles, a.nblk, a.nseg, a.seg_len, static_cast<int64_t>(a.ioff[a.ngroups]) * a.nseg);
 }
 
 // ---------------------------------------------------------------- per-group consensus

@@ -43,8 +43,8 @@ struct ms_handle {
     cudaEvent_t ev_k1[2] = {nullptr, nullptr};  // around the last K1 launch when timing is on
     cudaEvent_t ev_timer[2] = {nullptr, nullptr};  // ms_timer_start / ms_timer_stop
     int expand_ctas = 0, expand_ctas_nblk = -1;   // expand_events_kernel: resident CTAs per SM for row length nblk
-    cudaEvent_t ev_stage[15][2] = {};              // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
-    bool stage_seen[15] = {};
+    cudaEvent_t ev_stage[16][2] = {};              // when timing is on: around the last launch of MS_STAGE_* (ms_stage_kernel_ms)
+    bool stage_seen[16] = {};
     bool timing = false;
     int64_t k1_reads = 0;
     std::string err;
@@ -146,6 +146,13 @@ struct ms_handle {
     // read alignment (align.cu): the reference and its seed hash table, then per chunk of reads their bases and offsets, seeds,
     // the seed kernel's hit scratch, the band kernel's move-bit slabs and band-move bits, CIGAR slots, results, packed CIGARs
     int32_t aln_L = -1, aln_bits = 0;   // reference length (-1 = none set), log2 of the hash table's size
+    // in-frame indels (indel.cu): [L][2] k_del, n_ins | tally[sid] (one buffer: one all-reduce), the events, the call's buffer
+    int32_t indel_L = 0;                  // L of the layout the counts belong to; 0 = none
+    bool indel_reduced = false;           // the counts have been summed over the ranks
+    std::vector<int32_t> indel_col;       // per string id: its column ...
+    std::vector<std::string> indel_str;   // ... and its upper-cased string
+    DevBuf b_indel_cnt, b_indel_ev, b_indel_out;
+
     DevBuf b_aln_ref, b_aln_idx, b_aln_seq, b_aln_off, b_aln_seed, b_aln_scratch, b_aln_slab, b_aln_mbits, b_aln_cig, b_aln_res, b_aln_ctr,
         b_aln_dst, b_aln_pack;
 };

@@ -8,10 +8,12 @@
 // A third output kind, out.fasta (with --mode-phasing), holds the consensus sequence of every reported haplotype (restatement
 // choice U15): a grouped pile-up of each haplotype's reads on the GPU and fuse's column rule with thin columns written as 'N'.
 // --haplotype-abundance (restatement choice U18) fits every phased read, damaged ones included, to the reported haplotypes and
-// estimates their frequencies by EM over the reads' compatibility sets.
+// estimates their frequencies by EM over the reads' compatibility sets.  --indels (restatement choice U19) tests in-frame codon
+// deletions and insertions between codons with K2's model and reports them in an "indels" block.
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
+#include <cstring>
 #include <cstdlib>
 #include <ctime>
 #include <fstream>
@@ -38,11 +40,15 @@ static void usage() {
          "                                     Fisher tests for \"linked\" / \"exclusive\" after Bonferroni at --alpha)\n"
          "      --haplotype-abundance          with --mode-phasing: fit every read, damaged ones included, to the reported\n"
          "                                     haplotypes and estimate their frequencies by EM (\"haplotype_abundance\")\n"
+         "      --indels                       also call in-frame codon deletions and whole-codon insertions between codons\n"
+         "                                     (\"indels\"; DRM tokens such as 69ins, T69ins, 67del, D67del)\n"
          "      --min-perc <p>                 only variants with abundance > p %\n"
          "      --max-perc <p>                 only variants with abundance < p %\n"
          "      --drm-only                     only known drug-resistance mutations\n"
          "      --substitution-rate <r>        error model (default 5e-4)\n"
          "      --deletion-rate <r>            error model (default 3e-3)\n"
+         "      --insertion-rate <r>           error model of --indels: an inserted string of n bases has probability r^n\n"
+         "                                     (default 3e-3)\n"
          "      --alpha <a>                    significance after Bonferroni (default 0.01)\n"
          "      --min-haplotype-reads <n>      reads needed to report a haplotype (default 10)\n"
          "      --hap-min-coverage <n>         .fasta: a column with fewer votes of the haplotype's reads is written 'N'\n"
@@ -65,8 +71,8 @@ static bool ends_with(const std::string& s, const std::string& e) { return s.siz
 
 int main(int argc, char** argv) {
     std::string config, region, cmdline, timing_json;
-    bool phasing = false, drm_only = false, linkage = false, abundance = false;
-    double min_perc = -1, max_perc = -1, sub = 5e-4, del = 3e-3, alpha = 0.01;
+    bool phasing = false, drm_only = false, linkage = false, abundance = false, indels = false;
+    double min_perc = -1, max_perc = -1, sub = 5e-4, del = 3e-3, alpha = 0.01, ins_rate = 3e-3;
     int min_hap = 10, device = 0, ngpus = 1, hap_min_cov = 10;
     const int link_min_reads = 10;   // reads clean at both codons that a tested pair needs (the haplotype default, F21)
     mshost::QvFilter qv;
@@ -85,6 +91,8 @@ int main(int argc, char** argv) {
         else if (a == "--mode-phasing") phasing = true;
         else if (a == "--linkage") linkage = true;
         else if (a == "--haplotype-abundance") abundance = true;
+        else if (a == "--indels") indels = true;
+        else if (a == "--insertion-rate") ins_rate = atof(need("--insertion-rate").c_str());
         else if (a == "--drm-only") drm_only = true;
         else if (a == "--min-perc") min_perc = atof(need("--min-perc").c_str());
         else if (a == "--max-perc") max_perc = atof(need("--max-perc").c_str());
@@ -137,7 +145,7 @@ int main(int argc, char** argv) {
         std::vector<ms_handle*> hs(static_cast<size_t>(ngpus), nullptr);
         mshost::Alignments aln;
         const bool fasta = !out_fasta.empty();
-        mshost::load_alignments_overlapped(pos[0], qv, phasing, fasta, cfg.reference_sequence, aln, [&] {
+        mshost::load_alignments_overlapped(pos[0], qv, phasing, fasta || indels, cfg.reference_sequence, aln, [&] {
             char id[128];
             if (ngpus > 1 && ms_comm_unique_id(id) != MS_OK) mshost::die("NCCL is not available (libnccl.so.2): --gpus needs it");
             std::vector<std::string> errs(static_cast<size_t>(ngpus));
@@ -357,6 +365,74 @@ int main(int argc, char** argv) {
 
         lap(linkage ? "phasing + linkage" : "phasing");
 
+        // in-frame indels: every rank counts its reads (string ids from all the run's insertion events, so that they agree), one
+        // all-reduce inside ms_indel_call, the same list on every rank
+        msreport::IndelBlock ind;
+        if (indels) {
+            ms_indel_params ip;
+            ms_indel_params_default(&ip);
+            ip.deletion_rate = del; ip.insertion_rate = ins_rate; ip.alpha = alpha;
+            ip.min_perc = min_perc; ip.max_perc = max_perc; ip.region_begin = rb; ip.region_end = re;
+            std::vector<ms_indel> calls;
+            mshost::run_ranks(ngpus, [&](int r) {
+                ms_handle* h = hs[r];
+                const int64_t r0 = aln.nreads * r / ngpus, r1 = aln.nreads * (r + 1) / ngpus;
+                CKR(ms_indel_count_dev(h, rows_dev[r], r1 - r0, r0, aln.ins_read.data(), aln.ins_col.data(), aln.ins_off.data(), aln.ins_len.data(),
+                                       static_cast<int64_t>(aln.ins_read.size()), aln.ins_pool.data(), static_cast<int64_t>(aln.ins_pool.size())));
+                std::vector<ms_indel> my(256);
+                int64_t n = 0;
+                for (;;) {
+                    const int rc = ms_indel_call(h, mg.data(), static_cast<int32_t>(mg.size()), ref, &ip, my.data(), static_cast<int64_t>(my.size()), &n);
+                    if (rc == MS_ERR_CAPACITY) { my.resize(n); continue; }
+                    CKR(rc);
+                    break;
+                }
+                my.resize(n);
+                if (r == 0) calls.swap(my);
+            });
+            for (const std::string& e : errs)
+                if (!e.empty()) mshost::die(e);
+            ind.deletion_rate = del;
+            ind.insertion_rate = ins_rate;
+            for (const ms_indel& c : calls) {
+                msreport::IndelRow row;
+                const bool ins = c.kind == MS_INDEL_INSERTION;
+                auto aa = [](int32_t codon) { return codon >= 0 ? mscfg::translate(codon) : '?'; };
+                row.gene = c.gene;
+                row.type = ins ? "insertion" : "deletion";
+                row.ref_position = c.codon_index + 1;
+                row.abs_pos = c.col + 1;
+                row.count = c.count; row.coverage = c.coverage; row.expected = c.expected; row.ntests = c.ntests; row.pvalue = c.pvalue;
+                row.label = std::string(1, aa(c.ref_codon)) + std::to_string(row.ref_position);
+                if (ins) {
+                    std::vector<char> buf(static_cast<size_t>(L) + 1);
+                    int64_t len = 0;
+                    for (;;) {
+                        const int rc = ms_indel_inserted(h, c.sid, nullptr, buf.data(), static_cast<int64_t>(buf.size()), &len);
+                        if (rc == MS_ERR_CAPACITY) { buf.resize(static_cast<size_t>(len)); continue; }
+                        if (rc != MS_OK) mshost::die(std::string("ms_indel_inserted failed: ") + ms_last_error(h));
+                        break;
+                    }
+                    row.inserted.assign(buf.data(), static_cast<size_t>(len));
+                    row.label += "_" + std::string(1, aa(c.next_codon)) + std::to_string(row.ref_position + 1) + "ins";
+                    for (size_t q = 0; q + 3 <= row.inserted.size(); q += 3) {
+                        const int codon = 16 * (strchr("ACGT", row.inserted[q]) - "ACGT") + 4 * (strchr("ACGT", row.inserted[q + 1]) - "ACGT") +
+                                          (strchr("ACGT", row.inserted[q + 2]) - "ACGT");
+                        const char t = mscfg::translate(codon);
+                        row.label += t == 'X' ? '*' : t;
+                    }
+                } else {
+                    row.label += "del";
+                }
+                for (const mscfg::Drm& d : genes[c.gene].drms)
+                    for (const mscfg::DrmPosition& p : d.positions)
+                        if (mscfg::drm_matches_indel(p, row.ref_position, aa(c.ref_codon), ins)) { row.drugs.push_back(d.name); break; }
+                if (drm_only && row.drugs.empty()) continue;
+                ind.calls.push_back(row);
+            }
+            lap("indels");
+        }
+
         // haplotype abundance: every rank fits its reads to the same reported patterns; classes and EM are merged inside the library
         msreport::AbundanceBlock ab;
         if (abundance) {
@@ -456,7 +532,7 @@ int main(int argc, char** argv) {
         if (getenv("MS_FIXED_TIMESTAMP")) snprintf(ts, sizeof ts, "%s", getenv("MS_FIXED_TIMESTAMP"));
 
         const msjson::Value report = msreport::build(ts, pos[0], cmdline, MS_VERSION, cfg, L, genes, rows, col, L, phasing, haps, counters,
-                                                     linkage ? &link : nullptr, abundance ? &ab : nullptr);
+                                                     linkage ? &link : nullptr, abundance ? &ab : nullptr, indels ? &ind : nullptr);
         if (!out_json.empty()) {
             std::ofstream f(out_json);
             if (!f) mshost::die("cannot write " + out_json);

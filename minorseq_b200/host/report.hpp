@@ -71,6 +71,23 @@ struct AbundanceBlock {
     std::vector<AbundanceRow> haplotypes;   // report order
 };
 
+// in-frame codon deletions and insertions (--indels, restatement choice U19)
+struct IndelRow {
+    int gene = 0;
+    std::string type;          // "deletion" / "insertion"
+    std::string label;         // D67del, T69_S70insSS
+    int ref_position = 0;      // 1-based codon of the deletion / before the insertion
+    int abs_pos = 0;           // 1-based column: the deleted codon's first, or the one the insertion follows
+    std::string inserted;      // upper-cased inserted bases ("" for a deletion)
+    unsigned count = 0, coverage = 0, expected = 0, ntests = 0;
+    double pvalue = 0;
+    std::vector<std::string> drugs;
+};
+struct IndelBlock {
+    double deletion_rate = 0, insertion_rate = 0;
+    std::vector<IndelRow> calls;   // (gene, codon, deletion first, inserted)
+};
+
 // "%": two significant digits as in the screenshots (1.1, 0.91, 98, 100)
 inline std::string perc2(double p) {
     char b[32];
@@ -91,7 +108,7 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
                    const mscfg::TargetConfig& cfg, int ref_length, const std::vector<mscfg::Gene>& genes,
                    const std::vector<VariantRow>& variants, const std::vector<unsigned>& col_counts /* L*8 */, int L,
                    bool phasing, const std::vector<HaplotypeRow>& haps, const unsigned long long counters[6],
-                   const LinkageBlock* linkage = nullptr, const AbundanceBlock* abundance = nullptr) {
+                   const LinkageBlock* linkage = nullptr, const AbundanceBlock* abundance = nullptr, const IndelBlock* indels = nullptr) {
     Value root = Value::object();
     Value& in = root.set("input", Value::object());
     in.set("timestamp", Value::string(timestamp));
@@ -181,6 +198,14 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             i = j;
         }
     }
+    if (indels)
+        for (const IndelRow& r : indels->calls) {
+            const std::string label = r.label + " (" + genes[r.gene].name + ", " + perc2(100.0 * r.count / r.coverage) + " %)";
+            for (const std::string& d : r.drugs) {
+                if (!drug_summary.count(d)) drug_order.push_back(d);
+                drug_summary[d].push_back(label);
+            }
+        }
     Value& dsum = root.set("drug_summaries", Value::array());
     for (const std::string& d : drug_order) {
         Value& o = dsum.push(Value::object());
@@ -233,6 +258,32 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             o.set("pValue", Value::number(r.pvalue));
             o.set("pValueCorrected", Value::number(r.pvalue_corrected));
             o.set("relation", Value::string(r.relation));
+        }
+    }
+    if (indels) {
+        Value& ib = root.set("indels", Value::object());
+        ib.set("deletion_rate", Value::number(indels->deletion_rate));
+        ib.set("insertion_rate", Value::number(indels->insertion_rate));
+        Value& cs = ib.set("calls", Value::array());
+        for (const IndelRow& r : indels->calls) {
+            Value& o = cs.push(Value::object());
+            const double freq = static_cast<double>(r.count) / static_cast<double>(r.coverage);
+            o.set("gene", Value::string(genes[r.gene].name));
+            o.set("type", Value::string(r.type));
+            o.set("label", Value::string(r.label));
+            o.set("ref_position", Value::integer(r.ref_position));
+            o.set("abs_pos", Value::integer(r.abs_pos));
+            o.set("inserted", Value::string(r.inserted));
+            o.set("count", Value::integer(r.count));
+            o.set("coverage", Value::integer(r.coverage));
+            o.set("frequency", Value::number(freq));
+            o.set("percentage", Value::string(perc2(100.0 * freq)));
+            o.set("expected", Value::integer(r.expected));
+            o.set("pValue", Value::number(r.pvalue));
+            o.set("pValueCorrected", Value::number(std::min(1.0, r.pvalue * r.ntests)));
+            std::string known;
+            for (size_t d = 0; d < r.drugs.size(); ++d) known += (d ? " + " : "") + r.drugs[d];
+            o.set("known_drm", Value::string(known));
         }
     }
     if (abundance) {
@@ -444,6 +495,25 @@ inline std::string to_html(const Value& root) {
                 h += "<td>" + esc(r.get_string("em_percentage")) + "</td></tr>\n";
             }
         h += "</table></details>\n";
+    }
+    if (const Value* ib = root.get("indels")) {
+        char b[160];
+        snprintf(b, sizeof b, "Error model: deletion rate %g, insertion rate %g", ib->get_number("deletion_rate"), ib->get_number("insertion_rate"));
+        h += "<details open><summary>In-frame Insertions and Deletions</summary><p>" + std::string(b) + "</p>";
+        const Value* cs = ib->get("calls");
+        if (cs && !cs->arr.empty()) {
+            h += "<table><tr><th>Gene</th><th>Indel</th><th>Pos</th><th>Inserted</th><th>%</th><th>Count</th><th>Coverage</th>"
+                 "<th>p (corrected)</th><th>Affected Drugs</th></tr>\n";
+            for (const Value& r : cs->arr) {
+                snprintf(b, sizeof b, "<td>%.2e</td>", r.get_number("pValueCorrected"));
+                h += "<tr><td>" + esc(r.get_string("gene")) + "</td><td>" + esc(r.get_string("label")) + "</td><td>" +
+                     std::to_string(static_cast<long long>(r.get_number("abs_pos"))) + "</td><td><tt>" + esc(r.get_string("inserted")) + "</tt></td><td>" +
+                     esc(r.get_string("percentage")) + "</td><td>" + std::to_string(static_cast<long long>(r.get_number("count"))) + "</td><td>" +
+                     std::to_string(static_cast<long long>(r.get_number("coverage"))) + "</td>" + b + "<td>" + esc(r.get_string("known_drm")) + "</td></tr>\n";
+            }
+            h += "</table>";
+        }
+        h += "</details>\n";
     }
     h += "</body></html>\n";
     return h;

@@ -17,11 +17,15 @@
 
 namespace mscfg {
 
-struct DrmPosition {          // "M103LKA": ref aa (or '*'), position, allowed mutant aas (empty = '*')
+// "M103LKA": ref aa (or '*'), position, allowed mutant aas (empty = '*', which also matches an indel there).
+// "T69ins" / "69ins": an in-frame insertion after codon 69; "D67del" / "67del": a deletion of codon 67 (restatement choice U19).
+enum DrmKind { kDrmSubstitution = 0, kDrmInsertion = 1, kDrmDeletion = 2 };
+struct DrmPosition {
     char ref_aa = '*';
     int pos = 0;
     std::string mut_aas;
     std::string text;
+    int kind = kDrmSubstitution;
 };
 struct Drm { std::string name; std::vector<DrmPosition> positions; };
 struct Gene { std::string name; int begin = 0, end = 0; std::vector<Drm> drms; };
@@ -41,14 +45,26 @@ inline DrmPosition parse_drm_position(const std::string& s) {
     if (j == i) throw std::runtime_error("DRM position without a number: " + s);
     p.pos = std::stoi(s.substr(i, j - i));
     p.mut_aas = s.substr(j);
+    if (p.mut_aas == "ins" || p.mut_aas == "del") {
+        p.kind = p.mut_aas == "ins" ? kDrmInsertion : kDrmDeletion;
+        p.mut_aas.clear();
+    }
     return p;
 }
 
 // does a variant (1-based amino-acid position in the gene, reference aa, variant aa) hit this DRM entry?
 inline bool drm_matches(const DrmPosition& p, int aa_pos, char ref_aa, char var_aa) {
-    if (p.pos != aa_pos) return false;
+    if (p.kind != kDrmSubstitution || p.pos != aa_pos) return false;
     if (p.ref_aa != '*' && p.ref_aa != ref_aa) return false;
     return p.mut_aas.empty() || p.mut_aas.find(var_aa) != std::string::npos;
+}
+
+// does an in-frame indel hit this DRM entry?  aa_pos / ref_aa: the deleted codon, or the codon before the insertion
+inline bool drm_matches_indel(const DrmPosition& p, int aa_pos, char ref_aa, bool insertion) {
+    if (p.pos != aa_pos) return false;
+    if (p.ref_aa != '*' && p.ref_aa != ref_aa) return false;
+    if (p.kind == kDrmSubstitution) return p.mut_aas.empty();   // a bare position is a wildcard
+    return p.kind == (insertion ? kDrmInsertion : kDrmDeletion);
 }
 
 inline TargetConfig from_json(const msjson::Value& root) {
