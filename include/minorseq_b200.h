@@ -382,6 +382,27 @@ int ms_indel_inserted(ms_handle *h, int32_t sid, int32_t *col, char *buf, int64_
 int ms_indel_call(ms_handle *h, const ms_gene *genes, int32_t ngenes, const char *refseq, const ms_indel_params *prm,
                   ms_indel *out, int64_t cap, int64_t *n);
 
+/* ---- in-frame indels in phasing (restatement choice U20) ------------------------------------------------------
+ * Key order: the V substitution keys (the pooled, sorted (column, codon) list, bits [0, V) as with ms_phase_begin), then ndel
+ * deletion keys (start columns s, as given: ascending in juliet), then nins insertion keys (string ids of ms_indel_call, as
+ * given: by column, then string).  For read r ("clean" = A/C/G/T):
+ *   deletion key s:      B = '-' at s, s+1 and s+2;  M = B, or the three columns all clean;
+ *   insertion key (c,x): M = c and c+1 both clean;   B = M and r's first insertion event at c is x (the kept events of
+ *                        ms_indel_count_dev: in frame, A/C/G/T, upper-cased);
+ *   substitution keys:   B and M as with ms_phase_begin (a codon the read deletes is not clean: its bit is 0).
+ * Damage: r is not phased when some key's columns are not informative (M = 0).  The columns that cause it give the
+ * categories: '-' gaps, QV-filtered N heteroduplex, not spanned partial.  Substitution codons are judged as with
+ * ms_phase_begin, except that the three columns of a deletion key that r carries in full are never damage (also where a
+ * substitution codon, of any frame, covers them); a partial gap there is still a gap.  Insertion columns c, c+1 are judged
+ * like codon columns.  Pairwise linkage takes s and c as the keys' columns (|col_v - col_w| >= 3 as before).  After it,
+ * ms_phase_dev, ms_phase_groups, ms_phase_haplotypes, ms_phase_assign, ms_phase_hap_device, ms_linkage, ms_linkage_device
+ * and ms_haplotype_abundance work over the V + ndel + nins keys unchanged. */
+/* ms_phase_begin with the indel keys of restatement choice U20 after the V substitution keys: ndel deletion start
+ * columns, then nins insertion keys given by ms_indel_call's sid.  Needs ms_indel_count_dev on this handle for the same
+ * reads that the following ms_phase_dev receives (MS_ERR_ARG otherwise).  ndel = nins = 0 is ms_phase_begin. */
+int ms_phase_begin_indels(ms_handle *h, const int32_t *var_col, const int32_t *var_codon, int32_t V,
+                          const int32_t *del_col, int32_t ndel, const int32_t *ins_sid, int32_t nins, int64_t max_reads);
+
 /* ---- the whole juliet pass in one call ------------------------------------------------------
  * reset -> pileup -> (all-reduce when a communicator is attached) -> codon test -> phasing, i.e. everything
  * juliet does between BAM decode and report writing.  The caller owns the result buffers; on

@@ -188,6 +188,7 @@ _SIGNATURES = {
     "ms_indel_inserted": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32), _P, C.c_int64, C.POINTER(C.c_int64)]),
     "ms_indel_call": (C.c_int, [_P, C.POINTER(Gene), C.c_int32, C.c_char_p, C.POINTER(IndelParams), C.POINTER(Indel), C.c_int64,
                                 C.POINTER(C.c_int64)]),
+    "ms_phase_begin_indels": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int64]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

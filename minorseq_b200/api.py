@@ -295,14 +295,22 @@ class Juliet:
 
     # -- K3
     def phase_device(self, variants, d_packed_ptr: int, nreads: int, want_hap_id=True, host_merge=False, cap=4096,
-                     linkage=False, abundance=False) -> Haplotypes:
+                     linkage=False, abundance=False, indels=None) -> Haplotypes:
         """linkage / abundance: also record which reads are clean at each key, for Juliet.linkage / Juliet.haplotype_abundance
-        afterwards"""
+        afterwards.  indels: the Indels record of Juliet.indels on the same reads (restatement choice U20): its calls become
+        keys after the substitution keys, ("del", s) for the distinct deletion columns, then ("ins", c, x) for the distinct
+        inserted strings by column and string."""
         import torch.distributed as dist
         keys = sorted({(v.col, v.codon) for v in variants})
-        V = len(keys)
+        Vs = len(keys)
         vc = np.array([k[0] for k in keys], dtype=np.int32)
         vd = np.array([k[1] for k in keys], dtype=np.int32)
+        dcol, isid = np.zeros(0, dtype=np.int32), np.zeros(0, dtype=np.int32)
+        if indels is not None:
+            dcol = np.array(sorted({int(c) for k, c in zip(indels.kind, indels.col) if k == 0}), dtype=np.int32)
+            isid = np.array(sorted({int(s) for k, s in zip(indels.kind, indels.sid) if k == 1}), dtype=np.int32)   # ids: by column, string
+            keys = keys + [("del", int(s)) for s in dcol] + [("ins", int(indels.string_col[s]), indels.strings[s]) for s in isid]
+        V = len(keys)
         nw = max(1, (V + 31) // 32)
         self._V = V
         self._keys = keys
@@ -310,7 +318,8 @@ class Juliet:
         self._reported = None
         check(self.lib.ms_set_linkage(self.hd.h, 1 if linkage else 0), self.hd.h)
         check(self.lib.ms_set_abundance(self.hd.h, 1 if abundance else 0), self.hd.h)
-        check(self.lib.ms_phase_begin(self.hd.h, _ptr(vc), _ptr(vd), V, nreads), self.hd.h)
+        check(self.lib.ms_phase_begin_indels(self.hd.h, _ptr(vc), _ptr(vd), Vs, _ptr(dcol), len(dcol), _ptr(isid), len(isid), nreads),
+              self.hd.h)
         check(self.lib.ms_phase_dev(self.hd.h, C.c_void_p(d_packed_ptr), nreads), self.hd.h)
         if not host_merge and (getattr(self.hd, "native_comm", False) or _torch_world() == 1):
             hap = self._haplotypes_device(V, nw, nreads, want_hap_id, cap)

@@ -93,6 +93,10 @@ struct ms_handle {
     int32_t V = 0, vwords = 0;
     int64_t phase_cap = 0, phase_n = 0;
     int32_t nblocklist = 0;
+    // in-frame indel keys of ms_phase_begin_indels (phase_indel.cu) at bits [V - pi_nkeys, V): per key two words (block slot |
+    // kind | column in the block; bit index), the 32-column blocks they touch, and string id -> bit index (-1: no key)
+    int32_t pi_nkeys = 0, pi_nblk = 0;
+    DevBuf b_pi_keys, b_pi_blocks, b_pi_sid;
     int32_t phase_nrec = 0;          // words of phase_bits_kernel's variant stream
     bool phase_ordered = true;       // the stream visits the words of the bit-vector one after the other
     bool phase_partial_all = false;  // some variant lies outside the reference: every read is partial
@@ -149,6 +153,7 @@ struct ms_handle {
     // in-frame indels (indel.cu): [L][2] k_del, n_ins | tally[sid] (one buffer: one all-reduce), the events, the call's buffer
     int32_t indel_L = 0;                  // L of the layout the counts belong to; 0 = none
     bool indel_reduced = false;           // the counts have been summed over the ranks
+    int64_t indel_R = 0, indel_nev = 0;   // reads counted, and this rank's kept events in b_indel_ev: (local read, c, sid)
     std::vector<int32_t> indel_col;       // per string id: its column ...
     std::vector<std::string> indel_str;   // ... and its upper-cased string
     DevBuf b_indel_cnt, b_indel_ev, b_indel_out;

@@ -248,6 +248,8 @@ int ms_indel_count_dev(ms_handle* h, const uint32_t* d_packed, int64_t R, int64_
     MS_CUDA(h, cudaMemsetAsync(cnt, 0, words * 4, h->stream));
     h->indel_L = L;
     h->indel_reduced = false;
+    h->indel_R = R;
+    h->indel_nev = R > 0 ? nev : 0;
     if (R > 0) {
         ms::IndelCountArgs a;
         a.tiles = reinterpret_cast<const uint4*>(d_packed);

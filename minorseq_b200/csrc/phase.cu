@@ -643,22 +643,34 @@ void ms_phase_free_internal(ms_handle* h) {
                      &h->b_gslot, &h->b_mt_key, &h->b_mt_cnt, &h->b_mt_rep, &h->b_mslot, &h->b_mindex, &h->b_m_cnt, &h->b_m_pat, &h->b_m_rank,
                      &h->b_ord, &h->b_keys, &h->b_out, &h->b_tc_tiles,
                      &h->b_nw_seq, &h->b_nw_hrow, &h->b_nw_hcol, &h->b_nw_dir,
-                     &h->b_mbits, &h->b_link_gram, &h->b_link_col, &h->b_link_sig, &h->b_link_rows, &h->b_link_out};
+                     &h->b_mbits, &h->b_link_gram, &h->b_link_col, &h->b_link_sig, &h->b_link_rows, &h->b_link_out,
+                     &h->b_pi_keys, &h->b_pi_blocks, &h->b_pi_sid};
     for (DevBuf* b : all) b->release();
     if (h->h_stage) cudaFreeHost(h->h_stage);
     h->h_stage = nullptr; h->h_stage_cap = 0;
     if (h->plan_stage) cudaFreeHost(h->plan_stage);
     h->plan_stage = nullptr;
-    h->phase_cap = h->phase_n = 0; h->V = 0; h->vwords = 0; h->table_valid = false;
+    h->phase_cap = h->phase_n = 0; h->V = 0; h->vwords = 0; h->table_valid = false; h->pi_nkeys = 0;
     h->link_ready = h->gram_valid = false;
     h->hap_ranked = h->hap_assigned = false;
 }
 
 int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codon, int32_t V, int64_t max_reads) {
-    if (!h || h->L <= 0 || V < 0 || max_reads < 0 || (V > 0 && (!var_col || !var_codon))) return MS_ERR_ARG;
+    return ms::phase_begin_keys(h, var_col, var_codon, V, nullptr, 0, std::vector<uint32_t>(), max_reads);
+}
+
+}  // extern "C"
+
+namespace ms {
+
+int phase_begin_keys(ms_handle* h, const int32_t* var_col, const int32_t* var_codon, int32_t V, const int32_t* extra_col, int32_t nextra,
+                     const std::vector<uint32_t>& exclude, int64_t max_reads) {
+    if (!h || h->L <= 0 || V < 0 || nextra < 0 || max_reads < 0 || (V > 0 && (!var_col || !var_codon)) || (nextra > 0 && !extra_col))
+        return MS_ERR_ARG;
     MS_CUDA(h, cudaSetDevice(h->device));
-    h->V = V;
-    h->vwords = std::max(1, (V + 31) / 32);
+    h->V = V + nextra;
+    h->vwords = std::max(1, (V + nextra + 31) / 32);
+    h->pi_nkeys = 0;
     h->phase_cap = std::max<int64_t>(1, max_reads);
     h->phase_n = 0;
     h->table_valid = false;
@@ -696,6 +708,8 @@ int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codo
             }
             by_block[std::lower_bound(blocks.begin(), blocks.end(), var_col[v] >> 5) - blocks.begin()].push_back(v);
         }
+        if (!exclude.empty())
+            for (int32_t sl = 0; sl < NBl; ++sl) cover[sl] &= ~exclude[blocks[sl]];
     }
     std::vector<uint32_t> vd;
     bool ordered = true;
@@ -777,6 +791,7 @@ int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codo
     if (h->linkage || h->abundance) {   // the clean-codon matrix of pairwise linkage and haplotype abundance, same shape as the bit matrix
         MS_CUDA(h, h->b_mbits.ensure(static_cast<size_t>(h->phase_cap) * h->vwords * 4));
         h->link_col.assign(var_col, var_col + V);
+        h->link_col.insert(h->link_col.end(), extra_col, extra_col + nextra);
         h->link_ready = true;
     }
     MS_CUDA(h, h->b_var.ensure(vd.size() * 4));
@@ -806,10 +821,16 @@ int ms_phase_begin(ms_handle* h, const int32_t* var_col, const int32_t* var_codo
     return MS_OK;
 }
 
+}  // namespace ms
+
+extern "C" {
+
 int ms_phase_dev(ms_handle* h, const uint32_t* d_packed, int64_t R) {
     MsRange nvtx_range("K3 phase bits");
     if (!h || !h->b_bits.p || R < 0 || (R > 0 && !d_packed)) return MS_ERR_ARG;
     if (h->phase_n + R > h->phase_cap) MS_FAIL(h, MS_ERR_CAPACITY, "more reads than ms_phase_begin(max_reads)");
+    if (h->pi_nkeys > 0 && (h->phase_n != 0 || R != h->indel_R || h->indel_L != h->L))
+        MS_FAIL(h, MS_ERR_ARG, "ms_phase_dev: indel keys need the reads of the last ms_indel_count_dev, in one call");
     if (R == 0) return MS_OK;
     MS_CUDA(h, cudaSetDevice(h->device));
     h->table_valid = false;
@@ -848,6 +869,10 @@ int ms_phase_dev(ms_handle* h, const uint32_t* d_packed, int64_t R) {
     MS_STAGE_END(h, MS_STAGE_PHASE_BITS);
     h->launches++;
     MS_CUDA(h, cudaGetLastError());
+    if (h->pi_nkeys > 0) {
+        const int rc = ms::phase_indel_dev(h, pk, R, bits, mbits, flags);
+        if (rc != MS_OK) return rc;
+    }
     h->phase_n += R;
     return MS_OK;
 }
@@ -865,6 +890,7 @@ int ms_phase_planned_dev(ms_handle* h, const ms_variant* d_calls, const unsigned
     h->V = 0;                       // known after the download of the plan (ms_phase_planned_adopt)
     h->vwords = 1;
     h->link_ready = h->gram_valid = false;   // this pass writes no clean-codon matrix
+    h->pi_nkeys = 0;
     h->hap_ranked = h->hap_assigned = false;
     h->phase_cap = std::max<int64_t>(1, R);
     h->phase_n = 0;

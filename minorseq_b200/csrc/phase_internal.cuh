@@ -1,6 +1,7 @@
 // phase_internal.cuh -- pieces of K3 shared by phase.cu (bit-vectors, local grouping table) and
 // phase_order.cu (cross-rank merge + ordering on the device).
 #pragma once
+#include <vector>
 #include "handle.h"
 
 namespace ms {
@@ -112,5 +113,13 @@ int phase_build_table(ms_handle* h, int attempt);
 int phase_compact(ms_handle* h, uint32_t* g_cnt, uint32_t* g_pat, int32_t* g_slot, int64_t cap);
 // after a host look at ctr[6]: grow the table (x8) for the next build; fails at the maximum size
 int phase_grow_table(ms_handle* h);
+
+// ms_phase_begin with nextra keys after the V (column, codon) keys, at bits [V, V + nextra): phase_bits_kernel leaves them 0 and
+// pairwise linkage takes extra_col as their columns.  exclude (empty, or one word per 32-column block of the layout): columns
+// left out of phase_bits_kernel's damage mask `cover`.
+int phase_begin_keys(ms_handle* h, const int32_t* var_col, const int32_t* var_codon, int32_t V, const int32_t* extra_col, int32_t nextra,
+                     const std::vector<uint32_t>& exclude, int64_t max_reads);
+// after phase_bits_kernel on the same reads: the indel keys' bits, clean bits (mbits may be null) and damage (phase_indel.cu)
+int phase_indel_dev(ms_handle* h, const uint4* packed, int64_t R, uint32_t* bits, uint32_t* mbits, uint8_t* flags);
 
 }  // namespace ms

@@ -9,7 +9,8 @@
 // choice U15): a grouped pile-up of each haplotype's reads on the GPU and fuse's column rule with thin columns written as 'N'.
 // --haplotype-abundance (restatement choice U18) fits every phased read, damaged ones included, to the reported haplotypes and
 // estimates their frequencies by EM over the reads' compatibility sets.  --indels (restatement choice U19) tests in-frame codon
-// deletions and insertions between codons with K2's model and reports them in an "indels" block.
+// deletions and insertions between codons with K2's model and reports them in an "indels" block.  --phase-indels (restatement
+// choice U20) adds the reported indels to the phasing keys: haplotypes, linkage, abundance and the FASTA then see them.
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -42,6 +43,8 @@ static void usage() {
          "                                     haplotypes and estimate their frequencies by EM (\"haplotype_abundance\")\n"
          "      --indels                       also call in-frame codon deletions and whole-codon insertions between codons\n"
          "                                     (\"indels\"; DRM tokens such as 69ins, T69ins, 67del, D67del)\n"
+         "      --phase-indels                 with --mode-phasing and --indels: phase the reported indels with the variants\n"
+         "                                     (haplotypes, linkage, abundance and the .fasta carry them)\n"
          "      --min-perc <p>                 only variants with abundance > p %\n"
          "      --max-perc <p>                 only variants with abundance < p %\n"
          "      --drm-only                     only known drug-resistance mutations\n"
@@ -71,7 +74,7 @@ static bool ends_with(const std::string& s, const std::string& e) { return s.siz
 
 int main(int argc, char** argv) {
     std::string config, region, cmdline, timing_json;
-    bool phasing = false, drm_only = false, linkage = false, abundance = false, indels = false;
+    bool phasing = false, drm_only = false, linkage = false, abundance = false, indels = false, phase_indels = false;
     double min_perc = -1, max_perc = -1, sub = 5e-4, del = 3e-3, alpha = 0.01, ins_rate = 3e-3;
     int min_hap = 10, device = 0, ngpus = 1, hap_min_cov = 10;
     const int link_min_reads = 10;   // reads clean at both codons that a tested pair needs (the haplotype default, F21)
@@ -92,6 +95,7 @@ int main(int argc, char** argv) {
         else if (a == "--linkage") linkage = true;
         else if (a == "--haplotype-abundance") abundance = true;
         else if (a == "--indels") indels = true;
+        else if (a == "--phase-indels") phase_indels = true;
         else if (a == "--insertion-rate") ins_rate = atof(need("--insertion-rate").c_str());
         else if (a == "--drm-only") drm_only = true;
         else if (a == "--min-perc") min_perc = atof(need("--min-perc").c_str());
@@ -120,6 +124,8 @@ int main(int argc, char** argv) {
     if (!out_fasta.empty() && !phasing) mshost::die("a .fasta output holds the haplotypes' sequences: it needs --mode-phasing");
     if (hap_min_cov < 0) mshost::die("--hap-min-coverage expects a count >= 0");
     if (abundance && !phasing) mshost::die("--haplotype-abundance fits the reads to the reported haplotypes: it needs --mode-phasing");
+    if (phase_indels && (!phasing || !indels))
+        mshost::die("--phase-indels puts the reported indels into the haplotypes: it needs --mode-phasing and --indels");
     int rb = 0, re = 0;
     if (!region.empty()) {
         if (sscanf(region.c_str(), "%d-%d", &rb, &re) != 2 || rb < 1 || re <= rb) mshost::die("--region expects <begin-end>");
@@ -200,10 +206,45 @@ int main(int argc, char** argv) {
         int64_t link_tested = 0;
         std::vector<const uint32_t*> rows_dev(static_cast<size_t>(ngpus), nullptr);   // each rank's reads on its GPU (tiles)
         std::vector<std::string> errs(static_cast<size_t>(ngpus));
+        std::vector<std::vector<ms_indel>> calls_rank(static_cast<size_t>(ngpus));   // --phase-indels: each rank's copy of the calls
 #define CKR(call)                                                                                      \
     do {                                                                                               \
         if ((call) != MS_OK) { errs[r] = std::string(#call) + " failed: " + ms_last_error(h); return; } \
     } while (0)
+        // in-frame indels: every rank counts its reads (string ids from all the run's insertion events, so that they agree), one
+        // all-reduce inside ms_indel_call, the same list on every rank
+        ms_indel_params ip;
+        ms_indel_params_default(&ip);
+        ip.deletion_rate = del; ip.insertion_rate = ins_rate; ip.alpha = alpha;
+        ip.min_perc = min_perc; ip.max_perc = max_perc; ip.region_begin = rb; ip.region_end = re;
+        std::vector<ms_indel> calls;
+        auto indel_rank = [&](int r) {
+            ms_handle* h = hs[r];
+            const int64_t r0 = aln.nreads * r / ngpus, r1 = aln.nreads * (r + 1) / ngpus;
+            CKR(ms_indel_count_dev(h, rows_dev[r], r1 - r0, r0, aln.ins_read.data(), aln.ins_col.data(), aln.ins_off.data(), aln.ins_len.data(),
+                                   static_cast<int64_t>(aln.ins_read.size()), aln.ins_pool.data(), static_cast<int64_t>(aln.ins_pool.size())));
+            std::vector<ms_indel> my(256);
+            int64_t n = 0;
+            for (;;) {
+                const int rc = ms_indel_call(h, mg.data(), static_cast<int32_t>(mg.size()), ref, &ip, my.data(), static_cast<int64_t>(my.size()), &n);
+                if (rc == MS_ERR_CAPACITY) { my.resize(n); continue; }
+                CKR(rc);
+                break;
+            }
+            my.resize(n);
+            if (r == 0) calls.swap(my);
+            else if (phase_indels) calls_rank[r].swap(my);
+        };
+        auto indel_aa = [](int32_t codon) { return codon >= 0 ? mscfg::translate(codon) : '?'; };
+        auto indel_drugs = [&](const ms_indel& c) {
+            std::vector<std::string> d;
+            for (const mscfg::Drm& x : genes[c.gene].drms)
+                for (const mscfg::DrmPosition& p : x.positions)
+                    if (mscfg::drm_matches_indel(p, c.codon_index + 1, indel_aa(c.ref_codon), c.kind == MS_INDEL_INSERTION)) { d.push_back(x.name); break; }
+            return d;
+        };
+        // --phase-indels: the reported calls' keys, deletion columns ascending, then insertion string ids (by column, string)
+        std::vector<int32_t> key_del, key_sid;
         mshost::run_ranks(ngpus, [&](int r) {
             ms_handle* h = hs[r];
             const int64_t r0 = aln.nreads * r / ngpus, r1 = aln.nreads * (r + 1) / ngpus;
@@ -251,6 +292,21 @@ int main(int argc, char** argv) {
                 lap("call + DRM annotation");
                 CKR(ms_get_counts(h, col.data(), nullptr));
             }
+            std::vector<int32_t> my_del, my_sid;
+            if (phase_indels) {
+                indel_rank(r);
+                if (!errs[r].empty()) return;
+                if (r == 0) lap("indels");
+                for (const ms_indel& c : r == 0 ? calls : calls_rank[r]) {
+                    if (drm_only && indel_drugs(c).empty()) continue;
+                    if (c.kind == MS_INDEL_DELETION) my_del.push_back(c.col);
+                    else my_sid.push_back(c.sid);
+                }
+                for (std::vector<int32_t>* k : {&my_del, &my_sid}) {
+                    std::sort(k->begin(), k->end());
+                    k->erase(std::unique(k->begin(), k->end()), k->end());
+                }
+            }
             if (phasing || linkage) {
                 // one global variant list over all genes (screenshot juliet_hiv-phasing.png: same columns in every table)
                 std::vector<std::pair<int, int>> my_keys;
@@ -258,12 +314,13 @@ int main(int argc, char** argv) {
                 std::sort(my_keys.begin(), my_keys.end());
                 my_keys.erase(std::unique(my_keys.begin(), my_keys.end()), my_keys.end());
                 const int32_t V = static_cast<int32_t>(my_keys.size());
-                const int32_t nw = std::max(1, (V + 31) / 32);
+                const int32_t nw = std::max(1, (V + static_cast<int32_t>(my_del.size() + my_sid.size()) + 31) / 32);
                 std::vector<int32_t> vc(V), vk(V);
                 for (int32_t i = 0; i < V; ++i) { vc[i] = my_keys[i].first; vk[i] = my_keys[i].second; }
                 CKR(ms_set_linkage(h, linkage ? 1 : 0));
                 CKR(ms_set_abundance(h, abundance ? 1 : 0));
-                CKR(ms_phase_begin(h, vc.data(), vk.data(), V, r1 - r0));
+                CKR(ms_phase_begin_indels(h, vc.data(), vk.data(), V, my_del.data(), static_cast<int32_t>(my_del.size()), my_sid.data(),
+                                          static_cast<int32_t>(my_sid.size()), r1 - r0));
                 CKR(ms_phase_dev(h, d_rows, r1 - r0));
                 if (linkage) {
                     // every rank computes the same list from the all-reduced counts (a collective: all ranks call it)
@@ -301,7 +358,7 @@ int main(int argc, char** argv) {
                         pat.swap(my_pat); cnt.swap(my_cnt); nrep_all = nrep;
                     }
                 }
-                if (r == 0) keys.swap(my_keys);
+                if (r == 0) { keys.swap(my_keys); key_del.swap(my_del); key_sid.swap(my_sid); }
             }
             if (r == 0) rows.swap(my_rows);
         });
@@ -309,9 +366,53 @@ int main(int argc, char** argv) {
             if (!e.empty()) mshost::die(e);
         ms_handle* h = hs[0];
 
+        msreport::IndelBlock ind;
+        const int32_t V = static_cast<int32_t>(keys.size());
+        // the report rows of the calls; with --phase-indels each row's key index (V + position among the indel keys)
+        auto indel_rows = [&]() {
+            ind.deletion_rate = del;
+            ind.insertion_rate = ins_rate;
+            for (const ms_indel& c : calls) {
+                msreport::IndelRow row;
+                const bool ins = c.kind == MS_INDEL_INSERTION;
+                row.gene = c.gene;
+                row.type = ins ? "insertion" : "deletion";
+                row.ref_position = c.codon_index + 1;
+                row.abs_pos = c.col + 1;
+                row.count = c.count; row.coverage = c.coverage; row.expected = c.expected; row.ntests = c.ntests; row.pvalue = c.pvalue;
+                row.label = std::string(1, indel_aa(c.ref_codon)) + std::to_string(row.ref_position);
+                if (ins) {
+                    std::vector<char> buf(static_cast<size_t>(L) + 1);
+                    int64_t len = 0;
+                    for (;;) {
+                        const int rc = ms_indel_inserted(h, c.sid, nullptr, buf.data(), static_cast<int64_t>(buf.size()), &len);
+                        if (rc == MS_ERR_CAPACITY) { buf.resize(static_cast<size_t>(len)); continue; }
+                        if (rc != MS_OK) mshost::die(std::string("ms_indel_inserted failed: ") + ms_last_error(h));
+                        break;
+                    }
+                    row.inserted.assign(buf.data(), static_cast<size_t>(len));
+                    row.label += "_" + std::string(1, indel_aa(c.next_codon)) + std::to_string(row.ref_position + 1) + "ins";
+                    for (size_t q = 0; q + 3 <= row.inserted.size(); q += 3) {
+                        const int codon = 16 * (strchr("ACGT", row.inserted[q]) - "ACGT") + 4 * (strchr("ACGT", row.inserted[q + 1]) - "ACGT") +
+                                          (strchr("ACGT", row.inserted[q + 2]) - "ACGT");
+                        const char t = mscfg::translate(codon);
+                        row.label += t == 'X' ? '*' : t;
+                    }
+                } else {
+                    row.label += "del";
+                }
+                row.drugs = indel_drugs(c);
+                if (drm_only && row.drugs.empty()) continue;
+                if (phase_indels)
+                    row.key = ins ? V + static_cast<int>(key_del.size() + (std::lower_bound(key_sid.begin(), key_sid.end(), c.sid) - key_sid.begin()))
+                                  : V + static_cast<int>(std::lower_bound(key_del.begin(), key_del.end(), c.col) - key_del.begin());
+                ind.calls.push_back(row);
+            }
+        };
+        if (phase_indels) indel_rows();
+
         if (phasing) {
-            const int32_t V = static_cast<int32_t>(keys.size());
-            const int32_t nw = std::max(1, (V + 31) / 32);
+            const int32_t nw = std::max(1, (V + static_cast<int32_t>(key_del.size() + key_sid.size()) + 31) / 32);
             const int64_t nrep = nrep_all;
             haps.resize(nrep);
             for (int64_t k = 0; k < nrep; ++k) {
@@ -325,6 +426,14 @@ int main(int argc, char** argv) {
                     const bool on = (pat[static_cast<size_t>(k) * nw + (v >> 5)] >> (v & 31)) & 1u;
                     haps[k].codons.push_back(on ? mscfg::codon_string(keys[v].second, cb) : "");
                 }
+                for (int32_t v = V; v < V + static_cast<int32_t>(key_del.size() + key_sid.size()); ++v)
+                    if ((pat[static_cast<size_t>(k) * nw + (v >> 5)] >> (v & 31)) & 1u)
+                        for (const msreport::IndelRow& row : ind.calls)
+                            if (row.key == v) haps[k].indels.push_back(genes[row.gene].name + " " + row.label);
+            }
+            for (msreport::IndelRow& row : ind.calls) {
+                row.haplotype_hit.resize(nrep);
+                for (int64_t k = 0; k < nrep; ++k) row.haplotype_hit[k] = (pat[static_cast<size_t>(k) * nw + (row.key >> 5)] >> (row.key & 31)) & 1u;
             }
             for (int64_t r = 0; r < aln.nreads; ++r)
                 if (hap[r] >= 0 && hap[r] < nrep) haps[hap[r]].read_names.push_back(aln.names[r]);
@@ -343,6 +452,15 @@ int main(int argc, char** argv) {
             auto variant = [&](int32_t v) {
                 msreport::LinkageVariant o;
                 char cb[4];
+                if (v >= V) {      // an indel key: "---" or "+" and the inserted bases
+                    for (const msreport::IndelRow& row : ind.calls)
+                        if (row.key == v) {
+                            o.abs_pos = row.abs_pos;
+                            o.codon = row.type == "deletion" ? "---" : "+" + row.inserted;
+                            o.labels.push_back(genes[row.gene].name + " " + row.label);
+                        }
+                    return o;
+                }
                 o.abs_pos = keys[v].first + 1;
                 o.codon = mscfg::codon_string(keys[v].second, cb);
                 for (const msreport::VariantRow& r : rows)
@@ -365,71 +483,11 @@ int main(int argc, char** argv) {
 
         lap(linkage ? "phasing + linkage" : "phasing");
 
-        // in-frame indels: every rank counts its reads (string ids from all the run's insertion events, so that they agree), one
-        // all-reduce inside ms_indel_call, the same list on every rank
-        msreport::IndelBlock ind;
-        if (indels) {
-            ms_indel_params ip;
-            ms_indel_params_default(&ip);
-            ip.deletion_rate = del; ip.insertion_rate = ins_rate; ip.alpha = alpha;
-            ip.min_perc = min_perc; ip.max_perc = max_perc; ip.region_begin = rb; ip.region_end = re;
-            std::vector<ms_indel> calls;
-            mshost::run_ranks(ngpus, [&](int r) {
-                ms_handle* h = hs[r];
-                const int64_t r0 = aln.nreads * r / ngpus, r1 = aln.nreads * (r + 1) / ngpus;
-                CKR(ms_indel_count_dev(h, rows_dev[r], r1 - r0, r0, aln.ins_read.data(), aln.ins_col.data(), aln.ins_off.data(), aln.ins_len.data(),
-                                       static_cast<int64_t>(aln.ins_read.size()), aln.ins_pool.data(), static_cast<int64_t>(aln.ins_pool.size())));
-                std::vector<ms_indel> my(256);
-                int64_t n = 0;
-                for (;;) {
-                    const int rc = ms_indel_call(h, mg.data(), static_cast<int32_t>(mg.size()), ref, &ip, my.data(), static_cast<int64_t>(my.size()), &n);
-                    if (rc == MS_ERR_CAPACITY) { my.resize(n); continue; }
-                    CKR(rc);
-                    break;
-                }
-                my.resize(n);
-                if (r == 0) calls.swap(my);
-            });
+        if (indels && !phase_indels) {
+            mshost::run_ranks(ngpus, indel_rank);
             for (const std::string& e : errs)
                 if (!e.empty()) mshost::die(e);
-            ind.deletion_rate = del;
-            ind.insertion_rate = ins_rate;
-            for (const ms_indel& c : calls) {
-                msreport::IndelRow row;
-                const bool ins = c.kind == MS_INDEL_INSERTION;
-                auto aa = [](int32_t codon) { return codon >= 0 ? mscfg::translate(codon) : '?'; };
-                row.gene = c.gene;
-                row.type = ins ? "insertion" : "deletion";
-                row.ref_position = c.codon_index + 1;
-                row.abs_pos = c.col + 1;
-                row.count = c.count; row.coverage = c.coverage; row.expected = c.expected; row.ntests = c.ntests; row.pvalue = c.pvalue;
-                row.label = std::string(1, aa(c.ref_codon)) + std::to_string(row.ref_position);
-                if (ins) {
-                    std::vector<char> buf(static_cast<size_t>(L) + 1);
-                    int64_t len = 0;
-                    for (;;) {
-                        const int rc = ms_indel_inserted(h, c.sid, nullptr, buf.data(), static_cast<int64_t>(buf.size()), &len);
-                        if (rc == MS_ERR_CAPACITY) { buf.resize(static_cast<size_t>(len)); continue; }
-                        if (rc != MS_OK) mshost::die(std::string("ms_indel_inserted failed: ") + ms_last_error(h));
-                        break;
-                    }
-                    row.inserted.assign(buf.data(), static_cast<size_t>(len));
-                    row.label += "_" + std::string(1, aa(c.next_codon)) + std::to_string(row.ref_position + 1) + "ins";
-                    for (size_t q = 0; q + 3 <= row.inserted.size(); q += 3) {
-                        const int codon = 16 * (strchr("ACGT", row.inserted[q]) - "ACGT") + 4 * (strchr("ACGT", row.inserted[q + 1]) - "ACGT") +
-                                          (strchr("ACGT", row.inserted[q + 2]) - "ACGT");
-                        const char t = mscfg::translate(codon);
-                        row.label += t == 'X' ? '*' : t;
-                    }
-                } else {
-                    row.label += "del";
-                }
-                for (const mscfg::Drm& d : genes[c.gene].drms)
-                    for (const mscfg::DrmPosition& p : d.positions)
-                        if (mscfg::drm_matches_indel(p, row.ref_position, aa(c.ref_codon), ins)) { row.drugs.push_back(d.name); break; }
-                if (drm_only && row.drugs.empty()) continue;
-                ind.calls.push_back(row);
-            }
+            indel_rows();
             lap("indels");
         }
 
@@ -532,7 +590,7 @@ int main(int argc, char** argv) {
         if (getenv("MS_FIXED_TIMESTAMP")) snprintf(ts, sizeof ts, "%s", getenv("MS_FIXED_TIMESTAMP"));
 
         const msjson::Value report = msreport::build(ts, pos[0], cmdline, MS_VERSION, cfg, L, genes, rows, col, L, phasing, haps, counters,
-                                                     linkage ? &link : nullptr, abundance ? &ab : nullptr, indels ? &ind : nullptr);
+                                                     linkage ? &link : nullptr, abundance ? &ab : nullptr, indels ? &ind : nullptr, phase_indels);
         if (!out_json.empty()) {
             std::ofstream f(out_json);
             if (!f) mshost::die("cannot write " + out_json);

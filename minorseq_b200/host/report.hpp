@@ -34,6 +34,7 @@ struct HaplotypeRow {
     unsigned long long reads = 0;
     double frequency = 0;           // of the reported reads (screenshot juliet_hiv-phasing.png sums to 100)
     std::vector<std::string> codons;  // per variant column: codon string if carried, else ""
+    std::vector<std::string> indels;  // --phase-indels: "<gene> <label>" of the indel calls it carries
     std::vector<std::string> read_names;
 };
 
@@ -82,6 +83,8 @@ struct IndelRow {
     unsigned count = 0, coverage = 0, expected = 0, ntests = 0;
     double pvalue = 0;
     std::vector<std::string> drugs;
+    int key = -1;                          // --phase-indels: the call's index in the phasing keys
+    std::vector<bool> haplotype_hit;       // --phase-indels: per reported haplotype
 };
 struct IndelBlock {
     double deletion_rate = 0, insertion_rate = 0;
@@ -108,7 +111,8 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
                    const mscfg::TargetConfig& cfg, int ref_length, const std::vector<mscfg::Gene>& genes,
                    const std::vector<VariantRow>& variants, const std::vector<unsigned>& col_counts /* L*8 */, int L,
                    bool phasing, const std::vector<HaplotypeRow>& haps, const unsigned long long counters[6],
-                   const LinkageBlock* linkage = nullptr, const AbundanceBlock* abundance = nullptr, const IndelBlock* indels = nullptr) {
+                   const LinkageBlock* linkage = nullptr, const AbundanceBlock* abundance = nullptr, const IndelBlock* indels = nullptr,
+                   bool phase_indels = false) {
     Value root = Value::object();
     Value& in = root.set("input", Value::object());
     in.set("timestamp", Value::string(timestamp));
@@ -223,6 +227,10 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             o.set("percentage", Value::string(perc1(100.0 * h.frequency)));
             Value& cs = o.set("codons", Value::array());
             for (const std::string& c : h.codons) cs.push(Value::string(c));
+            if (phase_indels) {
+                Value& is = o.set("indels", Value::array());
+                for (const std::string& c : h.indels) is.push(Value::string(c));
+            }
             Value& rn = o.set("read_names", Value::array());
             for (const std::string& n : h.read_names) rn.push(Value::string(n));
         }
@@ -284,6 +292,10 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             std::string known;
             for (size_t d = 0; d < r.drugs.size(); ++d) known += (d ? " + " : "") + r.drugs[d];
             o.set("known_drm", Value::string(known));
+            if (phase_indels) {
+                Value& hh = o.set("haplotype_hit", Value::array());
+                for (bool b : r.haplotype_hit) hh.push(Value::boolean(b));
+            }
         }
     }
     if (abundance) {
@@ -502,14 +514,24 @@ inline std::string to_html(const Value& root) {
         h += "<details open><summary>In-frame Insertions and Deletions</summary><p>" + std::string(b) + "</p>";
         const Value* cs = ib->get("calls");
         if (cs && !cs->arr.empty()) {
+            // with --phase-indels one column per reported haplotype marks the calls it carries, as in Variant Discovery
+            const size_t nhi = cs->arr[0].get("haplotype_hit") ? nh : 0;
             h += "<table><tr><th>Gene</th><th>Indel</th><th>Pos</th><th>Inserted</th><th>%</th><th>Count</th><th>Coverage</th>"
-                 "<th>p (corrected)</th><th>Affected Drugs</th></tr>\n";
+                 "<th>p (corrected)</th><th>Affected Drugs</th>";
+            for (size_t k = 0; k < nhi; ++k) h += "<th style=\"color:" + std::string(palette[k % 10]) + "\">" + esc(haps->arr[k].get_string("name")) + "</th>";
+            h += "</tr>\n";
             for (const Value& r : cs->arr) {
                 snprintf(b, sizeof b, "<td>%.2e</td>", r.get_number("pValueCorrected"));
                 h += "<tr><td>" + esc(r.get_string("gene")) + "</td><td>" + esc(r.get_string("label")) + "</td><td>" +
                      std::to_string(static_cast<long long>(r.get_number("abs_pos"))) + "</td><td><tt>" + esc(r.get_string("inserted")) + "</tt></td><td>" +
                      esc(r.get_string("percentage")) + "</td><td>" + std::to_string(static_cast<long long>(r.get_number("count"))) + "</td><td>" +
-                     std::to_string(static_cast<long long>(r.get_number("coverage"))) + "</td>" + b + "<td>" + esc(r.get_string("known_drm")) + "</td></tr>\n";
+                     std::to_string(static_cast<long long>(r.get_number("coverage"))) + "</td>" + b + "<td>" + esc(r.get_string("known_drm")) + "</td>";
+                const Value* hh = r.get("haplotype_hit");
+                for (size_t k = 0; k < nhi; ++k) {
+                    const bool hit = hh && k < hh->arr.size() && hh->arr[k].b;
+                    h += hit ? "<td class=\"hap\" style=\"background:" + std::string(palette[k % 10]) + "\"></td>" : "<td class=\"hap\"></td>";
+                }
+                h += "</tr>\n";
             }
             h += "</table>";
         }
