@@ -304,6 +304,38 @@ int ms_linkage(ms_handle *h, const ms_linkage_params *prm, ms_linkage_pair *out,
  * Owned by the handle; same caching and collective rule as ms_linkage.                                              */
 int ms_linkage_device(ms_handle *h, int32_t **d_gram, int32_t *dim);
 
+/* ---- sub-threshold variant linkage (restatement choice U21) ---------------------------------------
+ * A minor strain below K2's Bonferroni threshold still leaves its codons on the same reads.  Candidates are codons (s, c),
+ * c != the reference codon, of K2's positions with count >= min_reads and K2's uncorrected p < candidate_alpha that no gene
+ * calls (p * ntests >= alpha there, whatever min_perc / max_perc say).  One record per (s, c): the gene with the smallest p
+ * (ties: the lowest gene index).  At most MS_RARE_MAX_CANDIDATES are kept (smallest p, ties by (column, codon)).
+ * Phase the called keys followed by the candidates (ms_set_linkage(h, 1), ms_phase_begin, ms_phase_dev); ms_rare_linkage
+ * then tests the pairs (v, w), v < w, w >= first_candidate, |col_v - col_w| >= 3, n >= min_reads on the table of
+ * ms_linkage, with the linked tail only: linked iff p_together * m_r < alpha, m_r = the number of tested pairs.        */
+#define MS_RARE_MAX_CANDIDATES 2048
+typedef struct {
+    double candidate_alpha;    /* K2's uncorrected p must be below it (default 0.1) */
+    int32_t min_reads;         /* reads carrying the codon (default 5) */
+} ms_rare_params;
+void ms_rare_params_default(ms_rare_params *p);
+/* The candidates of the handle's (all-reduced) counts with K2's arguments, ordered by (column, codon).  *n receives their
+ * number (<= MS_RARE_MAX_CANDIDATES; may exceed cap: call again), *dropped how many the cap on candidates left out.     */
+int ms_rare_candidates(ms_handle *h, const ms_gene *genes, int32_t ngenes, const char *refseq, const ms_call_params *prm,
+                       const ms_rare_params *rp, ms_variant *out, int64_t cap, int64_t *n, int64_t *dropped);
+/* The linked pairs (relation MS_LINKED) of the phased keys with w >= first_candidate, ordered by v, then w; *n their number
+ * (may exceed cap), *ntested m_r.  Reads phased with ms_set_linkage(h, 1).  A collective when a communicator is attached
+ * (the Gram matrix of ms_linkage_device, all-reduced once per read set).                                              */
+int ms_rare_linkage(ms_handle *h, int32_t first_candidate, const ms_linkage_params *prm, ms_linkage_pair *out, int64_t cap,
+                    int64_t *n, int64_t *ntested);
+/* Key sets (G rows of ceil(V/32) words over the phased keys; bits >= V ignored, a row must not be empty): carriers[g] = reads
+ * with B = 1 at every key of row g, informative[g] = reads with M = 1 at every key.  Summed over the ranks in one all-reduce
+ * when a communicator is attached (a collective).                                                                      */
+int ms_rare_support(ms_handle *h, const uint32_t *masks, int64_t G, uint64_t *carriers, uint64_t *informative);
+/* Pure host logic: the connected components of the candidate-candidate pairs (v, w >= first_candidate) among pairs[0, npairs)
+ * with at least two members, numbered by their smallest key: group[k] = the component of key k, -1 for none (V entries).
+ * Returns the number of groups (>= 0) or MS_ERR_ARG.                                                                    */
+int ms_rare_groups(const ms_linkage_pair *pairs, int64_t npairs, int32_t first_candidate, int32_t V, int32_t *group);
+
 /* ---- haplotype abundance (restatement choice U18) ------------------------------------------------
  * Phasing counts a haplotype's reads among the reads that are clean at EVERY key; abundance also uses the damaged ones.
  * With B (read carries key v's codon) and M (key v's three columns are all A/C/G/T) as in linkage, read r is compatible

@@ -52,6 +52,10 @@ class LinkagePair(C.Structure):
                 ("neither", C.c_uint32), ("d_prime", C.c_double), ("r2", C.c_double), ("pvalue", C.c_double), ("relation", C.c_int32)]
 
 
+class RareParams(C.Structure):
+    _fields_ = [("candidate_alpha", C.c_double), ("min_reads", C.c_int32)]
+
+
 class AbundanceParams(C.Structure):
     _fields_ = [("tolerance", C.c_double), ("max_iterations", C.c_int32)]
 
@@ -189,6 +193,13 @@ _SIGNATURES = {
     "ms_indel_call": (C.c_int, [_P, C.POINTER(Gene), C.c_int32, C.c_char_p, C.POINTER(IndelParams), C.POINTER(Indel), C.c_int64,
                                 C.POINTER(C.c_int64)]),
     "ms_phase_begin_indels": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int64]),
+    "ms_rare_params_default": (None, [C.POINTER(RareParams)]),
+    "ms_rare_candidates": (C.c_int, [_P, C.POINTER(Gene), C.c_int32, C.c_char_p, C.POINTER(CallParams), C.POINTER(RareParams),
+                                     C.POINTER(Variant), C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "ms_rare_linkage": (C.c_int, [_P, C.c_int32, C.POINTER(LinkageParams), C.POINTER(LinkagePair), C.c_int64, C.POINTER(C.c_int64),
+                                  C.POINTER(C.c_int64)]),
+    "ms_rare_support": (C.c_int, [_P, _P, C.c_int64, _P, _P]),
+    "ms_rare_groups": (C.c_int, [C.POINTER(LinkagePair), C.c_int64, C.c_int32, C.c_int32, _P]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -13,7 +13,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _lib
-from ._lib import (AbundanceCounters, AbundanceParams, AbundanceRow, AlignParams, CallParams, FuseParams, Gene, Indel, IndelParams, LinkagePair, LinkageParams, PhaseCounters, ReadAlignment, SynthParams, Variant,
+from ._lib import (AbundanceCounters, AbundanceParams, AbundanceRow, AlignParams, CallParams, FuseParams, Gene, Indel, IndelParams, LinkagePair, LinkageParams, PhaseCounters, RareParams, ReadAlignment, SynthParams, Variant,
                    check)
 from .synth import start_mask_words, tile_rows, untile_rows
 
@@ -116,6 +116,32 @@ class Indels:
     tally: np.ndarray
     strings: list
     string_col: np.ndarray
+
+
+@dataclass
+class RareLinkage:
+    """Sub-threshold variant linkage (Juliet.rare_linkage, restatement choice U21).  keys = the called keys, then the candidates
+    from index first_candidate on (candidates[i] is key first_candidate + i).  The linked pairs, ordered by v then w, as a
+    record array with the fields of ms_linkage_pair; tested = m_r; dropped = candidates beyond MS_RARE_MAX_CANDIDATES.  groups:
+    the connected components of the linked candidate-candidate pairs (lists of key indices, ordered by their smallest key),
+    with the reads carrying every member and the reads clean at every member."""
+    candidates: list
+    keys: list
+    first_candidate: int
+    pairs: np.ndarray
+    tested: int
+    dropped: int
+    groups: list
+    carriers: np.ndarray
+    informative: np.ndarray
+
+    @property
+    def frequency(self):
+        return np.where(self.informative > 0, self.carriers / np.maximum(self.informative, 1), 0.0)
+
+    def linked_called(self, k):
+        """the called keys linked to candidate key k"""
+        return sorted(int(v) for v, w in zip(self.pairs["v"], self.pairs["w"]) if w == k and v < self.first_candidate)
 
 
 def translate_dna(x: str) -> str:
@@ -460,6 +486,70 @@ class Juliet:
                          em_frequency=rec["em_frequency"].copy(), counters=counters, reads_used=counters["unique"] + counters["ambiguous"],
                          iterations=int(it.value), converged=bool(conv.value), log_likelihood=float(ll.value), tolerance=float(tol),
                          max_iterations=int(max_iter))
+
+    def rare_candidates(self, min_reads=5, candidate_alpha=0.1, cap=256):
+        """-> (candidates, dropped): K2's sub-threshold codons of the (all-reduced) counts (ms_rare_candidates)"""
+        rp = RareParams()
+        self.lib.ms_rare_params_default(C.byref(rp))
+        rp.min_reads, rp.candidate_alpha = int(min_reads), float(candidate_alpha)
+        genes = (Gene * max(1, len(self.genes)))(*[Gene(b, e) for (b, e) in self.genes])
+        ref = self.refseq.encode() if self.refseq else None
+        n, dropped = C.c_int64(), C.c_int64()
+        while True:
+            out = (Variant * max(1, cap))()
+            check(self.lib.ms_rare_candidates(self.hd.h, genes, len(self.genes), ref, C.byref(self.params), C.byref(rp), out, cap, C.byref(n),
+                                              C.byref(dropped)), self.hd.h)
+            if n.value <= cap:
+                break
+            cap = int(n.value)
+        return [Variant.from_buffer_copy(out[i]) for i in range(n.value)], int(dropped.value)
+
+    def rare_linkage(self, d_packed_ptr: int, nreads: int, variants=None, min_reads=5, candidate_alpha=0.1, alpha=None,
+                     link_min_reads=10, cap=1024) -> RareLinkage:
+        """Sub-threshold variant linkage (restatement choice U21) of this rank's reads (device tiles; the counts must be the
+        all-reduced ones of the same reads).  variants: the reported calls (None = Juliet.call()).  The keys are phased anew
+        with the clean-codon matrix, which replaces the handle's phasing state: run it after whatever uses that state.  With
+        several ranks the handle needs its own communicator (Handle.attach_comm); every rank calls it."""
+        if not getattr(self.hd, "native_comm", False) and _torch_world() > 1:
+            raise _lib.MsError("rare linkage over several ranks needs the handle's own communicator (Handle.attach_comm)")
+        if variants is None:
+            variants = self.call()
+        called = sorted({(v.col, v.codon) for v in variants})
+        cands, dropped = self.rare_candidates(min_reads, candidate_alpha)
+        keys = called + [(c.col, c.codon) for c in cands]
+        V, fc = len(keys), len(called)
+        vc = np.array([k[0] for k in keys], dtype=np.int32)
+        vd = np.array([k[1] for k in keys], dtype=np.int32)
+        check(self.lib.ms_set_linkage(self.hd.h, 1), self.hd.h)
+        check(self.lib.ms_phase_begin(self.hd.h, _ptr(vc), _ptr(vd), V, nreads), self.hd.h)
+        check(self.lib.ms_phase_dev(self.hd.h, C.c_void_p(d_packed_ptr), nreads), self.hd.h)
+        self._V, self._keys, self._reported, self._nreported = V, list(keys), None, None
+        p = LinkageParams()
+        self.lib.ms_linkage_params_default(C.byref(p))
+        p.alpha = self.params.alpha if alpha is None else float(alpha)
+        p.min_reads = int(link_min_reads)
+        n, m = C.c_int64(), C.c_int64()
+        while True:
+            out = (LinkagePair * max(1, cap))()
+            check(self.lib.ms_rare_linkage(self.hd.h, fc, C.byref(p), out, cap, C.byref(n), C.byref(m)), self.hd.h)
+            if n.value <= cap:
+                break
+            cap = int(n.value)
+        pairs = np.ctypeslib.as_array(out)[: n.value].copy()
+        group = np.full(max(1, V), -1, dtype=np.int32)
+        ng = self.lib.ms_rare_groups(out, n.value, fc, V, _ptr(group))
+        if ng < 0:
+            raise _lib.MsError(f"ms_rare_groups failed ({ng})")
+        groups = [np.nonzero(group[:V] == g)[0].tolist() for g in range(ng)]
+        nw = max(1, (V + 31) // 32)
+        masks = np.zeros((max(1, ng), nw), dtype=np.uint32)
+        for g, mem in enumerate(groups):
+            for k in mem:
+                masks[g, k >> 5] |= np.uint32(1 << (k & 31))
+        car, inf = np.zeros(max(1, ng), dtype=np.uint64), np.zeros(max(1, ng), dtype=np.uint64)
+        check(self.lib.ms_rare_support(self.hd.h, _ptr(masks), ng, _ptr(car), _ptr(inf)), self.hd.h)
+        return RareLinkage(candidates=cands, keys=keys, first_candidate=fc, pairs=pairs, tested=int(m.value), dropped=dropped,
+                           groups=groups, carriers=car[:ng].copy(), informative=inf[:ng].copy())
 
     # -- in-frame indels (restatement choice U19)
     def indels(self, d_packed_ptr: int, nreads: int, insertions=None, read0=0, deletion_rate=None, insertion_rate=3e-3,

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libminorseq_b200.so")
-SOURCES = ["abi_core.cu", "pileup.cu", "format.cu", "synth.cu", "call.cu", "phase.cu", "phase_order.cu", "cooc_tc.cu", "fuse.cu", "comm.cu", "pass.cu", "nw.cu", "events.cu", "tiles.cu", "linkage.cu", "group.cu", "align.cu", "abundance.cu", "indel.cu", "phase_indel.cu"]
+SOURCES = ["abi_core.cu", "pileup.cu", "format.cu", "synth.cu", "call.cu", "phase.cu", "phase_order.cu", "cooc_tc.cu", "fuse.cu", "comm.cu", "pass.cu", "nw.cu", "events.cu", "tiles.cu", "linkage.cu", "group.cu", "align.cu", "abundance.cu", "indel.cu", "phase_indel.cu", "rare.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-fmad=false",  # K2's fp64 path must not contract a*b+c (fisher_core.h)

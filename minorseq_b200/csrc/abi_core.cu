@@ -123,7 +123,8 @@ void ms_destroy(ms_handle* h) {
     cudaEventDestroy(h->ev_k1[0]); cudaEventDestroy(h->ev_k1[1]);
     cudaEventDestroy(h->ev_timer[0]); cudaEventDestroy(h->ev_timer[1]);
     for (DevBuf* b : {&h->b_ab_pat, &h->b_ab_mask, &h->b_ab_flag, &h->b_ab_slot, &h->b_ab_tab_key, &h->b_ab_tab_cnt, &h->b_ab_tab_rep, &h->b_ab_ctr,
-                      &h->b_ab_blk, &h->b_ab_out, &h->b_ab_em, &h->b_indel_cnt, &h->b_indel_ev, &h->b_indel_out})
+                      &h->b_ab_blk, &h->b_ab_out, &h->b_ab_em, &h->b_indel_cnt, &h->b_indel_ev, &h->b_indel_out,
+                      &h->b_rare_pos, &h->b_rare_out, &h->b_rare_pairs, &h->b_rare_sup})
         b->release();
     for (int s = 1; s < 16; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
     cudaStreamDestroy(h->own_stream); cudaStreamDestroy(h->copy_stream);

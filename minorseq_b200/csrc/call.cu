@@ -80,6 +80,71 @@ __global__ void call_kernel(const uint32_t* __restrict__ codon, const CallPos* _
     }
 }
 
+// Sub-threshold candidates (restatement choice U21): K2's test on call_kernel's position table, one warp per position.  The tail
+// only has to be exact below max(alpha / ntests, candidate_alpha): below alpha / ntests it decides K2's call exactly as K2 does,
+// below candidate_alpha it is the candidate's p.  Every codon with count >= min_reads that K2 calls, or whose p is below
+// candidate_alpha, is written with its call flag: a (column, codon) called in one gene is no candidate in any, which the host
+// decides after all genes are in.
+struct RareRec {
+    ms_variant v;
+    int32_t called, pad;
+};
+
+struct RareConst {
+    double P[4];
+    double alpha, candidate_alpha;
+    uint32_t min_reads;
+};
+
+__global__ void rare_candidate_kernel(const uint32_t* __restrict__ codon, const CallPos* __restrict__ pos, int32_t npos, RareConst rc,
+                                      RareRec* __restrict__ out, unsigned long long* __restrict__ nout, unsigned long long cap) {
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (warp >= npos) return;
+    const CallPos ps = pos[warp];
+    const uint32_t* h = codon + static_cast<size_t>(ps.col) * 64;
+    const uint32_t k0 = h[lane], k1 = h[lane + 32];
+    uint32_t n = k0 + k1;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+    if (n == 0) return;
+    int ref = ps.ref_codon;
+    if (ref < 0) {
+        uint32_t bc = k0, bi = lane;
+        if (k1 > bc) { bc = k1; bi = lane + 32; }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const uint32_t oc = __shfl_xor_sync(0xffffffffu, bc, o), oi = __shfl_xor_sync(0xffffffffu, bi, o);
+            if (oc > bc || (oc == bc && oi < bi)) { bc = oc; bi = oi; }
+        }
+        ref = static_cast<int>(bi);
+    }
+    const double nt = static_cast<double>(ps.ntests);
+    const double bound = fmax(rc.alpha / nt, rc.candidate_alpha);
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {
+        const int c = lane + 32 * half;
+        const uint32_t k = half ? k1 : k0;
+        if (c == ref || k < rc.min_reads) continue;
+        int nm = 0;
+#pragma unroll
+        for (int i = 0; i < 3; ++i) nm += (((ref >> (2 * i)) & 3) != ((c >> (2 * i)) & 3)) ? 1 : 0;
+        const double ex = ceil(static_cast<double>(n) * rc.P[nm]);
+        const uint32_t e = ex >= static_cast<double>(n) ? n : static_cast<uint32_t>(ex);
+        if (k <= e && 0.5 >= bound) continue;    // p >= 1/2 (call_kernel): neither called nor a candidate
+        const double p = fisher_upper(k, n - k, e, n - e, 1.000001 * bound);
+        const bool called = p * nt < rc.alpha;
+        if (!called && !(p < rc.candidate_alpha)) continue;
+        const unsigned long long slot = atomicAdd(nout, 1ULL);
+        if (slot < cap) {
+            RareRec r;
+            r.v.gene = ps.gene; r.v.codon_index = ps.codon_index; r.v.col = ps.col; r.v.ref_codon = ref; r.v.codon = c;
+            r.v.count = k; r.v.coverage = n; r.v.expected = e; r.v.ntests = ps.ntests; r.v.pvalue = p;
+            r.called = called ? 1 : 0; r.pad = 0;
+            out[slot] = r;
+        }
+    }
+}
+
 static int base_code(char ch) {
     switch (ch) {
     case 'A': case 'a': return 0;
@@ -88,6 +153,38 @@ static int base_code(char ch) {
     case 'T': case 't': return 3;
     default: return -1;
     }
+}
+
+// K2's position table: every tested codon start of every gene (inside --region), its reference codon and the gene's ntests
+int call_positions(ms_handle* h, const ms_gene* genes, int32_t ngenes, const char* refseq, const ms_call_params* prm,
+                   std::vector<CallPos>& pos) {
+    const int32_t L = h->L;
+    const size_t reflen = refseq ? strnlen(refseq, static_cast<size_t>(L)) : 0;
+    int32_t lo = 0, hi = L;
+    if (prm->region_end > prm->region_begin) {
+        lo = std::max(0, prm->region_begin - 1);
+        hi = std::min(L, prm->region_end - 1);
+    }
+    pos.clear();
+    for (int32_t g = 0; g < ngenes; ++g) {
+        const int32_t gb = genes[g].begin - 1, ge = std::min(genes[g].end - 1, L);
+        const size_t first = pos.size();
+        for (int32_t s = gb, ci = 0; s + 3 <= ge; s += 3, ++ci) {
+            if (!(s >= lo && s + 3 <= hi && s >= 0)) continue;
+            if (!((h->h_start[s >> 5] >> (s & 31)) & 1u))
+                MS_FAIL(h, MS_ERR_ARG, "gene codon start not in the layout's start mask");
+            CallPos p;
+            p.gene = g; p.codon_index = ci; p.col = s; p.ref_codon = -1; p.ntests = 0;
+            if (static_cast<size_t>(s) + 3 <= reflen) {
+                const int b0 = base_code(refseq[s]), b1 = base_code(refseq[s + 1]), b2 = base_code(refseq[s + 2]);
+                if (b0 >= 0 && b1 >= 0 && b2 >= 0) p.ref_codon = 16 * b0 + 4 * b1 + b2;
+            }
+            pos.push_back(p);
+        }
+        const uint32_t nt = static_cast<uint32_t>(pos.size() - first);
+        for (size_t i = first; i < pos.size(); ++i) pos[i].ntests = nt;
+    }
+    return MS_OK;
 }
 
 }  // namespace ms
@@ -111,31 +208,9 @@ int ms_call_launch(ms_handle* h, const ms_gene* genes, int32_t ngenes, const cha
     if (!h->count_codons) MS_FAIL(h, MS_ERR_ARG, "ms_set_layout was called without a codon start mask");
     MS_CUDA(h, cudaSetDevice(h->device));
     const int32_t L = h->L;
-    const size_t reflen = refseq ? strnlen(refseq, static_cast<size_t>(L)) : 0;
-    int32_t lo = 0, hi = L;
-    if (prm->region_end > prm->region_begin) {
-        lo = std::max(0, prm->region_begin - 1);
-        hi = std::min(L, prm->region_end - 1);
-    }
     std::vector<ms::CallPos> pos;
-    for (int32_t g = 0; g < ngenes; ++g) {
-        const int32_t gb = genes[g].begin - 1, ge = std::min(genes[g].end - 1, L);
-        const size_t first = pos.size();
-        for (int32_t s = gb, ci = 0; s + 3 <= ge; s += 3, ++ci) {
-            if (!(s >= lo && s + 3 <= hi && s >= 0)) continue;
-            if (!((h->h_start[s >> 5] >> (s & 31)) & 1u))
-                MS_FAIL(h, MS_ERR_ARG, "gene codon start not in the layout's start mask");
-            ms::CallPos p;
-            p.gene = g; p.codon_index = ci; p.col = s; p.ref_codon = -1; p.ntests = 0;
-            if (static_cast<size_t>(s) + 3 <= reflen) {
-                const int b0 = ms::base_code(refseq[s]), b1 = ms::base_code(refseq[s + 1]), b2 = ms::base_code(refseq[s + 2]);
-                if (b0 >= 0 && b1 >= 0 && b2 >= 0) p.ref_codon = 16 * b0 + 4 * b1 + b2;
-            }
-            pos.push_back(p);
-        }
-        const uint32_t nt = static_cast<uint32_t>(pos.size() - first);
-        for (size_t i = first; i < pos.size(); ++i) pos[i].ntests = nt;
-    }
+    const int prc = ms::call_positions(h, genes, ngenes, refseq, prm, pos);
+    if (prc != MS_OK) return prc;
     h->call_npos = pos.size();
     if (d_calls) *d_calls = nullptr;
     if (d_ncalls) *d_ncalls = nullptr;
@@ -230,6 +305,92 @@ int ms_call(ms_handle* h, const ms_gene* genes, int32_t ngenes, const char* refs
     int rc = ms_call_launch(h, genes, ngenes, refseq, prm, nullptr, nullptr, nullptr);
     if (rc != MS_OK) return rc;
     return ms_call_collect(h, false, out, cap, n);
+}
+
+}  // extern "C"
+
+extern "C" {
+
+void ms_rare_params_default(ms_rare_params* p) {
+    if (!p) return;
+    p->candidate_alpha = 0.1;
+    p->min_reads = 5;
+}
+
+int ms_rare_candidates(ms_handle* h, const ms_gene* genes, int32_t ngenes, const char* refseq, const ms_call_params* prm,
+                       const ms_rare_params* rp, ms_variant* out, int64_t cap, int64_t* n, int64_t* dropped) {
+    MsRange nvtx_range("rare candidates");
+    if (!h || !h->d_counts || !genes || ngenes < 0 || !prm || !rp || !n || cap < 0 || (cap > 0 && !out)) return MS_ERR_ARG;
+    if (rp->min_reads < 1 || !(rp->candidate_alpha > 0.0) || !(prm->alpha > 0.0)) MS_FAIL(h, MS_ERR_ARG, "ms_rare_candidates: bad parameters");
+    if (!h->count_codons) MS_FAIL(h, MS_ERR_ARG, "ms_set_layout was called without a codon start mask");
+    MS_CUDA(h, cudaSetDevice(h->device));
+    *n = 0;
+    if (dropped) *dropped = 0;
+    std::vector<ms::CallPos> pos;
+    int rc = ms::call_positions(h, genes, ngenes, refseq, prm, pos);
+    if (rc != MS_OK) return rc;
+    if (pos.empty()) return MS_OK;
+    const size_t npos = pos.size();
+    MS_CUDA(h, h->b_rare_pos.ensure(npos * sizeof(ms::CallPos)));
+    MS_CUDA(h, cudaMemcpyAsync(h->b_rare_pos.p, pos.data(), npos * sizeof(ms::CallPos), cudaMemcpyHostToDevice, h->stream));
+    ms::RareConst cc;
+    ms::codon_error_table(prm->substitution_rate, prm->deletion_rate, cc.P);
+    cc.alpha = prm->alpha; cc.candidate_alpha = rp->candidate_alpha; cc.min_reads = static_cast<uint32_t>(rp->min_reads);
+    // the records are few (codons seen min_reads times with a small p); the buffer grows and the kernel runs again if not
+    size_t dev_cap = std::min<size_t>(npos * 63, 1 << 16);
+    unsigned long long cnt = 0;
+    for (;;) {
+        MS_CUDA(h, h->b_rare_out.ensure(64 + dev_cap * sizeof(ms::RareRec)));
+        unsigned long long* d_n = h->b_rare_out.as<unsigned long long>();
+        MS_CUDA(h, cudaMemsetAsync(d_n, 0, 8, h->stream));
+        const int threads = 128;
+        const int blocks = static_cast<int>((npos * 32 + threads - 1) / threads);
+        ms::rare_candidate_kernel<<<blocks, threads, 0, h->stream>>>(h->d_counts + static_cast<size_t>(h->L) * 8, h->b_rare_pos.as<ms::CallPos>(),
+                                                                     static_cast<int32_t>(npos), cc,
+                                                                     reinterpret_cast<ms::RareRec*>(h->b_rare_out.as<uint8_t>() + 64), d_n, dev_cap);
+        h->launches++;
+        MS_CUDA(h, cudaGetLastError());
+        MS_CUDA(h, cudaMemcpyAsync(&cnt, d_n, 8, cudaMemcpyDeviceToHost, h->stream));
+        MS_CUDA(h, cudaStreamSynchronize(h->stream));
+        if (cnt <= dev_cap) break;
+        dev_cap = static_cast<size_t>(cnt);
+    }
+    std::vector<ms::RareRec> rec(cnt);
+    if (cnt) {
+        MS_CUDA(h, cudaMemcpyAsync(rec.data(), h->b_rare_out.as<uint8_t>() + 64, cnt * sizeof(ms::RareRec), cudaMemcpyDeviceToHost, h->stream));
+        MS_CUDA(h, cudaStreamSynchronize(h->stream));
+    }
+    std::sort(rec.begin(), rec.end(), [](const ms::RareRec& a, const ms::RareRec& b) {
+        if (a.v.col != b.v.col) return a.v.col < b.v.col;
+        if (a.v.codon != b.v.codon) return a.v.codon < b.v.codon;
+        return a.v.gene < b.v.gene;
+    });
+    // one record per (column, codon) that no gene calls: the gene with the smallest p, the lowest gene index on ties
+    std::vector<ms_variant> cand;
+    for (size_t i = 0; i < rec.size();) {
+        size_t j = i;
+        bool called = false;
+        size_t best = i;
+        for (; j < rec.size() && rec[j].v.col == rec[i].v.col && rec[j].v.codon == rec[i].v.codon; ++j) {
+            called = called || rec[j].called;
+            if (rec[j].v.pvalue < rec[best].v.pvalue) best = j;
+        }
+        if (!called) cand.push_back(rec[best].v);
+        i = j;
+    }
+    const auto by_col = [](const ms_variant& a, const ms_variant& b) { return a.col != b.col ? a.col < b.col : a.codon < b.codon; };
+    if (cand.size() > MS_RARE_MAX_CANDIDATES) {
+        std::sort(cand.begin(), cand.end(), [&](const ms_variant& a, const ms_variant& b) {
+            if (a.pvalue != b.pvalue) return a.pvalue < b.pvalue;
+            return by_col(a, b);
+        });
+        if (dropped) *dropped = static_cast<int64_t>(cand.size()) - MS_RARE_MAX_CANDIDATES;
+        cand.resize(MS_RARE_MAX_CANDIDATES);
+        std::sort(cand.begin(), cand.end(), by_col);
+    }
+    *n = static_cast<int64_t>(cand.size());
+    for (int64_t i = 0; i < std::min<int64_t>(cap, *n); ++i) out[i] = cand[i];
+    return MS_OK;
 }
 
 }  // extern "C"

@@ -157,6 +157,9 @@ struct ms_handle {
     std::vector<int32_t> indel_col;       // per string id: its column ...
     std::vector<std::string> indel_str;   // ... and its upper-cased string
     DevBuf b_indel_cnt, b_indel_ev, b_indel_out;
+    // sub-threshold linkage (call.cu, rare.cu): the candidate kernel's position table and records, the linked pairs, the group
+    // support scratch (masks | counters)
+    DevBuf b_rare_pos, b_rare_out, b_rare_pairs, b_rare_sup;
 
     DevBuf b_aln_ref, b_aln_idx, b_aln_seq, b_aln_off, b_aln_seed, b_aln_scratch, b_aln_slab, b_aln_mbits, b_aln_cig, b_aln_res, b_aln_ctr,
         b_aln_dst, b_aln_pack;

@@ -16,6 +16,7 @@
 // The order (v ascending, then w) and every value depend on the integer counts only: the same bytes on every run and rank.
 #include <algorithm>
 #include <vector>
+#include "link_table.cuh"
 #include "linkage_core.h"
 #include "phase_internal.cuh"
 
@@ -25,19 +26,6 @@ int ms_comm_allreduce_i32(ms_handle* h, int32_t* d, size_t count);
 namespace ms {
 
 constexpr int kLinkThreads = 128;
-
-struct LinkTable { uint32_t a, b, c, n; };
-
-// the 2x2 table of pair (v, w) from the stacked Gram matrix (dim x dim, half = dim / 2)
-__device__ __forceinline__ LinkTable link_table(const int32_t* __restrict__ G, int32_t dim, int32_t v, int32_t w) {
-    const int32_t half = dim >> 1;
-    LinkTable t;
-    t.a = static_cast<uint32_t>(G[static_cast<size_t>(v) * dim + w]);
-    t.n = static_cast<uint32_t>(G[static_cast<size_t>(half + v) * dim + half + w]);
-    t.b = static_cast<uint32_t>(G[static_cast<size_t>(v) * dim + half + w]) - t.a;     // B_v . M_w - a
-    t.c = static_cast<uint32_t>(G[static_cast<size_t>(w) * dim + half + v]) - t.a;     // M_v . B_w - a
-    return t;
-}
 
 __device__ __forceinline__ bool link_tested(const int32_t* __restrict__ col, const LinkTable& t, int32_t v, int32_t w, int32_t min_reads) {
     const int32_t dc = col[v] - col[w];

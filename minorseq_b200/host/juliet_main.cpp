@@ -11,6 +11,8 @@
 // estimates their frequencies by EM over the reads' compatibility sets.  --indels (restatement choice U19) tests in-frame codon
 // deletions and insertions between codons with K2's model and reports them in an "indels" block.  --phase-indels (restatement
 // choice U20) adds the reported indels to the phasing keys: haplotypes, linkage, abundance and the FASTA then see them.
+// --rare-linkage (restatement choice U21) looks for minor strains below K2's threshold: codons that K2 does not call but whose
+// uncorrected p is small, tested for linkage to each other and to the called variants on the reads clean at both codons.
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -45,6 +47,10 @@ static void usage() {
          "                                     (\"indels\"; DRM tokens such as 69ins, T69ins, 67del, D67del)\n"
          "      --phase-indels                 with --mode-phasing and --indels: phase the reported indels with the variants\n"
          "                                     (haplotypes, linkage, abundance and the .fasta carry them)\n"
+         "      --rare-linkage                 sub-threshold variant linkage: uncalled codons with a small uncorrected p, tested\n"
+         "                                     for linkage over the reads; linked groups and their reads (\"rare_linkage\")\n"
+         "      --rare-min-reads <n>           reads a --rare-linkage candidate needs (default 5)\n"
+         "      --rare-candidate-alpha <a>     uncorrected p a --rare-linkage candidate needs to stay below (default 0.1)\n"
          "      --min-perc <p>                 only variants with abundance > p %\n"
          "      --max-perc <p>                 only variants with abundance < p %\n"
          "      --drm-only                     only known drug-resistance mutations\n"
@@ -74,9 +80,9 @@ static bool ends_with(const std::string& s, const std::string& e) { return s.siz
 
 int main(int argc, char** argv) {
     std::string config, region, cmdline, timing_json;
-    bool phasing = false, drm_only = false, linkage = false, abundance = false, indels = false, phase_indels = false;
-    double min_perc = -1, max_perc = -1, sub = 5e-4, del = 3e-3, alpha = 0.01, ins_rate = 3e-3;
-    int min_hap = 10, device = 0, ngpus = 1, hap_min_cov = 10;
+    bool phasing = false, drm_only = false, linkage = false, abundance = false, indels = false, phase_indels = false, rare_linkage = false;
+    double min_perc = -1, max_perc = -1, sub = 5e-4, del = 3e-3, alpha = 0.01, ins_rate = 3e-3, rare_alpha = 0.1;
+    int min_hap = 10, device = 0, ngpus = 1, hap_min_cov = 10, rare_min_reads = 5;
     const int link_min_reads = 10;   // reads clean at both codons that a tested pair needs (the haplotype default, F21)
     mshost::QvFilter qv;
     std::vector<std::string> pos;
@@ -96,6 +102,9 @@ int main(int argc, char** argv) {
         else if (a == "--haplotype-abundance") abundance = true;
         else if (a == "--indels") indels = true;
         else if (a == "--phase-indels") phase_indels = true;
+        else if (a == "--rare-linkage") rare_linkage = true;
+        else if (a == "--rare-min-reads") rare_min_reads = atoi(need("--rare-min-reads").c_str());
+        else if (a == "--rare-candidate-alpha") rare_alpha = atof(need("--rare-candidate-alpha").c_str());
         else if (a == "--insertion-rate") ins_rate = atof(need("--insertion-rate").c_str());
         else if (a == "--drm-only") drm_only = true;
         else if (a == "--min-perc") min_perc = atof(need("--min-perc").c_str());
@@ -126,6 +135,8 @@ int main(int argc, char** argv) {
     if (abundance && !phasing) mshost::die("--haplotype-abundance fits the reads to the reported haplotypes: it needs --mode-phasing");
     if (phase_indels && (!phasing || !indels))
         mshost::die("--phase-indels puts the reported indels into the haplotypes: it needs --mode-phasing and --indels");
+    if (rare_min_reads < 1) mshost::die("--rare-min-reads expects a count >= 1");
+    if (!(rare_alpha > 0.0 && rare_alpha <= 1.0)) mshost::die("--rare-candidate-alpha expects a value in (0, 1]");
     int rb = 0, re = 0;
     if (!region.empty()) {
         if (sscanf(region.c_str(), "%d-%d", &rb, &re) != 2 || rb < 1 || re <= rb) mshost::die("--region expects <begin-end>");
@@ -578,6 +589,138 @@ int main(int argc, char** argv) {
             }
             lap("haplotype consensus");
         }
+        // sub-threshold linkage: every rank phases the called keys and the candidates anew (the handle's phasing state is no longer
+        // needed by the steps above) and takes the same turns through the collectives: the Gram all-reduce, the support all-reduce
+        msreport::RareBlock rare;
+        if (rare_linkage) {
+            std::vector<std::pair<int, int>> called;
+            for (const msreport::VariantRow& vr : rows) called.emplace_back(vr.col, vr.codon);
+            std::sort(called.begin(), called.end());
+            called.erase(std::unique(called.begin(), called.end()), called.end());
+            const int32_t fc = static_cast<int32_t>(called.size());
+            ms_rare_params rp;
+            ms_rare_params_default(&rp);
+            rp.min_reads = rare_min_reads;
+            rp.candidate_alpha = rare_alpha;
+            ms_linkage_params lp;
+            ms_linkage_params_default(&lp);
+            lp.alpha = alpha;
+            lp.min_reads = link_min_reads;
+            std::vector<ms_variant> cands;
+            std::vector<ms_linkage_pair> rpairs;
+            std::vector<int32_t> rgroup;
+            std::vector<uint64_t> rcar, rinf;
+            int64_t rdropped = 0, rtested = 0;
+            mshost::run_ranks(ngpus, [&](int r) {
+                ms_handle* h = hs[r];
+                const int64_t r0 = aln.nreads * r / ngpus, r1 = aln.nreads * (r + 1) / ngpus;
+                std::vector<ms_variant> my_c(256);
+                int64_t nc = 0, dropped = 0;
+                for (;;) {
+                    CKR(ms_rare_candidates(h, mg.data(), static_cast<int32_t>(mg.size()), ref, &prm, &rp, my_c.data(), static_cast<int64_t>(my_c.size()), &nc,
+                                           &dropped));
+                    if (nc <= static_cast<int64_t>(my_c.size())) break;
+                    my_c.resize(nc);
+                }
+                my_c.resize(nc);
+                const int32_t V = fc + static_cast<int32_t>(nc);
+                std::vector<int32_t> vc(V), vk(V);
+                for (int32_t i = 0; i < fc; ++i) { vc[i] = called[i].first; vk[i] = called[i].second; }
+                for (int32_t i = 0; i < nc; ++i) { vc[fc + i] = my_c[i].col; vk[fc + i] = my_c[i].codon; }
+                CKR(ms_set_linkage(h, 1));
+                CKR(ms_phase_begin(h, vc.data(), vk.data(), V, r1 - r0));
+                CKR(ms_phase_dev(h, rows_dev[r], r1 - r0));
+                std::vector<ms_linkage_pair> my_p(64);
+                int64_t np = 0, nt = 0;
+                for (;;) {
+                    CKR(ms_rare_linkage(h, fc, &lp, my_p.data(), static_cast<int64_t>(my_p.size()), &np, &nt));
+                    if (np <= static_cast<int64_t>(my_p.size())) break;
+                    my_p.resize(np);
+                }
+                my_p.resize(np);
+                std::vector<int32_t> grp(static_cast<size_t>(std::max(1, V)), -1);
+                const int ng = ms_rare_groups(my_p.data(), np, fc, V, grp.data());
+                if (ng < 0) { errs[r] = "ms_rare_groups failed"; return; }
+                const int32_t nw = std::max(1, (V + 31) / 32);
+                std::vector<uint32_t> masks(static_cast<size_t>(std::max(1, ng)) * nw, 0u);
+                for (int32_t k = 0; k < V; ++k)
+                    if (grp[k] >= 0) masks[static_cast<size_t>(grp[k]) * nw + (k >> 5)] |= 1u << (k & 31);
+                std::vector<uint64_t> car(static_cast<size_t>(std::max(1, ng))), inf(car.size());
+                CKR(ms_rare_support(h, masks.data(), ng, car.data(), inf.data()));
+                if (r == 0) {
+                    cands.swap(my_c); rpairs.swap(my_p); rgroup.swap(grp); car.resize(ng); inf.resize(ng); rcar.swap(car); rinf.swap(inf);
+                    rdropped = dropped; rtested = nt;
+                }
+            });
+            for (const std::string& e : errs)
+                if (!e.empty()) mshost::die(e);
+            rare.min_reads = rare_min_reads;
+            rare.candidate_alpha = rare_alpha;
+            rare.alpha = alpha;
+            rare.pair_min_reads = link_min_reads;
+            rare.max_candidates = MS_RARE_MAX_CANDIDATES;
+            rare.candidates_tested = static_cast<long long>(cands.size());
+            rare.dropped_candidates = rdropped;
+            rare.tested_pairs = rtested;
+            auto cand_label = [&](const ms_variant& c) {
+                return std::string(1, mscfg::translate(c.ref_codon)) + std::to_string(c.codon_index + 1) + mscfg::translate(c.codon);
+            };
+            auto key_variant = [&](int32_t k) {
+                msreport::LinkageVariant o;
+                char cb[4];
+                if (k >= fc) {
+                    const ms_variant& c = cands[k - fc];
+                    o.abs_pos = c.col + 1;
+                    o.codon = mscfg::codon_string(c.codon, cb);
+                    o.labels.push_back(genes[c.gene].name + " " + cand_label(c));
+                    return o;
+                }
+                o.abs_pos = called[k].first + 1;
+                o.codon = mscfg::codon_string(called[k].second, cb);
+                for (const msreport::VariantRow& vr : rows)
+                    if (vr.col == called[k].first && vr.codon == called[k].second)
+                        o.labels.push_back(genes[vr.gene].name + " " + mscfg::translate(vr.ref_codon) + std::to_string(vr.aa_pos) + mscfg::translate(vr.codon));
+                return o;
+            };
+            std::vector<std::vector<std::string>> linked_called(cands.size());
+            std::vector<char> in_pair(cands.size(), 0);
+            for (const ms_linkage_pair& p : rpairs) {
+                msreport::LinkageRow lr;
+                lr.a = key_variant(p.v);
+                lr.b = key_variant(p.w);
+                lr.reads = static_cast<unsigned long long>(p.both) + p.v_only + p.w_only + p.neither;
+                lr.both = p.both; lr.a_only = p.v_only; lr.b_only = p.w_only; lr.neither = p.neither;
+                lr.d_prime = p.d_prime; lr.r2 = p.r2; lr.pvalue = p.pvalue;
+                lr.pvalue_corrected = std::min(1.0, p.pvalue * static_cast<double>(rtested));
+                lr.relation = "linked";
+                rare.pairs.push_back(lr);
+                in_pair[p.w - fc] = 1;
+                if (p.v >= fc) in_pair[p.v - fc] = 1;
+                else for (const std::string& l : lr.a.labels) linked_called[p.w - fc].push_back(l);
+            }
+            rare.groups.resize(rcar.size());
+            for (size_t g = 0; g < rcar.size(); ++g) { rare.groups[g].carriers = rcar[g]; rare.groups[g].informative = rinf[g]; }
+            for (size_t i = 0; i < cands.size(); ++i) {
+                const ms_variant& c = cands[i];
+                const int32_t g = rgroup[fc + i];
+                if (g >= 0) rare.groups[g].members.push_back(genes[c.gene].name + " " + cand_label(c));
+                if (!in_pair[i]) continue;
+                msreport::RareCandidate rc;
+                char cb[4];
+                rc.gene = genes[c.gene].name;
+                rc.label = cand_label(c);
+                rc.position = c.codon_index + 1;
+                rc.abs_pos = c.col + 1;
+                rc.ref_codon = mscfg::codon_string(c.ref_codon, cb);
+                rc.codon = mscfg::codon_string(c.codon, cb);
+                rc.count = c.count; rc.coverage = c.coverage; rc.expected = c.expected; rc.pvalue = c.pvalue;
+                rc.group = g;
+                rc.linked_called = linked_called[i];
+                rare.candidates.push_back(rc);
+            }
+            lap("rare linkage");
+        }
+
         char ts[40];
         const auto now = std::chrono::system_clock::now();
         const std::time_t tt = std::chrono::system_clock::to_time_t(now);
@@ -590,7 +733,8 @@ int main(int argc, char** argv) {
         if (getenv("MS_FIXED_TIMESTAMP")) snprintf(ts, sizeof ts, "%s", getenv("MS_FIXED_TIMESTAMP"));
 
         const msjson::Value report = msreport::build(ts, pos[0], cmdline, MS_VERSION, cfg, L, genes, rows, col, L, phasing, haps, counters,
-                                                     linkage ? &link : nullptr, abundance ? &ab : nullptr, indels ? &ind : nullptr, phase_indels);
+                                                     linkage ? &link : nullptr, abundance ? &ab : nullptr, indels ? &ind : nullptr, phase_indels,
+                                                     rare_linkage ? &rare : nullptr);
         if (!out_json.empty()) {
             std::ofstream f(out_json);
             if (!f) mshost::die("cannot write " + out_json);

@@ -57,6 +57,29 @@ struct LinkageBlock {
     std::vector<LinkageRow> pairs;
 };
 
+// sub-threshold variant linkage (--rare-linkage, restatement choice U21): K2's uncalled candidates, their linked pairs and groups
+struct RareCandidate {
+    std::string gene, label;          // label as a variant row's, e.g. "K103N"
+    int position = 0, abs_pos = 0;    // amino-acid position in the gene; 1-based first column
+    std::string ref_codon, codon;
+    unsigned long long count = 0, coverage = 0, expected = 0;
+    double pvalue = 0;
+    int group = -1;                   // index into RareBlock::groups, -1 = none
+    std::vector<std::string> linked_called;   // labels of the called variants it is linked to
+};
+struct RareGroup {
+    std::vector<std::string> members;         // "<gene> <label>" of each member
+    unsigned long long carriers = 0, informative = 0;
+};
+struct RareBlock {
+    int min_reads = 0, pair_min_reads = 0, max_candidates = 0;
+    double candidate_alpha = 0, alpha = 0;
+    long long candidates_tested = 0, dropped_candidates = 0, tested_pairs = 0;
+    std::vector<RareCandidate> candidates;    // those in at least one linked pair
+    std::vector<LinkageRow> pairs;
+    std::vector<RareGroup> groups;
+};
+
 // haplotype abundance (--haplotype-abundance, restatement choice U18): every phased read fitted to the reported haplotypes
 struct AbundanceRow {
     std::string name;
@@ -112,7 +135,7 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
                    const std::vector<VariantRow>& variants, const std::vector<unsigned>& col_counts /* L*8 */, int L,
                    bool phasing, const std::vector<HaplotypeRow>& haps, const unsigned long long counters[6],
                    const LinkageBlock* linkage = nullptr, const AbundanceBlock* abundance = nullptr, const IndelBlock* indels = nullptr,
-                   bool phase_indels = false) {
+                   bool phase_indels = false, const RareBlock* rare = nullptr) {
     Value root = Value::object();
     Value& in = root.set("input", Value::object());
     in.set("timestamp", Value::string(timestamp));
@@ -326,6 +349,67 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             o.set("em_percentage", Value::string(b));
         }
     }
+    if (rare) {
+        Value& rl = root.set("rare_linkage", Value::object());
+        rl.set("min_reads", Value::integer(rare->min_reads));
+        rl.set("candidate_alpha", Value::number(rare->candidate_alpha));
+        rl.set("alpha", Value::number(rare->alpha));
+        rl.set("pair_min_reads", Value::integer(rare->pair_min_reads));
+        rl.set("max_candidates", Value::integer(rare->max_candidates));
+        rl.set("candidates_tested", Value::integer(rare->candidates_tested));
+        rl.set("dropped_candidates", Value::integer(rare->dropped_candidates));
+        rl.set("tested_pairs", Value::integer(rare->tested_pairs));
+        Value& cs = rl.set("candidates", Value::array());
+        for (const RareCandidate& c : rare->candidates) {
+            Value& o = cs.push(Value::object());
+            o.set("gene", Value::string(c.gene));
+            o.set("label", Value::string(c.label));
+            o.set("position", Value::integer(c.position));
+            o.set("abs_pos", Value::integer(c.abs_pos));
+            o.set("ref_codon", Value::string(c.ref_codon));
+            o.set("codon", Value::string(c.codon));
+            o.set("count", Value::integer(static_cast<long long>(c.count)));
+            o.set("coverage", Value::integer(static_cast<long long>(c.coverage)));
+            o.set("expected", Value::integer(static_cast<long long>(c.expected)));
+            o.set("percentage", Value::string(perc2(c.coverage ? 100.0 * static_cast<double>(c.count) / static_cast<double>(c.coverage) : 0.0)));
+            o.set("pValue", Value::number(c.pvalue));
+            o.set("group", Value::integer(c.group));
+            Value& lc = o.set("linked_called", Value::array());
+            for (const std::string& l : c.linked_called) lc.push(Value::string(l));
+        }
+        Value& ps = rl.set("pairs", Value::array());
+        auto variant = [](const LinkageVariant& v) {
+            Value o = Value::object();
+            o.set("abs_pos", Value::integer(v.abs_pos));
+            o.set("codon", Value::string(v.codon));
+            Value& ls = o.set("labels", Value::array());
+            for (const std::string& l : v.labels) ls.push(Value::string(l));
+            return o;
+        };
+        for (const LinkageRow& r : rare->pairs) {
+            Value& o = ps.push(Value::object());
+            o.set("a", variant(r.a));
+            o.set("b", variant(r.b));
+            o.set("reads", Value::integer(static_cast<long long>(r.reads)));
+            o.set("both", Value::integer(static_cast<long long>(r.both)));
+            o.set("a_only", Value::integer(static_cast<long long>(r.a_only)));
+            o.set("b_only", Value::integer(static_cast<long long>(r.b_only)));
+            o.set("neither", Value::integer(static_cast<long long>(r.neither)));
+            o.set("d_prime", Value::number(r.d_prime));
+            o.set("r2", Value::number(r.r2));
+            o.set("pValue", Value::number(r.pvalue));
+            o.set("pValueCorrected", Value::number(r.pvalue_corrected));
+        }
+        Value& gs = rl.set("groups", Value::array());
+        for (const RareGroup& g : rare->groups) {
+            Value& o = gs.push(Value::object());
+            Value& ms = o.set("members", Value::array());
+            for (const std::string& m : g.members) ms.push(Value::string(m));
+            o.set("carriers", Value::integer(static_cast<long long>(g.carriers)));
+            o.set("informative", Value::integer(static_cast<long long>(g.informative)));
+            o.set("frequency", Value::number(g.informative ? static_cast<double>(g.carriers) / static_cast<double>(g.informative) : 0.0));
+        }
+    }
     return root;
 }
 
@@ -532,6 +616,48 @@ inline std::string to_html(const Value& root) {
                     h += hit ? "<td class=\"hap\" style=\"background:" + std::string(palette[k % 10]) + "\"></td>" : "<td class=\"hap\"></td>";
                 }
                 h += "</tr>\n";
+            }
+            h += "</table>";
+        }
+        h += "</details>\n";
+    }
+    if (const Value* rl = root.get("rare_linkage")) {
+        char b[256];
+        snprintf(b, sizeof b, "Candidates: %lld codons with at least %lld reads and uncorrected p &lt; %g that are not called (%lld left out by "
+                 "the cap of %lld); pairs tested: %lld (at least %lld reads clean at both codons; linked at %g after Bonferroni)",
+                 static_cast<long long>(rl->get_number("candidates_tested")), static_cast<long long>(rl->get_number("min_reads")),
+                 rl->get_number("candidate_alpha"), static_cast<long long>(rl->get_number("dropped_candidates")),
+                 static_cast<long long>(rl->get_number("max_candidates")), static_cast<long long>(rl->get_number("tested_pairs")),
+                 static_cast<long long>(rl->get_number("pair_min_reads")), rl->get_number("alpha"));
+        h += "<details open><summary>Linked sub-threshold variants</summary><p>" + std::string(b) + "</p>";
+        const Value* gs = rl->get("groups");
+        if (gs && !gs->arr.empty()) {
+            h += "<table><tr><th>Group</th><th>Members</th><th>Carriers</th><th>Informative</th><th>%</th></tr>\n";
+            for (size_t g = 0; g < gs->arr.size(); ++g) {
+                const Value& r = gs->arr[g];
+                std::string m;
+                if (const Value* ms = r.get("members"))
+                    for (const Value& x : ms->arr) m += (m.empty() ? "" : "<br>") + esc(x.str);
+                snprintf(b, sizeof b, "<td>%.2f</td>", 100.0 * r.get_number("frequency"));
+                h += "<tr><td>" + std::to_string(g + 1) + "</td><td>" + m + "</td><td>" + std::to_string(static_cast<long long>(r.get_number("carriers"))) +
+                     "</td><td>" + std::to_string(static_cast<long long>(r.get_number("informative"))) + "</td>" + b + "</tr>\n";
+            }
+            h += "</table>";
+        }
+        const Value* cs = rl->get("candidates");
+        if (cs && !cs->arr.empty()) {
+            h += "<table><tr><th>Gene</th><th>Variant</th><th>Codon</th><th>%</th><th>Count</th><th>Coverage</th><th>p</th><th>Group</th>"
+                 "<th>Linked called variants</th></tr>\n";
+            for (const Value& r : cs->arr) {
+                std::string lc;
+                if (const Value* l = r.get("linked_called"))
+                    for (const Value& x : l->arr) lc += (lc.empty() ? "" : "<br>") + esc(x.str);
+                const long long g = static_cast<long long>(r.get_number("group"));
+                snprintf(b, sizeof b, "<td>%.2e</td>", r.get_number("pValue"));
+                h += "<tr><td>" + esc(r.get_string("gene")) + "</td><td>" + esc(r.get_string("label")) + "</td><td><tt>" + esc(r.get_string("ref_codon")) +
+                     " &rarr; " + esc(r.get_string("codon")) + "</tt></td><td>" + esc(r.get_string("percentage")) + "</td><td>" +
+                     std::to_string(static_cast<long long>(r.get_number("count"))) + "</td><td>" + std::to_string(static_cast<long long>(r.get_number("coverage"))) +
+                     "</td>" + b + "<td>" + (g >= 0 ? std::to_string(g + 1) : std::string()) + "</td><td>" + lc + "</td></tr>\n";
             }
             h += "</table>";
         }
