@@ -13,12 +13,6 @@
 #include "cleric.hpp"
 #include "host_common.hpp"
 
-#define CK(h, call)                                                                            \
-    do {                                                                                       \
-        int rc_ = (call);                                                                      \
-        if (rc_ != MS_OK) mshost::die(std::string(#call) + " failed: " + ms_last_error(h));     \
-    } while (0)
-
 // IUPAC complement (the codes a BAM SEQ can hold: =ACMGRSVTWYHKDBN), so a stored-reverse record keeps every code
 static char complement(char c) {
     switch (c) {

@@ -13,12 +13,6 @@
 #include "cleric.hpp"
 #include "host_common.hpp"
 
-#define CK(h, call)                                                                            \
-    do {                                                                                       \
-        int rc_ = (call);                                                                      \
-        if (rc_ != MS_OK) mshost::die(std::string(#call) + " failed: " + ms_last_error(h));     \
-    } while (0)
-
 int main(int argc, char** argv) {
     int device = 0;
     std::vector<std::string> pos;

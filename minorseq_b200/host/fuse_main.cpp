@@ -5,16 +5,9 @@
 #include <cstdlib>
 #include <fstream>
 #include <string>
-#include <thread>
 #include <vector>
 #include <unistd.h>
 #include "host_common.hpp"
-
-#define CK(h, call)                                                                            \
-    do {                                                                                       \
-        int rc_ = (call);                                                                      \
-        if (rc_ != MS_OK) mshost::die(std::string(#call) + " failed: " + ms_last_error(h));     \
-    } while (0)
 
 int main(int argc, char** argv) {
     ms_fuse_params prm;
@@ -46,52 +39,25 @@ int main(int argc, char** argv) {
     if (ngpus < 1 || ngpus > 64) mshost::die("--gpus expects 1..64");
     try {
         // the CUDA contexts come up (~0.5 s, one thread per GPU) while a helper thread inflates and indexes the BAM
-        std::vector<ms_handle*> hs(static_cast<size_t>(ngpus), nullptr);
+        std::vector<ms_handle*> hs;
         mshost::Alignments aln;
-        mshost::load_alignments_overlapped(pos[0], qv, false, true, std::string(), aln, [&] {
-            char id[128];
-            if (ngpus > 1 && ms_comm_unique_id(id) != MS_OK) mshost::die("NCCL is not available (libnccl.so.2): --gpus needs it");
-            std::vector<std::string> errs(static_cast<size_t>(ngpus));
-            mshost::run_ranks(ngpus, [&](int r) {
-                if (ms_create(device + r, &hs[r]) != MS_OK) { errs[r] = ms_last_error(nullptr); return; }   // there is no CPU path
-                if (ngpus > 1 && ms_comm_init(hs[r], id, r, ngpus) != MS_OK) errs[r] = ms_last_error(hs[r]);
-            });
-            for (const std::string& e : errs)
-                if (!e.empty()) mshost::die(e);
-        });
+        mshost::load_alignments_overlapped(pos[0], qv, false, true, std::string(), aln, [&] { hs = mshost::open_ranks(device, ngpus); });
         if (aln.nreads == 0) mshost::die("no primary or supplementary alignments in " + pos[0]);
         // every rank piles up its contiguous range of the reads; the all-reduce leaves the column counts of all reads on rank 0
-        {
-            std::vector<std::string> errs(static_cast<size_t>(ngpus));
-            mshost::run_ranks(ngpus, [&](int r) {
-                ms_handle* hr = hs[r];
-                const int64_t r0 = aln.nreads * r / ngpus, r1 = aln.nreads * (r + 1) / ngpus;
-                if (ms_set_layout(hr, aln.L, nullptr) != MS_OK || ms_set_base(hr, aln.base.data()) != MS_OK) { errs[r] = ms_last_error(hr); return; }
-                ms_read_hdr* my_hdr = ngpus > 1 ? nullptr : aln.hdr;      // the reads as event rows (base = majority of a sample of them)
-                const uint8_t* my_ev = aln.events;
-                if (ngpus > 1) {
-                    try { my_ev = mshost::shard_events(aln, r0, r1, &my_hdr); } catch (const std::exception& e) { errs[r] = e.what(); return; }
-                }
-                const bool ok = ms_pileup_events_host(hr, my_hdr, my_ev, r1 - r0, nullptr) == MS_OK && ms_allreduce_counts(hr) == MS_OK &&
-                                ms_synchronize(hr) == MS_OK;
-                if (!ok) errs[r] = ms_last_error(hr);
-                if (ngpus > 1) { ms_synchronize(hr); ms_free_pinned(my_hdr); }
-            });
-            for (const std::string& e : errs)
-                if (!e.empty()) mshost::die("pile-up failed: " + e);
-        }
+        mshost::for_ranks(ngpus, [&](int r) {
+            CK(hs[r], ms_set_layout(hs[r], aln.L, nullptr));
+            CK(hs[r], ms_set_base(hs[r], aln.base.data()));   // the reads as event rows (base = majority of a sample of them)
+            mshost::pileup_shard(hs[r], aln, r, ngpus);
+        });
         ms_handle* h = hs[0];
         std::string seq(static_cast<size_t>(aln.L) + aln.ins_pool.size() + 16, '\0');
         int64_t len = 0;
         CK(h, ms_fuse(h, &prm, aln.ins_col.data(), aln.ins_off.data(), aln.ins_len.data(), static_cast<int64_t>(aln.ins_col.size()),
                       aln.ins_pool.data(), static_cast<int64_t>(aln.ins_pool.size()), &seq[0], static_cast<int64_t>(seq.size()), &len));
         seq.resize(static_cast<size_t>(len));
-        std::string stem = pos[0];
-        const size_t sl = stem.find_last_of('/');
-        if (sl != std::string::npos) stem = stem.substr(sl + 1);
         std::ofstream f(pos[1]);
         if (!f) mshost::die("cannot write " + pos[1]);
-        f << ">" << stem << "|fuse|" << aln.ref_name << "\n";
+        f << ">" << mshost::file_name(pos[0]) << "|fuse|" << aln.ref_name << "\n";
         for (size_t i = 0; i < seq.size(); i += 70) f << seq.substr(i, 70) << "\n";
         fprintf(stderr, "fuse: %lld reads, consensus length %lld\n", static_cast<long long>(aln.nreads), static_cast<long long>(len));
         f.close();

@@ -1,4 +1,4 @@
-// host_common.hpp -- what juliet and fuse share in front of the C ABI: the BAM loop.
+// host_common.hpp -- what juliet and fuse share in front of the C ABI: the BAM loop, the ranks, the checks of the calls.
 //
 // For every record: admission filter (/root/reference/doc/JULIET.md:58), CIGAR walk into one packed row
 // (:49-58, `M` rejected), rich-QV base filter -> 'N' (:256-259,:273-276), optional insertion events (fuse).
@@ -7,9 +7,11 @@
 #include <cstdlib>
 #include <cstring>
 #include <algorithm>
+#include <exception>
 #include <stdexcept>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 #include "../../include/minorseq_b200.h"
 #include "bgzf_bam.hpp"
@@ -110,6 +112,34 @@ inline void die(const std::string& m) {
     exit(1);
 }
 
+// throws "<what> failed: <the library's message>" unless rc is MS_OK
+inline void check(ms_handle* h, int rc, const char* what) {
+    if (rc != MS_OK) throw std::runtime_error(std::string(what) + " failed: " + ms_last_error(h));
+}
+#define CK(h, call) mshost::check((h), (call), #call)
+
+// The list of one of the ABI's list calls: call(out, cap, &n) -> ms_status, first with initial_cap entries, then again with
+// cap = n while the list did not fit.  Both conventions of the ABI count as "did not fit": MS_ERR_CAPACITY, and MS_OK with
+// n > cap.  Any other failure throws as check() does.
+template <class T, class Call>
+inline std::vector<T> fetch(ms_handle* h, const char* what, int64_t initial_cap, Call call) {
+    std::vector<T> out(static_cast<size_t>(initial_cap));
+    int64_t n = 0;
+    for (;;) {
+        const int rc = call(out.data(), static_cast<int64_t>(out.size()), &n);
+        if (rc == MS_ERR_CAPACITY || (rc == MS_OK && n > static_cast<int64_t>(out.size()))) { out.resize(static_cast<size_t>(n)); continue; }
+        check(h, rc, what);
+        out.resize(static_cast<size_t>(n));
+        return out;
+    }
+}
+
+// "in.bam" of "dir/in.bam": the input's name in the FASTA headers
+inline std::string file_name(const std::string& path) { return path.substr(path.find_last_of('/') + 1); }
+
+// rank r's contiguous range [r0, r1) of nreads reads over n ranks
+inline std::pair<int64_t, int64_t> shard(int64_t nreads, int r, int n) { return {nreads * r / n, nreads * (r + 1) / n}; }
+
 // f(rank) for rank 0..n-1: on this thread when n == 1, else one thread per rank (one rank per GPU; the ranks meet inside the
 // library's collectives, so they have to run concurrently)
 template <class F>
@@ -118,6 +148,32 @@ inline void run_ranks(int n, F f) {
     std::vector<std::thread> th;
     for (int r = 0; r < n; ++r) th.emplace_back([&f, r] { f(r); });
     for (std::thread& t : th) t.join();
+}
+
+// run_ranks where f may throw: a rank's thread must never exit() the process (the other ranks may be inside a collective),
+// so each rank's exception is kept, and after the join the first failing rank's (in rank order) is rethrown on this thread
+template <class F>
+inline void for_ranks(int n, F f) {
+    std::vector<std::exception_ptr> errs(static_cast<size_t>(n));
+    run_ranks(n, [&](int r) { try { f(r); } catch (...) { errs[r] = std::current_exception(); } });
+    for (const std::exception_ptr& e : errs)
+        if (e) std::rethrow_exception(e);
+}
+
+// One handle per GPU (devices device..device+n-1, one thread each), sharing one NCCL communicator when n > 1.  Dies rather
+// than throws: it runs while the BAM decode thread of load_alignments_overlapped is joinable.
+inline std::vector<ms_handle*> open_ranks(int device, int n) {
+    std::vector<ms_handle*> hs(static_cast<size_t>(n), nullptr);
+    char id[128];
+    if (n > 1 && ms_comm_unique_id(id) != MS_OK) die("NCCL is not available (libnccl.so.2): --gpus needs it");
+    try {
+        for_ranks(n, [&](int r) {
+            // ms_create's error text is one for all threads, rewritten by each failing create: it is read after the join
+            if (ms_create(device + r, &hs[r]) != MS_OK) throw std::runtime_error("");
+            if (n > 1 && ms_comm_init(hs[r], id, r, n) != MS_OK) throw std::runtime_error(ms_last_error(hs[r]));
+        });
+    } catch (const std::exception& e) { die(*e.what() ? e.what() : ms_last_error(nullptr)); }   // there is no CPU path
+    return hs;
 }
 
 // One record -> one packed row (+ optional insertion events appended to the caller's vectors).
@@ -245,9 +301,8 @@ inline void expand_alignments(const Decoded& d, const QvFilter& qv, bool want_na
     };
     nt = static_cast<unsigned>(std::min<size_t>(nt, keep.size()));
     std::vector<Part> parts(nt);
-    std::vector<std::string> errs(nt);      // a corrupt record throws on its worker: carried to the caller after the join
     const int64_t bound = ms_events_bound(L);
-    auto work = [&](unsigned t) { try {
+    for_ranks(static_cast<int>(nt), [&](int t) {      // a corrupt record throws on its worker: carried to the caller after the join
         const size_t i0 = keep.size() * t / nt, i1 = keep.size() * (t + 1) / nt;
         Part& P = parts[t];
         P.hdr.resize(i1 - i0);
@@ -268,16 +323,7 @@ inline void expand_alignments(const Decoded& d, const QvFilter& qv, bool want_na
                 throw std::runtime_error("record " + rec.name + ": cannot encode the expanded row");
             if (want_names) out.names[k] = rec.name;
         }
-    } catch (const std::exception& e) { errs[t] = e.what(); } };
-    auto run_all = [&](auto&& f) {
-        if (nt == 1) { f(0u); return; }
-        std::vector<std::thread> th;
-        for (unsigned t = 0; t < nt; ++t) th.emplace_back(f, t);
-        for (auto& x : th) x.join();
-    };
-    run_all(work);
-    for (const std::string& e : errs)
-        if (!e.empty()) throw std::runtime_error(e);
+    });
     // ---- one pinned header array and one pinned event array; the threads copy their parts into place
     std::vector<int64_t> ev0(nt + 1, 0);
     for (unsigned t = 0; t < nt; ++t) ev0[t + 1] = ev0[t] + parts[t].nbytes;
@@ -286,7 +332,7 @@ inline void expand_alignments(const Decoded& d, const QvFilter& qv, bool want_na
     out.hdr = static_cast<ms_read_hdr*>(ms_alloc_pinned((keep.size() + 1) * sizeof(ms_read_hdr)));
     out.events = static_cast<uint8_t*>(ms_alloc_pinned(static_cast<size_t>(out.ev_bytes) + 64));
     if (!out.hdr || !out.events) throw std::runtime_error("cannot allocate pinned host memory for the event rows");
-    run_all([&](unsigned t) {
+    run_ranks(static_cast<int>(nt), [&](int t) {
         const size_t i0 = keep.size() * t / nt;
         const Part& P = parts[t];
         for (size_t k = 0; k < P.hdr.size(); ++k) {
@@ -325,6 +371,25 @@ inline void load_alignments_overlapped(const std::string& path, const QvFilter& 
     dec.join();
     if (!err.empty()) throw std::runtime_error(err);
     expand_alignments(d, qv, want_names, want_insertions, refseq, out);
+}
+
+// Rank r of n piles up its shard of the reads (event rows, ~112 B instead of 1504 B per 3 kb read on the link, expanded into
+// tiles on the GPU) and all-reduces the counts; returns the rank's reads on its GPU (tiles, owned by the handle).
+inline const uint32_t* pileup_shard(ms_handle* h, const Alignments& a, int r, int n) {
+    const std::pair<int64_t, int64_t> s = shard(a.nreads, r, n);
+    ms_read_hdr* hdr = a.hdr;
+    const uint8_t* ev = a.events;
+    if (n > 1) ev = shard_events(a, s.first, s.second, &hdr);
+    const uint32_t* rows = nullptr;
+    const int rc = ms_pileup_events_host(h, hdr, ev, s.second - s.first, &rows);
+    if (n > 1) {
+        if (rc == MS_OK) ms_synchronize(h);     // the shard's header copy is ours to free once the upload is done
+        ms_free_pinned(hdr);
+    }
+    check(h, rc, "ms_pileup_events_host");
+    CK(h, ms_allreduce_counts(h));
+    CK(h, ms_synchronize(h));
+    return rows;
 }
 
 }  // namespace mshost

@@ -1,8 +1,11 @@
 // host_selftest.cpp -- CPU-only checks of the C++ host layer (no GPU calls): BAM write/read round trip,
-// aux tags, target-config JSON + DRM grammar, report JSON -> HTML.  Exit code 0 = all good.
+// aux tags, target-config JSON + DRM grammar, report JSON -> HTML, the rank and capacity helpers.  Exit code 0 = all good.
+#include <algorithm>
+#include <chrono>
 #include <cstdio>
 #include <cstdlib>
 #include <string>
+#include <thread>
 #include <vector>
 #include <zlib.h>
 #include "bgzf_bam.hpp"
@@ -10,6 +13,9 @@
 #include "json.hpp"
 #include "report.hpp"
 #include "target_config.hpp"
+
+// the one library function the helpers under test reach (their error message); the self test runs without the library
+extern "C" const char* ms_last_error(const ms_handle*) { return "fake library error"; }
 
 #define REQUIRE(c)                                                          \
     do {                                                                    \
@@ -311,18 +317,26 @@ int main(int argc, char** argv) {
     {   // ---- report: formatting rules read off the screenshots, JSON -> HTML
         REQUIRE(msreport::perc2(1.107) == "1.1" && msreport::perc2(0.912) == "0.91" && msreport::perc2(98.4) == "98" && msreport::perc2(100.0) == "100");
         REQUIRE(msreport::perc1(92.52) == "92.5" && msreport::perc1(1.0) == "1" && msreport::perc1(0.74) == "0.7");
-        mscfg::TargetConfig cfg = mscfg::load("HIV");
-        std::vector<msreport::VariantRow> rows(1);
+        msreport::Report in;
+        in.timestamp = "2017-05-16T11:00:12.187Z"; in.input_file = "in.bam"; in.command_line = "juliet in.bam out.json"; in.version = "test";
+        in.cfg = mscfg::load("HIV");
+        in.genes = in.cfg.genes;
+        in.L = 9719;
+        std::vector<msreport::VariantRow>& rows = in.variants;
+        rows.resize(1);
         rows[0].gene = 7; rows[0].aa_pos = 46; rows[0].col = 2252 + 45 * 3; rows[0].ref_codon = 14; rows[0].codon = 12;  // ATG -> ATA (M46I)
         rows[0].count = 28; rows[0].coverage = 2529; rows[0].expected = 1; rows[0].ntests = 99; rows[0].pvalue = 5.2e-8;
         rows[0].drugs = {"ATV/r", "NFV"};
         rows[0].haplotype_hit = {false, true};
-        std::vector<unsigned> col(9719 * 8, 7);
-        std::vector<msreport::HaplotypeRow> haps(2);
+        in.col_counts.assign(9719 * 8, 7);
+        in.phasing = true;
+        std::vector<msreport::HaplotypeRow>& haps = in.haplotypes;
+        haps.resize(2);
         haps[0].name = "A"; haps[0].reads = 900; haps[0].frequency = 0.9; haps[0].codons = {""}; haps[0].read_names = {"r1", "r2"};
         haps[1].name = "B"; haps[1].reads = 100; haps[1].frequency = 0.1; haps[1].codons = {"ATA"}; haps[1].read_names = {"r3"};
         const unsigned long long ctr[6] = {1000, 5, 20, 3, 15, 4};
-        const msjson::Value rep = msreport::build("2017-05-16T11:00:12.187Z", "in.bam", "juliet in.bam out.json", "test", cfg, 9719, cfg.genes, rows, col, 9719, true, haps, ctr);
+        std::copy(ctr, ctr + 6, in.counters);
+        const msjson::Value rep = msreport::build(in);
         const std::string js = msjson::dump(rep);
         const msjson::Value back = msjson::Parser(js).parse();
         REQUIRE(msjson::dump(back) == js);                                                   // writer/parser round trip
@@ -332,6 +346,50 @@ int main(int argc, char** argv) {
         const std::string html = msreport::to_html(back);
         for (const char* needle : {"Input data", "Target config", "Variant Discovery", "Drug Summaries", "Haplotypes %", "ATV/r + NFV", "2017-05-16T11:00:12.187Z", "M46I"})
             REQUIRE(html.find(needle) != std::string::npos);
+    }
+    {   // ---- the rank and capacity helpers of the binaries, with fake library calls
+        // fetch: both ways of the ABI to say "too small", a list that needs two growths, a failure
+        int calls = 0;
+        auto grows_by_status = [&](int* out, int64_t cap, int64_t* n) {   // MS_ERR_CAPACITY with the size it needs: 10, then 50
+            ++calls;
+            *n = calls == 1 ? 10 : 50;
+            if (cap < *n) return static_cast<int>(MS_ERR_CAPACITY);
+            for (int64_t i = 0; i < *n; ++i) out[i] = static_cast<int>(i);
+            return static_cast<int>(MS_OK);
+        };
+        std::vector<int> got = mshost::fetch<int>(nullptr, "grows_by_status", 4, grows_by_status);
+        REQUIRE(calls == 3 && got.size() == 50 && got[49] == 49);
+        calls = 0;
+        std::vector<int64_t> caps;
+        auto grows_by_count = [&](int* out, int64_t cap, int64_t* n) {   // MS_OK with n > cap (out holds the first cap)
+            caps.push_back(cap);
+            *n = ++calls == 1 ? 7 : 20;
+            for (int64_t i = 0; i < std::min(cap, *n); ++i) out[i] = static_cast<int>(100 + i);
+            return static_cast<int>(MS_OK);
+        };
+        got = mshost::fetch<int>(nullptr, "grows_by_count", 4, grows_by_count);
+        REQUIRE(calls == 3 && caps == std::vector<int64_t>({4, 7, 20}) && got.size() == 20 && got[19] == 119);
+        got = mshost::fetch<int>(nullptr, "fits", 4, [](int*, int64_t, int64_t* n) { *n = 3; return static_cast<int>(MS_OK); });
+        REQUIRE(got.size() == 3);
+        std::string msg;
+        try { mshost::fetch<int>(nullptr, "ms_broken", 4, [](int*, int64_t, int64_t*) { return static_cast<int>(MS_ERR_ARG); }); }
+        catch (const std::exception& e) { msg = e.what(); }
+        REQUIRE(msg == "ms_broken failed: fake library error");
+        // for_ranks: every rank runs; of the failing ranks 1 and 2, rank 1's message reaches the caller
+        std::vector<int> ran(3, 0);
+        msg.clear();
+        try {
+            mshost::for_ranks(3, [&](int r) {
+                ran[r] = 1;
+                if (r == 2) throw std::runtime_error("rank 2 failed");
+                if (r == 1) {
+                    std::this_thread::sleep_for(std::chrono::milliseconds(50));    // rank 2 fails first in time
+                    throw std::runtime_error("rank 1 failed");
+                }
+            });
+        } catch (const std::exception& e) { msg = e.what(); }
+        REQUIRE(msg == "rank 1 failed" && ran == std::vector<int>({1, 1, 1}));
+        REQUIRE(mshost::shard(10, 0, 3).second == 3 && mshost::shard(10, 2, 3).first == 6 && mshost::shard(10, 2, 3).second == 10);
     }
     puts("host selftest ok");
     return 0;

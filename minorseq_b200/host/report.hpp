@@ -12,6 +12,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <map>
+#include <optional>
 #include <string>
 #include <vector>
 #include "json.hpp"
@@ -111,7 +112,25 @@ struct IndelRow {
 };
 struct IndelBlock {
     double deletion_rate = 0, insertion_rate = 0;
+    bool phased = false;           // --phase-indels: the calls are phasing keys (haplotype_hit, the haplotypes' "indels")
     std::vector<IndelRow> calls;   // (gene, codon, deletion first, inserted)
+};
+
+// everything the report shows; the optional blocks are present when their option was given
+struct Report {
+    std::string timestamp, input_file, command_line, version;
+    mscfg::TargetConfig cfg;                     // its version, databaseVersion and referenceName
+    std::vector<mscfg::Gene> genes;              // the genes of the run (the config's, or one "unknown" ORF)
+    int L = 0;                                   // reference length
+    std::vector<unsigned> col_counts;            // L*8
+    std::vector<VariantRow> variants;
+    bool phasing = false;
+    std::vector<HaplotypeRow> haplotypes;
+    unsigned long long counters[6] = {0, 0, 0, 0, 0, 0};   // haplotype read categories
+    std::optional<LinkageBlock> linkage;
+    std::optional<AbundanceBlock> abundance;
+    std::optional<IndelBlock> indels;
+    std::optional<RareBlock> rare;
 };
 
 // "%": two significant digits as in the screenshots (1.1, 0.91, 98, 100)
@@ -130,23 +149,61 @@ inline std::string perc1(double p) {  // haplotype %: one decimal, trailing ".0"
     return s;
 }
 
-inline Value build(const std::string& timestamp, const std::string& input_file, const std::string& cmdline, const std::string& version,
-                   const mscfg::TargetConfig& cfg, int ref_length, const std::vector<mscfg::Gene>& genes,
-                   const std::vector<VariantRow>& variants, const std::vector<unsigned>& col_counts /* L*8 */, int L,
-                   bool phasing, const std::vector<HaplotypeRow>& haps, const unsigned long long counters[6],
-                   const LinkageBlock* linkage = nullptr, const AbundanceBlock* abundance = nullptr, const IndelBlock* indels = nullptr,
-                   bool phase_indels = false, const RareBlock* rare = nullptr) {
+inline Value known_drm(const std::vector<std::string>& drugs) {
+    std::string known;
+    for (size_t d = 0; d < drugs.size(); ++d) known += (d ? " + " : "") + drugs[d];
+    return Value::string(known);
+}
+
+inline Value haplotype_hit(const std::vector<bool>& hit) {
+    Value hh = Value::array();
+    for (bool b : hit) hh.push(Value::boolean(b));
+    return hh;
+}
+
+// the pairs of the linkage and the rare-linkage blocks; the rare block's are all "linked" and carry no "relation"
+inline Value linkage_pairs(const std::vector<LinkageRow>& pairs, bool relation) {
+    auto variant = [](const LinkageVariant& v) {
+        Value o = Value::object();
+        o.set("abs_pos", Value::integer(v.abs_pos));
+        o.set("codon", Value::string(v.codon));
+        Value& ls = o.set("labels", Value::array());
+        for (const std::string& l : v.labels) ls.push(Value::string(l));
+        return o;
+    };
+    Value ps = Value::array();
+    for (const LinkageRow& r : pairs) {
+        Value& o = ps.push(Value::object());
+        o.set("a", variant(r.a));
+        o.set("b", variant(r.b));
+        o.set("reads", Value::integer(static_cast<long long>(r.reads)));
+        o.set("both", Value::integer(static_cast<long long>(r.both)));
+        o.set("a_only", Value::integer(static_cast<long long>(r.a_only)));
+        o.set("b_only", Value::integer(static_cast<long long>(r.b_only)));
+        o.set("neither", Value::integer(static_cast<long long>(r.neither)));
+        o.set("d_prime", Value::number(r.d_prime));
+        o.set("r2", Value::number(r.r2));
+        o.set("pValue", Value::number(r.pvalue));
+        o.set("pValueCorrected", Value::number(r.pvalue_corrected));
+        if (relation) o.set("relation", Value::string(r.relation));
+    }
+    return ps;
+}
+
+inline Value build(const Report& rep) {
+    const std::vector<mscfg::Gene>& genes = rep.genes;
+    const std::vector<VariantRow>& variants = rep.variants;
     Value root = Value::object();
     Value& in = root.set("input", Value::object());
-    in.set("timestamp", Value::string(timestamp));
-    in.set("input_file", Value::string(input_file));
-    in.set("command_line", Value::string(cmdline));
-    in.set("juliet_version", Value::string(version));
+    in.set("timestamp", Value::string(rep.timestamp));
+    in.set("input_file", Value::string(rep.input_file));
+    in.set("command_line", Value::string(rep.command_line));
+    in.set("juliet_version", Value::string(rep.version));
     Value& tc = root.set("target_config", Value::object());
-    tc.set("version", Value::string(cfg.version));
-    tc.set("databaseVersion", Value::string(cfg.database_version));
-    tc.set("referenceName", Value::string(cfg.reference_name));
-    tc.set("referenceLength", Value::integer(ref_length));
+    tc.set("version", Value::string(rep.cfg.version));
+    tc.set("databaseVersion", Value::string(rep.cfg.database_version));
+    tc.set("referenceName", Value::string(rep.cfg.reference_name));
+    tc.set("referenceLength", Value::integer(rep.L));
     Value& tg = tc.set("genes", Value::array());
     for (const mscfg::Gene& g : genes) {
         Value& o = tg.push(Value::object());
@@ -164,6 +221,12 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
     Value& gs = root.set("genes", Value::array());
     std::map<std::string, std::vector<std::string>> drug_summary;
     std::vector<std::string> drug_order;
+    auto summarise = [&](const std::vector<std::string>& drugs, const std::string& label) {   // label under each of its drugs
+        for (const std::string& d : drugs) {
+            if (!drug_summary.count(d)) drug_order.push_back(d);
+            drug_summary[d].push_back(label);
+        }
+    };
     for (size_t gi = 0; gi < genes.size(); ++gi) {
         Value& go = gs.push(Value::object());
         go.set("name", Value::string(genes[gi].name));
@@ -197,42 +260,27 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
                 vc.set("expected", Value::integer(v.expected));
                 vc.set("pValue", Value::number(v.pvalue));
                 vc.set("pValueCorrected", Value::number(std::min(1.0, v.pvalue * v.ntests)));
-                std::string known;
-                for (size_t d = 0; d < v.drugs.size(); ++d) known += (d ? " + " : "") + v.drugs[d];
-                vc.set("known_drm", Value::string(known));
-                if (phasing) {
-                    Value& hh = vc.set("haplotype_hit", Value::array());
-                    for (bool b : v.haplotype_hit) hh.push(Value::boolean(b));
-                }
-                const std::string label = std::string(1, mscfg::translate(v.ref_codon)) + std::to_string(v.aa_pos) + aa + " (" + genes[gi].name + ", " +
-                                          perc2(100.0 * freq) + " %)";
-                for (const std::string& d : v.drugs) {
-                    if (!drug_summary.count(d)) drug_order.push_back(d);
-                    drug_summary[d].push_back(label);
-                }
+                vc.set("known_drm", known_drm(v.drugs));
+                if (rep.phasing) vc.set("haplotype_hit", haplotype_hit(v.haplotype_hit));
+                summarise(v.drugs, std::string(1, mscfg::translate(v.ref_codon)) + std::to_string(v.aa_pos) + aa + " (" + genes[gi].name + ", " +
+                                       perc2(100.0 * freq) + " %)");
             }
             // MSA context: relative positions -3..+5 around the codon's first column (screenshot juliet_hiv-context.png)
             Value& msa = vp.set("msa", Value::array());
             for (int rel = -3; rel <= 5; ++rel) {
                 const int c = f.col + rel;
-                if (c < 0 || c >= L) continue;
+                if (c < 0 || c >= rep.L) continue;
                 Value& row = msa.push(Value::object());
                 row.set("rel_pos", Value::integer(rel));
                 row.set("abs_pos", Value::integer(c + 1));
                 static const char* names[6] = {"A", "C", "G", "T", "-", "N"};
-                for (int s = 0; s < 6; ++s) row.set(names[s], Value::integer(col_counts[static_cast<size_t>(c) * 8 + s]));
+                for (int s = 0; s < 6; ++s) row.set(names[s], Value::integer(rep.col_counts[static_cast<size_t>(c) * 8 + s]));
             }
             i = j;
         }
     }
-    if (indels)
-        for (const IndelRow& r : indels->calls) {
-            const std::string label = r.label + " (" + genes[r.gene].name + ", " + perc2(100.0 * r.count / r.coverage) + " %)";
-            for (const std::string& d : r.drugs) {
-                if (!drug_summary.count(d)) drug_order.push_back(d);
-                drug_summary[d].push_back(label);
-            }
-        }
+    if (rep.indels)
+        for (const IndelRow& r : rep.indels->calls) summarise(r.drugs, r.label + " (" + genes[r.gene].name + ", " + perc2(100.0 * r.count / r.coverage) + " %)");
     Value& dsum = root.set("drug_summaries", Value::array());
     for (const std::string& d : drug_order) {
         Value& o = dsum.push(Value::object());
@@ -240,9 +288,9 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
         Value& vs = o.set("variants", Value::array());
         for (const std::string& l : drug_summary[d]) vs.push(Value::string(l));
     }
-    if (phasing) {
+    if (rep.phasing) {
         Value& hs = root.set("haplotypes", Value::array());
-        for (const HaplotypeRow& h : haps) {
+        for (const HaplotypeRow& h : rep.haplotypes) {
             Value& o = hs.push(Value::object());
             o.set("name", Value::string(h.name));
             o.set("reads", Value::integer(static_cast<long long>(h.reads)));
@@ -250,7 +298,7 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             o.set("percentage", Value::string(perc1(100.0 * h.frequency)));
             Value& cs = o.set("codons", Value::array());
             for (const std::string& c : h.codons) cs.push(Value::string(c));
-            if (phase_indels) {
+            if (rep.indels && rep.indels->phased) {
                 Value& is = o.set("indels", Value::array());
                 for (const std::string& c : h.indels) is.push(Value::string(c));
             }
@@ -259,39 +307,16 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
         }
         Value& hc = root.set("haplotype_read_categories", Value::object());
         static const char* names[6] = {"reported", "insufficient_coverage", "unsuitable", "unsuitable_gaps", "unsuitable_heteroduplex", "unsuitable_partial"};
-        for (int i = 0; i < 6; ++i) hc.set(names[i], Value::integer(static_cast<long long>(counters[i])));
+        for (int i = 0; i < 6; ++i) hc.set(names[i], Value::integer(static_cast<long long>(rep.counters[i])));
     }
-    if (linkage) {
+    if (const auto& linkage = rep.linkage) {
         Value& lk = root.set("linkage", Value::object());
         lk.set("min_reads", Value::integer(linkage->min_reads));
         lk.set("alpha", Value::number(linkage->alpha));
         lk.set("tested_pairs", Value::integer(linkage->tested_pairs));
-        Value& ps = lk.set("pairs", Value::array());
-        auto variant = [](const LinkageVariant& v) {
-            Value o = Value::object();
-            o.set("abs_pos", Value::integer(v.abs_pos));
-            o.set("codon", Value::string(v.codon));
-            Value& ls = o.set("labels", Value::array());
-            for (const std::string& l : v.labels) ls.push(Value::string(l));
-            return o;
-        };
-        for (const LinkageRow& r : linkage->pairs) {
-            Value& o = ps.push(Value::object());
-            o.set("a", variant(r.a));
-            o.set("b", variant(r.b));
-            o.set("reads", Value::integer(static_cast<long long>(r.reads)));
-            o.set("both", Value::integer(static_cast<long long>(r.both)));
-            o.set("a_only", Value::integer(static_cast<long long>(r.a_only)));
-            o.set("b_only", Value::integer(static_cast<long long>(r.b_only)));
-            o.set("neither", Value::integer(static_cast<long long>(r.neither)));
-            o.set("d_prime", Value::number(r.d_prime));
-            o.set("r2", Value::number(r.r2));
-            o.set("pValue", Value::number(r.pvalue));
-            o.set("pValueCorrected", Value::number(r.pvalue_corrected));
-            o.set("relation", Value::string(r.relation));
-        }
+        lk.set("pairs", linkage_pairs(linkage->pairs, true));
     }
-    if (indels) {
+    if (const auto& indels = rep.indels) {
         Value& ib = root.set("indels", Value::object());
         ib.set("deletion_rate", Value::number(indels->deletion_rate));
         ib.set("insertion_rate", Value::number(indels->insertion_rate));
@@ -312,16 +337,11 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             o.set("expected", Value::integer(r.expected));
             o.set("pValue", Value::number(r.pvalue));
             o.set("pValueCorrected", Value::number(std::min(1.0, r.pvalue * r.ntests)));
-            std::string known;
-            for (size_t d = 0; d < r.drugs.size(); ++d) known += (d ? " + " : "") + r.drugs[d];
-            o.set("known_drm", Value::string(known));
-            if (phase_indels) {
-                Value& hh = o.set("haplotype_hit", Value::array());
-                for (bool b : r.haplotype_hit) hh.push(Value::boolean(b));
-            }
+            o.set("known_drm", known_drm(r.drugs));
+            if (indels->phased) o.set("haplotype_hit", haplotype_hit(r.haplotype_hit));
         }
     }
-    if (abundance) {
+    if (const auto& abundance = rep.abundance) {
         Value& ab = root.set("haplotype_abundance", Value::object());
         ab.set("tolerance", Value::number(abundance->tolerance));
         ab.set("max_iterations", Value::integer(abundance->max_iterations));
@@ -349,7 +369,7 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             o.set("em_percentage", Value::string(b));
         }
     }
-    if (rare) {
+    if (const auto& rare = rep.rare) {
         Value& rl = root.set("rare_linkage", Value::object());
         rl.set("min_reads", Value::integer(rare->min_reads));
         rl.set("candidate_alpha", Value::number(rare->candidate_alpha));
@@ -377,29 +397,7 @@ inline Value build(const std::string& timestamp, const std::string& input_file, 
             Value& lc = o.set("linked_called", Value::array());
             for (const std::string& l : c.linked_called) lc.push(Value::string(l));
         }
-        Value& ps = rl.set("pairs", Value::array());
-        auto variant = [](const LinkageVariant& v) {
-            Value o = Value::object();
-            o.set("abs_pos", Value::integer(v.abs_pos));
-            o.set("codon", Value::string(v.codon));
-            Value& ls = o.set("labels", Value::array());
-            for (const std::string& l : v.labels) ls.push(Value::string(l));
-            return o;
-        };
-        for (const LinkageRow& r : rare->pairs) {
-            Value& o = ps.push(Value::object());
-            o.set("a", variant(r.a));
-            o.set("b", variant(r.b));
-            o.set("reads", Value::integer(static_cast<long long>(r.reads)));
-            o.set("both", Value::integer(static_cast<long long>(r.both)));
-            o.set("a_only", Value::integer(static_cast<long long>(r.a_only)));
-            o.set("b_only", Value::integer(static_cast<long long>(r.b_only)));
-            o.set("neither", Value::integer(static_cast<long long>(r.neither)));
-            o.set("d_prime", Value::number(r.d_prime));
-            o.set("r2", Value::number(r.r2));
-            o.set("pValue", Value::number(r.pvalue));
-            o.set("pValueCorrected", Value::number(r.pvalue_corrected));
-        }
+        rl.set("pairs", linkage_pairs(rare->pairs, false));
         Value& gs = rl.set("groups", Value::array());
         for (const RareGroup& g : rare->groups) {
             Value& o = gs.push(Value::object());
@@ -421,9 +419,20 @@ inline std::string esc(const std::string& s) {
     return o;
 }
 
+static const char* const palette[] = {"#e6391e", "#f18f00", "#e8ff0c", "#55e400", "#4fc3ff", "#4a7dff", "#a639ff", "#de0062", "#e6391e", "#8c564b"};
+
+// one cell per haplotype column, in the haplotype's colour where the row's haplotype_hit array says it carries the row
+inline std::string hap_cells(const Value* hh, size_t n) {
+    std::string h;
+    for (size_t k = 0; k < n; ++k) {
+        const bool hit = hh && k < hh->arr.size() && hh->arr[k].b;
+        h += hit ? "<td class=\"hap\" style=\"background:" + std::string(palette[k % 10]) + "\"></td>" : "<td class=\"hap\"></td>";
+    }
+    return h;
+}
+
 // HTML from the JSON value only (never from internal state): the 1:1 conversion of doc/JULIET.md:68-69.
 inline std::string to_html(const Value& root) {
-    static const char* palette[] = {"#e6391e", "#f18f00", "#e8ff0c", "#55e400", "#4fc3ff", "#4a7dff", "#a639ff", "#de0062", "#e6391e", "#8c564b"};
     std::string h;
     h += "<!DOCTYPE html>\n<html><head><meta charset=\"utf-8\"><title>juliet</title>\n<style>\n"
          "body{font-family:Helvetica,Arial,sans-serif;margin:1.5em}details{border-left:3px solid #222;border-radius:8px;padding:.4em 1em;margin:.8em 0}"
@@ -514,11 +523,7 @@ inline std::string to_html(const Value& root) {
                                 h += "<td>" + esc(va.get_string("amino_acid")) + "</td><td><tt>" + cm + "</tt></td><td>" + esc(vc.get_string("percentage")) +
                                      "</td><td class=\"cov\">" + std::to_string(static_cast<long long>(vp.get_number("coverage"))) + "</td><td class=\"drug\">" +
                                      esc(vc.get_string("known_drm")) + "</td>";
-                                const Value* hh = vc.get("haplotype_hit");
-                                for (size_t k = 0; k < nh; ++k) {
-                                    const bool hit = hh && k < hh->arr.size() && hh->arr[k].b;
-                                    h += hit ? "<td class=\"hap\" style=\"background:" + std::string(palette[k % 10]) + "\"></td>" : "<td class=\"hap\"></td>";
-                                }
+                                h += hap_cells(vc.get("haplotype_hit"), nh);
                                 h += "</tr>\n";
                             }
                 if (const Value* msa = vp.get("msa")) {
@@ -610,11 +615,7 @@ inline std::string to_html(const Value& root) {
                      std::to_string(static_cast<long long>(r.get_number("abs_pos"))) + "</td><td><tt>" + esc(r.get_string("inserted")) + "</tt></td><td>" +
                      esc(r.get_string("percentage")) + "</td><td>" + std::to_string(static_cast<long long>(r.get_number("count"))) + "</td><td>" +
                      std::to_string(static_cast<long long>(r.get_number("coverage"))) + "</td>" + b + "<td>" + esc(r.get_string("known_drm")) + "</td>";
-                const Value* hh = r.get("haplotype_hit");
-                for (size_t k = 0; k < nhi; ++k) {
-                    const bool hit = hh && k < hh->arr.size() && hh->arr[k].b;
-                    h += hit ? "<td class=\"hap\" style=\"background:" + std::string(palette[k % 10]) + "\"></td>" : "<td class=\"hap\"></td>";
-                }
+                h += hap_cells(r.get("haplotype_hit"), nhi);
                 h += "</tr>\n";
             }
             h += "</table>";
