@@ -375,10 +375,12 @@ int ms_haplotype_abundance(ms_handle *h, const ms_abundance_params *prm, const u
  *   length that is a multiple of 3 and >= 3, all A/C/G/T (upper-cased).  Other insertions stay in n and count for no x.
  * Test as K2: e = min(n, ceil(n P)) with P = deletion_rate^3 or insertion_rate^len(x), p = one-sided Fisher of
  * [[k, n-k], [e, n-e]], called iff p * ntests < alpha (ntests = the gene's tested codons, as K2), then min_perc / max_perc
- * on 100 k / n.  Needs the (all-reduced) K1 counts of the same reads.                                                 */
+ * on 100 k / n.  Needs the (all-reduced) K1 counts of the same reads.  Limit: n is summed in uint32, so a deletion's
+ * k + coverage (and an insertion's n) must stay <= 2^32 - 1.  ms_indel_call refuses (MS_ERR_ARG) a rate outside [0, 1], an
+ * alpha <= 0, and NaN in any of the three.                                                                               */
 typedef struct {
-    double deletion_rate, insertion_rate;      /* error model: P = deletion_rate^3, insertion_rate^len */
-    double alpha;                              /* call iff p * ntests < alpha */
+    double deletion_rate, insertion_rate;      /* error model: P = deletion_rate^3, insertion_rate^len; each in [0, 1] */
+    double alpha;                              /* call iff p * ntests < alpha; > 0 */
     double min_perc, max_perc;                 /* < 0 = off */
     int32_t region_begin, region_end;          /* 1-based [b,e); 0,0 = off */
 } ms_indel_params;

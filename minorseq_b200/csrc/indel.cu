@@ -10,7 +10,8 @@
 // counters through the grouped pile-up's walk (group.cuh); it counts every column, the call reads codon starts and
 // boundaries only.  indel_ins_kernel checks the two columns of each candidate event in the tiles.  The test is K2's
 // (U1-U3): e = min(n, ceil(n P)), the one-sided Fisher test of [[k, n-k], [e, n-e]], called iff p * ntests < alpha; for a
-// deletion n = k_del + K2's coverage (the reads with a clean codon at s, the sum of K1's codon histogram).
+// deletion n = k_del + K2's coverage (the reads with a clean codon at s, the sum of K1's codon histogram), summed in uint32:
+// a deletion's k_del + coverage must stay <= 2^32 - 1.
 #include <algorithm>
 #include <cstring>
 #include <map>
@@ -312,6 +313,13 @@ int ms_indel_call(ms_handle* h, const ms_gene* genes, int32_t ngenes, const char
     MsRange nvtx_range("indel call");
     if (!h || !genes || ngenes < 0 || !prm || !n || cap < 0 || (cap > 0 && !out)) return MS_ERR_ARG;
     *n = 0;
+    // a rate outside [0, 1] makes e = ceil(n P) negative or larger than n, and the kernel's conversion of a negative e to
+    // uint32 is undefined; NaN fails every comparison below and is refused with them
+    if (!(prm->deletion_rate >= 0.0 && prm->deletion_rate <= 1.0))
+        MS_FAIL(h, MS_ERR_ARG, "ms_indel_call: deletion_rate must lie in [0, 1]");
+    if (!(prm->insertion_rate >= 0.0 && prm->insertion_rate <= 1.0))
+        MS_FAIL(h, MS_ERR_ARG, "ms_indel_call: insertion_rate must lie in [0, 1]");
+    if (!(prm->alpha > 0.0)) MS_FAIL(h, MS_ERR_ARG, "ms_indel_call: alpha must be > 0");
     if (h->indel_L != h->L || h->L <= 0 || !h->d_counts) MS_FAIL(h, MS_ERR_ARG, "ms_indel_call: no indel counts (ms_indel_count_dev)");
     MS_CUDA(h, cudaSetDevice(h->device));
     const int32_t L = h->L;
