@@ -336,6 +336,32 @@ int ms_rare_support(ms_handle *h, const uint32_t *masks, int64_t G, uint64_t *ca
  * Returns the number of groups (>= 0) or MS_ERR_ARG.                                                                    */
 int ms_rare_groups(const ms_linkage_pair *pairs, int64_t npairs, int32_t first_candidate, int32_t V, int32_t *group);
 
+/* ---- control comparison (restatement choice U22) -------------------------------------------------
+ * K2's error model is the same at every column, so a systematic error (a PCR / RT hot spot, an alignment artefact) is called
+ * like a minor strain.  A control sample piled up with the same layout measures that background: on K2's positions and
+ * reference codon (referenceSequence, else the SAMPLE's major codon), each codon c != ref with sample count k >= 1 in the
+ * sample's coverage n is tested against the control's count k0 of c in its clean coverage n0 at the same column:
+ *     p = P(X >= k) for the top-left cell of [[k, n - k], [k0, n0 - k0]]   (one-sided "greater"; p = 1 when n0 = 0)
+ * called iff p * ntests < alpha and then min_perc / max_perc on 100 k / n, exactly as in K2.  No collective: every rank with
+ * the same (all-reduced) counts and capture computes the same list.
+ * Snapshot the handle's current (all-reduced) codon counts L*64 as the control: one device-to-device copy on the handle's
+ * stream.  Kept by ms_reset_counts, dropped by ms_set_layout.                                                             */
+int ms_control_capture(ms_handle *h);
+typedef struct {
+    int32_t gene, codon_index, col, ref_codon, codon;
+    uint32_t count, coverage, control_count, control_coverage, ntests;
+    int32_t called, listed;          /* control-test verdict; the codon was in `listed` */
+    double pvalue;                   /* uncorrected one-sided p, exact when called or listed */
+} ms_control_variant;
+/* One record per (gene, column, codon) that the control test calls or that `listed` names (K2's records, e.g. the report's
+ * calls: each must sit at one of the gene's tested positions, else MS_ERR_ARG; a listed codon that is the reference codon
+ * or has no reads gives no record), sorted by (gene, col, codon).  *n receives their number (may exceed cap: call again).
+ * *uncovered_positions (may be NULL): position-table entries the sample covers (n > 0) and the control does not (n0 = 0).
+ * MS_ERR_ARG without a capture for the current layout, or alpha <= 0.  Coverages are summed in uint32 as in K2.          */
+int ms_control_call(ms_handle *h, const ms_gene *genes, int32_t ngenes, const char *refseq, const ms_call_params *prm,
+                    const ms_variant *listed, int64_t nlisted, ms_control_variant *out, int64_t cap, int64_t *n,
+                    int64_t *uncovered_positions);
+
 /* ---- haplotype abundance (restatement choice U18) ------------------------------------------------
  * Phasing counts a haplotype's reads among the reads that are clean at EVERY key; abundance also uses the damaged ones.
  * With B (read carries key v's codon) and M (key v's three columns are all A/C/G/T) as in linkage, read r is compatible

@@ -56,6 +56,12 @@ class RareParams(C.Structure):
     _fields_ = [("candidate_alpha", C.c_double), ("min_reads", C.c_int32)]
 
 
+class ControlVariant(C.Structure):
+    _fields_ = [("gene", C.c_int32), ("codon_index", C.c_int32), ("col", C.c_int32), ("ref_codon", C.c_int32), ("codon", C.c_int32),
+                ("count", C.c_uint32), ("coverage", C.c_uint32), ("control_count", C.c_uint32), ("control_coverage", C.c_uint32),
+                ("ntests", C.c_uint32), ("called", C.c_int32), ("listed", C.c_int32), ("pvalue", C.c_double)]
+
+
 class AbundanceParams(C.Structure):
     _fields_ = [("tolerance", C.c_double), ("max_iterations", C.c_int32)]
 
@@ -200,6 +206,9 @@ _SIGNATURES = {
                                   C.POINTER(C.c_int64)]),
     "ms_rare_support": (C.c_int, [_P, _P, C.c_int64, _P, _P]),
     "ms_rare_groups": (C.c_int, [C.POINTER(LinkagePair), C.c_int64, C.c_int32, C.c_int32, _P]),
+    "ms_control_capture": (C.c_int, [_P]),
+    "ms_control_call": (C.c_int, [_P, C.POINTER(Gene), C.c_int32, C.c_char_p, C.POINTER(CallParams), C.POINTER(Variant), C.c_int64,
+                                  C.POINTER(ControlVariant), C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -13,7 +13,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _lib
-from ._lib import (AbundanceCounters, AbundanceParams, AbundanceRow, AlignParams, CallParams, FuseParams, Gene, Indel, IndelParams, LinkagePair, LinkageParams, PhaseCounters, RareParams, ReadAlignment, SynthParams, Variant,
+from ._lib import (AbundanceCounters, AbundanceParams, AbundanceRow, AlignParams, CallParams, ControlVariant, FuseParams, Gene, Indel, IndelParams, LinkagePair, LinkageParams, PhaseCounters, RareParams, ReadAlignment, SynthParams, Variant,
                    check)
 from .synth import start_mask_words, tile_rows, untile_rows
 
@@ -142,6 +142,15 @@ class RareLinkage:
     def linked_called(self, k):
         """the called keys linked to candidate key k"""
         return sorted(int(v) for v, w in zip(self.pairs["v"], self.pairs["w"]) if w == k and v < self.first_candidate)
+
+
+@dataclass
+class Control:
+    """Control comparison (Juliet.control_call, restatement choice U22): one ControlVariant per codon that the control test
+    calls or that was listed, sorted by (gene, col, codon); uncovered_positions = the positions the sample covers and the
+    control does not (p = 1 there)."""
+    rows: list
+    uncovered_positions: int
 
 
 def translate_dna(x: str) -> str:
@@ -550,6 +559,30 @@ class Juliet:
         check(self.lib.ms_rare_support(self.hd.h, _ptr(masks), ng, _ptr(car), _ptr(inf)), self.hd.h)
         return RareLinkage(candidates=cands, keys=keys, first_candidate=fc, pairs=pairs, tested=int(m.value), dropped=dropped,
                            groups=groups, carriers=car[:ng].copy(), informative=inf[:ng].copy())
+
+    # -- control comparison (restatement choice U22)
+    def capture_control(self):
+        """Keep the handle's current (all-reduced) codon counts as the control: pile up and all-reduce the control's reads,
+        capture, reset the counts, then pile up the sample.  Survives reset(), not a new Juliet on the same handle."""
+        check(self.lib.ms_control_capture(self.hd.h), self.hd.h)
+
+    def control_call(self, listed=None, cap=256) -> Control:
+        """Test the sample's codons against the captured control (ms_control_call).  listed: Variant records whose rows are
+        reported whatever the control says (None = Juliet.call(); [] = the control calls only)."""
+        if listed is None:
+            listed = self.call()
+        lv = (Variant * max(1, len(listed)))(*[Variant.from_buffer_copy(v) for v in listed])
+        genes = (Gene * max(1, len(self.genes)))(*[Gene(b, e) for (b, e) in self.genes])
+        ref = self.refseq.encode() if self.refseq else None
+        n, unc = C.c_int64(), C.c_int64()
+        while True:
+            out = (ControlVariant * max(1, cap))()
+            check(self.lib.ms_control_call(self.hd.h, genes, len(self.genes), ref, C.byref(self.params), lv, len(listed), out, cap, C.byref(n),
+                                           C.byref(unc)), self.hd.h)
+            if n.value <= cap:
+                break
+            cap = int(n.value)
+        return Control(rows=[ControlVariant.from_buffer_copy(out[i]) for i in range(n.value)], uncovered_positions=int(unc.value))
 
     # -- in-frame indels (restatement choice U19)
     def indels(self, d_packed_ptr: int, nreads: int, insertions=None, read0=0, deletion_rate=None, insertion_rate=3e-3,

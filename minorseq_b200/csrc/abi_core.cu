@@ -124,7 +124,7 @@ void ms_destroy(ms_handle* h) {
     cudaEventDestroy(h->ev_timer[0]); cudaEventDestroy(h->ev_timer[1]);
     for (DevBuf* b : {&h->b_ab_pat, &h->b_ab_mask, &h->b_ab_flag, &h->b_ab_slot, &h->b_ab_tab_key, &h->b_ab_tab_cnt, &h->b_ab_tab_rep, &h->b_ab_ctr,
                       &h->b_ab_blk, &h->b_ab_out, &h->b_ab_em, &h->b_indel_cnt, &h->b_indel_ev, &h->b_indel_out,
-                      &h->b_rare_pos, &h->b_rare_out, &h->b_rare_pairs, &h->b_rare_sup})
+                      &h->b_rare_pos, &h->b_rare_out, &h->b_rare_pairs, &h->b_rare_sup, &h->b_control, &h->b_control_pos, &h->b_control_out})
         b->release();
     for (int s = 1; s < 16; ++s) { cudaEventDestroy(h->ev_stage[s][0]); cudaEventDestroy(h->ev_stage[s][1]); }
     cudaStreamDestroy(h->own_stream); cudaStreamDestroy(h->copy_stream);
@@ -218,6 +218,7 @@ int ms_set_layout(ms_handle* h, int32_t L, const uint32_t* start_mask) {
     if (!h || L < 3) return MS_ERR_ARG;
     MS_CUDA(h, cudaSetDevice(h->device));
     h->indel_L = 0;   // the indel counts belong to the old layout
+    h->control_valid = false;   // and so does a captured control
     const int32_t nblk = (L + 31) / 32;
     // CTA shape.  W warps span a row or a column segment of it (31 counting lanes per warp -- lane 31 is the codon
     // look-ahead provider -- and 32 in the last), G row-groups per CTA with W*G <= 12.  With nseg > 1 CTA c handles

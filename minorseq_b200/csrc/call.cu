@@ -24,6 +24,19 @@ struct CallConst {
     double alpha, min_perc, max_perc;
 };
 
+// the major codon of a column whose 64 bins the warp holds as (lane, lane + 32), lowest index on ties: maximise (count, -index).
+// Integer-only, so every kernel that shares it picks the same codon.
+__device__ __forceinline__ int major_codon(uint32_t k0, uint32_t k1, int lane) {
+    uint32_t bc = k0, bi = lane;
+    if (k1 > bc) { bc = k1; bi = lane + 32; }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const uint32_t oc = __shfl_xor_sync(0xffffffffu, bc, o), oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (oc > bc || (oc == bc && oi < bi)) { bc = oc; bi = oi; }
+    }
+    return static_cast<int>(bi);
+}
+
 // one warp per codon position; lane tests codons lane and lane+32
 __global__ void call_kernel(const uint32_t* __restrict__ codon, const CallPos* __restrict__ pos, int32_t npos,
                             CallConst cc, ms_variant* __restrict__ out, unsigned long long* __restrict__ nout,
@@ -37,18 +50,7 @@ __global__ void call_kernel(const uint32_t* __restrict__ codon, const CallPos* _
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
     if (n == 0) return;
-    int ref = ps.ref_codon;
-    if (ref < 0) {
-        // major codon, lowest index wins ties: maximise (count, -index)
-        uint32_t bc = k0, bi = lane;
-        if (k1 > bc) { bc = k1; bi = lane + 32; }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const uint32_t oc = __shfl_xor_sync(0xffffffffu, bc, o), oi = __shfl_xor_sync(0xffffffffu, bi, o);
-            if (oc > bc || (oc == bc && oi < bi)) { bc = oc; bi = oi; }
-        }
-        ref = static_cast<int>(bi);
-    }
+    const int ref = ps.ref_codon >= 0 ? ps.ref_codon : major_codon(k0, k1, lane);
 #pragma unroll
     for (int half = 0; half < 2; ++half) {
         const int c = lane + 32 * half;
@@ -107,17 +109,7 @@ __global__ void rare_candidate_kernel(const uint32_t* __restrict__ codon, const 
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
     if (n == 0) return;
-    int ref = ps.ref_codon;
-    if (ref < 0) {
-        uint32_t bc = k0, bi = lane;
-        if (k1 > bc) { bc = k1; bi = lane + 32; }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const uint32_t oc = __shfl_xor_sync(0xffffffffu, bc, o), oi = __shfl_xor_sync(0xffffffffu, bi, o);
-            if (oc > bc || (oc == bc && oi < bi)) { bc = oc; bi = oi; }
-        }
-        ref = static_cast<int>(bi);
-    }
+    const int ref = ps.ref_codon >= 0 ? ps.ref_codon : major_codon(k0, k1, lane);
     const double nt = static_cast<double>(ps.ntests);
     const double bound = fmax(rc.alpha / nt, rc.candidate_alpha);
 #pragma unroll
@@ -141,6 +133,62 @@ __global__ void rare_candidate_kernel(const uint32_t* __restrict__ codon, const 
             r.v.count = k; r.v.coverage = n; r.v.expected = e; r.v.ntests = ps.ntests; r.v.pvalue = p;
             r.called = called ? 1 : 0; r.pad = 0;
             out[slot] = r;
+        }
+    }
+}
+
+// Control comparison (restatement choice U22): K2's position table and reference codon, but each codon c != ref of the sample,
+// seen k times in n, is tested against the control's count k0 of c in its clean coverage n0 at the same column:
+// p = P(X >= k) of [[k, n - k], [k0, n0 - k0]] (one-sided "greater"), p = 1 when n0 = 0.  Called iff p * ntests < alpha and the
+// percentage filters pass, as in K2.  The rows are unequal (n != n0), so K2's k <= e shortcut has no counterpart: every codon
+// with k >= 1 goes through fisher_upper, whose tail below the mode is 1 - P(X <= k - 1), summed away from the mode and short.
+// Listed codons (the report's K2 calls) get the whole tail, the others stop at alpha / ntests as K2's do.  The precise log:
+// the tables can have k close to n (a minor strain absent from the control).  ctr[0] = records, ctr[1] = positions that the
+// sample covers and the control does not.
+struct ControlConst {
+    double alpha, min_perc, max_perc;
+};
+
+__global__ void control_call_kernel(const uint32_t* __restrict__ codon, const uint32_t* __restrict__ control, const CallPos* __restrict__ pos,
+                                    const unsigned long long* __restrict__ listed, int32_t npos, ControlConst cc,
+                                    ms_control_variant* __restrict__ out, unsigned long long* __restrict__ ctr, unsigned long long cap) {
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (warp >= npos) return;
+    const CallPos ps = pos[warp];
+    const uint32_t* h = codon + static_cast<size_t>(ps.col) * 64;
+    const uint32_t* h0 = control + static_cast<size_t>(ps.col) * 64;
+    const uint32_t k0 = h[lane], k1 = h[lane + 32], c0 = h0[lane], c1 = h0[lane + 32];
+    uint32_t n = k0 + k1, n0 = c0 + c1;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        n += __shfl_xor_sync(0xffffffffu, n, o);
+        n0 += __shfl_xor_sync(0xffffffffu, n0, o);
+    }
+    if (n == 0) return;
+    if (n0 == 0 && lane == 0) atomicAdd(ctr + 1, 1ULL);
+    const int ref = ps.ref_codon >= 0 ? ps.ref_codon : major_codon(k0, k1, lane);
+    const unsigned long long lmask = listed[warp];
+    const double nt = static_cast<double>(ps.ntests);
+    const double enough = 1.000001 * cc.alpha / nt;
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {
+        const int c = lane + 32 * half;
+        const uint32_t k = half ? k1 : k0, kc = half ? c1 : c0;
+        if (c == ref || k == 0) continue;
+        const bool is_listed = (lmask >> c) & 1ULL;
+        const double p = n0 == 0 ? 1.0 : fisher_upper<true>(k, n - k, kc, n0 - kc, is_listed ? 2.0 : enough);
+        bool called = p * nt < cc.alpha;
+        const double perc = 100.0 * static_cast<double>(k) / static_cast<double>(n);
+        if (cc.min_perc >= 0.0 && !(perc > cc.min_perc)) called = false;
+        if (cc.max_perc >= 0.0 && !(perc < cc.max_perc)) called = false;
+        if (!called && !is_listed) continue;
+        const unsigned long long slot = atomicAdd(ctr, 1ULL);
+        if (slot < cap) {
+            ms_control_variant v;
+            v.gene = ps.gene; v.codon_index = ps.codon_index; v.col = ps.col; v.ref_codon = ref; v.codon = c;
+            v.count = k; v.coverage = n; v.control_count = kc; v.control_coverage = n0; v.ntests = ps.ntests;
+            v.called = called ? 1 : 0; v.listed = is_listed ? 1 : 0; v.pvalue = p;
+            out[slot] = v;
         }
     }
 }
@@ -390,6 +438,92 @@ int ms_rare_candidates(ms_handle* h, const ms_gene* genes, int32_t ngenes, const
     }
     *n = static_cast<int64_t>(cand.size());
     for (int64_t i = 0; i < std::min<int64_t>(cap, *n); ++i) out[i] = cand[i];
+    return MS_OK;
+}
+
+int ms_control_capture(ms_handle* h) {
+    if (!h || !h->d_counts) return MS_ERR_ARG;
+    if (!h->count_codons) MS_FAIL(h, MS_ERR_ARG, "ms_set_layout was called without a codon start mask");
+    MS_CUDA(h, cudaSetDevice(h->device));
+    const size_t bytes = static_cast<size_t>(h->L) * 64 * 4;
+    MS_CUDA(h, h->b_control.ensure(bytes));
+    MS_CUDA(h, cudaMemcpyAsync(h->b_control.p, h->d_counts + static_cast<size_t>(h->L) * 8, bytes, cudaMemcpyDeviceToDevice, h->stream));
+    h->control_valid = true;
+    return MS_OK;
+}
+
+int ms_control_call(ms_handle* h, const ms_gene* genes, int32_t ngenes, const char* refseq, const ms_call_params* prm,
+                    const ms_variant* listed, int64_t nlisted, ms_control_variant* out, int64_t cap, int64_t* n,
+                    int64_t* uncovered_positions) {
+    MsRange nvtx_range("control call");
+    if (!h || !h->d_counts || !genes || ngenes < 0 || !prm || !n || cap < 0 || (cap > 0 && !out) || nlisted < 0 || (nlisted > 0 && !listed))
+        return MS_ERR_ARG;
+    if (!(prm->alpha > 0.0)) MS_FAIL(h, MS_ERR_ARG, "ms_control_call: alpha must be > 0");
+    if (!h->count_codons) MS_FAIL(h, MS_ERR_ARG, "ms_set_layout was called without a codon start mask");
+    if (!h->control_valid) MS_FAIL(h, MS_ERR_ARG, "ms_control_call: no control captured for this layout (call ms_control_capture first)");
+    MS_CUDA(h, cudaSetDevice(h->device));
+    *n = 0;
+    if (uncovered_positions) *uncovered_positions = 0;
+    std::vector<ms::CallPos> pos;
+    int rc = ms::call_positions(h, genes, ngenes, refseq, prm, pos);
+    if (rc != MS_OK) return rc;
+    if (pos.empty()) return MS_OK;
+    const size_t npos = pos.size();
+    // listed codons -> one 64-bit mask per position table entry; a gene's entries are contiguous and ordered by column
+    std::vector<unsigned long long> mask(npos, 0ULL);
+    std::vector<size_t> gene_first(static_cast<size_t>(ngenes) + 1, npos);
+    for (size_t i = npos; i-- > 0;) gene_first[pos[i].gene] = i;
+    for (int32_t g = ngenes - 1; g >= 0; --g) gene_first[g] = std::min(gene_first[g], gene_first[g + 1]);
+    for (int64_t i = 0; i < nlisted; ++i) {
+        const ms_variant& v = listed[i];
+        if (v.gene < 0 || v.gene >= ngenes || v.codon < 0 || v.codon > 63) MS_FAIL(h, MS_ERR_ARG, "ms_control_call: a listed variant has no such gene or codon");
+        const auto b = pos.begin() + static_cast<std::ptrdiff_t>(gene_first[v.gene]), e = pos.begin() + static_cast<std::ptrdiff_t>(gene_first[v.gene + 1]);
+        const auto it = std::lower_bound(b, e, v.col, [](const ms::CallPos& p, int32_t col) { return p.col < col; });
+        if (it == e || it->col != v.col) MS_FAIL(h, MS_ERR_ARG, "ms_control_call: a listed variant is not at one of the gene's tested positions");
+        mask[static_cast<size_t>(it - pos.begin())] |= 1ULL << v.codon;
+    }
+    const size_t mask_bytes = npos * sizeof(unsigned long long);
+    MS_CUDA(h, h->b_control_pos.ensure(mask_bytes + npos * sizeof(ms::CallPos)));
+    unsigned long long* d_mask = h->b_control_pos.as<unsigned long long>();
+    ms::CallPos* d_pos = reinterpret_cast<ms::CallPos*>(h->b_control_pos.as<uint8_t>() + mask_bytes);
+    MS_CUDA(h, cudaMemcpyAsync(d_mask, mask.data(), mask_bytes, cudaMemcpyHostToDevice, h->stream));
+    MS_CUDA(h, cudaMemcpyAsync(d_pos, pos.data(), npos * sizeof(ms::CallPos), cudaMemcpyHostToDevice, h->stream));
+    ms::ControlConst cc;
+    cc.alpha = prm->alpha; cc.min_perc = prm->min_perc; cc.max_perc = prm->max_perc;
+    // the records are the listed codons and the control calls, few; the buffer grows and the kernel runs again if not
+    size_t dev_cap = std::min<size_t>(npos * 63, std::max<size_t>(1 << 12, 2 * static_cast<size_t>(nlisted)));
+    unsigned long long st[2] = {0, 0};
+    for (;;) {
+        MS_CUDA(h, h->b_control_out.ensure(64 + dev_cap * sizeof(ms_control_variant)));
+        unsigned long long* d_ctr = h->b_control_out.as<unsigned long long>();
+        MS_CUDA(h, cudaMemsetAsync(d_ctr, 0, 16, h->stream));
+        const int threads = 128;
+        const int blocks = static_cast<int>((npos * 32 + threads - 1) / threads);
+        ms::control_call_kernel<<<blocks, threads, 0, h->stream>>>(h->d_counts + static_cast<size_t>(h->L) * 8, h->b_control.as<uint32_t>(), d_pos,
+                                                                   d_mask, static_cast<int32_t>(npos), cc,
+                                                                   reinterpret_cast<ms_control_variant*>(h->b_control_out.as<uint8_t>() + 64), d_ctr,
+                                                                   dev_cap);
+        h->launches++;
+        MS_CUDA(h, cudaGetLastError());
+        MS_CUDA(h, cudaMemcpyAsync(st, d_ctr, 16, cudaMemcpyDeviceToHost, h->stream));
+        MS_CUDA(h, cudaStreamSynchronize(h->stream));
+        if (st[0] <= dev_cap) break;
+        dev_cap = static_cast<size_t>(st[0]);
+    }
+    std::vector<ms_control_variant> rec(st[0]);
+    if (st[0]) {
+        MS_CUDA(h, cudaMemcpyAsync(rec.data(), h->b_control_out.as<uint8_t>() + 64, st[0] * sizeof(ms_control_variant), cudaMemcpyDeviceToHost,
+                                   h->stream));
+        MS_CUDA(h, cudaStreamSynchronize(h->stream));
+    }
+    std::sort(rec.begin(), rec.end(), [](const ms_control_variant& a, const ms_control_variant& b) {
+        if (a.gene != b.gene) return a.gene < b.gene;
+        if (a.col != b.col) return a.col < b.col;
+        return a.codon < b.codon;
+    });
+    *n = static_cast<int64_t>(st[0]);
+    if (uncovered_positions) *uncovered_positions = static_cast<int64_t>(st[1]);
+    for (int64_t i = 0; i < std::min<int64_t>(cap, *n); ++i) out[i] = rec[i];
     return MS_OK;
 }
 

@@ -160,6 +160,10 @@ struct ms_handle {
     // sub-threshold linkage (call.cu, rare.cu): the candidate kernel's position table and records, the linked pairs, the group
     // support scratch (masks | counters)
     DevBuf b_rare_pos, b_rare_out, b_rare_pairs, b_rare_sup;
+    // control comparison (call.cu): the captured control codon counts [L*64], the position table with its listed-codon masks,
+    // the records; control_valid: b_control belongs to the current layout
+    bool control_valid = false;
+    DevBuf b_control, b_control_pos, b_control_out;
 
     DevBuf b_aln_ref, b_aln_idx, b_aln_seq, b_aln_off, b_aln_seed, b_aln_scratch, b_aln_slab, b_aln_mbits, b_aln_cig, b_aln_res, b_aln_ctr,
         b_aln_dst, b_aln_pack;

@@ -13,6 +13,8 @@
 // choice U20) adds the reported indels to the phasing keys: haplotypes, linkage, abundance and the FASTA then see them.
 // --rare-linkage (restatement choice U21) looks for minor strains below K2's threshold: codons that K2 does not call but whose
 // uncorrected p is small, tested for linkage to each other and to the called variants on the reads clean at both codons.
+// --control (restatement choice U22) piles up a control sample with the same layout and tests every codon of the sample against
+// the control's count at the same position (two-sample Fisher), so that a systematic error is told apart from a minor strain.
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -49,6 +51,9 @@ static void usage() {
          "                                     for linkage over the reads; linked groups and their reads (\"rare_linkage\")\n"
          "      --rare-min-reads <n>           reads a --rare-linkage candidate needs (default 5)\n"
          "      --rare-candidate-alpha <a>     uncorrected p a --rare-linkage candidate needs to stay below (default 0.1)\n"
+         "      --control <control.bam>        test each codon against a control sample (same reference) at the same position:\n"
+         "                                     two-sample one-sided Fisher, Bonferroni at --alpha (\"control\"; the rest of the\n"
+         "                                     report is unchanged)\n"
          "      --min-perc <p>                 only variants with abundance > p %\n"
          "      --max-perc <p>                 only variants with abundance < p %\n"
          "      --drm-only                     only known drug-resistance mutations\n"
@@ -71,7 +76,7 @@ static void usage() {
 static bool ends_with(const std::string& s, const std::string& e) { return s.size() >= e.size() && s.compare(s.size() - e.size(), e.size(), e) == 0; }
 
 struct Options {
-    std::string input, config, region, cmdline, timing_json, out_json, out_html, out_fasta;
+    std::string input, config, region, cmdline, timing_json, out_json, out_html, out_fasta, control;
     bool phasing = false, drm_only = false, linkage = false, abundance = false, indels = false, phase_indels = false, rare_linkage = false;
     double min_perc = -1, max_perc = -1, sub = 5e-4, del = 3e-3, alpha = 0.01, ins_rate = 3e-3, rare_alpha = 0.1;
     int min_hap = 10, device = 0, ngpus = 1, hap_min_cov = 10, rare_min_reads = 5;
@@ -102,6 +107,7 @@ static Options parse_options(int argc, char** argv) {
         else if (a == "--rare-linkage") o.rare_linkage = true;
         else if (a == "--rare-min-reads") o.rare_min_reads = atoi(need("--rare-min-reads").c_str());
         else if (a == "--rare-candidate-alpha") o.rare_alpha = atof(need("--rare-candidate-alpha").c_str());
+        else if (a == "--control") o.control = need("--control");
         else if (a == "--insertion-rate") o.ins_rate = atof(need("--insertion-rate").c_str());
         else if (a == "--drm-only") o.drm_only = true;
         else if (a == "--min-perc") o.min_perc = atof(need("--min-perc").c_str());
@@ -164,6 +170,7 @@ struct Run {
     ms_call_params prm;
     const char* ref = nullptr;                // the config's referenceSequence when it covers the reference
     mshost::Alignments aln;
+    mshost::Alignments ctl;                   // --control: the control's reads
     std::vector<ms_handle*> hs;               // one handle per GPU (rank)
     std::vector<const uint32_t*> rows_dev;    // each rank's reads on its GPU (tiles)
     std::vector<std::pair<int, int>> keys;    // the called variants' (col, codon), sorted: phasing keys 0..V-1
@@ -176,6 +183,8 @@ struct Run {
     std::vector<int32_t> hap;                 // per read: its haplotype's position in the report order (-1 = none)
     std::vector<ms_linkage_pair> link_pairs;
     int64_t link_tested = 0;
+    std::vector<ms_control_variant> control_rows;
+    int64_t control_uncovered = 0;
     msreport::Report rep;
     bool carries(int64_t k, int32_t v) const { return (pat[static_cast<size_t>(k) * nw + (v >> 5)] >> (v & 31)) & 1u; }
     std::string gene_label(int gene, const std::string& label) const { return rep.genes[gene].name + " " + label; }
@@ -205,6 +214,17 @@ static void load(Run& run) {
     run.lap("CUDA context || BAM inflate + CIGAR expansion + event encoding");
     if (run.aln.nreads == 0) mshost::die("no primary or supplementary alignments in " + o.input);
     const int32_t L = run.aln.L;
+    if (!o.control.empty()) {
+        // the control goes through the same admission rules and QV filter; it must be aligned to the sample's reference
+        mshost::Decoded d;
+        mshost::decode_alignments(o.control, d, run.ctl);
+        if (run.ctl.nreads == 0) mshost::die("no primary or supplementary alignments in the control " + o.control);
+        if (run.ctl.ref_name != run.aln.ref_name || run.ctl.L != L)
+            mshost::die("the control " + o.control + " is aligned to " + run.ctl.ref_name + " (" + std::to_string(run.ctl.L) + " bp), the sample to " +
+                        run.aln.ref_name + " (" + std::to_string(L) + " bp): --control needs the same reference");
+        mshost::expand_alignments(d, o.qv, false, false, run.cfg.reference_sequence, run.ctl);
+        run.lap("control BAM inflate + CIGAR expansion + event encoding");
+    }
 
     // genes: from the config, or one ORF labelled "unknown" (doc/JULIET.md:182-188)
     std::vector<mscfg::Gene>& genes = run.rep.genes;
@@ -232,6 +252,16 @@ static void load(Run& run) {
     run.rep.col_counts.resize(static_cast<size_t>(L) * 8);
     run.rows_dev.resize(static_cast<size_t>(o.ngpus));
     run.hap.resize(o.phasing ? run.aln.nreads : 0);
+}
+
+// the DRMs of gene `gene` that a codon change at 1-based amino-acid position aa_pos matches (doc/JULIET.md:104-107)
+static std::vector<std::string> variant_drugs(const Run& run, int gene, int aa_pos, int ref_codon, int codon) {
+    std::vector<std::string> d;
+    const char ra = mscfg::translate(ref_codon), va = mscfg::translate(codon);
+    for (const mscfg::Drm& x : run.rep.genes[gene].drms)
+        for (const mscfg::DrmPosition& p : x.positions)
+            if (mscfg::drm_matches(p, aa_pos, ra, va)) { d.push_back(x.name); break; }
+    return d;
 }
 
 static char indel_aa(int32_t codon) { return codon >= 0 ? mscfg::translate(codon) : '?'; }
@@ -272,6 +302,14 @@ static void rank_pass(Run& run) {
         const std::pair<int64_t, int64_t> s = mshost::shard(run.aln.nreads, r, o.ngpus);
         const int64_t nr = s.second - s.first;
         CK(h, ms_set_layout(h, run.aln.L, run.start.data()));
+        if (!o.control.empty()) {
+            // the control first: the sample's reads have to stay on the device for phasing and indels
+            CK(h, ms_set_base(h, run.ctl.base.data()));
+            mshost::pileup_shard(h, run.ctl, r, o.ngpus);
+            CK(h, ms_control_capture(h));
+            CK(h, ms_reset_counts(h));
+            if (r == 0) run.lap(o.ngpus > 1 ? "control: H2D events + expand + pileup + all-reduce" : "control: H2D events + expand + pileup");
+        }
         CK(h, ms_set_base(h, run.aln.base.data()));
         run.rows_dev[r] = mshost::pileup_shard(h, run.aln, r, o.ngpus);
         if (r == 0) run.lap(o.ngpus > 1 ? "H2D events + expand + pileup + all-reduce" : "H2D events + expand + pileup");
@@ -281,21 +319,31 @@ static void rank_pass(Run& run) {
         });
         // DRM annotation and --drm-only (doc/JULIET.md:104-107,:370)
         std::vector<msreport::VariantRow> rows;
+        std::vector<ms_variant> listed;       // the calls behind `rows`
         for (const ms_variant& v : mv) {
             msreport::VariantRow vr;
             vr.gene = v.gene; vr.aa_pos = v.codon_index + 1; vr.col = v.col; vr.ref_codon = v.ref_codon; vr.codon = v.codon;
             vr.count = v.count; vr.coverage = v.coverage; vr.expected = v.expected; vr.ntests = v.ntests; vr.pvalue = v.pvalue;
-            const char ra = mscfg::translate(v.ref_codon), va = mscfg::translate(v.codon);
-            for (const mscfg::Drm& d : run.rep.genes[v.gene].drms)
-                for (const mscfg::DrmPosition& p : d.positions)
-                    if (mscfg::drm_matches(p, vr.aa_pos, ra, va)) { vr.drugs.push_back(d.name); break; }
+            vr.drugs = variant_drugs(run, v.gene, vr.aa_pos, v.ref_codon, v.codon);
             if (o.drm_only && vr.drugs.empty()) continue;
             rows.push_back(vr);
+            listed.push_back(v);
         }
-        if (r == 0) {
-            run.lap("call + DRM annotation");
-            CK(h, ms_get_counts(h, run.rep.col_counts.data(), nullptr));
+        if (r == 0) run.lap("call + DRM annotation");
+        if (!o.control.empty()) {
+            // replicated: every rank tests the same all-reduced counts against the same capture
+            int64_t unc = 0;
+            std::vector<ms_control_variant> cv = mshost::fetch<ms_control_variant>(h, "ms_control_call", 256, [&](ms_control_variant* out, int64_t cap, int64_t* n) {
+                return ms_control_call(h, run.mg.data(), static_cast<int32_t>(run.mg.size()), run.ref, &run.prm, listed.data(),
+                                       static_cast<int64_t>(listed.size()), out, cap, n, &unc);
+            });
+            if (r == 0) {
+                run.control_rows.swap(cv);
+                run.control_uncovered = unc;
+                run.lap("control comparison");
+            }
         }
+        if (r == 0) CK(h, ms_get_counts(h, run.rep.col_counts.data(), nullptr));
         // one global variant list over all genes (screenshot juliet_hiv-phasing.png: same columns in every table)
         std::vector<std::pair<int, int>> keys;
         for (const msreport::VariantRow& vr : rows) keys.emplace_back(vr.col, vr.codon);
@@ -661,6 +709,34 @@ static msreport::RareBlock rare_block(Run& run) {
     return rare;
 }
 
+// the control comparison's rows: the control calls and the report's variants, DRM-annotated (--drm-only drops the rest)
+static msreport::ControlBlock control_block(const Run& run) {
+    msreport::ControlBlock cb;
+    cb.input_file = run.o.control;
+    cb.reads = run.ctl.nreads;
+    cb.alpha = run.o.alpha;
+    cb.uncovered_positions = run.control_uncovered;
+    for (const ms_control_variant& v : run.control_rows) {
+        msreport::ControlRow row;
+        char cb4[4];
+        row.gene = run.rep.genes[v.gene].name;
+        row.position = v.codon_index + 1;
+        row.label = aa_change(v.ref_codon, row.position, v.codon);
+        row.abs_pos = v.col + 1;
+        row.ref_codon = mscfg::codon_string(v.ref_codon, cb4);
+        row.codon = mscfg::codon_string(v.codon, cb4);
+        row.count = v.count; row.coverage = v.coverage; row.control_count = v.control_count; row.control_coverage = v.control_coverage;
+        row.pvalue = v.pvalue;
+        row.pvalue_corrected = std::min(1.0, v.pvalue * static_cast<double>(v.ntests));
+        row.control_call = v.called != 0;
+        row.model_call = v.listed != 0;
+        row.drugs = variant_drugs(run, v.gene, row.position, v.ref_codon, v.codon);
+        if (run.o.drm_only && row.drugs.empty()) continue;
+        cb.rows.push_back(row);
+    }
+    return cb;
+}
+
 static void write_file(const std::string& path, const std::string& text) {
     std::ofstream f(path);
     if (!f) mshost::die("cannot write " + path);
@@ -730,6 +806,7 @@ int main(int argc, char** argv) {
         if (o.abundance) run.rep.abundance = abundance_block(run);
         const std::string fasta = o.out_fasta.empty() ? std::string() : haplotype_fasta(run);
         if (o.rare_linkage) run.rep.rare = rare_block(run);   // replaces the handles' phasing state: last
+        if (!o.control.empty()) run.rep.control = control_block(run);
         write_outputs(run, fasta);
         fprintf(stderr, "juliet: %lld reads (%lld skipped), %zu variants%s\n", static_cast<long long>(run.aln.nreads),
                 static_cast<long long>(run.aln.nskipped), run.rep.variants.size(),

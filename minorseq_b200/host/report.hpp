@@ -116,6 +116,23 @@ struct IndelBlock {
     std::vector<IndelRow> calls;   // (gene, codon, deletion first, inserted)
 };
 
+// control comparison (--control, restatement choice U22): the union of the control calls and the report's variants
+struct ControlRow {
+    std::string gene, label;          // label as a variant row's, e.g. "K65R"
+    int position = 0, abs_pos = 0;    // amino-acid position in the gene; 1-based first column
+    std::string ref_codon, codon;
+    unsigned long long count = 0, coverage = 0, control_count = 0, control_coverage = 0;
+    double pvalue = 0, pvalue_corrected = 0;
+    bool control_call = false, model_call = false;
+    std::vector<std::string> drugs;
+};
+struct ControlBlock {
+    std::string input_file;
+    long long reads = 0, uncovered_positions = 0;
+    double alpha = 0;
+    std::vector<ControlRow> rows;     // (gene, column, codon)
+};
+
 // everything the report shows; the optional blocks are present when their option was given
 struct Report {
     std::string timestamp, input_file, command_line, version;
@@ -131,6 +148,7 @@ struct Report {
     std::optional<AbundanceBlock> abundance;
     std::optional<IndelBlock> indels;
     std::optional<RareBlock> rare;
+    std::optional<ControlBlock> control;
 };
 
 // "%": two significant digits as in the screenshots (1.1, 0.91, 98, 100)
@@ -408,6 +426,35 @@ inline Value build(const Report& rep) {
             o.set("frequency", Value::number(g.informative ? static_cast<double>(g.carriers) / static_cast<double>(g.informative) : 0.0));
         }
     }
+    if (const auto& control = rep.control) {
+        Value& cb = root.set("control", Value::object());
+        cb.set("input_file", Value::string(control->input_file));
+        cb.set("reads", Value::integer(control->reads));
+        cb.set("alpha", Value::number(control->alpha));
+        cb.set("uncovered_positions", Value::integer(control->uncovered_positions));
+        Value& rs = cb.set("rows", Value::array());
+        auto perc = [](unsigned long long k, unsigned long long n) { return perc2(n ? 100.0 * static_cast<double>(k) / static_cast<double>(n) : 0.0); };
+        for (const ControlRow& r : control->rows) {
+            Value& o = rs.push(Value::object());
+            o.set("gene", Value::string(r.gene));
+            o.set("label", Value::string(r.label));
+            o.set("position", Value::integer(r.position));
+            o.set("abs_pos", Value::integer(r.abs_pos));
+            o.set("ref_codon", Value::string(r.ref_codon));
+            o.set("codon", Value::string(r.codon));
+            o.set("count", Value::integer(static_cast<long long>(r.count)));
+            o.set("coverage", Value::integer(static_cast<long long>(r.coverage)));
+            o.set("percentage", Value::string(perc(r.count, r.coverage)));
+            o.set("control_count", Value::integer(static_cast<long long>(r.control_count)));
+            o.set("control_coverage", Value::integer(static_cast<long long>(r.control_coverage)));
+            o.set("control_percentage", Value::string(perc(r.control_count, r.control_coverage)));
+            o.set("pValue", Value::number(r.pvalue));
+            o.set("pValueCorrected", Value::number(r.pvalue_corrected));
+            o.set("control_call", Value::boolean(r.control_call));
+            o.set("model_call", Value::boolean(r.model_call));
+            o.set("known_drm", known_drm(r.drugs));
+        }
+    }
     return root;
 }
 
@@ -659,6 +706,30 @@ inline std::string to_html(const Value& root) {
                      " &rarr; " + esc(r.get_string("codon")) + "</tt></td><td>" + esc(r.get_string("percentage")) + "</td><td>" +
                      std::to_string(static_cast<long long>(r.get_number("count"))) + "</td><td>" + std::to_string(static_cast<long long>(r.get_number("coverage"))) +
                      "</td>" + b + "<td>" + (g >= 0 ? std::to_string(g + 1) : std::string()) + "</td><td>" + lc + "</td></tr>\n";
+            }
+            h += "</table>";
+        }
+        h += "</details>\n";
+    }
+    if (const Value* cb = root.get("control")) {
+        char b[256];
+        snprintf(b, sizeof b, "Control: %lld reads; codons tested against the control's count at the same position (one-sided Fisher, "
+                 "significance %g after Bonferroni); %lld positions without control coverage", static_cast<long long>(cb->get_number("reads")),
+                 cb->get_number("alpha"), static_cast<long long>(cb->get_number("uncovered_positions")));
+        h += "<details open><summary>Control Comparison</summary><p>" + esc(cb->get_string("input_file")) + "<br>" + std::string(b) + "</p>";
+        const Value* rs = cb->get("rows");
+        if (rs && !rs->arr.empty()) {
+            h += "<table><tr><th>Gene</th><th>Variant</th><th>Codon</th><th>%</th><th>Count</th><th>Coverage</th><th>Control %</th>"
+                 "<th>Control count</th><th>Control coverage</th><th>p (corrected)</th><th>Control call</th><th>Model call</th><th>Affected Drugs</th></tr>\n";
+            auto yes = [](const Value* v) { return std::string(v && v->b ? "yes" : "no"); };
+            for (const Value& r : rs->arr) {
+                snprintf(b, sizeof b, "<td>%.2e</td>", r.get_number("pValueCorrected"));
+                h += "<tr><td>" + esc(r.get_string("gene")) + "</td><td>" + esc(r.get_string("label")) + "</td><td><tt>" + esc(r.get_string("ref_codon")) +
+                     " &rarr; " + esc(r.get_string("codon")) + "</tt></td><td>" + esc(r.get_string("percentage")) + "</td><td>" +
+                     std::to_string(static_cast<long long>(r.get_number("count"))) + "</td><td>" + std::to_string(static_cast<long long>(r.get_number("coverage"))) +
+                     "</td><td>" + esc(r.get_string("control_percentage")) + "</td><td>" + std::to_string(static_cast<long long>(r.get_number("control_count"))) +
+                     "</td><td>" + std::to_string(static_cast<long long>(r.get_number("control_coverage"))) + "</td>" + b + "<td>" + yes(r.get("control_call")) +
+                     "</td><td>" + yes(r.get("model_call")) + "</td><td>" + esc(r.get_string("known_drm")) + "</td></tr>\n";
             }
             h += "</table>";
         }
